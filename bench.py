@@ -1,6 +1,6 @@
 """bench.py — audio-seconds per wall-second of the level-1/level-2 hot path at 4096 streams per B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--only sweep|config3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--only sweep|config3] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -560,6 +560,30 @@ def config3_leg(torch, dist, dev, stream, local_rank, rank, world, word, pool_de
     return leg
 
 
+def dump_outputs(out_dir, results, events, last_tick):
+    """--dump-outputs: what the device-resident timed path computed in its last step, one DIR/<name>.npy per array:
+    every stream's result record (`stream_score`, `stream_flags`: the caller's ewk_stream_result buffer) and each field
+    of the events the step's ticks produced (`event_<field>`, in ewk_poll's order).  float32 values stay float32,
+    integers become float64 (exact).  A score is NaN where none exists (a stream before its first level-2 evaluation,
+    a timeout event): it is written as 0 with `<name>_valid` = 0 beside it, so that every value written is finite."""
+    from easywakeword_b200 import _lib
+    os.makedirs(out_dir, exist_ok=True)
+    rec = results.cpu().numpy()
+    origin = events["tick"] + (events["kind"] == _lib.EV_TIMEOUT)      # a timeout event carries the tick before the one that raised it
+    ev = events[origin > last_tick - TICKS_PER_STEP]
+    arrays = {"stream_score": rec[:, 0].copy().view(np.float32),
+              "stream_flags": rec[:, 1].copy().view(np.uint32).astype(np.float64)}
+    for f in _lib.EVENT_DTYPE.names:
+        arrays[f"event_{f}"] = ev[f] if ev[f].dtype == np.float32 else ev[f].astype(np.float64)
+    for name in ("stream_score", "event_score"):
+        valid = np.isfinite(arrays[name])
+        arrays[name] = np.where(valid, arrays[name], np.float32(0))
+        arrays[f"{name}_valid"] = valid.astype(np.float32)
+    for name, a in arrays.items():
+        assert np.isfinite(a).all(), name
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # ----------------------------------------------------------------------------------------------
 def run_ours(args):
     import torch
@@ -674,6 +698,8 @@ def run_ours(args):
             step(where, True)
         blocks = []
         for _ in range(repeats):
+            if not read_back:
+                bank.poll()         # untimed: the event queue holds one block's events, none of them dropped for lack of room
             gc.collect()
             gc.disable()            # a collection inside a 3 ms block stalls the enqueueing thread for longer than the queue is deep
             barrier()
@@ -718,7 +744,12 @@ def run_ours(args):
         sampler.start()
     R = max(1, args.repeats)
     ms_dev, launches, _, dev_blocks = timed(_lib.DEVICE, False, K, R)      # inputs resident in HBM
-    bank.poll()
+    ev_dev = bank.poll()
+    if args.dump_outputs and rank == 0:
+        if ctx.dropped:
+            raise SystemExit(f"bench.py: the event queue dropped {ctx.dropped} events in the last timed block, so its "
+                             "last step is incomplete and is not dumped; use fewer --steps")
+        dump_outputs(args.dump_outputs, results, ev_dev, ctx.status(0).tick)
     ms_e2e, _, n_events, e2e_blocks = timed(_lib.HOST, True, K, R)         # host PCM -> rings -> events on host
 
     # the same end-to-end step fed with G.711 mu-law codes (ewk_push_g711: 1 byte per sample over PCIe, expanded on the
@@ -1099,7 +1130,14 @@ def main():
     ap.add_argument("--only", default="all", choices=["all", "sweep", "config3"],
                     help="run one secondary leg on its own instead of the whole line")
     ap.add_argument("--sweep-seconds", type=int, default=SWEEP_SECONDS, help="audio seconds per stream the sweep leg measures")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline (device-resident) path computed for rank 0's "
+                         "streams as DIR/<name>.npy: per-stream result records and that step's events")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.only != "all"):
+        ap.error("--dump-outputs applies to the GPU line (--impl ours, --only all)")
     if args.impl == "reference":
         run_reference(args)
     elif args.only != "all":

@@ -110,6 +110,9 @@ DETECT_CASES = [
          params=dict(speech_duration_min=0.5, speech_duration_max=1.6, timeout=20, similarity_threshold=98.0)),
     dict(name="b320_zero_gaps", seed=2007, seconds=40, block=320, noise=0.004, gain=(2.0, 4.0), zero_gaps=6,
          params=dict(speech_duration_min=0.69, speech_duration_max=1.38, timeout=30)),
+    # a short timeout with restarts at block 512 and 0.6-1.5 s durations, which no case above covers
+    dict(name="b512_timeout8", seed=4242, seconds=25, block=512, noise=0.003, gain=(2.0, 4.0),
+         params=dict(speech_duration_min=0.6, speech_duration_max=1.5, timeout=8)),
 ]
 
 

@@ -2,9 +2,8 @@
 
 `-m "not gpu"` runs here (no GPU): oracle vs the reference-generated goldens, host logic,
 C-ABI symbol checks, gloo world_size-2 paths.  `-m gpu` runs on a B200 and compares the
-CUDA path (through the C-ABI) with the oracle and the goldens.  Nothing here reads
-/root/reference at run time except tests explicitly marked `needs_reference`, which skip
-when the tree is absent (GPU box).
+CUDA path (through the C-ABI) with the oracle and the goldens.  Every input is in the
+repository (tests/golden) or generated from a seed.
 """
 import json
 import os
@@ -21,19 +20,15 @@ GOLDEN = os.path.join(REPO, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (B200); deselected on the CPU box")
-    config.addinivalue_line("markers", "needs_reference: imports /root/reference (build container only)")
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isfile("/root/reference/easywakeword/wakeword.py")
     try:
         import torch
         have_gpu = torch.cuda.is_available()
     except Exception:
         have_gpu = False
     for item in items:
-        if "needs_reference" in item.keywords and not have_ref:
-            item.add_marker(pytest.mark.skip(reason="/root/reference not present on this box"))
         if "gpu" in item.keywords and not have_gpu:
             item.add_marker(pytest.mark.skip(reason="no CUDA device"))
 
