@@ -12,6 +12,7 @@ LIB_PATH = os.path.join(HERE, "libewk.so")
 
 EWK_OK, EWK_ERR_ARG, EWK_ERR_NO_TEMPLATE, EWK_ERR_CUDA, EWK_ERR_STATE, EWK_ERR_NOMEM = 0, -1, -2, -3, -4, -5
 PCM_F32, PCM_I16 = 0, 1
+IN_ULAW, IN_ALAW = 2, 3          # input formats of ewk_push_resampled beside PCM_F32 / PCM_I16
 HOST, DEVICE = 0, 1
 
 
@@ -293,6 +294,8 @@ def _declare_stream_protos(lib):
         "ewk_set_stream_params": (C.c_int, [vp, i32, _p(StreamParams)]),
         "ewk_push": (C.c_int, [vp, i32, i32, vp, i64, i64, i32]),
         "ewk_push_g711": (C.c_int, [vp, i32, i32, vp, i64, i64, i32, i32]),
+        "ewk_push_resampled": (C.c_int, [vp, i32, i32, vp, i32, i64, i64, i32, i32]),
+        "ewk_stream_input": (C.c_int, [vp, i32, _p(C.c_int32), _p(i64)]),
         "ewk_tick": (C.c_int, [vp, i32]),
         "ewk_set_overlap": (C.c_int, [vp, i32]),
         "ewk_join": (C.c_int, [vp]),
@@ -413,6 +416,44 @@ def _bank_methods():
             stride = a.strides[0] if ns > 1 else n
             ptr = a.ctypes.data
         self._ck(self.lib.ewk_push_g711(self.h, stream0, ns, ptr, n, stride, where, 1 if law == "alaw" else 0))
+
+    def push_resampled(self, pcm_or_codes, sr_in, stream0=0, where=HOST, fmt=None):
+        """A native-rate feed [n_streams, n] at sr_in Hz, converted to 16 kHz on the device and landed in the rings (K8;
+        include/ewk.h: ewk_push_resampled).  The input format follows the dtype: float32, int16, or uint8 G.711 codes with
+        fmt="ulaw" / "alaw" (into either ring format).  A device input is (ptr, n_streams, n, stride, dtype).
+        Returns the number of 16 kHz samples landed per stream."""
+        if isinstance(pcm_or_codes, tuple):
+            ptr, ns, n, stride, dt = pcm_or_codes
+            dt = np.dtype(dt)
+        else:
+            a = pcm_or_codes if pcm_or_codes.ndim == 2 else pcm_or_codes.reshape(1, -1)
+            if a.strides[1] != a.itemsize:
+                a = np.ascontiguousarray(a)
+            ns, n = a.shape
+            stride = a.strides[0] // a.itemsize if ns > 1 else n
+            ptr, dt = a.ctypes.data, a.dtype
+        if dt == np.uint8:
+            if fmt not in ("ulaw", "alaw"):
+                raise ValueError('uint8 input is G.711: fmt must be "ulaw" or "alaw"')
+            code = IN_ULAW if fmt == "ulaw" else IN_ALAW
+        elif fmt is not None:
+            raise ValueError("fmt selects G.711 for uint8 input only")
+        elif dt == np.int16:
+            code = PCM_I16
+        elif dt == np.float32:
+            code = PCM_F32
+        else:
+            raise TypeError(f"push_resampled takes float32, int16 or uint8 G.711 input, got {dt}")
+        rc = self.lib.ewk_push_resampled(self.h, stream0, ns, ptr, code, n, stride, where, int(sr_in))
+        if rc < 0:
+            self._ck(rc)
+        return rc
+
+    def stream_input(self, stream):
+        """-> (input rate latched by the stream's first push (0: none yet), input samples received)."""
+        sr, n = C.c_int32(), C.c_int64()
+        self._ck(self.lib.ewk_stream_input(self.h, int(stream), C.byref(sr), C.byref(n)))
+        return sr.value, n.value
 
     def tick(self, n_ticks=1, trace=False):
         if not trace:
@@ -541,10 +582,12 @@ def _bank_methods():
         ms = (C.c_double * 8)()
         n = (C.c_int64 * 8)()
         self._ck(self.lib.ewk_profile_read(self.h, ms, n))
-        names = ["ring_push", "tick_gate", "segment_queue", "segment_batch", "dense_score", "segment_prepare", "publish"]
+        names = ["ring_push", "tick_gate", "segment_queue", "segment_batch", "dense_score", "segment_prepare", "publish",
+                 "resample_push"]
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
-    for f in (prepare_segments, dense_scores, profile, profile_read, set_stream_params, push, push_g711, tick, poll, status, read_last, read_segment, results, results_device_ptr,
+    for f in (prepare_segments, dense_scores, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
+              stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
               set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count):
         setattr(Context, f.__name__, f)
 

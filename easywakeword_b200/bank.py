@@ -22,7 +22,11 @@ EV_TIMEOUT, EV_SCORED = _lib.EV_TIMEOUT, _lib.EV_SCORED
 
 
 class WakeWordBank:
-    """N independent 16 kHz streams, one GPU.
+    """N independent audio streams, one GPU.
+
+    sample_rate: the rate of the blocks push / push_g711 / step / run take.  Any rate other than 16000 (8 kHz telephony,
+    44.1 / 48 kHz devices) is converted to 16 kHz on the device as it lands (K8); the rings, the timing and
+    samples_pushed are in 16 kHz samples.
 
     templates: list of float32 arrays or WAV paths (slot i = templates[i]); every stream is scored
     against all of them (best score wins) unless set_stream(..., template_first=, template_count=).
@@ -34,7 +38,8 @@ class WakeWordBank:
                  pre_speech_silence: float = 0.8, speech_duration_min: Optional[float] = None,
                  speech_duration_max: Optional[float] = None, post_speech_silence: float = 0.4,
                  timeout: float = 30.0, max_push_seconds: float = 1.0, max_events: int = 0,
-                 cuda_stream: Optional[int] = None, overlap: bool = False, preemphasis: float = 0.0, n_mfcc: int = 20):
+                 cuda_stream: Optional[int] = None, overlap: bool = False, preemphasis: float = 0.0, n_mfcc: int = 20,
+                 sample_rate: int = 16000):
         if n_streams < 1:
             raise ValueError("n_streams must be at least 1")
         if buffer_seconds <= 0:
@@ -42,6 +47,9 @@ class WakeWordBank:
         if not templates:
             raise ValueError("at least one template is required")
         self.n_streams = n_streams
+        self.sample_rate = int(sample_rate)
+        if self.sample_rate != 16000:
+            _lib.resample_info(self.sample_rate)                 # ValueError for rates the device filter does not support
         self.pcm_dtype = np.dtype(pcm_dtype)
         if self.pcm_dtype not in (np.dtype(np.int16), np.dtype(np.float32)):
             raise ValueError("pcm_dtype must be int16 or float32")
@@ -90,12 +98,24 @@ class WakeWordBank:
 
     # ---- data plane
     def push(self, pcm, where=_lib.HOST):
-        """pcm[n_streams, n] in the bank's dtype: n new samples for every stream (K1 / direct H2D)."""
+        """pcm[n_streams, n]: n new samples for every stream (K1 / direct H2D) in the bank's dtype; at another
+        sample_rate, float32 or int16 at that rate (K8; a device input is (ptr, n_streams, n, stride, dtype))."""
+        if self.sample_rate != 16000:
+            self.samples_pushed += self.ctx.push_resampled(pcm, self.sample_rate, stream0=0, where=where)
+            return
         self.ctx.push(pcm, stream0=0, where=where)
         self.samples_pushed += pcm[2] if isinstance(pcm, tuple) else pcm.shape[-1]
 
     def push_g711(self, codes, law: str = "ulaw", where=_lib.HOST):
-        """codes[n_streams, n] uint8: a G.711 mu-law / A-law feed, expanded to PCM16 on the device (int16 banks)."""
+        """codes[n_streams, n] uint8: a G.711 mu-law / A-law feed, expanded on the device (16 kHz: int16 banks only; at
+        another sample_rate the codes are converted by K8 into either ring format)."""
+        if self.sample_rate != 16000:
+            if law not in ("ulaw", "alaw"):
+                raise ValueError("law must be 'ulaw' or 'alaw'")
+            if isinstance(codes, tuple):
+                codes = (*codes[:4], np.uint8)
+            self.samples_pushed += self.ctx.push_resampled(codes, self.sample_rate, stream0=0, where=where, fmt=law)
+            return
         self.ctx.push_g711(codes, stream0=0, where=where, law=law)
         self.samples_pushed += codes[2] if isinstance(codes, tuple) else codes.shape[-1]
 
@@ -105,8 +125,7 @@ class WakeWordBank:
         return self.ctx.tick(n_ticks, trace=trace)
 
     def step(self, pcm, where=_lib.HOST):
-        """push + as many ticks as the pushed audio covers."""
-        n = pcm[2] if isinstance(pcm, tuple) else pcm.shape[-1]
+        """push + as many ticks as the landed audio covers."""
         self.push(pcm, where)
         due = self.samples_pushed // TICK_SAMPLES - self.ticks
         if due > 0:
@@ -131,16 +150,21 @@ class WakeWordBank:
         return self.ctx.read_segment(int(event["stream"]), int(event["seg_start"]), int(event["seg_len"]))
 
     def dense_sweep(self, blocks: Iterable[np.ndarray], template_first: int = 0, template_count: Optional[int] = None):
-        """Offline sweep (BASELINE config 5): push each [n_streams, n] block (n a multiple of 160) and yield
-        (first_hop, scores[n_streams, n // 160, T]) for the hops it completes — every template scored at every hop."""
+        """Offline sweep (BASELINE config 5): push each [n_streams, n] block (at 16 kHz, n a multiple of 160; at another
+        sample_rate, any n) and yield (first_hop, scores[n_streams, hops, T]) for the hops the landed audio completes —
+        every template scored at every hop."""
         self.ctx.set_stream_params(-1, **dict(self.params, live=1))     # no ticks here: pushes run free of the gate's guard
         for blk in blocks:
-            n = blk.shape[-1]
-            if n % 160:
+            if self.sample_rate == 16000 and blk.shape[-1] % 160:
                 raise ValueError("dense_sweep blocks must hold a multiple of 160 samples")
             hop0 = self.samples_pushed // 160 + 1
             self.push(blk)
-            yield hop0, self.dense_scores(hop0, n // 160, template_first, template_count)
+            n_hops = self.samples_pushed // 160 + 1 - hop0
+            if n_hops == 0:
+                T = len(self.templates) - template_first if template_count is None else template_count
+                yield hop0, np.zeros((self.n_streams, 0, T), np.float32)
+                continue
+            yield hop0, self.dense_scores(hop0, n_hops, template_first, template_count)
 
     def prepare_for_transcription(self, events) -> list:
         """Batched level-3 pre-processing on the device (wakeword.py:1020-1025) of the word_audio of `events`

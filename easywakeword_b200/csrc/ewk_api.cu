@@ -495,7 +495,8 @@ extern "C" int ewk_resample(ewk_ctx* ctx, const void* in, int pcm_format, int wh
     int rc = ctx->resample_table(sr_in, &t);
     if (rc) return rc;
     const size_t esz = pcm_format == EWK_PCM_I16 ? 2 : 4;
-    ResampleArgs A{};
+    if (n_rows > 65535) { ctx->fail("ewk_resample: at most 65535 rows per call"); return EWK_ERR_ARG; }
+    RsPushArgs A{};
     A.in = in; A.in_stride = in_stride;
     if (where_in == EWK_HOST) {
         CK(ctx->b_rs_in.ensure(esz * (size_t)n_rows * (size_t)std::max<int64_t>(n_in, 1)));
@@ -509,18 +510,11 @@ extern "C" int ewk_resample(ewk_ctx* ctx, const void* in, int pcm_format, int wh
         CK(ctx->b_rs_out.ensure(sizeof(float) * (size_t)n_rows * (size_t)n_out));
         A.out = (float*)ctx->b_rs_out.p; A.out_stride = n_out;
     }
-    A.H = t->H; A.n_in = n_in; A.in_first = in_first; A.out_first = out_first; A.n_out = n_out;
-    A.L = t->d.L; A.M = t->d.M; A.Minv = t->d.Minv; A.W = t->d.W; A.fmt = pcm_format == EWK_PCM_I16 ? 1 : 0;
-    const long long g0 = out_first / A.L, g1 = (out_first + n_out + A.L - 1) / A.L;
-    const long long threads = (g1 - g0) * A.L;
-    const dim3 grid((unsigned)((threads + RS_THREADS - 1) / RS_THREADS), (unsigned)n_rows);
-    if (n_rows > 65535) { ctx->fail("ewk_resample: at most 65535 rows per call"); return EWK_ERR_ARG; }
-    cudaEvent_t pe = ctx->prof_begin(3);
-    if (A.fmt == 1) resample_kernel<short><<<grid, RS_THREADS, 0, ctx->stream>>>(A);
-    else resample_kernel<float><<<grid, RS_THREADS, 0, ctx->stream>>>(A);
-    ctx->prof_end(pe, 3);
-    CK(cudaGetLastError());
-    ctx->launches++;
+    // the input buffer is absolute samples [in_first, in_first + n_in), zeros elsewhere: no tail
+    A.n_in = n_in; A.c = A.t0_old = A.t0_new = in_first; A.o0 = out_first; A.o1 = out_first + n_out;
+    A.in_fmt = pcm_format; A.H = t->H; A.L = t->d.L; A.M = t->d.M; A.W = t->d.W;
+    rc = ctx->launch_fir(*t, A, n_rows, 3, "ewk_resample");
+    if (rc) return rc;
     if (where_out == EWK_HOST) {
         CK(cudaMemcpy2DAsync(out, sizeof(float) * (size_t)out_stride, ctx->b_rs_out.p, sizeof(float) * (size_t)n_out,
                              sizeof(float) * (size_t)n_out, (size_t)n_rows, cudaMemcpyDeviceToHost, ctx->stream));
@@ -619,6 +613,8 @@ int ewk_ctx::init_streams() {
     h_visible_lb.assign(n, 0);
     h_tick.assign(n, 0);
     h_frame_size.assign(n, 0);
+    h_rate.assign(n, 0);
+    h_inputs.assign(n, 0);
     CK(cudaFuncSetAttribute(segment_queue_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                             (int)seg_smem_bytes(SEG_SMEM_FRAMES)));
     CK(cudaFuncSetAttribute(segment_queue_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -645,6 +641,7 @@ void ewk_ctx::release_streams() {
         cudaFree(bank.k3_trace);
     }
 #endif
+    if (d_rs_tail) { cudaFree(d_rs_tail); d_rs_tail = nullptr; rs_tail_cap = 0; }
     for (void* p : {bank.ring, (void*)bank.st, (void*)bank.prm, (void*)bank.chunk_ms, (void*)bank.events,
                     (void*)bank.ev_count, (void*)bank.block_ss, (void*)bank.lm_ws, own_results, (void*)bank.frow,
                     (void*)bank.frame_ev, (void*)bank.ev_done, (void*)bank.bk_count, (void*)bank.bk_list})
@@ -799,7 +796,24 @@ int ewk_ctx::land(int stream0, int n_streams, const void* d_src, long long d_str
 int ewk_ctx::flush_pending() {
     if (!pending.valid) return EWK_OK;
     pending.valid = false;
+    if (pending.rs_rate)
+        return land_resampled(pending.stream0, pending.n_streams, b_raw[pending.slot].p, pending.rs_n_in, pending.rs_fmt,
+                              pending.rs_n_in, pending.rs_rate, pending.rs_c, pending.slot);
     return land(pending.stream0, pending.n_streams, b_stage2[pending.slot].p, pending.n, pending.n, pending.slot);
+}
+
+// A stream's input rate is fixed by its first push: 16 kHz pushes (ewk_push, ewk_push_g711) refuse a native-rate stream.
+static int check_16k(ewk_ctx* ctx, const char* who, int stream0, int n_streams) {
+    for (int s = stream0; s < stream0 + n_streams; s++)
+        if (ctx->h_rate[s] != 0 && ctx->h_rate[s] != RS_TARGET) {
+            ctx->fail("%s: stream %d takes %d Hz input through ewk_push_resampled", who, s, ctx->h_rate[s]);
+            return EWK_ERR_STATE;
+        }
+    return EWK_OK;
+}
+
+static void latch_16k(ewk_ctx* ctx, int stream0, int n_streams, long long n) {
+    for (int s = stream0; s < stream0 + n_streams; s++) { ctx->h_rate[s] = RS_TARGET; ctx->h_inputs[s] += n; }
 }
 
 extern "C" int ewk_push(ewk_ctx* ctx, int stream0, int n_streams, const void* pcm, int64_t n, int64_t stride, int where) {
@@ -812,6 +826,8 @@ extern "C" int ewk_push(ewk_ctx* ctx, int stream0, int n_streams, const void* pc
         return EWK_ERR_ARG;
     }
     if (n > B.P - B.R && n > B.R) { ctx->fail("ewk_push: %lld samples exceed the ring (%d)", (long long)n, B.R); return EWK_ERR_ARG; }
+    rc = check_16k(ctx, "ewk_push", stream0, n_streams);
+    if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
     rc = ctx->flush_pending();
     if (rc) return rc;
@@ -833,6 +849,7 @@ extern "C" int ewk_push(ewk_ctx* ctx, int stream0, int n_streams, const void* pc
         }
     }
     const size_t esz = B.fmt == 1 ? 2 : 4;
+    latch_16k(ctx, stream0, n_streams, n);
     if (where != EWK_HOST) return ctx->land(stream0, n_streams, pcm, stride, n, -1);
     // Host PCM: H2D on a dedicated copy stream into one of two staging buffers.  Contiguous sources
     // ([n_streams][n]) go as ONE linear copy (55 GB/s over PCIe 5 vs 47 GB/s pitched).
@@ -846,6 +863,7 @@ extern "C" int ewk_push(ewk_ctx* ctx, int stream0, int n_streams, const void* pc
         CK(cudaMemcpy2DAsync(ctx->b_stage2[b].p, (size_t)n * esz, pcm, (size_t)stride * esz, (size_t)n * esz, n_streams,
                              cudaMemcpyHostToDevice, ctx->copy_stream));
     CK(cudaEventRecord(ctx->ev_ready[b], ctx->copy_stream));
+    ctx->pending = ewk_ctx::Pending{};
     ctx->pending.valid = true; ctx->pending.slot = b; ctx->pending.stream0 = stream0; ctx->pending.n_streams = n_streams;
     ctx->pending.n = n;
     return EWK_OK;
@@ -866,6 +884,8 @@ extern "C" int ewk_push_g711(ewk_ctx* ctx, int stream0, int n_streams, const uin
         return EWK_ERR_ARG;
     }
     if (n > B.P - B.R && n > B.R) { ctx->fail("ewk_push_g711: %lld samples exceed the ring (%d)", (long long)n, B.R); return EWK_ERR_ARG; }
+    rc = check_16k(ctx, "ewk_push_g711", stream0, n_streams);
+    if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
     rc = ctx->flush_pending();
     if (rc) return rc;
@@ -885,6 +905,7 @@ extern "C" int ewk_push_g711(ewk_ctx* ctx, int stream0, int n_streams, const uin
             return EWK_ERR_STATE;
         }
     }
+    latch_16k(ctx, stream0, n_streams, n);
     const int b = ctx->stage_idx;
     ctx->stage_idx ^= 1;
     CK(ctx->b_stage2[b].ensure(sizeof(short) * (size_t)n * n_streams));
@@ -910,8 +931,191 @@ extern "C" int ewk_push_g711(ewk_ctx* ctx, int stream0, int n_streams, const uin
     CK(cudaGetLastError());
     ctx->launches++;
     CK(cudaEventRecord(ctx->ev_ready[b], ctx->copy_stream));
+    ctx->pending = ewk_ctx::Pending{};
     ctx->pending.valid = true; ctx->pending.slot = b; ctx->pending.stream0 = stream0; ctx->pending.n_streams = n_streams;
     ctx->pending.n = n;
+    return EWK_OK;
+}
+
+// ------------------------------------------------------------------------------------------ K8 native-rate push
+// outputs whose W inputs of look-ahead have arrived after c inputs (StreamResampler.push's rule)
+static long long rs_ready(long long c, const ResampleDesign& d) {
+    const long long a = c - d.W;
+    return a <= 0 ? 0 : (a * d.L + d.M - 1) / d.M;
+}
+// first input sample any output from ready(c) on reads
+static long long rs_tail_start(long long c, const ResampleDesign& d) {
+    return std::max(0LL, rs_ready(c, d) * d.M / d.L - d.W + 1);
+}
+static size_t rs_in_size(int in_fmt) { return in_fmt == EWK_PCM_F32 ? 4 : in_fmt == EWK_PCM_I16 ? 2 : 1; }
+
+// The FIR (K8) over rows [0, n_rows) of A: plans the work mapping (fast or generic path, tile, staged span) and launches.
+int ewk_ctx::launch_fir(const ResampleTable& t, RsPushArgs& A, int n_rows, int prof_cls, const char* who) {
+    ewk_ctx* ctx = this;
+    const ResampleDesign& d = t.d;
+    const int taps = 2 * d.W;
+    A.table_smem = (long long)taps * d.L <= RSP_TABLE_SMEM;
+    // fast path: warp-uniform phases and register windows; its tile must leave the tail (if any) to CTA 0 alone
+    int fast_m = 0;
+    if ((d.L == 1 || d.L == 2 || d.L == 4 || d.L == 8) && d.M <= 3 && A.table_smem &&
+        (RSP_THREADS / d.L) * rsp_k(d.M) * d.M >= taps + d.M)
+        fast_m = d.M;
+    long long first;
+    if (fast_m) {
+        A.tile = RSP_THREADS * rsp_k(d.M);
+        A.span = (RSP_THREADS / d.L) * rsp_k(d.M) * d.M + taps + d.M + 1;
+        first = (A.o0 / d.L) * d.L;
+    } else {
+        auto span = [&](long long tile) { return (tile * d.M + d.L - 1) / d.L + taps + 1; };
+        long long tile = RSP_GENERIC_TILE;
+        while (tile > RSP_THREADS && span(tile) > 24576) tile /= 2;
+        const long long need = ((long long)taps * d.L + d.M - 1) / d.M;      // tile M / L >= 2W: CTAs >= 1 start past the tail
+        tile = std::max(tile, (need + RSP_THREADS - 1) / RSP_THREADS * RSP_THREADS);
+        A.tile = (int)tile;
+        A.span = (int)span(tile);
+        first = A.o0;
+    }
+    const size_t smem = sizeof(float) * ((size_t)256 + A.tail_cap + (A.table_smem ? (size_t)taps * d.L : 0) + A.span);
+    if (smem > (size_t)200 * 1024) { fail("%s: %d Hz needs %zu bytes of shared memory", who, d.sr_in, smem); return EWK_ERR_ARG; }
+    const dim3 grid((unsigned)std::max<long long>(1, (A.o1 - first + A.tile - 1) / A.tile), (unsigned)n_rows);
+    auto k8 = fast_m == 1 ? resample_push_kernel<1> : fast_m == 2 ? resample_push_kernel<2> : fast_m == 3 ? resample_push_kernel<3>
+                                                                                        : resample_push_kernel<0>;
+    CK(cudaFuncSetAttribute(k8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cudaEvent_t pe = prof_begin(prof_cls);
+    k8<<<grid, RSP_THREADS, smem, stream>>>(bank, A);
+    prof_end(pe, prof_cls);
+    CK(cudaGetLastError());
+    launches++;
+    return EWK_OK;
+}
+
+// K8 on device-resident input (the caller's buffer or a staging slot): every stream of the call has received c inputs
+int ewk_ctx::land_resampled(int stream0, int n_streams, const void* d_src, long long d_stride, int in_fmt, long long n_in,
+                            int sr_in, long long c, int stage_slot) {
+    ewk_ctx* ctx = this;
+    const ResampleTable* t = nullptr;
+    int rc = resample_table(sr_in, &t);
+    if (rc) return rc;
+    const ResampleDesign& d = t->d;
+    RsPushArgs A{};
+    A.in = d_src; A.in_stride = d_stride; A.n_in = n_in; A.in_fmt = in_fmt;
+    A.tail = d_rs_tail; A.tail_cap = rs_tail_cap; A.H = t->H;
+    A.L = d.L; A.M = d.M; A.W = d.W; A.stream0 = stream0;
+    A.c = c; A.o0 = rs_ready(c, d); A.o1 = rs_ready(c + n_in, d);
+    A.t0_old = rs_tail_start(c, d); A.t0_new = rs_tail_start(c + n_in, d);
+    A.frame_latch = (int)ewk_resample_out_len(n_in, sr_in);
+    if (stage_slot >= 0) CK(cudaStreamWaitEvent(stream, ev_ready[stage_slot], 0));
+    rc = launch_fir(*t, A, n_streams, 7, "ewk_push_resampled");
+    if (rc) return rc;
+    if (stage_slot >= 0) {
+        CK(cudaEventRecord(ev_free[stage_slot], stream));
+        ev_free_valid[stage_slot] = true;
+    }
+    all_presummed = false;                  // K8 forms no block sums: K2 reads these samples
+    pushes_since_tick++;
+    for (int s = stream0; s < stream0 + n_streams; s++) {
+        h_written[s] = A.o1;
+        if (h_frame_size[s] == 0) h_frame_size[s] = h_prm[s].frame_size > 0 ? h_prm[s].frame_size : A.frame_latch;
+    }
+    return EWK_OK;
+}
+
+extern "C" int ewk_push_resampled(ewk_ctx* ctx, int stream0, int n_streams, const void* in, int in_format, int64_t n_in,
+                                  int64_t stride, int where, int sr_in) {
+    if (!ctx) return EWK_ERR_ARG;
+    int rc = need_streams(ctx, "ewk_push_resampled", false);
+    if (rc) return rc;
+    BankView& B = ctx->bank;
+    if (!in || n_streams < 1 || stream0 < 0 || stream0 + n_streams > B.n_streams || n_in < 1 || stride < n_in ||
+        in_format < EWK_PCM_F32 || in_format > EWK_IN_ALAW || n_in > (int64_t)1 << 34) {
+        ctx->fail("ewk_push_resampled: bad arguments (stream0=%d n_streams=%d n_in=%lld stride=%lld in_format=%d)", stream0,
+                  n_streams, (long long)n_in, (long long)stride, in_format);
+        return EWK_ERR_ARG;
+    }
+    ResampleDesign d;
+    if (sr_in == RS_TARGET || sr_in < 1000 || sr_in > 768000 || !rs_design(sr_in, d)) {
+        ctx->fail("ewk_push_resampled: %d Hz is not a supported input rate (16000 Hz input goes through ewk_push)", sr_in);
+        return EWK_ERR_ARG;
+    }
+    const long long c = ctx->h_inputs[stream0];
+    for (int s = stream0; s < stream0 + n_streams; s++) {
+        if (ctx->h_rate[s] != 0 && ctx->h_rate[s] != sr_in) {
+            ctx->fail("ewk_push_resampled: stream %d already takes %d Hz input", s, ctx->h_rate[s]);
+            return EWK_ERR_STATE;
+        }
+        if (ctx->h_inputs[s] != c) {
+            ctx->fail("ewk_push_resampled: streams %d and %d have received %lld and %lld input samples; one call takes streams "
+                      "at the same position", stream0, s, c, ctx->h_inputs[s]);
+            return EWK_ERR_STATE;
+        }
+    }
+    const long long n = rs_ready(c + n_in, d) - rs_ready(c, d);            // samples this call lands
+    if (n > B.P - B.R && n > B.R) { ctx->fail("ewk_push_resampled: %lld samples exceed the ring (%d)", n, B.R); return EWK_ERR_ARG; }
+    CK(cudaSetDevice(ctx->device));
+    rc = ctx->flush_pending();
+    if (rc) return rc;
+    for (int s = stream0; s < stream0 + n_streams; s++) {     // same guard as ewk_push, on the landed count
+        if (ctx->h_prm[s].live) continue;
+        const long long ahead = ctx->h_written[s] + n - ctx->h_visible_lb[s];
+        if (ctx->h_visible_lb[s] >= B.R && ahead > (long long)(B.P - B.R)) {
+            ctx->fail("ewk_push_resampled: stream %d would hold %lld un-gated samples, more than slack_samples=%d; call "
+                      "ewk_tick first", s, ahead, B.P - B.R);
+            return EWK_ERR_STATE;
+        }
+        if (ctx->h_visible_lb[s] < B.R && ctx->h_written[s] + n > (long long)B.P) {
+            ctx->fail("ewk_push_resampled: stream %d would hold %lld samples before its first full tick, more than the physical "
+                      "ring (%d); call ewk_tick first", s, ctx->h_written[s] + n, B.P);
+            return EWK_ERR_STATE;
+        }
+    }
+    const ewk_ctx::ResampleTable* t = nullptr;
+    rc = ctx->resample_table(sr_in, &t);
+    if (rc) return rc;
+    if (ctx->rs_tail_cap < 2 * d.W) {
+        // tails for the widest filter in use; rows of streams already running move with their content
+        const int cap = 2 * d.W;
+        float* nt = nullptr;
+        CK(cudaMalloc(&nt, sizeof(float) * (size_t)B.n_streams * cap));
+        if (ctx->d_rs_tail) {
+            CK(cudaMemcpy2DAsync(nt, sizeof(float) * cap, ctx->d_rs_tail, sizeof(float) * ctx->rs_tail_cap,
+                                 sizeof(float) * ctx->rs_tail_cap, B.n_streams, cudaMemcpyDeviceToDevice, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
+            CK(cudaFree(ctx->d_rs_tail));
+        }
+        ctx->d_rs_tail = nt;
+        ctx->rs_tail_cap = cap;
+    }
+    for (int s = stream0; s < stream0 + n_streams; s++) { ctx->h_rate[s] = sr_in; ctx->h_inputs[s] = c + n_in; }
+    if (where != EWK_HOST) {
+        rc = ctx->land_resampled(stream0, n_streams, in, stride, in_format, n_in, sr_in, c, -1);
+        return rc ? rc : (int)n;
+    }
+    // host input: its compact bytes cross PCIe on the copy stream and land lazily, as with ewk_push
+    const size_t esz = rs_in_size(in_format);
+    const int b = ctx->stage_idx;
+    ctx->stage_idx ^= 1;
+    CK(ctx->b_raw[b].ensure(esz * (size_t)n_in * n_streams));
+    if (ctx->ev_free_valid[b]) CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_free[b], 0));
+    if (stride == n_in)
+        CK(cudaMemcpyAsync(ctx->b_raw[b].p, in, esz * (size_t)n_in * n_streams, cudaMemcpyHostToDevice, ctx->copy_stream));
+    else
+        CK(cudaMemcpy2DAsync(ctx->b_raw[b].p, esz * (size_t)n_in, in, esz * (size_t)stride, esz * (size_t)n_in, n_streams,
+                             cudaMemcpyHostToDevice, ctx->copy_stream));
+    CK(cudaEventRecord(ctx->ev_ready[b], ctx->copy_stream));
+    ctx->pending = ewk_ctx::Pending{};
+    ctx->pending.valid = true; ctx->pending.slot = b; ctx->pending.stream0 = stream0; ctx->pending.n_streams = n_streams;
+    ctx->pending.n = n;
+    ctx->pending.rs_rate = sr_in; ctx->pending.rs_fmt = in_format; ctx->pending.rs_n_in = n_in; ctx->pending.rs_c = c;
+    return (int)n;
+}
+
+extern "C" int ewk_stream_input(ewk_ctx* ctx, int stream, int32_t* sr_in, int64_t* n_in) {
+    if (!ctx) return EWK_ERR_ARG;
+    int rc = need_streams(ctx, "ewk_stream_input", false);
+    if (rc) return rc;
+    if (stream < 0 || stream >= ctx->bank.n_streams) { ctx->fail("ewk_stream_input: bad stream %d", stream); return EWK_ERR_ARG; }
+    if (sr_in) *sr_in = ctx->h_rate[stream];
+    if (n_in) *n_in = ctx->h_inputs[stream];
     return EWK_OK;
 }
 

@@ -12,6 +12,7 @@
 #include "ewk_dense.cuh"
 #include "ewk_vad.cuh"
 #include "ewk_resample.cuh"
+#include "ewk_resample_push.cuh"
 #include "ewk_tables.hpp"
 
 #define EWK_MAX_TEMPLATES 64
@@ -59,11 +60,17 @@ struct ewk_ctx {
     cudaStream_t last_match_stream = nullptr;   // where the latest ewk_tick launched K3
     int join_match();
     int stage_idx = 0;
-    struct Pending { bool valid = false; int slot = 0, stream0 = 0, n_streams = 0; long long n = 0; } pending;
+    // n: samples that land in the rings; rs_rate != 0 marks a native-rate push (K8) of rs_n_in inputs at that rate
+    struct Pending {
+        bool valid = false; int slot = 0, stream0 = 0, n_streams = 0; long long n = 0;
+        int rs_rate = 0, rs_fmt = 0; long long rs_n_in = 0, rs_c = 0;
+    } pending;
     int land(int stream0, int n_streams, const void* d_src, long long d_stride, long long n, int stage_slot);
+    int land_resampled(int stream0, int n_streams, const void* d_src, long long d_stride, int in_fmt, long long n_in,
+                       int sr_in, long long c, int stage_slot);
     int flush_pending();
     ewk::DevBuf b_stage2[2];
-    ewk::DevBuf b_raw[2];                    // G.711 codes of a host push (ewk_push_g711), decoded into b_stage2
+    ewk::DevBuf b_raw[2];                    // compact host input: G.711 codes (ewk_push_g711, decoded into b_stage2) or a native-rate feed
     ewk::DeviceTables* d_tables = nullptr;
     ewk::TemplateFeat* d_tmpl = nullptr;
     std::vector<ewk::TemplateFeat> h_tmpl;
@@ -87,6 +94,10 @@ struct ewk_ctx {
     std::vector<long long> h_visible_lb;   // lower bound of StreamState.visible (audio-clock overrun check)
     std::vector<long long> h_tick;
     std::vector<int> h_frame_size;         // latched frame size per stream (0: no push yet)
+    std::vector<int> h_rate;               // input rate latched by the stream's first push (0: none yet; 16000: ewk_push)
+    std::vector<long long> h_inputs;       // input samples the stream received (at its own rate)
+    float* d_rs_tail = nullptr;            // K8 input tails [n_streams][rs_tail_cap], sized by the rates in use
+    int rs_tail_cap = 0;
     int gate_chunks() const;               // largest R / frame_size in use
     // per-kernel event timing (ewk_profile)
     bool prof_on = false;
@@ -110,4 +121,5 @@ struct ewk_ctx {
     std::map<int, ResampleTable> rs_tables;
     ewk::DevBuf b_rs_in, b_rs_out;
     int resample_table(int sr_in, const ResampleTable** out);
+    int launch_fir(const ResampleTable& t, ewk::RsPushArgs& A, int n_rows, int prof_cls, const char* who);
 };

@@ -1,4 +1,4 @@
-// K7 — resample_kernel: sample-rate conversion to 16 kHz on the device (SURVEY §8(f) row N3), what the reference
+// K7 — sample-rate conversion to 16 kHz on the device: the filter design and its table (SURVEY §8(f) row N3), what the reference
 // obtains from librosa.load(sr=16000) / librosa.resample (/root/reference/easywakeword/wakeword.py:588, 866-870;
 // examples/tune_threshold.py:33-47; soxr HQ underneath).  soxr is not restated bit for bit (see
 // oracle/resample_restated.py: PARITY UNPINNED); the filter meets soxr HQ's published specification — linear
@@ -6,9 +6,8 @@
 // polyphase stage:    out[n] = sum_k x[k] g(n M / L - k),   L / M = 16000 / sr_in in lowest terms.
 //
 // Table H[j][p] (float32, [2W][L], built on the host in double): tap of input sample k_c - W + 1 + j for phase p,
-// k_c = floor(n M / L), p = n M mod L.  Thread mapping: a group of L consecutive outputs is handled by L
-// consecutive threads ordered by PHASE (thread p computes output g L + (p M^-1 mod L)), so that a warp's table
-// reads are one contiguous row segment; the PCM reads are an L1-resident gather over the group's input span.
+// k_c = floor(n M / L), p = n M mod L.  The FIR that evaluates it for ewk_resample and ewk_push_resampled is K8
+// (ewk_resample_push.cuh).
 #pragma once
 #include <cmath>
 #include <cstdint>
@@ -20,10 +19,9 @@ namespace ewk {
 
 constexpr int RS_TARGET = 16000;
 constexpr int RS_MAX_PHASES = 4096;
-constexpr int RS_THREADS = 256;
 
 struct ResampleDesign {
-    int sr_in = 0, L = 0, M = 0, Minv = 0, W = 0;
+    int sr_in = 0, L = 0, M = 0, W = 0;
     double fc = 0, beta = 0;
 };
 
@@ -52,8 +50,6 @@ inline bool rs_design(int sr_in, ResampleDesign& d) {
     const int n_taps = (int)std::ceil((att - 8.0) / (2.285 * d_omega));
     d.W = (n_taps + 1) / 2;
     d.fc = 0.5 * (f_pass + f_stop) / sr_in;
-    d.Minv = 0;
-    for (int i = 1; i < d.L; i++) if ((long long)i * d.M % d.L == 1) { d.Minv = i; break; }
     return true;
 }
 
@@ -71,49 +67,6 @@ inline void rs_build_table(const ResampleDesign& d, std::vector<float>& H) {
             }
             H[(size_t)j * d.L + p] = (float)v;
         }
-}
-
-struct ResampleArgs {
-    const void* in;         // [rows][in_stride] float32 or int16
-    float* out;             // [rows][out_stride]
-    const float* H;         // [2W][L]
-    long long in_stride, n_in, in_first;      // in[r][i] is absolute input sample in_first + i
-    long long out_stride, out_first, n_out;   // out[r][i] is absolute output sample out_first + i
-    int L, M, Minv, W, fmt;                   // fmt 0 f32, 1 i16
-};
-
-template <typename T>
-__device__ __forceinline__ float rs_load(const T* p);
-template <>
-__device__ __forceinline__ float rs_load<float>(const float* p) { return __ldg(p); }
-template <>
-__device__ __forceinline__ float rs_load<short>(const short* p) { return (float)__ldg(p) * (1.0f / 32768.0f); }
-
-template <typename T>
-__global__ void __launch_bounds__(RS_THREADS) resample_kernel(ResampleArgs A) {
-    const long long idx = (long long)blockIdx.x * RS_THREADS + threadIdx.x;
-    const long long g0 = A.out_first / A.L;
-    const long long g = g0 + idx / A.L;
-    const int p = (int)(idx % A.L);
-    const long long n = g * A.L + (A.L > 1 ? (long long)p * A.Minv % A.L : 0);
-    if (n < A.out_first || n >= A.out_first + A.n_out) return;
-    const long long kc = n * A.M / A.L;                       // n M mod L == p by construction
-    const T* x = reinterpret_cast<const T*>(A.in) + (size_t)blockIdx.y * A.in_stride;
-    const float* h = A.H + p;
-    const long long i0 = kc - A.W + 1 - A.in_first;           // buffer index of tap 0
-    const int taps = 2 * A.W;
-    float acc = 0.f;
-    if (i0 >= 0 && i0 + taps <= A.n_in) {
-        const T* xp = x + i0;
-#pragma unroll 4
-        for (int j = 0; j < taps; j++) acc = fmaf(rs_load(xp + j), h[(size_t)j * A.L], acc);
-    } else {
-        for (int j = 0; j < taps; j++) {
-            const long long i = i0 + j;
-            if (i >= 0 && i < A.n_in) acc = fmaf(rs_load(x + i), h[(size_t)j * A.L], acc);
-        }
-    }
-    A.out[(size_t)blockIdx.y * A.out_stride + (n - A.out_first)] = acc;
 }
 
 }  // namespace ewk

@@ -42,6 +42,13 @@ def resample_to_16k(y, sr_native: int, sr_target: int = TARGET_SR, *, ctx=None, 
     return c.resample(y, sr_native)
 
 
+def ready_outputs(n_in: int, half_width: int, up: int, down: int) -> int:
+    """16 kHz outputs computable from the first n_in input samples: output n needs input up to floor(n * down / up) + W
+    (what ``StreamResampler.push`` emits, and what ``Context.push_resampled`` lands)."""
+    a = n_in - half_width
+    return (a * up + down - 1) // down if a > 0 else 0
+
+
 class StreamResampler:
     """Chunked conversion of [rows, n] feeds to 16 kHz whose concatenated output equals the one-shot result
     sample for sample: every call is given the filter's half-width of history and emits only the outputs whose
@@ -74,10 +81,7 @@ class StreamResampler:
         chunk = np.asarray(chunk, self.dtype).reshape(self.rows, -1)
         self.hist = np.concatenate([self.hist, chunk], axis=1)
         self.n_in += chunk.shape[1]
-        # output n needs input up to floor(n * down / up) + W
-        a = self.n_in - 1 - self.W
-        ready = ((a + 1) * self.up + self.down - 1) // self.down if a >= 0 else 0
-        return self._emit(max(ready, self.n_out))
+        return self._emit(max(ready_outputs(self.n_in, self.W, self.up, self.down), self.n_out))
 
     def flush(self) -> np.ndarray:
         total = int(_lib.load().ewk_resample_out_len(self.n_in, self.sr_in))

@@ -229,6 +229,26 @@ int64_t ewk_resample_out_len(int64_t n_in, int sr_in);
 int ewk_resample(ewk_ctx* ctx, const void* in, int pcm_format, int where_in, int n_rows, int64_t n_in, int64_t in_stride,
                  int sr_in, int64_t in_first, int64_t out_first, int64_t n_out, float* out, int64_t out_stride,
                  int where_out);
+/* Native-rate feeds into the rings (K8): telephony G.711 at 8 kHz, 44.1 / 48 kHz from WebRTC or sound cards.
+ * ewk_push_resampled takes n_in samples per stream at sr_in Hz (stream s reads in + s*stride, in samples of in_format:
+ * EWK_PCM_F32, EWK_PCM_I16 = int16 / 32768, or 8-bit G.711 codes EWK_IN_ULAW / EWK_IN_ALAW = the standard's 16-bit
+ * value / 32768; any format into either ring format) and lands their 16 kHz conversion in the rings in one fused launch.
+ * Sample a of a stream's ring is exactly output a of a one-shot ewk_resample of everything pushed to the stream (int16
+ * rings store rint(y * 32768) clamped to [-32768, 32767], ties to even).  After c input samples, outputs
+ * [0, ready(c)) are in the ring, ready(c) = max(0, ceil((c - W) * up / down)) with W, up, down of ewk_resample_info:
+ * an output lands once its W input samples of look-ahead have arrived (the last W inputs wait for the next push; there
+ * is no final flush).  Returns the number of samples landed per stream (>= 0) or a status.
+ * A stream's input rate is fixed by its first push of any kind.  EWK_ERR_STATE: streams of one call that have received
+ * different numbers of input samples, a different rate than the stream's, a 16 kHz stream, and ewk_push /
+ * ewk_push_g711 onto a native-rate stream.  EWK_ERR_ARG: sr_in = 16000 or a rate ewk_resample rejects.
+ * With frame_size 0 the stream latches ewk_resample_out_len(n_in, sr_in) of its first call, so the audio clock stays on
+ * the nominal 16 kHz grid.  Push guards, host staging (pinned or pageable, on the copy stream, landing lazily) and
+ * overlap mode behave as for ewk_push, on the landed count.  The device keeps each stream's last <= 2W input samples. */
+enum { EWK_IN_ULAW = 2, EWK_IN_ALAW = 3 };
+int ewk_push_resampled(ewk_ctx* ctx, int stream0, int n_streams, const void* in, int in_format, int64_t n_in, int64_t stride,
+                       int where, int sr_in);
+/* rate latched by the stream's first push (0: none yet; 16000: ewk_push / ewk_push_g711) and input samples received */
+int ewk_stream_input(ewk_ctx* ctx, int stream, int32_t* sr_in, int64_t* n_in);
 /* Dense per-hop scoring (SURVEY §8(a) A9; usage shape of examples/tune_threshold.py:86-116 at hop
  * granularity): for every stream, every hop h in [hop0, hop0 + n_hops) (hop h <-> 160*h samples pushed)
  * and every template slot k in [template_first, template_first + template_count), the value
@@ -286,7 +306,8 @@ int ewk_host_free(void* p);
 int64_t ewk_launch_count(const ewk_ctx* ctx);
 /* Per-kernel device timing with CUDA events on the context's stream.  ewk_profile(ctx, 1) starts
  * bracketing every kernel launch with an event pair; ewk_profile_read synchronises and returns, per
- * kernel class (0 ring_push, 1 tick_gate, 2 segment_queue, 3 segment_batch, 4 dense_score, 5 segment_prepare, 6 publish), the summed
+ * kernel class (0 ring_push, 1 tick_gate, 2 segment_queue, 3 segment_batch, 4 dense_score, 5 segment_prepare, 6 publish,
+ * 7 resample_push), the summed
  * milliseconds and the number of launches since profiling was enabled, then resets the sums. */
 enum { EWK_PROF_CLASSES = 8 };
 int ewk_profile(ewk_ctx* ctx, int enable);
