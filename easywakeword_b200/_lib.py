@@ -295,7 +295,9 @@ def _declare_stream_protos(lib):
         "ewk_push": (C.c_int, [vp, i32, i32, vp, i64, i64, i32]),
         "ewk_push_g711": (C.c_int, [vp, i32, i32, vp, i64, i64, i32, i32]),
         "ewk_push_resampled": (C.c_int, [vp, i32, i32, vp, i32, i64, i64, i32, i32]),
+        "ewk_push_resampled_each": (C.c_int, [vp, i32, i32, vp, i32, i64, i64, i32, i32, _p(i64)]),
         "ewk_stream_input": (C.c_int, [vp, i32, _p(C.c_int32), _p(i64)]),
+        "ewk_reset_streams": (C.c_int, [vp, _p(C.c_int32), i32]),
         "ewk_tick": (C.c_int, [vp, i32]),
         "ewk_set_overlap": (C.c_int, [vp, i32]),
         "ewk_join": (C.c_int, [vp]),
@@ -378,6 +380,36 @@ class PinnedArray:
             pass
 
 
+def _resampled_input(pcm_or_codes, fmt):
+    """(ptr, n_streams, n, stride, in_format) of a native-rate feed: an array [n_streams, n] (float32, int16, or uint8
+    G.711 codes with fmt "ulaw" / "alaw") or a device input (ptr, n_streams, n, stride, dtype), and the array behind
+    ptr, which the caller keeps alive across the call."""
+    a = None
+    if isinstance(pcm_or_codes, tuple):
+        ptr, ns, n, stride, dt = pcm_or_codes
+        dt = np.dtype(dt)
+    else:
+        a = pcm_or_codes if pcm_or_codes.ndim == 2 else pcm_or_codes.reshape(1, -1)
+        if a.strides[1] != a.itemsize:
+            a = np.ascontiguousarray(a)
+        ns, n = a.shape
+        stride = a.strides[0] // a.itemsize if ns > 1 else n
+        ptr, dt = a.ctypes.data, a.dtype
+    if dt == np.uint8:
+        if fmt not in ("ulaw", "alaw"):
+            raise ValueError('uint8 input is G.711: fmt must be "ulaw" or "alaw"')
+        code = IN_ULAW if fmt == "ulaw" else IN_ALAW
+    elif fmt is not None:
+        raise ValueError("fmt selects G.711 for uint8 input only")
+    elif dt == np.int16:
+        code = PCM_I16
+    elif dt == np.float32:
+        code = PCM_F32
+    else:
+        raise TypeError(f"push_resampled takes float32, int16 or uint8 G.711 input, got {dt}")
+    return ptr, ns, n, stride, code, a
+
+
 def _bank_methods():
     def set_stream_params(self, stream=-1, params=None, **over):
         p = params if params is not None else default_stream_params(**over)
@@ -422,32 +454,29 @@ def _bank_methods():
         include/ewk.h: ewk_push_resampled).  The input format follows the dtype: float32, int16, or uint8 G.711 codes with
         fmt="ulaw" / "alaw" (into either ring format).  A device input is (ptr, n_streams, n, stride, dtype).
         Returns the number of 16 kHz samples landed per stream."""
-        if isinstance(pcm_or_codes, tuple):
-            ptr, ns, n, stride, dt = pcm_or_codes
-            dt = np.dtype(dt)
-        else:
-            a = pcm_or_codes if pcm_or_codes.ndim == 2 else pcm_or_codes.reshape(1, -1)
-            if a.strides[1] != a.itemsize:
-                a = np.ascontiguousarray(a)
-            ns, n = a.shape
-            stride = a.strides[0] // a.itemsize if ns > 1 else n
-            ptr, dt = a.ctypes.data, a.dtype
-        if dt == np.uint8:
-            if fmt not in ("ulaw", "alaw"):
-                raise ValueError('uint8 input is G.711: fmt must be "ulaw" or "alaw"')
-            code = IN_ULAW if fmt == "ulaw" else IN_ALAW
-        elif fmt is not None:
-            raise ValueError("fmt selects G.711 for uint8 input only")
-        elif dt == np.int16:
-            code = PCM_I16
-        elif dt == np.float32:
-            code = PCM_F32
-        else:
-            raise TypeError(f"push_resampled takes float32, int16 or uint8 G.711 input, got {dt}")
+        ptr, ns, n, stride, code, _keep = _resampled_input(pcm_or_codes, fmt)
         rc = self.lib.ewk_push_resampled(self.h, stream0, ns, ptr, code, n, stride, where, int(sr_in))
         if rc < 0:
             self._ck(rc)
         return rc
+
+    def push_resampled_each(self, pcm_or_codes, sr_in, stream0=0, where=HOST, fmt=None):
+        """push_resampled for streams at their own input positions (recycled streams restart at 0), in one launch
+        (include/ewk.h: ewk_push_resampled_each).  Returns int64 [n_streams]: the 16 kHz samples landed per stream."""
+        ptr, ns, n, stride, code, _keep = _resampled_input(pcm_or_codes, fmt)
+        landed = np.zeros(ns, np.int64)
+        self._ck(self.lib.ewk_push_resampled_each(self.h, stream0, ns, ptr, code, n, stride, where, int(sr_in),
+                                                  landed.ctypes.data_as(_p(C.c_int64))))
+        return landed
+
+    def reset_streams(self, streams):
+        """Return the listed streams to the state of a new context (include/ewk.h: ewk_reset_streams); their parameters
+        stay.  The event queue must be empty (poll first)."""
+        lst = np.ascontiguousarray(np.asarray(streams, dtype=np.int64).reshape(-1))
+        if lst.size and (lst.min() < -2**31 or lst.max() >= 2**31):
+            raise ValueError("stream index out of range")
+        lst = lst.astype(np.int32)
+        self._ck(self.lib.ewk_reset_streams(self.h, lst.ctypes.data_as(_p(C.c_int32)), int(lst.size)))
 
     def stream_input(self, stream):
         """-> (input rate latched by the stream's first push (0: none yet), input samples received)."""
@@ -587,7 +616,7 @@ def _bank_methods():
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
     for f in (prepare_segments, dense_scores, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
-              stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
+              push_resampled_each, reset_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
               set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count):
         setattr(Context, f.__name__, f)
 

@@ -28,6 +28,12 @@ class WakeWordBank:
     44.1 / 48 kHz devices) is converted to 16 kHz on the device as it lands (K8); the rings, the timing and
     samples_pushed are in 16 kHz samples.
 
+    Streams are recycled with reset(streams): a stream that served one call takes the next without touching the others.
+    A recycled stream's event ticks and seg_start count from its reset, as in a new bank.  At a sample_rate other than
+    16000 its input restarts at position 0 while the others go on, and one push still serves them all;
+    samples_pushed (the clock step() ticks by) then advances by the largest count landed, and status(s).written holds a
+    stream's own count.
+
     templates: list of float32 arrays or WAV paths (slot i = templates[i]); every stream is scored
     against all of them (best score wins) unless set_stream(..., template_first=, template_count=).
     Timing defaults are the reference's (wakeword.py:38-41); speech_duration_min/max default to the
@@ -96,12 +102,25 @@ class WakeWordBank:
         p.update(overrides)
         self.ctx.set_stream_params(stream, **p)
 
+    def reset(self, streams, **overrides) -> np.ndarray:
+        """Recycle `streams` (a new call on each slot): drains the event queue and returns those events (handle them as
+        poll()'s; no event of the old sessions can surface afterwards), then returns the streams to the state of a new
+        bank in one launch (include/ewk.h: ewk_reset_streams).  Their parameters stay unless `overrides` are given:
+        those are applied to each stream through set_stream (e.g. another template range or threshold)."""
+        events = self.poll()
+        lst = [int(s) for s in np.asarray(streams, dtype=np.int64).reshape(-1)]
+        self.ctx.reset_streams(lst)
+        if overrides:
+            for s in dict.fromkeys(lst):
+                self.set_stream(s, **overrides)
+        return events
+
     # ---- data plane
     def push(self, pcm, where=_lib.HOST):
         """pcm[n_streams, n]: n new samples for every stream (K1 / direct H2D) in the bank's dtype; at another
         sample_rate, float32 or int16 at that rate (K8; a device input is (ptr, n_streams, n, stride, dtype))."""
         if self.sample_rate != 16000:
-            self.samples_pushed += self.ctx.push_resampled(pcm, self.sample_rate, stream0=0, where=where)
+            self.samples_pushed += int(self.ctx.push_resampled_each(pcm, self.sample_rate, stream0=0, where=where).max())
             return
         self.ctx.push(pcm, stream0=0, where=where)
         self.samples_pushed += pcm[2] if isinstance(pcm, tuple) else pcm.shape[-1]
@@ -114,7 +133,8 @@ class WakeWordBank:
                 raise ValueError("law must be 'ulaw' or 'alaw'")
             if isinstance(codes, tuple):
                 codes = (*codes[:4], np.uint8)
-            self.samples_pushed += self.ctx.push_resampled(codes, self.sample_rate, stream0=0, where=where, fmt=law)
+            self.samples_pushed += int(self.ctx.push_resampled_each(codes, self.sample_rate, stream0=0, where=where,
+                                                                    fmt=law).max())
             return
         self.ctx.push_g711(codes, stream0=0, where=where, law=law)
         self.samples_pushed += codes[2] if isinstance(codes, tuple) else codes.shape[-1]

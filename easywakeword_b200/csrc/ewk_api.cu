@@ -8,6 +8,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/ewk.h"
@@ -199,7 +200,12 @@ void ewk_ctx::release() {
         ev_ready[i] = ev_free[i] = nullptr;
         b_stage2[i].free();
         b_raw[i].free();
+        if (ev_pos[i]) cudaEventDestroy(ev_pos[i]);
+        if (h_pos[i]) cudaFreeHost(h_pos[i]);
+        ev_pos[i] = nullptr; h_pos[i] = nullptr;
+        b_pos[i].free();
     }
+    b_reset.free();
     if (own_stream) cudaStreamDestroy(own_stream);
     d_tables = nullptr; d_tmpl = nullptr; own_stream = nullptr; copy_stream = nullptr;
 }
@@ -796,9 +802,12 @@ int ewk_ctx::land(int stream0, int n_streams, const void* d_src, long long d_str
 int ewk_ctx::flush_pending() {
     if (!pending.valid) return EWK_OK;
     pending.valid = false;
-    if (pending.rs_rate)
+    if (pending.rs_rate) {
+        const bool each = pending.rs_pos_slot >= 0;
         return land_resampled(pending.stream0, pending.n_streams, b_raw[pending.slot].p, pending.rs_n_in, pending.rs_fmt,
-                              pending.rs_n_in, pending.rs_rate, pending.rs_c, pending.slot);
+                              pending.rs_n_in, pending.rs_rate, each ? pending.rs_pos.data() : &pending.rs_c,
+                              each ? (const long long*)b_pos[pending.rs_pos_slot].p : nullptr, pending.slot);
+    }
     return land(pending.stream0, pending.n_streams, b_stage2[pending.slot].p, pending.n, pending.n, pending.slot);
 }
 
@@ -950,7 +959,8 @@ static long long rs_tail_start(long long c, const ResampleDesign& d) {
 static size_t rs_in_size(int in_fmt) { return in_fmt == EWK_PCM_F32 ? 4 : in_fmt == EWK_PCM_I16 ? 2 : 1; }
 
 // The FIR (K8) over rows [0, n_rows) of A: plans the work mapping (fast or generic path, tile, staged span) and launches.
-int ewk_ctx::launch_fir(const ResampleTable& t, RsPushArgs& A, int n_rows, int prof_cls, const char* who) {
+int ewk_ctx::launch_fir(const ResampleTable& t, RsPushArgs& A, int n_rows, int prof_cls, const char* who,
+                        const long long* pos) {
     ewk_ctx* ctx = this;
     const ResampleDesign& d = t.d;
     const int taps = 2 * d.W;
@@ -960,11 +970,9 @@ int ewk_ctx::launch_fir(const ResampleTable& t, RsPushArgs& A, int n_rows, int p
     if ((d.L == 1 || d.L == 2 || d.L == 4 || d.L == 8) && d.M <= 3 && A.table_smem &&
         (RSP_THREADS / d.L) * rsp_k(d.M) * d.M >= taps + d.M)
         fast_m = d.M;
-    long long first;
     if (fast_m) {
         A.tile = RSP_THREADS * rsp_k(d.M);
         A.span = (RSP_THREADS / d.L) * rsp_k(d.M) * d.M + taps + d.M + 1;
-        first = (A.o0 / d.L) * d.L;
     } else {
         auto span = [&](long long tile) { return (tile * d.M + d.L - 1) / d.L + taps + 1; };
         long long tile = RSP_GENERIC_TILE;
@@ -973,13 +981,24 @@ int ewk_ctx::launch_fir(const ResampleTable& t, RsPushArgs& A, int n_rows, int p
         tile = std::max(tile, (need + RSP_THREADS - 1) / RSP_THREADS * RSP_THREADS);
         A.tile = (int)tile;
         A.span = (int)span(tile);
-        first = A.o0;
     }
     const size_t smem = sizeof(float) * ((size_t)256 + A.tail_cap + (A.table_smem ? (size_t)taps * d.L : 0) + A.span);
     if (smem > (size_t)200 * 1024) { fail("%s: %d Hz needs %zu bytes of shared memory", who, d.sr_in, smem); return EWK_ERR_ARG; }
-    const dim3 grid((unsigned)std::max<long long>(1, (A.o1 - first + A.tile - 1) / A.tile), (unsigned)n_rows);
-    auto k8 = fast_m == 1 ? resample_push_kernel<1> : fast_m == 2 ? resample_push_kernel<2> : fast_m == 3 ? resample_push_kernel<3>
-                                                                                        : resample_push_kernel<0>;
+    // output tiles of a row: its outputs [o0, o1) from the first tile start (fast path: o0 rounded down to a phase group)
+    auto tiles = [&](long long o0, long long o1) {
+        const long long first = fast_m ? (o0 / d.L) * d.L : o0;
+        return std::max<long long>(1, (o1 - first + A.tile - 1) / A.tile);
+    };
+    long long n_tiles = tiles(A.o0, A.o1);
+    if (pos)
+        for (int y = 0; y < n_rows; y++) n_tiles = std::max(n_tiles, tiles(rs_ready(pos[y], d), rs_ready(pos[y] + A.n_in, d)));
+    const dim3 grid((unsigned)n_tiles, (unsigned)n_rows);
+    auto pick = [&](auto each) {
+        constexpr bool E = decltype(each)::value;
+        return fast_m == 1 ? resample_push_kernel<1, E> : fast_m == 2 ? resample_push_kernel<2, E>
+             : fast_m == 3 ? resample_push_kernel<3, E> : resample_push_kernel<0, E>;
+    };
+    auto k8 = A.pos ? pick(std::true_type{}) : pick(std::false_type{});
     CK(cudaFuncSetAttribute(k8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaEvent_t pe = prof_begin(prof_cls);
     k8<<<grid, RSP_THREADS, smem, stream>>>(bank, A);
@@ -989,14 +1008,16 @@ int ewk_ctx::launch_fir(const ResampleTable& t, RsPushArgs& A, int n_rows, int p
     return EWK_OK;
 }
 
-// K8 on device-resident input (the caller's buffer or a staging slot): every stream of the call has received c inputs
+// K8 on device-resident input (the caller's buffer or a staging slot): stream stream0 + i has received pos[i] inputs
+// (d_pos: the device copy of pos[0 .. n_streams) when they differ; null: every stream sits at pos[0])
 int ewk_ctx::land_resampled(int stream0, int n_streams, const void* d_src, long long d_stride, int in_fmt, long long n_in,
-                            int sr_in, long long c, int stage_slot) {
+                            int sr_in, const long long* pos, const long long* d_pos, int stage_slot) {
     ewk_ctx* ctx = this;
     const ResampleTable* t = nullptr;
     int rc = resample_table(sr_in, &t);
     if (rc) return rc;
     const ResampleDesign& d = t->d;
+    const long long c = pos[0];
     RsPushArgs A{};
     A.in = d_src; A.in_stride = d_stride; A.n_in = n_in; A.in_fmt = in_fmt;
     A.tail = d_rs_tail; A.tail_cap = rs_tail_cap; A.H = t->H;
@@ -1004,67 +1025,82 @@ int ewk_ctx::land_resampled(int stream0, int n_streams, const void* d_src, long 
     A.c = c; A.o0 = rs_ready(c, d); A.o1 = rs_ready(c + n_in, d);
     A.t0_old = rs_tail_start(c, d); A.t0_new = rs_tail_start(c + n_in, d);
     A.frame_latch = (int)ewk_resample_out_len(n_in, sr_in);
+    A.pos = d_pos;
     if (stage_slot >= 0) CK(cudaStreamWaitEvent(stream, ev_ready[stage_slot], 0));
-    rc = launch_fir(*t, A, n_streams, 7, "ewk_push_resampled");
+    rc = launch_fir(*t, A, n_streams, 7, "ewk_push_resampled", d_pos ? pos : nullptr);
     if (rc) return rc;
     if (stage_slot >= 0) {
         CK(cudaEventRecord(ev_free[stage_slot], stream));
         ev_free_valid[stage_slot] = true;
     }
+    if (d_pos) {                            // the positions' slot is free once this K8 has read them
+        const int k = (int)(d_pos == (const long long*)b_pos[1].p);
+        CK(cudaEventRecord(ev_pos[k], stream));
+        ev_pos_valid[k] = true;
+    }
     all_presummed = false;                  // K8 forms no block sums: K2 reads these samples
     pushes_since_tick++;
-    for (int s = stream0; s < stream0 + n_streams; s++) {
-        h_written[s] = A.o1;
+    for (int i = 0; i < n_streams; i++) {
+        const int s = stream0 + i;
+        h_written[s] = rs_ready((d_pos ? pos[i] : c) + n_in, d);
         if (h_frame_size[s] == 0) h_frame_size[s] = h_prm[s].frame_size > 0 ? h_prm[s].frame_size : A.frame_latch;
     }
     return EWK_OK;
 }
 
-extern "C" int ewk_push_resampled(ewk_ctx* ctx, int stream0, int n_streams, const void* in, int in_format, int64_t n_in,
-                                  int64_t stride, int where, int sr_in) {
-    if (!ctx) return EWK_ERR_ARG;
-    int rc = need_streams(ctx, "ewk_push_resampled", false);
+// ewk_push_resampled (each = false: every stream of the call at the same input position, returns the landed count) and
+// ewk_push_resampled_each (streams at their own positions, landed counts into landed[])
+static int push_resampled_impl(ewk_ctx* ctx, const char* who, int stream0, int n_streams, const void* in, int in_format,
+                               int64_t n_in, int64_t stride, int where, int sr_in, bool each, int64_t* landed) {
+    int rc = need_streams(ctx, who, false);
     if (rc) return rc;
     BankView& B = ctx->bank;
     if (!in || n_streams < 1 || stream0 < 0 || stream0 + n_streams > B.n_streams || n_in < 1 || stride < n_in ||
-        in_format < EWK_PCM_F32 || in_format > EWK_IN_ALAW || n_in > (int64_t)1 << 34) {
-        ctx->fail("ewk_push_resampled: bad arguments (stream0=%d n_streams=%d n_in=%lld stride=%lld in_format=%d)", stream0,
-                  n_streams, (long long)n_in, (long long)stride, in_format);
+        in_format < EWK_PCM_F32 || in_format > EWK_IN_ALAW || n_in > (int64_t)1 << 34 || (each && !landed)) {
+        ctx->fail("%s: bad arguments (stream0=%d n_streams=%d n_in=%lld stride=%lld in_format=%d%s)", who, stream0,
+                  n_streams, (long long)n_in, (long long)stride, in_format, each && !landed ? ", landed is NULL" : "");
         return EWK_ERR_ARG;
     }
     ResampleDesign d;
     if (sr_in == RS_TARGET || sr_in < 1000 || sr_in > 768000 || !rs_design(sr_in, d)) {
-        ctx->fail("ewk_push_resampled: %d Hz is not a supported input rate (16000 Hz input goes through ewk_push)", sr_in);
+        ctx->fail("%s: %d Hz is not a supported input rate (16000 Hz input goes through ewk_push)", who, sr_in);
         return EWK_ERR_ARG;
     }
     const long long c = ctx->h_inputs[stream0];
+    bool uniform = true;
     for (int s = stream0; s < stream0 + n_streams; s++) {
         if (ctx->h_rate[s] != 0 && ctx->h_rate[s] != sr_in) {
-            ctx->fail("ewk_push_resampled: stream %d already takes %d Hz input", s, ctx->h_rate[s]);
+            ctx->fail("%s: stream %d already takes %d Hz input", who, s, ctx->h_rate[s]);
             return EWK_ERR_STATE;
         }
         if (ctx->h_inputs[s] != c) {
-            ctx->fail("ewk_push_resampled: streams %d and %d have received %lld and %lld input samples; one call takes streams "
-                      "at the same position", stream0, s, c, ctx->h_inputs[s]);
-            return EWK_ERR_STATE;
+            if (!each) {
+                ctx->fail("%s: streams %d and %d have received %lld and %lld input samples; one call takes streams "
+                          "at the same position", who, stream0, s, c, ctx->h_inputs[s]);
+                return EWK_ERR_STATE;
+            }
+            uniform = false;
         }
     }
-    const long long n = rs_ready(c + n_in, d) - rs_ready(c, d);            // samples this call lands
-    if (n > B.P - B.R && n > B.R) { ctx->fail("ewk_push_resampled: %lld samples exceed the ring (%d)", n, B.R); return EWK_ERR_ARG; }
+    for (int s = stream0; s < stream0 + n_streams; s++) {
+        const long long n = rs_ready(ctx->h_inputs[s] + n_in, d) - rs_ready(ctx->h_inputs[s], d);   // samples it lands
+        if (n > B.P - B.R && n > B.R) { ctx->fail("%s: %lld samples exceed the ring (%d)", who, n, B.R); return EWK_ERR_ARG; }
+    }
     CK(cudaSetDevice(ctx->device));
     rc = ctx->flush_pending();
     if (rc) return rc;
-    for (int s = stream0; s < stream0 + n_streams; s++) {     // same guard as ewk_push, on the landed count
+    for (int s = stream0; s < stream0 + n_streams; s++) {     // same guard as ewk_push, on the stream's landed count
         if (ctx->h_prm[s].live) continue;
+        const long long n = rs_ready(ctx->h_inputs[s] + n_in, d) - rs_ready(ctx->h_inputs[s], d);
         const long long ahead = ctx->h_written[s] + n - ctx->h_visible_lb[s];
         if (ctx->h_visible_lb[s] >= B.R && ahead > (long long)(B.P - B.R)) {
-            ctx->fail("ewk_push_resampled: stream %d would hold %lld un-gated samples, more than slack_samples=%d; call "
-                      "ewk_tick first", s, ahead, B.P - B.R);
+            ctx->fail("%s: stream %d would hold %lld un-gated samples, more than slack_samples=%d; call "
+                      "ewk_tick first", who, s, ahead, B.P - B.R);
             return EWK_ERR_STATE;
         }
         if (ctx->h_visible_lb[s] < B.R && ctx->h_written[s] + n > (long long)B.P) {
-            ctx->fail("ewk_push_resampled: stream %d would hold %lld samples before its first full tick, more than the physical "
-                      "ring (%d); call ewk_tick first", s, ctx->h_written[s] + n, B.P);
+            ctx->fail("%s: stream %d would hold %lld samples before its first full tick, more than the physical "
+                      "ring (%d); call ewk_tick first", who, s, ctx->h_written[s] + n, B.P);
             return EWK_ERR_STATE;
         }
     }
@@ -1085,10 +1121,35 @@ extern "C" int ewk_push_resampled(ewk_ctx* ctx, int stream0, int n_streams, cons
         ctx->d_rs_tail = nt;
         ctx->rs_tail_cap = cap;
     }
-    for (int s = stream0; s < stream0 + n_streams; s++) { ctx->h_rate[s] = sr_in; ctx->h_inputs[s] = c + n_in; }
+    std::vector<long long> pos(ctx->h_inputs.begin() + stream0, ctx->h_inputs.begin() + stream0 + n_streams);
+    for (int i = 0; i < n_streams; i++) {
+        if (landed) landed[i] = rs_ready(pos[i] + n_in, d) - rs_ready(pos[i], d);
+        ctx->h_rate[stream0 + i] = sr_in;
+        ctx->h_inputs[stream0 + i] = pos[i] + n_in;
+    }
+    const int n_ret = (int)(rs_ready(c + n_in, d) - rs_ready(c, d));
+    // streams at different positions: their positions go to the device in a slot of their own, which a later push
+    // reuses only after the K8 that reads them has run
+    int k = -1;
+    cudaStream_t on = where == EWK_HOST ? ctx->copy_stream : ctx->stream;
+    if (!uniform) {
+        k = ctx->pos_idx;
+        ctx->pos_idx ^= 1;
+        const size_t bytes = sizeof(long long) * (size_t)B.n_streams;
+        if (!ctx->h_pos[k]) {
+            CK(cudaHostAlloc((void**)&ctx->h_pos[k], bytes, cudaHostAllocDefault));
+            CK(cudaEventCreateWithFlags(&ctx->ev_pos[k], cudaEventDisableTiming));
+        }
+        CK(ctx->b_pos[k].ensure(bytes));
+        if (ctx->ev_pos_valid[k]) CK(cudaEventSynchronize(ctx->ev_pos[k]));
+        std::memcpy(ctx->h_pos[k], pos.data(), sizeof(long long) * (size_t)n_streams);
+        // host input: on the copy stream ahead of the input's copy, so the K8 that waits for that copy finds them
+        CK(cudaMemcpyAsync(ctx->b_pos[k].p, ctx->h_pos[k], sizeof(long long) * (size_t)n_streams, cudaMemcpyHostToDevice, on));
+    }
+    const long long* d_pos = k >= 0 ? (const long long*)ctx->b_pos[k].p : nullptr;
     if (where != EWK_HOST) {
-        rc = ctx->land_resampled(stream0, n_streams, in, stride, in_format, n_in, sr_in, c, -1);
-        return rc ? rc : (int)n;
+        rc = ctx->land_resampled(stream0, n_streams, in, stride, in_format, n_in, sr_in, pos.data(), d_pos, -1);
+        return rc ? rc : (each ? EWK_OK : n_ret);
     }
     // host input: its compact bytes cross PCIe on the copy stream and land lazily, as with ewk_push
     const size_t esz = rs_in_size(in_format);
@@ -1104,9 +1165,24 @@ extern "C" int ewk_push_resampled(ewk_ctx* ctx, int stream0, int n_streams, cons
     CK(cudaEventRecord(ctx->ev_ready[b], ctx->copy_stream));
     ctx->pending = ewk_ctx::Pending{};
     ctx->pending.valid = true; ctx->pending.slot = b; ctx->pending.stream0 = stream0; ctx->pending.n_streams = n_streams;
-    ctx->pending.n = n;
+    ctx->pending.n = n_ret;
     ctx->pending.rs_rate = sr_in; ctx->pending.rs_fmt = in_format; ctx->pending.rs_n_in = n_in; ctx->pending.rs_c = c;
-    return (int)n;
+    if (k >= 0) { ctx->pending.rs_pos_slot = k; ctx->pending.rs_pos = std::move(pos); }
+    return each ? EWK_OK : n_ret;
+}
+
+extern "C" int ewk_push_resampled(ewk_ctx* ctx, int stream0, int n_streams, const void* in, int in_format, int64_t n_in,
+                                  int64_t stride, int where, int sr_in) {
+    if (!ctx) return EWK_ERR_ARG;
+    return push_resampled_impl(ctx, "ewk_push_resampled", stream0, n_streams, in, in_format, n_in, stride, where, sr_in,
+                               false, nullptr);
+}
+
+extern "C" int ewk_push_resampled_each(ewk_ctx* ctx, int stream0, int n_streams, const void* in, int in_format,
+                                       int64_t n_in, int64_t stride, int where, int sr_in, int64_t* landed) {
+    if (!ctx) return EWK_ERR_ARG;
+    return push_resampled_impl(ctx, "ewk_push_resampled_each", stream0, n_streams, in, in_format, n_in, stride, where,
+                               sr_in, true, landed);
 }
 
 extern "C" int ewk_stream_input(ewk_ctx* ctx, int stream, int32_t* sr_in, int64_t* n_in) {
@@ -1116,6 +1192,48 @@ extern "C" int ewk_stream_input(ewk_ctx* ctx, int stream, int32_t* sr_in, int64_
     if (stream < 0 || stream >= ctx->bank.n_streams) { ctx->fail("ewk_stream_input: bad stream %d", stream); return EWK_ERR_ARG; }
     if (sr_in) *sr_in = ctx->h_rate[stream];
     if (n_in) *n_in = ctx->h_inputs[stream];
+    return EWK_OK;
+}
+
+// K9: streams back to the state ewk_create gives them, in one launch; host mirrors with them.  all_presummed may stay
+// set: K2 takes a stream's block sums only for ticks at or past its ss_from (reset to 0, as in a new context), a stream
+// with nothing written reads no samples at all, and the next push of the stream restarts its sums or clears the flag.
+extern "C" int ewk_reset_streams(ewk_ctx* ctx, const int32_t* streams, int n) {
+    if (!ctx) return EWK_ERR_ARG;
+    int rc = need_streams(ctx, "ewk_reset_streams");       // overlap mode: K3 still reads the rings
+    if (rc) return rc;
+    BankView& B = ctx->bank;
+    if (n < 0 || (n > 0 && !streams)) { ctx->fail("ewk_reset_streams: bad stream list (n=%d)", n); return EWK_ERR_ARG; }
+    for (int i = 0; i < n; i++)
+        if (streams[i] < 0 || streams[i] >= B.n_streams) {
+            ctx->fail("ewk_reset_streams: bad stream %d (context has %d)", streams[i], B.n_streams);
+            return EWK_ERR_ARG;
+        }
+    if (n == 0) return EWK_OK;
+    CK(cudaSetDevice(ctx->device));
+    rc = ctx->flush_pending();                              // a pending host push belongs to the old sessions
+    if (rc) return rc;
+    // events carry no session: one polled after its stream restarted would point at the new session's audio
+    int cnt[2] = {0, 0};
+    CK(cudaMemcpyAsync(cnt, B.ev_count, sizeof(cnt), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (cnt[0] != 0 || cnt[1] != 0) {
+        ctx->fail("ewk_reset_streams: %d events are queued; poll first", cnt[0]);
+        return EWK_ERR_STATE;
+    }
+    CK(ctx->b_reset.ensure(sizeof(int32_t) * (size_t)n));
+    CK(cudaMemcpyAsync(ctx->b_reset.p, streams, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    const size_t row_bytes = (size_t)B.P * (B.fmt == 1 ? 2 : 4);
+    const dim3 grid((unsigned)((row_bytes + RESET_SLICE - 1) / RESET_SLICE), (unsigned)std::min(n, 65535));
+    stream_reset_kernel<<<grid, RESET_THREADS, 0, ctx->stream>>>(B, (const int*)ctx->b_reset.p, n,
+                                                                 (long long*)ctx->b_keep_end.p);
+    CK(cudaGetLastError());
+    ctx->launches++;
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        ctx->h_written[s] = 0; ctx->h_visible_lb[s] = 0; ctx->h_tick[s] = 0;
+        ctx->h_frame_size[s] = 0; ctx->h_rate[s] = 0; ctx->h_inputs[s] = 0;
+    }
     return EWK_OK;
 }
 

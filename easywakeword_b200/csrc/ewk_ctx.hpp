@@ -60,14 +60,25 @@ struct ewk_ctx {
     cudaStream_t last_match_stream = nullptr;   // where the latest ewk_tick launched K3
     int join_match();
     int stage_idx = 0;
-    // n: samples that land in the rings; rs_rate != 0 marks a native-rate push (K8) of rs_n_in inputs at that rate
+    // n: samples that land in the rings; rs_rate != 0 marks a native-rate push (K8) of rs_n_in inputs at that rate, from
+    // input position rs_c, or from the per-stream positions rs_pos (device copy in pos slot rs_pos_slot) when they differ
     struct Pending {
         bool valid = false; int slot = 0, stream0 = 0, n_streams = 0; long long n = 0;
         int rs_rate = 0, rs_fmt = 0; long long rs_n_in = 0, rs_c = 0;
+        int rs_pos_slot = -1; std::vector<long long> rs_pos;
     } pending;
     int land(int stream0, int n_streams, const void* d_src, long long d_stride, long long n, int stage_slot);
+    // pos: host positions of the call's streams; d_pos: their device copy, null when they are all equal (uniform K8)
     int land_resampled(int stream0, int n_streams, const void* d_src, long long d_stride, int in_fmt, long long n_in,
-                       int sr_in, long long c, int stage_slot);
+                       int sr_in, const long long* pos, const long long* d_pos, int stage_slot);
+    // per-stream K8 input positions of a push at different positions (ewk_push_resampled_each): two slots of pinned host
+    // + device memory, each reused only once the K8 that read it has finished (ev_pos)
+    long long* h_pos[2] = {nullptr, nullptr};
+    ewk::DevBuf b_pos[2];
+    cudaEvent_t ev_pos[2] = {nullptr, nullptr};
+    bool ev_pos_valid[2] = {false, false};
+    int pos_idx = 0;
+    ewk::DevBuf b_reset;                     // K9's stream list
     int flush_pending();
     ewk::DevBuf b_stage2[2];
     ewk::DevBuf b_raw[2];                    // compact host input: G.711 codes (ewk_push_g711, decoded into b_stage2) or a native-rate feed
@@ -121,5 +132,7 @@ struct ewk_ctx {
     std::map<int, ResampleTable> rs_tables;
     ewk::DevBuf b_rs_in, b_rs_out;
     int resample_table(int sr_in, const ResampleTable** out);
-    int launch_fir(const ResampleTable& t, ewk::RsPushArgs& A, int n_rows, int prof_cls, const char* who);
+    // pos (host, optional): per-row input positions; the grid covers the row with the most output tiles
+    int launch_fir(const ResampleTable& t, ewk::RsPushArgs& A, int n_rows, int prof_cls, const char* who,
+                   const long long* pos = nullptr);
 };

@@ -45,7 +45,30 @@ struct RsPushArgs {
     int tail_cap, in_fmt, L, M, W, stream0, frame_latch, tile, table_smem, span;   // span: staged input floats per CTA
     float* out;                 // non-null: ewk_resample — outputs [o0, o1) of row y go to out + y * out_stride as float32;
     long long out_stride;       //   the input holds absolute samples [c, c + n_in) (c = t0_old, no tail); no ring, no commit
+    const long long* pos;       // non-null: [n_streams] inputs row y's stream had received before the call; the row's c, o0,
+                                //   o1, t0_old and t0_new follow from it (rsp_row) instead of the uniform values above
 };
+
+// outputs whose W inputs of look-ahead have arrived after c inputs, and the first input any later output reads (the
+// host's rs_ready / rs_tail_start)
+__device__ __forceinline__ long long rsp_ready(long long c, const RsPushArgs& A) {
+    const long long a = c - A.W;
+    return a <= 0 ? 0 : (a * A.L + A.M - 1) / A.M;
+}
+__device__ __forceinline__ long long rsp_tail_start(long long c, const RsPushArgs& A) {
+    const long long t = rsp_ready(c, A) * A.M / A.L - A.W + 1;
+    return t > 0 ? t : 0;
+}
+
+// the positions of row y: per-row (EACH: A.pos, ewk_push_resampled_each) or the call's uniform values.  The uniform
+// instance keeps them in the parameter bank, which leaves its register count (and occupancy) as it was
+struct RsRow { long long c, o0, o1, t0_old, t0_new; };
+template <bool EACH>
+__device__ __forceinline__ RsRow rsp_row(const RsPushArgs& A, int y) {
+    if (!EACH) return RsRow{A.c, A.o0, A.o1, A.t0_old, A.t0_new};
+    const long long c = A.pos[y];
+    return RsRow{c, rsp_ready(c, A), rsp_ready(c + A.n_in, A), rsp_tail_start(c, A), rsp_tail_start(c + A.n_in, A)};
+}
 
 __device__ __forceinline__ float g711_value(int code, int alaw) {
     int v;
@@ -72,11 +95,11 @@ __device__ __forceinline__ float rsp_chunk(const RsPushArgs& A, const void* row,
 
 // absolute input sample k of the stream: zeros before 0 and beyond what has arrived.  Below t0_old (> 0 once the stream
 // is under way) only outputs before o0 read, which this call computes on the fast path but does not store.
-__device__ __forceinline__ float rsp_input(const RsPushArgs& A, const float* tail, const void* row, long long k,
-                                           const float* lut) {
-    if (k < A.t0_old) return 0.f;
-    if (k < A.c) return tail[k - A.t0_old];
-    if (k < A.c + A.n_in) return rsp_chunk(A, row, k - A.c, lut);
+__device__ __forceinline__ float rsp_input(const RsPushArgs& A, const RsRow& R, const float* tail, const void* row,
+                                           long long k, const float* lut) {
+    if (k < R.t0_old) return 0.f;
+    if (k < R.c) return tail[k - R.t0_old];
+    if (k < R.c + A.n_in) return rsp_chunk(A, row, k - R.c, lut);
     return 0.f;
 }
 
@@ -124,7 +147,7 @@ __device__ __forceinline__ void rsp_fir_windows(const float* __restrict__ xs, in
     }
 }
 
-template <int M>
+template <int M, bool EACH>
 __global__ void __launch_bounds__(RSP_THREADS, 2) resample_push_kernel(BankView B, RsPushArgs A) {
     extern __shared__ float smem[];
     float* lut = smem;                                          // [256]
@@ -144,22 +167,25 @@ __global__ void __launch_bounds__(RSP_THREADS, 2) resample_push_kernel(BankView 
     const float* h = A.table_smem ? hs : A.H;
 
     // the CTA's outputs [n0, n0 + tile) and the input span they read, from absolute sample s0
+    const RsRow R = rsp_row<EACH>(A, blockIdx.y);
     const bool fast = M > 0;
     long long n0, s0;
     if (fast) {
-        n0 = (A.o0 / A.L) * A.L + (long long)blockIdx.x * A.tile;
+        n0 = (R.o0 / A.L) * A.L + (long long)blockIdx.x * A.tile;
         s0 = (n0 / A.L) * M - A.W + 1;
     } else {
-        n0 = A.o0 + (long long)blockIdx.x * A.tile;
+        n0 = R.o0 + (long long)blockIdx.x * A.tile;
         s0 = n0 * A.M / A.L - A.W + 1;
     }
-    for (int i = tid; i < A.span; i += RSP_THREADS) xs[i] = rsp_input(A, tail, row, s0 + i, lut);
+    // rows at different positions: the grid covers the row with the most tiles; CTA 0 always runs (tail, commit)
+    if (blockIdx.x > 0 && n0 >= R.o1) return;
+    for (int i = tid; i < A.span; i += RSP_THREADS) xs[i] = rsp_input(A, R, tail, row, s0 + i, lut);
     if (blockIdx.x == 0)
-        for (int i = tid; i < (int)(A.c - A.t0_old); i += RSP_THREADS) tail_s[i] = tail[i];
+        for (int i = tid; i < (int)(R.c - R.t0_old); i += RSP_THREADS) tail_s[i] = tail[i];
     __syncthreads();
 
     void* ring = A.out ? nullptr : reinterpret_cast<char*>(B.ring) + (size_t)s * B.P * (B.fmt == 1 ? 2 : 4);
-    float* out = A.out ? A.out + (size_t)blockIdx.y * A.out_stride - A.o0 : nullptr;
+    float* out = A.out ? A.out + (size_t)blockIdx.y * A.out_stride - R.o0 : nullptr;
     const int p_n0 = A.out ? 0 : (int)(n0 % B.P);               // ring position of n0: one 64-bit modulo per CTA
     auto store = [&](long long n, float y) {
         if (out) { out[n] = y; return; }
@@ -167,7 +193,7 @@ __global__ void __launch_bounds__(RSP_THREADS, 2) resample_push_kernel(BankView 
         while (i >= B.P) i -= B.P;
         rsp_store(ring, B.fmt, i, y);
     };
-    const long long lo = A.o0 > n0 ? A.o0 : n0, hi = A.o1 < n0 + A.tile ? A.o1 : n0 + A.tile;
+    const long long lo = R.o0 > n0 ? R.o0 : n0, hi = R.o1 < n0 + A.tile ? R.o1 : n0 + A.tile;
     if (fast) {
         constexpr int MM = M > 0 ? M : 1, RSP_K = rsp_k(MM);
         const int tp = RSP_THREADS / A.L;                       // threads per phase (a multiple of 32)
@@ -199,10 +225,10 @@ __global__ void __launch_bounds__(RSP_THREADS, 2) resample_push_kernel(BankView 
 
     if (blockIdx.x == 0 && !A.out) {
         // the tail for the next call: inputs [t0_new, c + n_in), from the old tail's copy or the new chunk
-        const int keep = (int)(A.c + A.n_in - A.t0_new);
+        const int keep = (int)(R.c + A.n_in - R.t0_new);
         for (int i = tid; i < keep; i += RSP_THREADS) {
-            const long long k = A.t0_new + i;
-            tail[i] = k < A.c ? tail_s[k - A.t0_old] : rsp_chunk(A, row, k - A.c, lut);
+            const long long k = R.t0_new + i;
+            tail[i] = k < R.c ? tail_s[k - R.t0_old] : rsp_chunk(A, row, k - R.c, lut);
         }
         if (tid == 0) {                                         // commit: what ring_commit_kernel does for an unsummed push
             StreamState& st = B.st[s];
@@ -210,8 +236,8 @@ __global__ void __launch_bounds__(RSP_THREADS, 2) resample_push_kernel(BankView 
                 const int fs = B.prm[s].frame_size;
                 st.frame_size = fs > 0 ? fs : A.frame_latch;
             }
-            st.written = A.o1;
-            st.ss_from = A.o1;
+            st.written = R.o1;
+            st.ss_from = R.o1;
         }
     }
 }

@@ -1421,4 +1421,37 @@ __global__ void peer_wait_kernel(const unsigned long long* __restrict__ sig_row,
     }
 }
 
+// ------------------------------------------------------------------------------------ K9 (stream recycling)
+// ewk_reset_streams: every listed stream back to the state init_streams gives it.  CTA (x, y) clears byte slice x of the
+// ring row of list[y] with 16-byte stores (rows are P * esz bytes, P a multiple of 64: 16-byte aligned); the CTAs of
+// slice 0 also write the StreamState, the block_ss and chunk_ms rows, the result record and K4's carried-row range.
+// The K8 input tail needs no clearing: a stream at input position 0 reads none of it and rewrites it on its next push.
+// HBM-bound: P * esz bytes per stream plus a few KB.
+constexpr int RESET_THREADS = 256;
+constexpr int RESET_SLICE = RESET_THREADS * 16 * 8;       // bytes of a ring row per CTA (8 stores per thread)
+
+__global__ void __launch_bounds__(RESET_THREADS)
+stream_reset_kernel(BankView B, const int* __restrict__ list, int n, long long* keep_end) {
+    const size_t row_bytes = (size_t)B.P * (B.fmt == 1 ? 2 : 4);
+    for (int y = blockIdx.y; y < n; y += gridDim.y) {
+        const int s = list[y];
+        int4* row = reinterpret_cast<int4*>(reinterpret_cast<char*>(B.ring) + (size_t)s * row_bytes);
+        const size_t w0 = (size_t)blockIdx.x * (RESET_SLICE / 16), w1 = min(w0 + RESET_SLICE / 16, row_bytes / 16);
+        for (size_t w = w0 + threadIdx.x; w < w1; w += RESET_THREADS) row[w] = make_int4(0, 0, 0, 0);   // np.zeros  wakeword.py:428
+        if (blockIdx.x != 0) continue;
+        if (threadIdx.x == 0) {
+            StreamState z;
+            memset(&z, 0, sizeof(z));
+            z.thr = 0.01; z.last_ev = -1;                                       // wakeword.py:431
+            B.st[s] = z;
+            store_result(B.results + s, StreamResult{__int_as_float(0x7fc00000), 0u});   // nanf(""), as init_streams
+            if (keep_end) { keep_end[2 * s] = 0; keep_end[2 * s + 1] = 0; }
+        }
+        double* ss = B.block_ss + (size_t)s * B.NB;
+        for (int i = threadIdx.x; i < B.NB; i += RESET_THREADS) ss[i] = 0.0;
+        double* ms = B.chunk_ms + (size_t)s * 2 * B.chunk_cap;                 // ms[cap] ++ sorted[cap]
+        for (int i = threadIdx.x; i < 2 * B.chunk_cap; i += RESET_THREADS) ms[i] = 0.0;
+    }
+}
+
 }  // namespace ewk

@@ -27,6 +27,19 @@ def owner_of(stream: int, n_total: int, world: int) -> tuple[int, int]:
     return rem + (stream - cut) // base, (stream - cut) % base
 
 
+def local_streams(global_streams, n_total: int, world: int, rank: int) -> list[int]:
+    """Local indices, in the given order, of the global stream ids that `rank` owns (the rest belong to other ranks)."""
+    out = []
+    for g in global_streams:
+        g = int(g)
+        if not 0 <= g < n_total:
+            raise ValueError(f"stream {g} outside [0, {n_total})")
+        r, i = owner_of(g, n_total, world)
+        if r == rank:
+            out.append(i)
+    return out
+
+
 def padded_shard(n_total: int, world: int) -> int:
     """Per-rank record count used for the fixed-size all-gather (ceil(n_total / world))."""
     return -(-n_total // world)
@@ -86,7 +99,7 @@ class ShardedBank:
         if exchange not in ("auto", "peer", "nccl"):
             raise ValueError("exchange must be 'auto', 'peer' or 'nccl'")
         self.first, self.last = shard_range(n_total, world, rank)
-        self.world = world
+        self.n_total, self.world, self.rank = n_total, world, rank
         self.bank = WakeWordBank(self.last - self.first, templates, device=device, **bank_kwargs)
         dev = torch.device("cuda", device)
         self.gatherer = ResultGather(n_total, world, rank, device=dev)
@@ -121,6 +134,13 @@ class ShardedBank:
             return self.peer.records(ctx.publish_parity())
         ctx.join()                        # overlap mode: the records are complete once K3 has been joined
         return self.gatherer.gather()
+
+    def reset(self, global_streams, **overrides):
+        """Recycle global streams: every rank is called with the same list and resets the streams it owns
+        (WakeWordBank.reset).  Returns this rank's drained events with global stream ids."""
+        ev = self.bank.reset(local_streams(global_streams, self.n_total, self.world, self.rank), **overrides)
+        ev["stream"] += self.first
+        return ev
 
     def poll_global(self):
         """Local events with global stream ids."""

@@ -49,6 +49,15 @@ def ready_outputs(n_in: int, half_width: int, up: int, down: int) -> int:
     return (a * up + down - 1) // down if a > 0 else 0
 
 
+def landed_counts(positions, n_in: int, sr_in: int) -> np.ndarray:
+    """16 kHz samples a push of n_in inputs at sr_in lands on streams that had received `positions` inputs
+    (ewk_push_resampled_each): ready(c + n_in) - ready(c) per stream."""
+    from . import _lib
+    W, L, M = _lib.resample_info(sr_in)
+    return np.array([ready_outputs(int(c) + n_in, W, L, M) - ready_outputs(int(c), W, L, M) for c in positions],
+                    dtype=np.int64)
+
+
 class StreamResampler:
     """Chunked conversion of [rows, n] feeds to 16 kHz whose concatenated output equals the one-shot result
     sample for sample: every call is given the filter's half-width of history and emits only the outputs whose

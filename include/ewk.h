@@ -247,8 +247,27 @@ int ewk_resample(ewk_ctx* ctx, const void* in, int pcm_format, int where_in, int
 enum { EWK_IN_ULAW = 2, EWK_IN_ALAW = 3 };
 int ewk_push_resampled(ewk_ctx* ctx, int stream0, int n_streams, const void* in, int in_format, int64_t n_in, int64_t stride,
                        int where, int sr_in);
+/* ewk_push_resampled for streams at their own input positions (recycled streams restart at 0): the same in every respect
+ * except that the streams of one call may have received different numbers of input samples, still in one launch.
+ * landed (host, required: EWK_ERR_ARG when NULL) receives, for stream stream0 + i, the number of 16 kHz samples landed,
+ * ready(c_i + n_in) - ready(c_i) for its position c_i.  Rings and input tails are bit-identical to one ewk_push_resampled
+ * per group of equal positions.  Returns EWK_OK or a status. */
+int ewk_push_resampled_each(ewk_ctx* ctx, int stream0, int n_streams, const void* in, int in_format, int64_t n_in,
+                            int64_t stride, int where, int sr_in, int64_t* landed);
 /* rate latched by the stream's first push (0: none yet; 16000: ewk_push / ewk_push_g711) and input samples received */
 int ewk_stream_input(ewk_ctx* ctx, int stream, int32_t* sr_in, int64_t* n_in);
+/* Stream recycling (a call ends, the slot takes the next one) without rebuilding the bank: return streams[0..n) to the
+ * state ewk_create gives a stream.  Afterwards stream s behaves exactly like stream s of a new context with the same
+ * ewk_config, templates and stream parameters given the same calls: events, result records, tick traces,
+ * ewk_stream_status, ewk_stream_input, ewk_read_last (zeros before the ring fills), ewk_read_segment, dense scores.  Its
+ * ticks and sample indices count from the reset.  Streams not listed are untouched.  Stream parameters are kept (change
+ * them with ewk_set_stream_params); the input-rate latch is cleared, so the next session may come at any rate.  A pending
+ * host push lands first (its samples belong to the old session and are cleared with it); in overlap mode the call joins
+ * K3 first.  One launch (K9) for the whole list; duplicates are harmless, n = 0 is a no-op.
+ * EWK_ERR_STATE while the event queue is not empty ("poll first": events carry no session, so an old session's event
+ * polled afterwards would point ewk_read_segment at the new session's audio) and for a context with n_streams = 0;
+ * EWK_ERR_ARG for a stream out of range or streams = NULL with n > 0.  Synchronises with the context's stream. */
+int ewk_reset_streams(ewk_ctx* ctx, const int32_t* streams, int n);
 /* Dense per-hop scoring (SURVEY §8(a) A9; usage shape of examples/tune_threshold.py:86-116 at hop
  * granularity): for every stream, every hop h in [hop0, hop0 + n_hops) (hop h <-> 160*h samples pushed)
  * and every template slot k in [template_first, template_first + template_count), the value
