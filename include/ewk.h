@@ -223,7 +223,13 @@ int ewk_analyze_templates(ewk_ctx* ctx, const float* pcm, int where, const int64
  * in_first = out_first = 0; streaming use passes each chunk with half_width samples of history and emits only
  * outputs whose half_width samples of look-ahead are present, which reproduces the one-shot result exactly.
  * in: float32 or int16 (pcm_format), rows in_stride samples apart; out: float32, rows out_stride apart.
- * Supported rates: those with 16000 / gcd(sr_in, 16000) <= 4096 (every standard rate). */
+ * Supported rates: 1000 to 768000 Hz with 16000 / gcd(sr_in, 16000) <= 4096 (every standard rate).
+ * Arithmetic: output n is the sequential fmaf chain, from +0, over taps j = 0 .. 2W-1 of H[j][p] * x[k_c - W + 1 + j]
+ * with the float32 table H (k_c = floor(n M / L), p = n M mod L), the same on every code path.  Its rounding error
+ * against the float64 sum of the same products grows with the filter length; measured on one B200 (1000 W) on full-scale
+ * square waves, worst output: at most 1.2e-6 (-118 dBFS) up to 24 kHz, 1.8e-6 up to 64 kHz, 2.2e-6 at 96 kHz,
+ * 1.5e-6 at 192 kHz, 5.5e-6 at 384 kHz and 8.1e-6 (-102 dBFS) at 768 kHz (DESIGN.md, K8).  The 125 dB above is the
+ * filter's stop-band design, not the arithmetic's noise floor. */
 int ewk_resample_info(int sr_in, int32_t* half_width, int32_t* up, int32_t* down);
 int64_t ewk_resample_out_len(int64_t n_in, int sr_in);
 int ewk_resample(ewk_ctx* ctx, const void* in, int pcm_format, int where_in, int n_rows, int64_t n_in, int64_t in_stride,

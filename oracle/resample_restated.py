@@ -88,3 +88,84 @@ def resample(y, sr_in: int, sr_out: int = TARGET_SR, *, in_first: int = 0, out_f
         ok = (idx >= 0) & (idx < len(ypad))
         out += np.where(ok, ypad[np.clip(idx, 0, len(ypad) - 1)], 0.0) * H[j, p]
     return out.astype(np.float32)
+
+
+# ------------------------------------------------------------------------------------------------ float32 chain
+# The device (K8, easywakeword_b200/csrc/ewk_resample_push.cuh) evaluates each output as one sequential fmaf chain
+# from +0 over taps j = 0 .. 2W-1 of the float32 table.  The functions below restate that arithmetic exactly, so a
+# test can compare the device with it bit for bit instead of within a tolerance.
+
+def fmaf32(a, b, c):
+    """C's fmaf on float32 arrays: a * b + c rounded once to float32 (round to nearest, ties to even).
+
+    The product of two float32 values is exact in float64; TwoSum gives the sum exactly as s + e.  Rounding s to
+    float32 is then correct unless s lies exactly on a float32 midpoint while e != 0, where the exact sum lies off
+    the midpoint on e's side (plain float32(float64(a * b) + c) rounds twice and gets such cases wrong)."""
+    a = np.asarray(a, np.float32)
+    b = np.asarray(b, np.float32)
+    c = np.asarray(c, np.float32)
+    p = a.astype(np.float64) * b.astype(np.float64)
+    cd = c.astype(np.float64)
+    s = p + cd
+    bb = s - p
+    e = (p - (s - bb)) + (cd - bb)
+    r = s.astype(np.float32)
+    rd = r.astype(np.float64)
+    away = np.nextafter(r, np.where(s > rd, np.float32(np.inf), np.float32(-np.inf)))
+    ad = away.astype(np.float64)
+    flip = (s != rd) & (s - rd == ad - s) & (e != 0) & (np.sign(e) == np.sign(ad - rd))
+    return np.where(flip, away, r)
+
+
+def chain_input(y, law=None):
+    """The float32 values the device's FIR reads: float32 as is, int16 / 32768, G.711 codes (uint8, law "ulaw" or
+    "alaw") through the ITU-T expansion table / 32768."""
+    y = np.asarray(y)
+    if law is not None:
+        if y.dtype != np.uint8:
+            raise TypeError("G.711 input is uint8 codes")
+        from easywakeword_b200.resample import ALAW_TABLE, ULAW_TABLE
+        table = {"ulaw": ULAW_TABLE, "alaw": ALAW_TABLE}[law]
+        return table[y].astype(np.float32) / np.float32(32768.0)
+    if y.dtype == np.int16:
+        return y.astype(np.float32) / np.float32(32768.0)
+    if y.dtype != np.float32:
+        raise TypeError(f"the device reads float32, int16 or G.711 input, not {y.dtype}")
+    return y
+
+
+def resample_chain(y, sr_in: int, *, in_first: int = 0, out_first: int = 0, n_out=None, law=None):
+    """float32 outputs [out_first, out_first + n_out) of the device's chain, with resample()'s framing: y ([n] or
+    [rows, n]) holds absolute input samples [in_first, in_first + n), zeros elsewhere.  Output n of a row is
+    acc = fmaf(H[j][p], x[k_c - W + 1 + j], acc) for j = 0 .. 2W-1 from acc = +0, k_c = floor(n M / L),
+    p = n M mod L, H = phase_table(d) rounded to float32."""
+    x = chain_input(y, law)
+    one_d = x.ndim == 1
+    x = x.reshape(1, -1) if one_d else x
+    d = design(sr_in)
+    W, L, M = d["W"], d["L"], d["M"]
+    if n_out is None:
+        n_out = out_len(x.shape[1], sr_in) - out_first
+    n_out = max(int(n_out), 0)
+    H = phase_table(d).astype(np.float32)
+    n = out_first + np.arange(n_out, dtype=np.int64)
+    kc, p = (n * M) // L, (n * M) % L
+    acc = np.zeros((x.shape[0], n_out), np.float32)
+    if n_out:
+        # absolute inputs [lo, hi) cover every tap of every output: zero-padded copy, one gather per tap
+        lo, hi = int(kc[0]) - W + 1, int(kc[-1]) + W + 1
+        xp = np.zeros((x.shape[0], hi - lo), np.float32)
+        a, b = max(lo, in_first), min(hi, in_first + x.shape[1])
+        if a < b:
+            xp[:, a - lo:b - lo] = x[:, a - in_first:b - in_first]
+        base = kc - W + 1 - lo
+        for j in range(2 * W):
+            acc = fmaf32(xp[:, base + j], H[j, p], acc)
+    return acc[0] if one_d else acc
+
+
+def ring_quantize(y):
+    """What an int16 ring stores for output y: clip(rint(y * 32768), -32768, 32767), ties to even.  Reading the ring
+    back gives the stored value / 32768."""
+    q = np.rint(np.asarray(y, np.float32).astype(np.float64) * 32768.0)
+    return np.clip(q, -32768, 32767).astype(np.int16)
