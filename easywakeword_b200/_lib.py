@@ -296,6 +296,8 @@ def _declare_stream_protos(lib):
         "ewk_push_g711": (C.c_int, [vp, i32, i32, vp, i64, i64, i32, i32]),
         "ewk_push_resampled": (C.c_int, [vp, i32, i32, vp, i32, i64, i64, i32, i32]),
         "ewk_push_resampled_each": (C.c_int, [vp, i32, i32, vp, i32, i64, i64, i32, i32, _p(i64)]),
+        "ewk_push_streams": (C.c_int, [vp, _p(C.c_int32), i32, vp, i32, _p(i64), _p(i64), i64, i32, i32, _p(i64)]),
+        "ewk_tick_ready": (C.c_int, [vp, i32, _p(C.c_int32), vp, vp, vp, vp]),
         "ewk_stream_input": (C.c_int, [vp, i32, _p(C.c_int32), _p(i64)]),
         "ewk_reset_streams": (C.c_int, [vp, _p(C.c_int32), i32]),
         "ewk_tick": (C.c_int, [vp, i32]),
@@ -469,6 +471,64 @@ def _bank_methods():
                                                   landed.ctypes.data_as(_p(C.c_int64))))
         return landed
 
+    def push_streams(self, streams, rows, sr_in=16000, fmt=None, where=HOST):
+        """Ragged push (include/ewk.h: ewk_push_streams): rows[i], a 1-D array of any length (0 included), goes to stream
+        streams[i]; the rows are packed into one buffer that crosses PCIe in one copy.  The format follows the dtype as in
+        push_resampled (uint8: G.711 with fmt "ulaw" / "alaw"); at sr_in = 16000 it must be the rings' dtype or G.711 into
+        int16 rings.  A device input is (ptr, offsets, lens, in_len, dtype).  Returns int64 [len(streams)]: the 16 kHz
+        samples landed per row."""
+        st = np.asarray(streams, dtype=np.int64).reshape(-1)
+        if st.size and (st.min() < -2**31 or st.max() >= 2**31):
+            raise ValueError("stream index out of range")
+        st = np.ascontiguousarray(st, dtype=np.int32)
+        if isinstance(rows, tuple):
+            ptr, off, ln, in_len, dt = rows
+            off = np.ascontiguousarray(off, dtype=np.int64)
+            ln = np.ascontiguousarray(ln, dtype=np.int64)
+            dt = np.dtype(dt)
+            buf = None
+        else:
+            rows = [np.asarray(r) for r in rows]
+            if len(rows) != len(st):
+                raise ValueError("one row per stream")
+            dts = {r.dtype for r in rows}
+            if len(dts) > 1:
+                raise TypeError(f"rows of one call share a dtype, got {sorted(map(str, dts))}")
+            dt = dts.pop() if dts else np.dtype(np.uint8 if fmt is not None else
+                                                np.int16 if self.cfg.pcm_format == PCM_I16 else np.float32)
+            ln = np.array([r.size for r in rows], np.int64)
+            off = np.zeros(len(rows), np.int64)
+            if len(rows) > 1:
+                off[1:] = np.cumsum(ln)[:-1]
+            buf = np.concatenate([r.reshape(-1) for r in rows]) if rows else np.zeros(0, dt)
+            ptr, in_len = (buf.ctypes.data if buf.size else None), int(buf.size)
+        if len(off) != len(st) or len(ln) != len(st):
+            raise ValueError("one offset and one length per stream")
+        _, _, _, _, code, _keep = _resampled_input((0, 1, 0, 0, dt), fmt)
+        landed = np.zeros(len(st), np.int64)
+        self._ck(self.lib.ewk_push_streams(self.h, st.ctypes.data_as(_p(C.c_int32)), len(st), ptr, code, i64ptr(off),
+                                           i64ptr(ln), int(in_len), where, int(sr_in), i64ptr(landed)))
+        return landed
+
+    def tick_ready(self, max_ticks, trace=False):
+        """Ticks paced by each stream's own landed audio (include/ewk.h: ewk_tick_ready): stream s takes
+        min(max_ticks, written_s // 1600 - tick_s) ticks (resample.due_ticks).  Returns taken (int32 [n_streams]), and
+        with trace=True also the trace dict of tick(trace=True) over [n_streams, max_ticks] (cells of ticks not taken:
+        state 255, thr / rms NaN; "silent" is then the raw uint8 with 255)."""
+        ns = self.cfg.n_streams
+        taken = np.zeros(ns, np.int32)
+        tp = taken.ctypes.data_as(_p(C.c_int32))
+        if not trace:
+            self._ck(self.lib.ewk_tick_ready(self.h, int(max_ticks), tp, None, None, None, None))
+            return taken
+        silent = np.empty((ns, max_ticks), np.uint8)
+        state = np.empty((ns, max_ticks), np.uint8)
+        thr = np.empty((ns, max_ticks), np.float64)
+        rms = np.empty((ns, max_ticks), np.float64)
+        self._ck(self.lib.ewk_tick_ready(self.h, int(max_ticks), tp, silent.ctypes.data, state.ctypes.data,
+                                         thr.ctypes.data, rms.ctypes.data))
+        return taken, {"silent": silent, "state": state, "thr": thr, "rms": rms}
+
     def reset_streams(self, streams):
         """Return the listed streams to the state of a new context (include/ewk.h: ewk_reset_streams); their parameters
         stay.  The event queue must be empty (poll first)."""
@@ -616,7 +676,7 @@ def _bank_methods():
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
     for f in (prepare_segments, dense_scores, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
-              push_resampled_each, reset_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
+              push_resampled_each, push_streams, tick_ready, reset_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
               set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count):
         setattr(Context, f.__name__, f)
 

@@ -34,6 +34,12 @@ class WakeWordBank:
     samples_pushed (the clock step() ticks by) then advances by the largest count landed, and status(s).written holds a
     stream's own count.
 
+    Feeds with jitter or a sparse set of active calls use push_streams / step_streams: any list of streams, each with its
+    own amount of audio, in one push, and ticks paced by each stream's own landed audio (include/ewk.h: ewk_push_streams,
+    ewk_tick_ready).  The same audio then gives the same events however it was split into pushes, and a slot that is not
+    fed takes no ticks and costs no PCIe bytes.  samples_pushed and ticks describe push / step only; read a stream's own
+    clock with status(s) (written, tick).
+
     templates: list of float32 arrays or WAV paths (slot i = templates[i]); every stream is scored
     against all of them (best score wins) unless set_stream(..., template_first=, template_count=).
     Timing defaults are the reference's (wakeword.py:38-41); speech_duration_min/max default to the
@@ -150,6 +156,23 @@ class WakeWordBank:
         due = self.samples_pushed // TICK_SAMPLES - self.ticks
         if due > 0:
             self.tick(due)
+
+    def push_streams(self, streams, blocks, where=_lib.HOST):
+        """blocks[i]: 1-D audio at the bank's sample_rate for stream streams[i], any length (0 included), in the bank's
+        dtype at 16 kHz (float32 or int16 at other rates).  One push for the whole list.  Returns the 16 kHz samples landed
+        per stream."""
+        return self.ctx.push_streams(streams, blocks, sr_in=self.sample_rate, where=where)
+
+    def step_streams(self, streams, blocks, where=_lib.HOST):
+        """push_streams, then every tick the landed audio pays for, stream by stream (ewk_tick_ready): no stream has a
+        due tick left when it returns.  Returns the ticks each stream took (int64 [n_streams])."""
+        self.push_streams(streams, blocks, where)
+        taken = np.zeros(self.n_streams, np.int64)
+        while True:
+            t = self.ctx.tick_ready(4096)
+            taken += t
+            if t.max() < 4096:
+                return taken
 
     def poll(self) -> np.ndarray:
         """Structured array of events since the last poll, sorted by (tick, stream):

@@ -3,6 +3,7 @@
 
 #include <algorithm>
 #include <cmath>
+#include <climits>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -632,7 +633,8 @@ int ewk_ctx::init_streams() {
     {
         const size_t big = sizeof(double) * 3 * (size_t)(std::min(chunk_cap, GATE_SMEM_CHUNKS) + 1) * GATE_WARPS;
         const size_t staged = sizeof(double) * 3 * (size_t)130 * GATE_WARPS + (size_t)2 * TICK * 4 * GATE_WARPS;
-        CK(cudaFuncSetAttribute(tick_gate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(big, staged)));
+        CK(cudaFuncSetAttribute(tick_gate_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(big, staged)));
+        CK(cudaFuncSetAttribute(tick_gate_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(big, staged)));
     }
     return EWK_OK;
 }
@@ -803,11 +805,13 @@ int ewk_ctx::flush_pending() {
     if (!pending.valid) return EWK_OK;
     pending.valid = false;
     if (pending.rs_rate) {
-        const bool each = pending.rs_pos_slot >= 0;
+        const bool each = pending.rows_slot >= 0;
         return land_resampled(pending.stream0, pending.n_streams, b_raw[pending.slot].p, pending.rs_n_in, pending.rs_fmt,
-                              pending.rs_n_in, pending.rs_rate, each ? pending.rs_pos.data() : &pending.rs_c,
-                              each ? (const long long*)b_pos[pending.rs_pos_slot].p : nullptr, pending.slot);
+                              pending.rs_n_in, pending.rs_rate, pending.rs_c, each ? pending.rows.data() : nullptr,
+                              pending.rows_slot, pending.n_items, pending.slot);
     }
+    if (pending.rows_slot >= 0)
+        return land_list(pending.rows, pending.rows_slot, pending.n_items, b_raw[pending.slot].p, pending.rs_fmt, pending.slot);
     return land(pending.stream0, pending.n_streams, b_stage2[pending.slot].p, pending.n, pending.n, pending.slot);
 }
 
@@ -958,47 +962,55 @@ static long long rs_tail_start(long long c, const ResampleDesign& d) {
 }
 static size_t rs_in_size(int in_fmt) { return in_fmt == EWK_PCM_F32 ? 4 : in_fmt == EWK_PCM_I16 ? 2 : 1; }
 
-// The FIR (K8) over rows [0, n_rows) of A: plans the work mapping (fast or generic path, tile, staged span) and launches.
-int ewk_ctx::launch_fir(const ResampleTable& t, RsPushArgs& A, int n_rows, int prof_cls, const char* who,
-                        const long long* pos) {
-    ewk_ctx* ctx = this;
-    const ResampleDesign& d = t.d;
+// K8's work mapping for a rate: fast or generic path, outputs per tile, staged input span
+struct FirPlan { int fast_m, tile, span, table_smem; };
+static FirPlan fir_plan(const ResampleDesign& d) {
+    FirPlan f{};
     const int taps = 2 * d.W;
-    A.table_smem = (long long)taps * d.L <= RSP_TABLE_SMEM;
+    f.table_smem = (long long)taps * d.L <= RSP_TABLE_SMEM;
     // fast path: warp-uniform phases and register windows; its tile must leave the tail (if any) to CTA 0 alone
-    int fast_m = 0;
-    if ((d.L == 1 || d.L == 2 || d.L == 4 || d.L == 8) && d.M <= 3 && A.table_smem &&
+    if ((d.L == 1 || d.L == 2 || d.L == 4 || d.L == 8) && d.M <= 3 && f.table_smem &&
         (RSP_THREADS / d.L) * rsp_k(d.M) * d.M >= taps + d.M)
-        fast_m = d.M;
-    if (fast_m) {
-        A.tile = RSP_THREADS * rsp_k(d.M);
-        A.span = (RSP_THREADS / d.L) * rsp_k(d.M) * d.M + taps + d.M + 1;
+        f.fast_m = d.M;
+    if (f.fast_m) {
+        f.tile = RSP_THREADS * rsp_k(d.M);
+        f.span = (RSP_THREADS / d.L) * rsp_k(d.M) * d.M + taps + d.M + 1;
     } else {
         auto span = [&](long long tile) { return (tile * d.M + d.L - 1) / d.L + taps + 1; };
         long long tile = RSP_GENERIC_TILE;
         while (tile > RSP_THREADS && span(tile) > 24576) tile /= 2;
         const long long need = ((long long)taps * d.L + d.M - 1) / d.M;      // tile M / L >= 2W: CTAs >= 1 start past the tail
         tile = std::max(tile, (need + RSP_THREADS - 1) / RSP_THREADS * RSP_THREADS);
-        A.tile = (int)tile;
-        A.span = (int)span(tile);
+        f.tile = (int)tile;
+        f.span = (int)span(tile);
     }
+    return f;
+}
+// output tiles of a row: its outputs [o0, o1) from the first tile start (fast path: o0 rounded down to a phase group)
+static long long fir_tiles(const FirPlan& f, const ResampleDesign& d, long long o0, long long o1) {
+    const long long first = f.fast_m ? (o0 / d.L) * d.L : o0;
+    return std::max<long long>(1, (o1 - first + f.tile - 1) / f.tile);
+}
+
+// The FIR (K8) over rows [0, n_rows) of A: plans the work mapping and launches.
+int ewk_ctx::launch_fir(const ResampleTable& t, RsPushArgs& A, int n_rows, int prof_cls, const char* who,
+                        long long n_items) {
+    ewk_ctx* ctx = this;
+    const ResampleDesign& d = t.d;
+    const int taps = 2 * d.W;
+    const FirPlan f = fir_plan(d);
+    const int fast_m = f.fast_m;
+    A.table_smem = f.table_smem; A.tile = f.tile; A.span = f.span;
     const size_t smem = sizeof(float) * ((size_t)256 + A.tail_cap + (A.table_smem ? (size_t)taps * d.L : 0) + A.span);
     if (smem > (size_t)200 * 1024) { fail("%s: %d Hz needs %zu bytes of shared memory", who, d.sr_in, smem); return EWK_ERR_ARG; }
-    // output tiles of a row: its outputs [o0, o1) from the first tile start (fast path: o0 rounded down to a phase group)
-    auto tiles = [&](long long o0, long long o1) {
-        const long long first = fast_m ? (o0 / d.L) * d.L : o0;
-        return std::max<long long>(1, (o1 - first + A.tile - 1) / A.tile);
-    };
-    long long n_tiles = tiles(A.o0, A.o1);
-    if (pos)
-        for (int y = 0; y < n_rows; y++) n_tiles = std::max(n_tiles, tiles(rs_ready(pos[y], d), rs_ready(pos[y] + A.n_in, d)));
-    const dim3 grid((unsigned)n_tiles, (unsigned)n_rows);
+    // per-row descriptors: one flat list of every row's tiles, so that rows of very different lengths leave no CTA idle
+    const dim3 grid = A.rows ? dim3((unsigned)n_items, 1) : dim3((unsigned)fir_tiles(f, d, A.o0, A.o1), (unsigned)n_rows);
     auto pick = [&](auto each) {
         constexpr bool E = decltype(each)::value;
         return fast_m == 1 ? resample_push_kernel<1, E> : fast_m == 2 ? resample_push_kernel<2, E>
              : fast_m == 3 ? resample_push_kernel<3, E> : resample_push_kernel<0, E>;
     };
-    auto k8 = A.pos ? pick(std::true_type{}) : pick(std::false_type{});
+    auto k8 = A.rows ? pick(std::true_type{}) : pick(std::false_type{});
     CK(cudaFuncSetAttribute(k8, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaEvent_t pe = prof_begin(prof_cls);
     k8<<<grid, RSP_THREADS, smem, stream>>>(bank, A);
@@ -1008,16 +1020,15 @@ int ewk_ctx::launch_fir(const ResampleTable& t, RsPushArgs& A, int n_rows, int p
     return EWK_OK;
 }
 
-// K8 on device-resident input (the caller's buffer or a staging slot): stream stream0 + i has received pos[i] inputs
-// (d_pos: the device copy of pos[0 .. n_streams) when they differ; null: every stream sits at pos[0])
+// K8 on device-resident input (the caller's buffer or a staging slot): uniform rows from position c, or per-row
+// descriptors (see ewk_ctx.hpp)
 int ewk_ctx::land_resampled(int stream0, int n_streams, const void* d_src, long long d_stride, int in_fmt, long long n_in,
-                            int sr_in, const long long* pos, const long long* d_pos, int stage_slot) {
+                            int sr_in, long long c, const RowDesc* rows, int rows_slot, long long n_items, int stage_slot) {
     ewk_ctx* ctx = this;
     const ResampleTable* t = nullptr;
     int rc = resample_table(sr_in, &t);
     if (rc) return rc;
     const ResampleDesign& d = t->d;
-    const long long c = pos[0];
     RsPushArgs A{};
     A.in = d_src; A.in_stride = d_stride; A.n_in = n_in; A.in_fmt = in_fmt;
     A.tail = d_rs_tail; A.tail_cap = rs_tail_cap; A.H = t->H;
@@ -1025,25 +1036,86 @@ int ewk_ctx::land_resampled(int stream0, int n_streams, const void* d_src, long 
     A.c = c; A.o0 = rs_ready(c, d); A.o1 = rs_ready(c + n_in, d);
     A.t0_old = rs_tail_start(c, d); A.t0_new = rs_tail_start(c + n_in, d);
     A.frame_latch = (int)ewk_resample_out_len(n_in, sr_in);
-    A.pos = d_pos;
+    if (rows_slot >= 0) { A.rows = (const RowDesc*)b_pos[rows_slot].p; A.n_rows = n_streams; }
     if (stage_slot >= 0) CK(cudaStreamWaitEvent(stream, ev_ready[stage_slot], 0));
-    rc = launch_fir(*t, A, n_streams, 7, "ewk_push_resampled", d_pos ? pos : nullptr);
+    rc = launch_fir(*t, A, n_streams, 7, "ewk_push_resampled", n_items);
     if (rc) return rc;
     if (stage_slot >= 0) {
         CK(cudaEventRecord(ev_free[stage_slot], stream));
         ev_free_valid[stage_slot] = true;
     }
-    if (d_pos) {                            // the positions' slot is free once this K8 has read them
-        const int k = (int)(d_pos == (const long long*)b_pos[1].p);
-        CK(cudaEventRecord(ev_pos[k], stream));
-        ev_pos_valid[k] = true;
+    if (rows_slot >= 0) {                   // the descriptors' slot is free once this K8 has read them
+        CK(cudaEventRecord(ev_pos[rows_slot], stream));
+        ev_pos_valid[rows_slot] = true;
     }
     all_presummed = false;                  // K8 forms no block sums: K2 reads these samples
     pushes_since_tick++;
     for (int i = 0; i < n_streams; i++) {
-        const int s = stream0 + i;
-        h_written[s] = rs_ready((d_pos ? pos[i] : c) + n_in, d);
-        if (h_frame_size[s] == 0) h_frame_size[s] = h_prm[s].frame_size > 0 ? h_prm[s].frame_size : A.frame_latch;
+        const int s = rows ? rows[i].stream : stream0 + i;
+        h_written[s] = rows ? rs_ready(rows[i].pos + rows[i].len, d) : rs_ready(c + n_in, d);
+        const int latch = rows ? rows[i].latch : A.frame_latch;
+        if (h_frame_size[s] == 0) h_frame_size[s] = h_prm[s].frame_size > 0 ? h_prm[s].frame_size : latch;
+    }
+    return EWK_OK;
+}
+
+int ewk_ctx::upload_rows(const std::vector<RowDesc>& rows, cudaStream_t on, int* slot) {
+    ewk_ctx* ctx = this;
+    const int k = pos_idx;
+    pos_idx ^= 1;
+    const size_t bytes = sizeof(RowDesc) * (size_t)bank.n_streams;
+    if (!h_pos[k]) {
+        CK(cudaHostAlloc((void**)&h_pos[k], bytes, cudaHostAllocDefault));
+        CK(cudaEventCreateWithFlags(&ev_pos[k], cudaEventDisableTiming));
+    }
+    CK(b_pos[k].ensure(bytes));
+    if (ev_pos_valid[k]) CK(cudaEventSynchronize(ev_pos[k]));
+    std::memcpy(h_pos[k], rows.data(), sizeof(RowDesc) * rows.size());
+    CK(cudaMemcpyAsync(b_pos[k].p, h_pos[k], sizeof(RowDesc) * rows.size(), cudaMemcpyHostToDevice, on));
+    *slot = k;
+    return EWK_OK;
+}
+
+// tails for the widest filter in use; rows of streams already running move with their content
+int ewk_ctx::ensure_rs_tail(int cap) {
+    ewk_ctx* ctx = this;
+    if (rs_tail_cap >= cap) return EWK_OK;
+    float* nt = nullptr;
+    CK(cudaMalloc(&nt, sizeof(float) * (size_t)bank.n_streams * cap));
+    if (d_rs_tail) {
+        CK(cudaMemcpy2DAsync(nt, sizeof(float) * cap, d_rs_tail, sizeof(float) * rs_tail_cap, sizeof(float) * rs_tail_cap,
+                             bank.n_streams, cudaMemcpyDeviceToDevice, stream));
+        CK(cudaStreamSynchronize(stream));
+        CK(cudaFree(d_rs_tail));
+    }
+    d_rs_tail = nt;
+    rs_tail_cap = cap;
+    return EWK_OK;
+}
+
+// K1L on device-resident input (the caller's buffer or a staging slot)
+int ewk_ctx::land_list(const std::vector<RowDesc>& rows, int rows_slot, long long n_items, const void* d_src, int in_fmt,
+                       int stage_slot) {
+    ewk_ctx* ctx = this;
+    if (stage_slot >= 0) CK(cudaStreamWaitEvent(stream, ev_ready[stage_slot], 0));
+    const RowDesc* d_rows = (const RowDesc*)b_pos[rows_slot].p;
+    cudaEvent_t pe = prof_begin(0);
+    if (bank.fmt == 1) ring_push_list_kernel<short><<<(unsigned)n_items, 256, 0, stream>>>(bank, d_src, in_fmt, d_rows, (int)rows.size());
+    else ring_push_list_kernel<float><<<(unsigned)n_items, 256, 0, stream>>>(bank, d_src, in_fmt, d_rows, (int)rows.size());
+    prof_end(pe, 0);
+    CK(cudaGetLastError());
+    launches++;
+    if (stage_slot >= 0) {
+        CK(cudaEventRecord(ev_free[stage_slot], stream));
+        ev_free_valid[stage_slot] = true;
+    }
+    CK(cudaEventRecord(ev_pos[rows_slot], stream));
+    ev_pos_valid[rows_slot] = true;
+    all_presummed = false;                  // K1L forms no block sums: K2 reads these samples
+    pushes_since_tick++;
+    for (const RowDesc& r : rows) {
+        h_written[r.stream] = r.pos + r.len;
+        if (h_frame_size[r.stream] == 0) h_frame_size[r.stream] = h_prm[r.stream].frame_size > 0 ? h_prm[r.stream].frame_size : r.latch;
     }
     return EWK_OK;
 }
@@ -1107,48 +1179,35 @@ static int push_resampled_impl(ewk_ctx* ctx, const char* who, int stream0, int n
     const ewk_ctx::ResampleTable* t = nullptr;
     rc = ctx->resample_table(sr_in, &t);
     if (rc) return rc;
-    if (ctx->rs_tail_cap < 2 * d.W) {
-        // tails for the widest filter in use; rows of streams already running move with their content
-        const int cap = 2 * d.W;
-        float* nt = nullptr;
-        CK(cudaMalloc(&nt, sizeof(float) * (size_t)B.n_streams * cap));
-        if (ctx->d_rs_tail) {
-            CK(cudaMemcpy2DAsync(nt, sizeof(float) * cap, ctx->d_rs_tail, sizeof(float) * ctx->rs_tail_cap,
-                                 sizeof(float) * ctx->rs_tail_cap, B.n_streams, cudaMemcpyDeviceToDevice, ctx->stream));
-            CK(cudaStreamSynchronize(ctx->stream));
-            CK(cudaFree(ctx->d_rs_tail));
-        }
-        ctx->d_rs_tail = nt;
-        ctx->rs_tail_cap = cap;
-    }
-    std::vector<long long> pos(ctx->h_inputs.begin() + stream0, ctx->h_inputs.begin() + stream0 + n_streams);
+    rc = ctx->ensure_rs_tail(2 * d.W);
+    if (rc) return rc;
+    // streams at different positions: per-row descriptors (identity streams, equal lengths) in a slot of their own,
+    // which a later push reuses only after the K8 that reads them has run
+    std::vector<RowDesc> rows;
+    long long n_items = 0;
+    const FirPlan f = fir_plan(d);
+    const int latch = (int)ewk_resample_out_len(n_in, sr_in);
     for (int i = 0; i < n_streams; i++) {
-        if (landed) landed[i] = rs_ready(pos[i] + n_in, d) - rs_ready(pos[i], d);
-        ctx->h_rate[stream0 + i] = sr_in;
-        ctx->h_inputs[stream0 + i] = pos[i] + n_in;
+        const int s = stream0 + i;
+        const long long p = ctx->h_inputs[s];
+        if (landed) landed[i] = rs_ready(p + n_in, d) - rs_ready(p, d);
+        if (!uniform) {
+            rows.push_back(RowDesc{(where == EWK_HOST ? n_in : stride) * i, n_in, p, s, (int)n_items, latch, 0});
+            n_items += fir_tiles(f, d, rs_ready(p, d), rs_ready(p + n_in, d));
+        }
+        ctx->h_rate[s] = sr_in;
+        ctx->h_inputs[s] = p + n_in;
     }
     const int n_ret = (int)(rs_ready(c + n_in, d) - rs_ready(c, d));
-    // streams at different positions: their positions go to the device in a slot of their own, which a later push
-    // reuses only after the K8 that reads them has run
     int k = -1;
-    cudaStream_t on = where == EWK_HOST ? ctx->copy_stream : ctx->stream;
+    // host input: on the copy stream ahead of the input's copy, so the K8 that waits for that copy finds them
     if (!uniform) {
-        k = ctx->pos_idx;
-        ctx->pos_idx ^= 1;
-        const size_t bytes = sizeof(long long) * (size_t)B.n_streams;
-        if (!ctx->h_pos[k]) {
-            CK(cudaHostAlloc((void**)&ctx->h_pos[k], bytes, cudaHostAllocDefault));
-            CK(cudaEventCreateWithFlags(&ctx->ev_pos[k], cudaEventDisableTiming));
-        }
-        CK(ctx->b_pos[k].ensure(bytes));
-        if (ctx->ev_pos_valid[k]) CK(cudaEventSynchronize(ctx->ev_pos[k]));
-        std::memcpy(ctx->h_pos[k], pos.data(), sizeof(long long) * (size_t)n_streams);
-        // host input: on the copy stream ahead of the input's copy, so the K8 that waits for that copy finds them
-        CK(cudaMemcpyAsync(ctx->b_pos[k].p, ctx->h_pos[k], sizeof(long long) * (size_t)n_streams, cudaMemcpyHostToDevice, on));
+        rc = ctx->upload_rows(rows, where == EWK_HOST ? ctx->copy_stream : ctx->stream, &k);
+        if (rc) return rc;
     }
-    const long long* d_pos = k >= 0 ? (const long long*)ctx->b_pos[k].p : nullptr;
     if (where != EWK_HOST) {
-        rc = ctx->land_resampled(stream0, n_streams, in, stride, in_format, n_in, sr_in, pos.data(), d_pos, -1);
+        rc = ctx->land_resampled(stream0, n_streams, in, stride, in_format, n_in, sr_in, c, k >= 0 ? rows.data() : nullptr,
+                                 k, n_items, -1);
         return rc ? rc : (each ? EWK_OK : n_ret);
     }
     // host input: its compact bytes cross PCIe on the copy stream and land lazily, as with ewk_push
@@ -1167,7 +1226,7 @@ static int push_resampled_impl(ewk_ctx* ctx, const char* who, int stream0, int n
     ctx->pending.valid = true; ctx->pending.slot = b; ctx->pending.stream0 = stream0; ctx->pending.n_streams = n_streams;
     ctx->pending.n = n_ret;
     ctx->pending.rs_rate = sr_in; ctx->pending.rs_fmt = in_format; ctx->pending.rs_n_in = n_in; ctx->pending.rs_c = c;
-    if (k >= 0) { ctx->pending.rs_pos_slot = k; ctx->pending.rs_pos = std::move(pos); }
+    if (k >= 0) { ctx->pending.rows_slot = k; ctx->pending.n_items = n_items; ctx->pending.rows = std::move(rows); }
     return each ? EWK_OK : n_ret;
 }
 
@@ -1192,6 +1251,136 @@ extern "C" int ewk_stream_input(ewk_ctx* ctx, int stream, int32_t* sr_in, int64_
     if (stream < 0 || stream >= ctx->bank.n_streams) { ctx->fail("ewk_stream_input: bad stream %d", stream); return EWK_ERR_ARG; }
     if (sr_in) *sr_in = ctx->h_rate[stream];
     if (n_in) *n_in = ctx->h_inputs[stream];
+    return EWK_OK;
+}
+
+// Ragged push to a list of streams: row i = in[offsets[i], offsets[i] + lens[i]) goes to stream streams[i].  Every rule
+// is the one of pushing the row alone with ewk_push / ewk_push_g711 (16 kHz) or ewk_push_resampled (other rates).
+extern "C" int ewk_push_streams(ewk_ctx* ctx, const int32_t* streams, int n, const void* in, int in_format,
+                                const int64_t* offsets, const int64_t* lens, int64_t in_len, int where, int sr_in,
+                                int64_t* landed) {
+    static const char* who = "ewk_push_streams";
+    if (!ctx) return EWK_ERR_ARG;
+    int rc = need_streams(ctx, who, false);
+    if (rc) return rc;
+    BankView& B = ctx->bank;
+    if (n == 0) return EWK_OK;
+    if (n < 0 || !streams || !offsets || !lens || (!in && in_len > 0) || in_len < 0 || in_format < EWK_PCM_F32 ||
+        in_format > EWK_IN_ALAW || !landed) {
+        ctx->fail("%s: bad arguments (n=%d in_len=%lld in_format=%d%s)", who, n, (long long)in_len, in_format,
+                  landed ? "" : ", landed is NULL");
+        return EWK_ERR_ARG;
+    }
+    const bool direct = sr_in == RS_TARGET;
+    ResampleDesign d;
+    if (!direct && (sr_in < 1000 || sr_in > 768000 || !rs_design(sr_in, d))) {
+        ctx->fail("%s: %d Hz is not a supported input rate", who, sr_in);
+        return EWK_ERR_ARG;
+    }
+    if (direct && in_format >= EWK_IN_ULAW && B.fmt != 1) {
+        ctx->fail("%s: G.711 at 16000 Hz needs int16 rings (pcm_format EWK_PCM_I16)", who);
+        return EWK_ERR_ARG;
+    }
+    if (direct && in_format < EWK_IN_ULAW && in_format != B.fmt) {
+        ctx->fail("%s: in_format %d at 16000 Hz must be the rings' pcm_format (%d) or G.711", who, in_format, B.fmt);
+        return EWK_ERR_ARG;
+    }
+    // samples row i lands: its own length at 16 kHz, else ready(c + len) - ready(c) from the stream's input position
+    auto lands = [&](int i) {
+        const long long c = ctx->h_inputs[streams[i]];
+        return direct ? (long long)lens[i] : rs_ready(c + lens[i], d) - rs_ready(c, d);
+    };
+    std::vector<char> seen((size_t)B.n_streams, 0);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        if (s < 0 || s >= B.n_streams) { ctx->fail("%s: bad stream %d (context has %d)", who, s, B.n_streams); return EWK_ERR_ARG; }
+        if (seen[s]) { ctx->fail("%s: stream %d is listed twice", who, s); return EWK_ERR_ARG; }
+        seen[s] = 1;
+        if (lens[i] < 0 || offsets[i] < 0 || offsets[i] > in_len - lens[i] || lens[i] > (int64_t)1 << 34) {
+            ctx->fail("%s: row %d of stream %d, [%lld, %lld + %lld), lies outside the input [0, %lld)", who, i, s,
+                      (long long)offsets[i], (long long)offsets[i], (long long)lens[i], (long long)in_len);
+            return EWK_ERR_ARG;
+        }
+        const long long m = lands(i);
+        if (m > B.P - B.R && m > B.R) {
+            ctx->fail("%s: stream %d: %lld samples exceed the ring (%d)", who, s, m, B.R);
+            return EWK_ERR_ARG;
+        }
+    }
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        if (lens[i] == 0) continue;
+        if (direct && ctx->h_rate[s] != 0 && ctx->h_rate[s] != RS_TARGET) {
+            ctx->fail("%s: stream %d takes %d Hz input through ewk_push_resampled", who, s, ctx->h_rate[s]);
+            return EWK_ERR_STATE;
+        }
+        if (!direct && ctx->h_rate[s] != 0 && ctx->h_rate[s] != sr_in) {
+            ctx->fail("%s: stream %d already takes %d Hz input", who, s, ctx->h_rate[s]);
+            return EWK_ERR_STATE;
+        }
+    }
+    CK(cudaSetDevice(ctx->device));
+    rc = ctx->flush_pending();
+    if (rc) return rc;
+    for (int i = 0; i < n; i++) {             // the guards of ewk_push, per stream on its landed count
+        const int s = streams[i];
+        if (lens[i] == 0 || ctx->h_prm[s].live) continue;
+        const long long m = lands(i);
+        const long long ahead = ctx->h_written[s] + m - ctx->h_visible_lb[s];
+        if (ctx->h_visible_lb[s] >= B.R && ahead > (long long)(B.P - B.R)) {
+            ctx->fail("%s: stream %d would hold %lld un-gated samples, more than slack_samples=%d; call ewk_tick first",
+                      who, s, ahead, B.P - B.R);
+            return EWK_ERR_STATE;
+        }
+        if (ctx->h_visible_lb[s] < B.R && ctx->h_written[s] + m > (long long)B.P) {
+            ctx->fail("%s: stream %d would hold %lld samples before its first full tick, more than the physical ring "
+                      "(%d); call ewk_tick first", who, s, ctx->h_written[s] + m, B.P);
+            return EWK_ERR_STATE;
+        }
+    }
+    const ewk_ctx::ResampleTable* t = nullptr;
+    if (!direct) {
+        rc = ctx->resample_table(sr_in, &t);
+        if (rc) return rc;
+        rc = ctx->ensure_rs_tail(2 * d.W);
+        if (rc) return rc;
+    }
+    // descriptors of the non-empty rows, and the flat work list: LIST_CHUNK-sample chunks (K1L) or output tiles (K8)
+    std::vector<RowDesc> rows;
+    long long n_items = 0;
+    const FirPlan f = direct ? FirPlan{} : fir_plan(d);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        landed[i] = lands(i);
+        if (lens[i] == 0) continue;
+        const long long c = ctx->h_inputs[s];
+        RowDesc r{offsets[i], lens[i], direct ? ctx->h_written[s] : c, s, (int)n_items,
+                  direct ? (int)lens[i] : (int)ewk_resample_out_len(lens[i], sr_in), 0};
+        n_items += direct ? (lens[i] + LIST_CHUNK - 1) / LIST_CHUNK : fir_tiles(f, d, rs_ready(c, d), rs_ready(c + lens[i], d));
+        if (n_items > INT_MAX) { ctx->fail("%s: too much input for one call", who); return EWK_ERR_ARG; }
+        rows.push_back(r);
+        ctx->h_rate[s] = direct ? RS_TARGET : sr_in;
+        ctx->h_inputs[s] = c + lens[i];
+    }
+    if (rows.empty()) return EWK_OK;
+    int k = -1;
+    rc = ctx->upload_rows(rows, where == EWK_HOST ? ctx->copy_stream : ctx->stream, &k);
+    if (rc) return rc;
+    if (where != EWK_HOST)
+        return direct ? ctx->land_list(rows, k, n_items, in, in_format, -1)
+                      : ctx->land_resampled(0, (int)rows.size(), in, 0, in_format, 0, sr_in, 0, rows.data(), k, n_items, -1);
+    // host input: [0, in_len) crosses PCIe as one copy on the copy stream and lands lazily, as with ewk_push
+    const size_t esz = rs_in_size(in_format);
+    const int b = ctx->stage_idx;
+    ctx->stage_idx ^= 1;
+    CK(ctx->b_raw[b].ensure(esz * (size_t)in_len));
+    if (ctx->ev_free_valid[b]) CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_free[b], 0));
+    CK(cudaMemcpyAsync(ctx->b_raw[b].p, in, esz * (size_t)in_len, cudaMemcpyHostToDevice, ctx->copy_stream));
+    CK(cudaEventRecord(ctx->ev_ready[b], ctx->copy_stream));
+    ctx->pending = ewk_ctx::Pending{};
+    ctx->pending.valid = true; ctx->pending.slot = b; ctx->pending.n_streams = (int)rows.size();
+    ctx->pending.rs_rate = direct ? 0 : sr_in; ctx->pending.rs_fmt = in_format;
+    ctx->pending.rows_slot = k; ctx->pending.n_items = n_items; ctx->pending.rows = std::move(rows);
     return EWK_OK;
 }
 
@@ -1237,21 +1426,42 @@ extern "C" int ewk_reset_streams(ewk_ctx* ctx, const int32_t* streams, int n) {
     return EWK_OK;
 }
 
-static int tick_impl(ewk_ctx* ctx, int n_ticks, uint8_t* silent, uint8_t* state, double* thr, double* rms) {
-    int rc = need_streams(ctx, "ewk_tick");
+// ewk_tick / ewk_tick_trace, and paced: ewk_tick_ready (n_ticks = max_ticks; stream s takes taken[s] of them)
+static int tick_impl(ewk_ctx* ctx, int n_ticks, bool paced, int32_t* taken, uint8_t* silent, uint8_t* state, double* thr,
+                     double* rms) {
+    const char* who = paced ? "ewk_tick_ready" : "ewk_tick";
+    int rc = need_streams(ctx, who);
     if (rc) return rc;
-    if (n_ticks < 1 || n_ticks > 4096) { ctx->fail("ewk_tick: n_ticks must be in [1, 4096]"); return EWK_ERR_ARG; }
+    if (n_ticks < 1 || n_ticks > 4096) { ctx->fail("%s: %s must be in [1, 4096]", who, paced ? "max_ticks" : "n_ticks"); return EWK_ERR_ARG; }
     BankView& B = ctx->bank;
     CK(cudaSetDevice(ctx->device));
+    // paced: the budgets depend on every landed sample
+    if (paced) { rc = ctx->flush_pending(); if (rc) return rc; }
     if (ctx->pending.valid) {
         // land the in-flight host push only if these ticks reach into its samples
         bool need = false;
-        for (int s = ctx->pending.stream0; !need && s < ctx->pending.stream0 + ctx->pending.n_streams; s++) {
+        const std::vector<RowDesc>& rows = ctx->pending.rows;
+        for (int i = 0; !need && i < ctx->pending.n_streams; i++) {
+            const int s = rows.empty() ? ctx->pending.stream0 + i : rows[i].stream;
             const int fs = ctx->h_frame_size[s] > 0 ? ctx->h_frame_size[s] : ctx->h_prm[s].frame_size;
             if (ctx->h_prm[s].live || fs <= 0) need = true;
             else need = ((ctx->h_tick[s] + n_ticks) * TICK / fs) * fs > ctx->h_written[s];
         }
         if (need) { rc = ctx->flush_pending(); if (rc) return rc; }
+    }
+    // the ticks each stream takes: the due rule of ewk_tick_ready on the host mirrors (K2 applies it to StreamState), and
+    // only as many K2 rounds as the largest budget needs (one at least: K2 stores every stream's record in every call)
+    std::vector<int> budget;
+    int rounds_ticks = n_ticks;
+    if (paced) {
+        budget.resize((size_t)B.n_streams);
+        int most = 0;
+        for (int s = 0; s < B.n_streams; s++) {
+            const long long due = ctx->h_written[s] / TICK - ctx->h_tick[s];
+            budget[s] = (int)std::max(0LL, std::min((long long)n_ticks, due));
+            most = std::max(most, budget[s]);
+        }
+        rounds_ticks = std::max(1, most);
     }
     TraceView tr{};
     const bool want = silent || state || thr || rms;
@@ -1263,6 +1473,8 @@ static int tick_impl(ewk_ctx* ctx, int n_ticks, uint8_t* silent, uint8_t* state,
         tr.rms = (double*)(base + cells * 8);
         tr.silent = (unsigned char*)(base + cells * 16);
         tr.state = (unsigned char*)(base + cells * 17);
+        // cells of ticks a stream does not take: silent = state = 255, thr = rms = NaN (all-ones bits)
+        if (paced) CK(cudaMemsetAsync(ctx->b_trace.p, 0xFF, cells * (2 + 16), ctx->stream));
     }
     int smem_chunks = ctx->gate_chunks();
     if (smem_chunks > GATE_SMEM_CHUNKS) {
@@ -1282,11 +1494,12 @@ static int tick_impl(ewk_ctx* ctx, int n_ticks, uint8_t* silent, uint8_t* state,
     if (B.n_pub > 0 && ctx->ev_pub_valid[B.pub_parity])   // K2 rewrites this parity's copy: its sender (two calls ago) is long done
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_pub[B.pub_parity], 0));
     cudaEvent_t pe = ctx->prof_begin(1);
-    for (int done = 0; done < n_ticks; done += GATE_MAX_TICKS) {
-        const int nt = std::min(GATE_MAX_TICKS, n_ticks - done);
-        tick_gate_kernel<<<(B.n_streams + GATE_WARPS - 1) / GATE_WARPS, GATE_THREADS,
-                           sizeof(double) * 3 * (size_t)smem_chunks * GATE_WARPS + (size_t)2 * stage_bytes * GATE_WARPS,
-                           ctx->stream>>>(B, nt, tr, n_ticks, done, smem_chunks, stage_bytes);
+    for (int done = 0; done < rounds_ticks; done += GATE_MAX_TICKS) {
+        const int nt = std::min(GATE_MAX_TICKS, rounds_ticks - done);
+        auto k2 = paced ? tick_gate_kernel<true> : tick_gate_kernel<false>;
+        k2<<<(B.n_streams + GATE_WARPS - 1) / GATE_WARPS, GATE_THREADS,
+             sizeof(double) * 3 * (size_t)smem_chunks * GATE_WARPS + (size_t)2 * stage_bytes * GATE_WARPS,
+             ctx->stream>>>(B, nt, tr, n_ticks, done, smem_chunks, stage_bytes);
         ctx->launches++;
     }
     ctx->prof_end(pe, 1);
@@ -1299,7 +1512,7 @@ static int tick_impl(ewk_ctx* ctx, int n_ticks, uint8_t* silent, uint8_t* state,
     cudaStream_t ks = ctx->stream;
     // ... plus the tail a cut drops: n_back = segment + n_drop, n_drop ~ (post_speech_silence + 0.05 s) and one tick of slop
     const long long drop_reserve = (long long)std::ceil((ctx->max_post + 0.15) * 16000.0);
-    if (ctx->overlap && (long long)B.R >= MAX_SEG + (long long)(n_ticks + 2) * TICK + drop_reserve && !want) {
+    if (ctx->overlap && (long long)B.R >= MAX_SEG + (long long)(rounds_ticks + 2) * TICK + drop_reserve && !want) {
         CK(cudaEventRecord(ctx->ev_gate, ctx->stream));
         CK(cudaStreamWaitEvent(ctx->match_stream, ctx->ev_gate, 0));
         ks = ctx->match_stream;
@@ -1336,7 +1549,9 @@ static int tick_impl(ewk_ctx* ctx, int n_ticks, uint8_t* silent, uint8_t* state,
     ctx->pushes_since_tick = 0;
     // host mirrors (audio clock): V after these ticks, given what has been pushed
     for (int s = 0; s < B.n_streams; s++) {
-        ctx->h_tick[s] += n_ticks;
+        const int k = paced ? budget[s] : n_ticks;
+        if (taken) taken[s] = k;
+        ctx->h_tick[s] += k;
         const StreamParams& p = ctx->h_prm[s];
         if (p.live) { ctx->h_visible_lb[s] = ctx->h_written[s]; continue; }
         const int fs = ctx->h_frame_size[s];
@@ -1357,12 +1572,18 @@ static int tick_impl(ewk_ctx* ctx, int n_ticks, uint8_t* silent, uint8_t* state,
 
 extern "C" int ewk_tick(ewk_ctx* ctx, int n_ticks) {
     if (!ctx) return EWK_ERR_ARG;
-    return tick_impl(ctx, n_ticks, nullptr, nullptr, nullptr, nullptr);
+    return tick_impl(ctx, n_ticks, false, nullptr, nullptr, nullptr, nullptr, nullptr);
 }
 
 extern "C" int ewk_tick_trace(ewk_ctx* ctx, int n_ticks, uint8_t* silent, uint8_t* state, double* thr, double* rms) {
     if (!ctx) return EWK_ERR_ARG;
-    return tick_impl(ctx, n_ticks, silent, state, thr, rms);
+    return tick_impl(ctx, n_ticks, false, nullptr, silent, state, thr, rms);
+}
+
+extern "C" int ewk_tick_ready(ewk_ctx* ctx, int max_ticks, int32_t* taken, uint8_t* silent, uint8_t* state, double* thr,
+                              double* rms) {
+    if (!ctx) return EWK_ERR_ARG;
+    return tick_impl(ctx, max_ticks, true, taken, silent, state, thr, rms);
 }
 
 extern "C" int ewk_poll(ewk_ctx* ctx, ewk_event* out, int cap, int* dropped) {
@@ -1544,8 +1765,9 @@ extern "C" int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int tmpl
         // a host push whose copy is still in flight lands now only if these hops reach into its samples: otherwise the copy
         // of the NEXT block keeps overlapping this call's kernel (offline sweeps: push block j + 1, then score block j)
         bool need = false;
-        for (int s = ctx->pending.stream0; !need && s < ctx->pending.stream0 + ctx->pending.n_streams; s++)
-            need = ctx->h_written[s] < 160LL * (hop0 + n_hops - 1);
+        const std::vector<RowDesc>& rows = ctx->pending.rows;
+        for (int i = 0; !need && i < ctx->pending.n_streams; i++)
+            need = ctx->h_written[rows.empty() ? ctx->pending.stream0 + i : rows[i].stream] < 160LL * (hop0 + n_hops - 1);
         if (need) { rc = ctx->flush_pending(); if (rc) return rc; }
     }
     if (!out || hop0 < 0 || n_hops < 1 || tmpl_count < 1 || tmpl_count > DENSE_MAX_T || tmpl_first < 0 ||

@@ -61,19 +61,27 @@ struct ewk_ctx {
     int join_match();
     int stage_idx = 0;
     // n: samples that land in the rings; rs_rate != 0 marks a native-rate push (K8) of rs_n_in inputs at that rate, from
-    // input position rs_c, or from the per-stream positions rs_pos (device copy in pos slot rs_pos_slot) when they differ
+    // input position rs_c.  rows_slot >= 0: a push of per-row descriptors `rows` (device copy in that slot) of n_items
+    // work items from the raw input (format rs_fmt): K8 when rs_rate != 0, else K1L (ewk_push_streams at 16 kHz)
     struct Pending {
         bool valid = false; int slot = 0, stream0 = 0, n_streams = 0; long long n = 0;
         int rs_rate = 0, rs_fmt = 0; long long rs_n_in = 0, rs_c = 0;
-        int rs_pos_slot = -1; std::vector<long long> rs_pos;
+        int rows_slot = -1; long long n_items = 0; std::vector<ewk::RowDesc> rows;
     } pending;
     int land(int stream0, int n_streams, const void* d_src, long long d_stride, long long n, int stage_slot);
-    // pos: host positions of the call's streams; d_pos: their device copy, null when they are all equal (uniform K8)
+    // rows_slot < 0: rows i < n_streams (d_stride apart) go to streams stream0 + i, all at input position c (uniform K8).
+    // rows_slot >= 0: per-row descriptors rows[0 .. n_streams) (host) and their device copy in that slot, n_items tiles
     int land_resampled(int stream0, int n_streams, const void* d_src, long long d_stride, int in_fmt, long long n_in,
-                       int sr_in, const long long* pos, const long long* d_pos, int stage_slot);
-    // per-stream K8 input positions of a push at different positions (ewk_push_resampled_each): two slots of pinned host
-    // + device memory, each reused only once the K8 that read it has finished (ev_pos)
-    long long* h_pos[2] = {nullptr, nullptr};
+                       int sr_in, long long c, const ewk::RowDesc* rows, int rows_slot, long long n_items, int stage_slot);
+    // K1L: the rows of a list push at 16 kHz (descriptors on the host and in slot rows_slot), from d_src in format in_fmt
+    int land_list(const std::vector<ewk::RowDesc>& rows, int rows_slot, long long n_items, const void* d_src, int in_fmt,
+                  int stage_slot);
+    // per-row descriptors -> the next slot (copied on stream `on`); *slot receives its index
+    int upload_rows(const std::vector<ewk::RowDesc>& rows, cudaStream_t on, int* slot);
+    // per-row descriptors of a list push (ewk_push_streams) or of a push at different input positions
+    // (ewk_push_resampled_each): two slots of pinned host + device memory for n_streams rows, each reused only once the
+    // kernel that read it has finished (ev_pos)
+    ewk::RowDesc* h_pos[2] = {nullptr, nullptr};
     ewk::DevBuf b_pos[2];
     cudaEvent_t ev_pos[2] = {nullptr, nullptr};
     bool ev_pos_valid[2] = {false, false};
@@ -109,6 +117,7 @@ struct ewk_ctx {
     std::vector<long long> h_inputs;       // input samples the stream received (at its own rate)
     float* d_rs_tail = nullptr;            // K8 input tails [n_streams][rs_tail_cap], sized by the rates in use
     int rs_tail_cap = 0;
+    int ensure_rs_tail(int cap);           // grows the tails to cap floats per stream
     int gate_chunks() const;               // largest R / frame_size in use
     // per-kernel event timing (ewk_profile)
     bool prof_on = false;
@@ -132,7 +141,7 @@ struct ewk_ctx {
     std::map<int, ResampleTable> rs_tables;
     ewk::DevBuf b_rs_in, b_rs_out;
     int resample_table(int sr_in, const ResampleTable** out);
-    // pos (host, optional): per-row input positions; the grid covers the row with the most output tiles
+    // A.rows set: the grid is the descriptors' n_items flat output tiles (fir_tiles per row)
     int launch_fir(const ResampleTable& t, ewk::RsPushArgs& A, int n_rows, int prof_cls, const char* who,
-                   const long long* pos = nullptr);
+                   long long n_items = 0);
 };

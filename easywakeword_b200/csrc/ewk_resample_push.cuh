@@ -11,7 +11,7 @@
 // calls).  A call with n new inputs lands outputs [ready(c), ready(c + n)).  The host picks the tile so that only CTA 0
 // of a stream reads the tail; CTA 0 copies it to shared memory and rewrites it in place after a barrier.
 //
-// Work mapping.  CTA = (output tile, stream); the tile's input span, the 256-entry G.711 expansion table and (when small)
+// Work mapping.  CTA = (output tile, stream), or flat tile x of a list of per-row descriptors (RsPushArgs.rows); the tile's input span, the 256-entry G.711 expansion table and (when small)
 // the filter table are staged in shared memory as float32.
 //   fast path (L in {1, 2, 4, 8}, M in {1, 2, 3}: 8, 12, 24, 32, 48 kHz): warp-uniform phase, each thread holds K
 //     outputs of that phase in consecutive groups, n_q = (g + q) L + r.  Their tap-j inputs are x[b + q M + j], so tap
@@ -45,8 +45,9 @@ struct RsPushArgs {
     int tail_cap, in_fmt, L, M, W, stream0, frame_latch, tile, table_smem, span;   // span: staged input floats per CTA
     float* out;                 // non-null: ewk_resample — outputs [o0, o1) of row y go to out + y * out_stride as float32;
     long long out_stride;       //   the input holds absolute samples [c, c + n_in) (c = t0_old, no tail); no ring, no commit
-    const long long* pos;       // non-null: [n_streams] inputs row y's stream had received before the call; the row's c, o0,
-                                //   o1, t0_old and t0_new follow from it (rsp_row) instead of the uniform values above
+    const RowDesc* rows;        // non-null: per-row descriptors [n_rows] (ewk_push_streams, ewk_push_resampled_each): CTA x
+    int n_rows;                 //   is flat output tile x; its row's stream, input, position and frame latch come from the
+                                //   descriptor, and c, o0, o1, t0_old, t0_new follow from them (rsp_row)
 };
 
 // outputs whose W inputs of look-ahead have arrived after c inputs, and the first input any later output reads (the
@@ -60,14 +61,19 @@ __device__ __forceinline__ long long rsp_tail_start(long long c, const RsPushArg
     return t > 0 ? t : 0;
 }
 
-// the positions of row y: per-row (EACH: A.pos, ewk_push_resampled_each) or the call's uniform values.  The uniform
-// instance keeps them in the parameter bank, which leaves its register count (and occupancy) as it was
-struct RsRow { long long c, o0, o1, t0_old, t0_new; };
+// row y of the call: per-row (EACH: descriptor A.rows[y]) or the call's uniform values (row y = stream stream0 + y at
+// in + y in_stride).  The uniform instance reads n_in and the latch from the parameter bank (rsp_n_in, rsp_latch),
+// which leaves its register count (and occupancy) as it was
+struct RsRow { long long c, n_in, o0, o1, t0_old, t0_new; int latch; };
+template <bool EACH> __device__ __forceinline__ long long rsp_n_in(const RsPushArgs& A, const RsRow& R) { return EACH ? R.n_in : A.n_in; }
+template <bool EACH> __device__ __forceinline__ int rsp_latch(const RsPushArgs& A, const RsRow& R) { return EACH ? R.latch : A.frame_latch; }
 template <bool EACH>
 __device__ __forceinline__ RsRow rsp_row(const RsPushArgs& A, int y) {
-    if (!EACH) return RsRow{A.c, A.o0, A.o1, A.t0_old, A.t0_new};
-    const long long c = A.pos[y];
-    return RsRow{c, rsp_ready(c, A), rsp_ready(c + A.n_in, A), rsp_tail_start(c, A), rsp_tail_start(c + A.n_in, A)};
+    if (!EACH) return RsRow{A.c, A.n_in, A.o0, A.o1, A.t0_old, A.t0_new, A.frame_latch};
+    const RowDesc d = A.rows[y];
+    const long long c = d.pos;
+    return RsRow{c, d.len, rsp_ready(c, A), rsp_ready(c + d.len, A), rsp_tail_start(c, A), rsp_tail_start(c + d.len, A),
+                 d.latch};
 }
 
 __device__ __forceinline__ float g711_value(int code, int alaw) {
@@ -95,11 +101,12 @@ __device__ __forceinline__ float rsp_chunk(const RsPushArgs& A, const void* row,
 
 // absolute input sample k of the stream: zeros before 0 and beyond what has arrived.  Below t0_old (> 0 once the stream
 // is under way) only outputs before o0 read, which this call computes on the fast path but does not store.
+template <bool EACH>
 __device__ __forceinline__ float rsp_input(const RsPushArgs& A, const RsRow& R, const float* tail, const void* row,
                                            long long k, const float* lut) {
     if (k < R.t0_old) return 0.f;
     if (k < R.c) return tail[k - R.t0_old];
-    if (k < R.c + A.n_in) return rsp_chunk(A, row, k - R.c, lut);
+    if (k < R.c + rsp_n_in<EACH>(A, R)) return rsp_chunk(A, row, k - R.c, lut);
     return 0.f;
 }
 
@@ -154,9 +161,15 @@ __global__ void __launch_bounds__(RSP_THREADS, 2) resample_push_kernel(BankView 
     float* tail_s = lut + 256;                                  // [tail_cap] CTA 0's copy of the stream's tail
     float* hs = tail_s + A.tail_cap;                            // [2W L] when A.table_smem
     float* xs = hs + (A.table_smem ? 2 * A.W * A.L : 0);        // [span]
-    const int s = A.stream0 + blockIdx.y;
-    const void* row = reinterpret_cast<const char*>(A.in) +
-                      (size_t)blockIdx.y * A.in_stride * (A.in_fmt == RSP_IN_F32 ? 4 : A.in_fmt == RSP_IN_I16 ? 2 : 1);
+    // the CTA's row and output tile: the grid's (tile, row), or flat tile x of the descriptors' list.  The uniform
+    // instance reads blockIdx where it needs them (held in registers across the FIR, they cost it 5 registers at M = 3)
+    const unsigned y_each = EACH ? (unsigned)row_of_item(A.rows, A.n_rows, blockIdx.x) : 0u;
+    const unsigned tile_each = EACH ? blockIdx.x - (unsigned)A.rows[y_each].item0 : 0u;
+    auto row_y = [&] { return EACH ? y_each : blockIdx.y; };
+    auto tile_x = [&] { return EACH ? tile_each : blockIdx.x; };
+    const int s = EACH ? A.rows[y_each].stream : A.stream0 + (int)blockIdx.y;
+    const void* row = reinterpret_cast<const char*>(A.in) + (EACH ? (size_t)A.rows[y_each].off : (size_t)blockIdx.y * A.in_stride) *
+                      (A.in_fmt == RSP_IN_F32 ? 4 : A.in_fmt == RSP_IN_I16 ? 2 : 1);
     float* tail = A.out ? nullptr : A.tail + (size_t)s * A.tail_cap;
     const int tid = threadIdx.x;
     if (A.in_fmt >= RSP_IN_ULAW) lut[tid] = g711_value(tid, A.in_fmt == RSP_IN_ALAW);
@@ -167,25 +180,25 @@ __global__ void __launch_bounds__(RSP_THREADS, 2) resample_push_kernel(BankView 
     const float* h = A.table_smem ? hs : A.H;
 
     // the CTA's outputs [n0, n0 + tile) and the input span they read, from absolute sample s0
-    const RsRow R = rsp_row<EACH>(A, blockIdx.y);
+    const RsRow R = rsp_row<EACH>(A, row_y());
     const bool fast = M > 0;
     long long n0, s0;
     if (fast) {
-        n0 = (R.o0 / A.L) * A.L + (long long)blockIdx.x * A.tile;
+        n0 = (R.o0 / A.L) * A.L + (long long)tile_x() * A.tile;
         s0 = (n0 / A.L) * M - A.W + 1;
     } else {
-        n0 = R.o0 + (long long)blockIdx.x * A.tile;
+        n0 = R.o0 + (long long)tile_x() * A.tile;
         s0 = n0 * A.M / A.L - A.W + 1;
     }
-    // rows at different positions: the grid covers the row with the most tiles; CTA 0 always runs (tail, commit)
-    if (blockIdx.x > 0 && n0 >= R.o1) return;
-    for (int i = tid; i < A.span; i += RSP_THREADS) xs[i] = rsp_input(A, R, tail, row, s0 + i, lut);
-    if (blockIdx.x == 0)
+    // tile 0 always runs (tail, commit)
+    if (tile_x() > 0 && n0 >= R.o1) return;
+    for (int i = tid; i < A.span; i += RSP_THREADS) xs[i] = rsp_input<EACH>(A, R, tail, row, s0 + i, lut);
+    if (tile_x() == 0)
         for (int i = tid; i < (int)(R.c - R.t0_old); i += RSP_THREADS) tail_s[i] = tail[i];
     __syncthreads();
 
     void* ring = A.out ? nullptr : reinterpret_cast<char*>(B.ring) + (size_t)s * B.P * (B.fmt == 1 ? 2 : 4);
-    float* out = A.out ? A.out + (size_t)blockIdx.y * A.out_stride - R.o0 : nullptr;
+    float* out = A.out ? A.out + (size_t)row_y() * A.out_stride - R.o0 : nullptr;
     const int p_n0 = A.out ? 0 : (int)(n0 % B.P);               // ring position of n0: one 64-bit modulo per CTA
     auto store = [&](long long n, float y) {
         if (out) { out[n] = y; return; }
@@ -223,9 +236,9 @@ __global__ void __launch_bounds__(RSP_THREADS, 2) resample_push_kernel(BankView 
         }
     }
 
-    if (blockIdx.x == 0 && !A.out) {
+    if (tile_x() == 0 && !A.out) {
         // the tail for the next call: inputs [t0_new, c + n_in), from the old tail's copy or the new chunk
-        const int keep = (int)(R.c + A.n_in - R.t0_new);
+        const int keep = (int)(R.c + rsp_n_in<EACH>(A, R) - R.t0_new);
         for (int i = tid; i < keep; i += RSP_THREADS) {
             const long long k = R.t0_new + i;
             tail[i] = k < R.c ? tail_s[k - R.t0_old] : rsp_chunk(A, row, k - R.c, lut);
@@ -234,7 +247,7 @@ __global__ void __launch_bounds__(RSP_THREADS, 2) resample_push_kernel(BankView 
             StreamState& st = B.st[s];
             if (st.frame_size == 0) {
                 const int fs = B.prm[s].frame_size;
-                st.frame_size = fs > 0 ? fs : A.frame_latch;
+                st.frame_size = fs > 0 ? fs : rsp_latch<EACH>(A, R);
             }
             st.written = R.o1;
             st.ss_from = R.o1;

@@ -157,28 +157,30 @@ struct TraceView {          // optional per-tick trace for parity tests: [n_stre
 };
 
 // ------------------------------------------------------------------------------------ K0 (G.711 ingest)
+// the 16-bit linear value of G.711 code c (mu-law, or A-law when alaw), from the standard's bit layout
+__device__ __forceinline__ short g711_linear(int c, int alaw) {
+    int v;
+    if (alaw) {
+        const int a = c ^ 0x55, e = (a >> 4) & 7, m = a & 0x0F;
+        v = e == 0 ? (m << 4) + 8 : ((m << 4) + 0x108) << (e - 1);
+        v = (a & 0x80) ? v : -v;
+    } else {
+        const int u = ~c & 0xFF;
+        v = ((((u & 0x0F) << 3) + 0x84) << ((u >> 4) & 7)) - 0x84;
+        v = (u & 0x80) ? -v : v;
+    }
+    return (short)v;
+}
+
 // 8-bit mu-law / A-law codes -> the 16-bit linear samples of ITU-T G.711 (what libsndfile hands librosa.load for such
 // files, and what a telephony feed carries): in[r * stride + i] -> out[r * n + i], i < n.  The 256-entry expansion table is
-// formed in shared memory from the standard's bit layout; 16 codes per thread per step (one 16-byte load, two stores).
+// formed in shared memory; 16 codes per thread per step (one 16-byte load, two stores).
 // HBM-bound: 1 byte read + 2 bytes written per sample.  It runs on the copy stream right behind the H2D copy of the
 // codes, so a host feed crosses PCIe at half the bytes of PCM16.
 __global__ void __launch_bounds__(256)
 g711_decode_kernel(const unsigned char* __restrict__ in, short* __restrict__ out, int n_rows, long long n, long long stride, int alaw) {
     __shared__ short lut[256];
-    {
-        const int c = threadIdx.x;
-        int v;
-        if (alaw) {
-            const int a = c ^ 0x55, e = (a >> 4) & 7, m = a & 0x0F;
-            v = e == 0 ? (m << 4) + 8 : ((m << 4) + 0x108) << (e - 1);
-            v = (a & 0x80) ? v : -v;
-        } else {
-            const int u = ~c & 0xFF;
-            v = ((((u & 0x0F) << 3) + 0x84) << ((u >> 4) & 7)) - 0x84;
-            v = (u & 0x80) ? -v : v;
-        }
-        lut[c] = (short)v;
-    }
+    lut[threadIdx.x] = g711_linear(threadIdx.x, alaw);
     __syncthreads();
     const bool vec = (n % 16) == 0 && (stride % 16) == 0 && ((size_t)in & 15) == 0 && ((size_t)out & 15) == 0;
     const long long per_row = vec ? n / 16 : n;
@@ -304,6 +306,77 @@ __global__ void ring_commit_kernel(BankView B, int stream0, int n_streams, int n
     if (!with_sums) st.ss_from = st.written + n;                        // nothing known about these samples
     else if (st.ss_from > st.written) st.ss_from = st.written;          // sums restart at this push
     st.written += n;
+}
+
+// ------------------------------------------------------------------------------------ K1L (list push)
+// One row of a list push (ewk_push_streams; K8's per-row instance reads the same descriptors).  The rows' work is one flat
+// list of items — K1L: LIST_CHUNK-sample chunks, K8: output tiles — and row y owns items [item0, next row's item0).
+struct RowDesc {
+    long long off;          // first input sample of the row in the call's buffer
+    long long len;          // input samples of the row (> 0)
+    long long pos;          // K1L: samples the stream had landed (its `written`); K8: input samples it had received
+    int stream;
+    int item0;
+    int latch;              // frame size latched by a stream's first push when frame_size is 0
+    int pad;
+};
+
+// the row that owns flat item `item` (rows' item0 ascend, every row owns at least one item)
+__device__ __forceinline__ int row_of_item(const RowDesc* __restrict__ rows, int n_rows, int item) {
+    int lo = 0, hi = n_rows - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(&rows[mid].item0) <= item) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+constexpr int LIST_THREADS = 256, LIST_PER = 16;
+constexpr int LIST_CHUNK = LIST_THREADS * LIST_PER;     // samples per K1L item
+
+// K1L: row y's samples in[off, off + len) -> ring of stream `stream` at absolute index pos + i, with wrap.  in_fmt: the
+// ring's format (0 f32, 1 int16), or G.711 codes (2 mu-law, 3 A-law) expanded through a shared-memory table into int16
+// rings, as K0 does.  The row's first item commits it: written = pos + len, the frame-size latch, and ss_from past the
+// new samples (no block sums: K2 reads them).  Nothing in the launch reads `written`, so the commit needs no barrier.
+// Rows start at any sample, so accesses are per sample; each thread issues its LIST_PER loads before its stores, which
+// keeps enough bytes in flight to stream at HBM rate.
+template <typename T>
+__global__ void __launch_bounds__(LIST_THREADS)
+ring_push_list_kernel(BankView B, const void* __restrict__ in, int in_fmt, const RowDesc* __restrict__ rows, int n_rows) {
+    __shared__ short lut[256];
+    if (in_fmt >= 2) lut[threadIdx.x] = g711_linear(threadIdx.x, in_fmt == 3);
+    __syncthreads();
+    const int y = row_of_item(rows, n_rows, blockIdx.x);
+    const RowDesc d = rows[y];
+    const long long i0 = (long long)(blockIdx.x - d.item0) * LIST_CHUNK;
+    const int n = (int)min((long long)LIST_CHUNK, d.len - i0);
+    T* ring = (T*)B.ring + (size_t)d.stream * B.P;
+    const int p0 = (int)((d.pos + i0) % B.P);
+    T v[LIST_PER];
+#pragma unroll
+    for (int u = 0; u < LIST_PER; u++) {
+        const int i = threadIdx.x + u * LIST_THREADS;
+        if (i < n) {
+            if (in_fmt >= 2) v[u] = (T)lut[__ldg((const unsigned char*)in + d.off + i0 + i)];
+            else v[u] = __ldg((const T*)in + d.off + i0 + i);
+        }
+    }
+#pragma unroll
+    for (int u = 0; u < LIST_PER; u++) {
+        const int i = threadIdx.x + u * LIST_THREADS;
+        int p = p0 + i;
+        if (p >= B.P) p -= B.P;
+        if (i < n) ring[p] = v[u];
+    }
+    if (i0 == 0 && threadIdx.x == 0) {
+        StreamState& st = B.st[d.stream];
+        if (st.frame_size == 0) {
+            const int fs = B.prm[d.stream].frame_size;
+            st.frame_size = fs > 0 ? fs : d.latch;
+        }
+        st.written = d.pos + d.len;
+        st.ss_from = d.pos + d.len;
+    }
 }
 
 // ------------------------------------------------------------------------------------ K2 helpers
@@ -739,6 +812,9 @@ __device__ __forceinline__ unsigned gate_state_step(const BankView& B, int s, St
 // phase 1: the warp sums every planned range (the only HBM traffic: each new sample is read once,
 // 16-byte loads, eight in flight per lane); phase 2: the ticks are replayed in order — chunk updates
 // into an incrementally maintained sorted array, percentile, threshold, is_silent, state machine.
+// PACED (ewk_tick_ready): each stream takes only the ticks its landed audio pays for, min(n_ticks, written / 1600 - tick),
+// possibly none; its result record is stored all the same, since peer publication relies on every record in every call.
+template <bool PACED>
 __global__ void __launch_bounds__(GATE_THREADS, 7)
 tick_gate_kernel(BankView B, int n_ticks, TraceView tr, int trace_stride, int trace_off, int smem_chunks, int stage_bytes) {
     extern __shared__ __align__(16) double sm_d[];
@@ -773,6 +849,7 @@ tick_gate_kernel(BankView B, int n_ticks, TraceView tr, int trace_stride, int tr
         for (int i = lane; i < spec; i += 32) { ms[i] = g_ms[i]; SA[i] = g_sorted[i]; }
     }
     __syncwarp();
+    if (PACED) n_ticks = (int)max(0LL, min((long long)n_ticks, st.written / TICK - st.tick));
     const int fs = st.frame_size;
     const long long tick0 = st.tick, visible0 = st.visible, written0 = st.written;
     const int valid0 = st.chunks_valid;
@@ -914,7 +991,7 @@ tick_gate_kernel(BankView B, int n_ticks, TraceView tr, int trace_stride, int tr
         }
         __syncwarp();
     }
-    const bool pipelined = !presummed && stage_bytes > 0 && all_alias;
+    const bool pipelined = !presummed && stage_bytes > 0 && all_alias && (!PACED || n_ticks > 0);
     unsigned long long* bar = mbar[warp];
     char* buf = stage + (size_t)warp * 2 * stage_bytes;
     const char* ring_s = (const char*)B.ring + (size_t)s * B.P * esz;

@@ -124,6 +124,17 @@ class ShardedBank:
     def step(self, pcm_local, where=0):
         self.bank.step(pcm_local, where)
 
+    def step_streams(self, global_streams, blocks):
+        """WakeWordBank.step_streams over global stream ids: every rank may be called with the whole list and keeps only
+        the rows of the streams it owns (dist.local_streams)."""
+        streams, rows = [], []
+        for g, blk in zip(global_streams, blocks):
+            loc = local_streams([g], self.n_total, self.world, self.rank)
+            if loc:
+                streams.append(loc[0])
+                rows.append(blk)
+        return self.bank.step_streams(streams, rows)
+
     def gather(self):
         ctx = self.bank.ctx
         if self.peer is not None and ctx.publish_seq() > 0:

@@ -58,6 +58,13 @@ def landed_counts(positions, n_in: int, sr_in: int) -> np.ndarray:
                     dtype=np.int64)
 
 
+def due_ticks(written, ticks, max_ticks=None) -> np.ndarray:
+    """Ticks a stream may take under ewk_tick_ready: tick k is due once 1600 k samples have landed, so a stream that
+    landed `written` 16 kHz samples and took `ticks` ticks has max(0, written // 1600 - ticks) due, at most max_ticks."""
+    due = np.maximum(0, np.asarray(written, dtype=np.int64) // 1600 - np.asarray(ticks, dtype=np.int64))
+    return due if max_ticks is None else np.minimum(due, int(max_ticks))
+
+
 class StreamResampler:
     """Chunked conversion of [rows, n] feeds to 16 kHz whose concatenated output equals the one-shot result
     sample for sample: every call is given the filter's half-width of history and emits only the outputs whose

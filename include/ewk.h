@@ -260,6 +260,29 @@ int ewk_push_resampled(ewk_ctx* ctx, int stream0, int n_streams, const void* in,
  * per group of equal positions.  Returns EWK_OK or a status. */
 int ewk_push_resampled_each(ewk_ctx* ctx, int stream0, int n_streams, const void* in, int in_format, int64_t n_in,
                             int64_t stride, int where, int sr_in, int64_t* landed);
+/* Ragged push to a list of streams.  Row i is in[offsets[i] .. offsets[i] + lens[i]) (in samples of in_format; the
+ * buffer holds in_len samples) and goes to stream streams[i].  sr_in = 16000 lands the samples directly (in_format = the
+ * ring's format, or EWK_IN_ULAW / EWK_IN_ALAW into int16 rings, as ewk_push / ewk_push_g711); any other rate converts
+ * them with K8, any input format into either ring format, as ewk_push_resampled.  landed[i] (host, required) receives
+ * the 16 kHz samples landed on streams[i] (lens[i] at 16 kHz).  lens[i] = 0 is allowed; n = 0 is a no-op.
+ * The result is bit-identical to pushing each row alone with ewk_push / ewk_push_g711 / ewk_push_resampled onto
+ * [streams[i], streams[i] + 1): rings, K8 input tails, rate and frame-size latches, ewk_stream_input.  A row of length 0
+ * changes nothing.  With frame_size 0 a stream latches its row's length (other rates: ewk_resample_out_len of it).
+ * EWK_ERR_ARG: a stream out of range or listed twice, a negative length or a row outside [0, in_len), landed = NULL, an
+ * unsupported rate, G.711 at 16 kHz into f32 rings, another in_format than the rings' at 16 kHz, a row larger than the
+ * ring.  EWK_ERR_STATE: a stream latched to another rate, and the push guards of ewk_push, per stream on its landed
+ * count.  Host input crosses PCIe as one copy of [0, in_len) on the copy stream and lands lazily (pinned or pageable), as
+ * with ewk_push; overlap mode behaves as for ewk_push.  Streams not listed are untouched and cost no bytes. */
+int ewk_push_streams(ewk_ctx* ctx, const int32_t* streams, int n, const void* in, int in_format,
+                     const int64_t* offsets, const int64_t* lens, int64_t in_len, int where, int sr_in, int64_t* landed);
+/* Ticks paced by each stream's own audio: stream s takes taken[s] = min(max_ticks, max(0, written_s / 1600 - tick_s))
+ * ticks (written_s after any pending host push has landed), i.e. tick k is taken once 1600 k samples have landed.
+ * Otherwise the same as ewk_tick_trace: any of taken / silent / state / thr / rms may be NULL; trace cells are
+ * [n_streams][max_ticks], and cells of ticks a stream did not take hold silent = 255, state = 255, thr = rms = NaN.
+ * A stream with nothing due (a parked slot) takes no tick and raises no event; its result record is still rewritten
+ * (bit 4 cleared) and published.  The same audio gives the same events however it was split into pushes.  Mixing with
+ * ewk_tick on one context is allowed: ewk_tick moves every stream.  max_ticks in [1, 4096]. */
+int ewk_tick_ready(ewk_ctx* ctx, int max_ticks, int32_t* taken, uint8_t* silent, uint8_t* state, double* thr, double* rms);
 /* rate latched by the stream's first push (0: none yet; 16000: ewk_push / ewk_push_g711) and input samples received */
 int ewk_stream_input(ewk_ctx* ctx, int stream, int32_t* sr_in, int64_t* n_in);
 /* Stream recycling (a call ends, the slot takes the next one) without rebuilding the bank: return streams[0..n) to the
