@@ -62,6 +62,8 @@ def load():
         "ewk_resample_info": (C.c_int, [i32, _p(C.c_int32), _p(C.c_int32), _p(C.c_int32)]),
         "ewk_resample_out_len": (i64, [i64, i32]),
         "ewk_resample": (C.c_int, [vp, vp, i32, i32, i32, i64, i64, i32, i64, i64, i64, vp, i64, i32]),
+        "ewk_dense_plan": (C.c_int, [_p(i64), i32, _p(C.c_int32)]),
+        "ewk_dense_last_plan": (C.c_int, [vp, _p(C.c_int32)]),
     }
     for name, (res, args) in protos.items():
         fn = getattr(lib, name)
@@ -90,6 +92,18 @@ def host_table(which):
     out = np.empty(n, dtype=np.float32)
     lib.ewk_host_table(which, f32ptr(out), n)
     return out
+
+
+def dense_plan(lens):
+    """(DH, threads, CTAs per SM, shared-memory bytes) that ewk_dense_scores launches for templates of these lengths
+    (samples).  Host code: needs no GPU."""
+    lib = load()
+    a = np.ascontiguousarray(lens, dtype=np.int64)
+    out = (C.c_int32 * 4)()
+    if lib.ewk_dense_plan(i64ptr(a), len(a), out) != EWK_OK:
+        raise ValueError(f"no dense plan for template lengths {a.tolist()} (1..8 templates of 640..48000 samples that fit "
+                         "shared memory)")
+    return tuple(int(v) for v in out)
 
 
 def check(lib, ctx, rc):
@@ -594,6 +608,12 @@ def _bank_methods():
                                            out.ctypes.data, HOST))
         return out
 
+    def dense_last_plan(self):
+        """(DH, threads, CTAs per SM, shared-memory bytes) of the latest dense_scores launch (zeros before the first)."""
+        out = (C.c_int32 * 4)()
+        self._ck(self.lib.ewk_dense_last_plan(self.h, out))
+        return tuple(int(v) for v in out)
+
     def prepare_segments(self, streams, starts, lens):
         """Level-3 pre-processing (wakeword.py:1020-1025) of many ring segments at once -> list of float32 arrays."""
         st = np.ascontiguousarray(streams, dtype=np.int32)
@@ -675,7 +695,7 @@ def _bank_methods():
                  "resample_push"]
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
-    for f in (prepare_segments, dense_scores, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
+    for f in (prepare_segments, dense_scores, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
               push_resampled_each, push_streams, tick_ready, reset_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
               set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count):
         setattr(Context, f.__name__, f)

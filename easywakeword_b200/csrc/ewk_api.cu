@@ -1755,6 +1755,56 @@ static bool dense_plan(const DenseArgs& A0, int n_min, int n_max, int n_re_u, De
     return false;
 }
 
+// Everything of a K4 call that follows from the template lengths alone (each in [DENSE_MIN_L, DENSE_MAX_L]): window
+// geometry per template, the right-edge frames templates share, and the launch geometry.  ewk_dense_plan reports what
+// ewk_dense_scores launches because both go through here.  False: the set does not fit shared memory.
+static bool dense_setup(const int64_t* lens, int n, DenseArgs& A, DensePlan& plan) {
+    A.T = n;
+    int max_n = 0, min_n = 1 << 30, g_back = 1 << 30, n_re_u = 0;
+    for (int k = 0; k < n; k++) {
+        const int L = (int)lens[k];
+        DenseTmplDev& t = A.t[k];
+        t.L = L; t.n = (L + HOP - 1) / HOP; t.F = 1 + L / HOP; t.t_hi = (L - N_FFT / 2) / HOP; t.r = t.F - 1 - t.t_hi;
+        t.inv_f = 1.0 / (double)t.F;
+        max_n = std::max(max_n, t.n); min_n = std::min(min_n, t.n);
+        g_back = std::min(g_back, t.n - t.t_hi);
+        // right-edge frame e: stream-grid frame (hop - goff) cut at sample 160 hop - delta.  Templates with the same
+        // (goff, delta) share it; the group is computed through the window of its shortest member
+        const int delta = HOP * t.n - L;
+        for (int e = 0; e < t.r; e++) {
+            const int goff = t.n - (t.t_hi + 1 + e);
+            int u = 0;
+            while (u < n_re_u && !(A.re_goff[u] == goff && A.re_delta[u] == delta)) u++;
+            if (u == n_re_u) {
+                A.re_goff[u] = goff; A.re_delta[u] = delta; A.re_rep[u] = k; A.re_rep_e[u] = e; A.re_nfirst[u] = t.n;
+                n_re_u++;
+            } else if (t.n < A.re_nfirst[u]) { A.re_rep[u] = k; A.re_rep_e[u] = e; A.re_nfirst[u] = t.n; }
+            t.re_u[e] = u;
+        }
+    }
+    if (!dense_plan(A, min_n, max_n, n_re_u, plan)) return false;
+    A.DH = plan.DH; A.DG = plan.DH + max_n + 2; A.DLE = plan.DH + max_n - min_n; A.n_re_u = n_re_u;
+    A.n_min = min_n; A.n_max = max_n; A.g_back = g_back;
+    return true;
+}
+
+extern "C" int ewk_dense_plan(const int64_t* template_lens, int n, int32_t out[4]) {
+    if (!template_lens || !out || n < 1 || n > DENSE_MAX_T) return EWK_ERR_ARG;
+    for (int k = 0; k < n; k++)
+        if (template_lens[k] < DENSE_MIN_L || template_lens[k] > DENSE_MAX_L) return EWK_ERR_ARG;
+    DenseArgs A{};
+    DensePlan plan;
+    if (!dense_setup(template_lens, n, A, plan)) return EWK_ERR_ARG;
+    out[0] = plan.DH; out[1] = plan.threads; out[2] = plan.per_sm; out[3] = (int32_t)plan.smem;
+    return EWK_OK;
+}
+
+extern "C" int ewk_dense_last_plan(const ewk_ctx* ctx, int32_t out[4]) {
+    if (!ctx || !out) return EWK_ERR_ARG;
+    for (int i = 0; i < 4; i++) out[i] = ctx->dense_plan_info[i];
+    return EWK_OK;
+}
+
 extern "C" int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int tmpl_first, int tmpl_count, float* out, int where) {
     if (!ctx) return EWK_ERR_ARG;
     int rc = need_streams(ctx, "ewk_dense_scores");
@@ -1776,46 +1826,28 @@ extern "C" int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int tmpl
                   n_hops, tmpl_first, tmpl_first + tmpl_count, DENSE_MAX_T);
         return EWK_ERR_ARG;
     }
-    DenseArgs A{};
-    A.hop0 = hop0; A.n_hops = n_hops; A.T = tmpl_count;
-    int max_n = 0, min_n = 1 << 30, g_back = 1 << 30, n_re_u = 0;
+    int64_t lens[DENSE_MAX_T];
     for (int k = 0; k < tmpl_count; k++) {
         const TemplateFeat& tf = ctx->h_tmpl[tmpl_first + k];
         if (!tf.valid) { ctx->fail("No reference word set. Call set_reference() first."); return EWK_ERR_NO_TEMPLATE; }
-        const int L = (int)tf.n_samples;
         if (tf.n_samples < DENSE_MIN_L || tf.n_samples > DENSE_MAX_L) {
             ctx->fail("ewk_dense_scores: template %d has %lld samples; dense scoring needs %d..%d", tmpl_first + k,
                       (long long)tf.n_samples, DENSE_MIN_L, DENSE_MAX_L);
             return EWK_ERR_ARG;
         }
-        DenseTmplDev& t = A.t[k];
-        t.L = L; t.n = (L + HOP - 1) / HOP; t.F = 1 + L / HOP; t.t_hi = (L - N_FFT / 2) / HOP; t.r = t.F - 1 - t.t_hi;
-        t.slot = tmpl_first + k;
-        t.inv_f = 1.0 / (double)t.F;
-        max_n = std::max(max_n, t.n); min_n = std::min(min_n, t.n);
-        g_back = std::min(g_back, t.n - t.t_hi);
-        // right-edge frame e: stream-grid frame (hop - goff) cut at sample 160 hop - delta.  Templates with the same
-        // (goff, delta) share it; the group is computed through the window of its shortest member
-        const int delta = HOP * t.n - L;
-        for (int e = 0; e < t.r; e++) {
-            const int goff = t.n - (t.t_hi + 1 + e);
-            int u = 0;
-            while (u < n_re_u && !(A.re_goff[u] == goff && A.re_delta[u] == delta)) u++;
-            if (u == n_re_u) {
-                A.re_goff[u] = goff; A.re_delta[u] = delta; A.re_rep[u] = k; A.re_rep_e[u] = e; A.re_nfirst[u] = t.n;
-                n_re_u++;
-            } else if (t.n < A.re_nfirst[u]) { A.re_rep[u] = k; A.re_rep_e[u] = e; A.re_nfirst[u] = t.n; }
-            t.re_u[e] = u;
-        }
+        lens[k] = tf.n_samples;
     }
+    DenseArgs A{};
     DensePlan plan;
-    if (!dense_plan(A, min_n, max_n, n_re_u, plan)) {
+    if (!dense_setup(lens, tmpl_count, A, plan)) {
         ctx->fail("ewk_dense_scores: this template set does not fit shared memory (%d templates, windows of %d..%d hops)",
-                  tmpl_count, min_n, max_n);
+                  tmpl_count, (int)((*std::min_element(lens, lens + tmpl_count) + HOP - 1) / HOP),
+                  (int)((*std::max_element(lens, lens + tmpl_count) + HOP - 1) / HOP));
         return EWK_ERR_ARG;
     }
-    A.DH = plan.DH; A.DG = plan.DH + max_n + 2; A.DLE = plan.DH + max_n - min_n; A.n_re_u = n_re_u;
-    A.n_min = min_n; A.n_max = max_n; A.g_back = g_back;
+    A.hop0 = hop0; A.n_hops = n_hops;
+    for (int k = 0; k < tmpl_count; k++) A.t[k].slot = tmpl_first + k;
+    const int max_n = A.n_max;
     if ((long long)B.P < 160LL * (max_n + plan.DH + 4) + N_FFT) {        // the kernel wraps ring positions once
         ctx->fail("ewk_dense_scores: ring of %d samples is too short for a template of %d hops", B.P, max_n);
         return EWK_ERR_ARG;

@@ -102,7 +102,7 @@ struct ewk_ctx {
     ewk::BankView bank{};
     void* own_results = nullptr;
     ewk::DevBuf b_trace, b_read, b_dense, b_keep_rows, b_keep_end, b_g2;
-    int dense_plan_info[4] = {0, 0, 0, 0};  // K4 geometry of the latest ewk_dense_scores: hops per sub-chunk, threads, CTAs per SM, smem bytes
+    int dense_plan_info[4] = {0, 0, 0, 0};  // K4 geometry of the latest ewk_dense_scores: hops per sub-chunk, threads, CTAs per SM, smem bytes (ewk_dense_last_plan)
     int chunk_cap = 0;
     bool all_presummed = false;            // K1's block sums cover every sample pushed since the last tick
     int pushes_since_tick = 0;

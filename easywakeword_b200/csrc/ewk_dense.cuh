@@ -108,12 +108,16 @@ __device__ __forceinline__ int quant16(float x) {           // rint(x * 2^16) of
     return __float2int_rn(x * 65536.0f);
 }
 
-// (S1, S2) over F frames -> mean, std (ddof 0) as float32; the same function serves windows and templates
-__device__ __forceinline__ void dense_stats(long long S1, long long S2, double invf, float& mean, float& sd) {
+// (S1, S2) over F frames -> mean, std (ddof 0) as float32; the same function serves windows and templates.
+// Rows that are all equal (digital silence, a constant signal) have variance exactly 0, but once S2 passes 2^53 the
+// double formula leaves a rounding residue there: such a window would get a std, and a score, where the reference's
+// std is 0 and its cosine 0 / 0 = NaN.  F S2 == S1^2 (exact in 128 bits) detects them.
+__device__ __forceinline__ void dense_stats(long long S1, long long S2, int F, double invf, float& mean, float& sd) {
     const double s1 = (double)S1, s2 = (double)S2;
     mean = (float)(s1 * invf * (1.0 / 65536.0));
     const double var = (s2 - s1 * s1 * invf) * invf * (1.0 / 4294967296.0);
-    sd = sqrtf(fmaxf((float)var, 0.f));
+    const bool flat = (__int128)S1 * S1 == (__int128)F * S2;
+    sd = flat ? 0.f : sqrtf(fmaxf((float)var, 0.f));
 }
 
 // Template features for this kernel: the integer statistics of the template's own MFCC frames (K3's frames_out).
@@ -127,7 +131,7 @@ __global__ void dense_template_features_kernel(const float* __restrict__ frames,
             S2 += (long long)q * q;
         }
     float mean, sd;
-    dense_stats(S1, S2, 1.0 / (double)F, mean, sd);
+    dense_stats(S1, S2, F, 1.0 / (double)F, mean, sd);
     if (lane < N_MFCC) {
         out40[lane] = lane < n_mfcc ? mean : 0.f;
         out40[N_MFCC + lane] = lane < n_mfcc ? sd : 0.f;
@@ -323,7 +327,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
                 v = quant16(RE[(tp.re_u[e] * DH + hl) * ROW + c]);
                 S1 += v; S2 += (long long)v * v;
             }
-            dense_stats(S1, S2, tp.inv_f, mean_o, sd_o);
+            dense_stats(S1, S2, tp.F, tp.inv_f, mean_o, sd_o);
         }
     };
 
@@ -607,7 +611,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
                 }
                 // the same exact sums as a way window's, so the same (mean, std) bits: phase E scores both alike
                 float mean, sd;
-                dense_stats(S1, S2, tp.inv_f, mean, sd);
+                dense_stats(S1, S2, tp.F, tp.inv_f, mean, sd);
                 if (lane < n_mfcc) MS[((size_t)k * N_MFCC + lane) * DH + hl] = make_float2(mean, sd);
                 if (lane == 0) WAY[k * DH + hl] = DENSE_WAYS;
             }

@@ -311,6 +311,13 @@ int ewk_reset_streams(ewk_ctx* ctx, const int32_t* streams, int n);
  * `where` tells whether `out` is host or device memory. */
 int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int template_first, int template_count,
                      float* out, int where);
+/* Launch geometry ewk_dense_scores chooses for templates of these lengths (samples, n <= 8, each 640..48000):
+ * out = {hops per sub-chunk (32 or 64), threads per CTA, CTAs per SM, dynamic shared memory bytes}.  Host code only
+ * (no context, no device): the function ewk_dense_scores itself plans with.  EWK_ERR_ARG for lengths out of range or a
+ * set that does not fit shared memory. */
+int ewk_dense_plan(const int64_t* template_lens, int n, int32_t out[4]);
+/* The geometry (same layout) the context's latest ewk_dense_scores launched; zeros before the first call. */
+int ewk_dense_last_plan(const ewk_ctx* ctx, int32_t out[4]);
 /* Copy the dense per-stream results [n_streams] to host memory. */
 int ewk_stream_results(ewk_ctx* ctx, ewk_stream_result* out);
 /* Device pointer of that array (ewk_stream_result[n_streams]); or make the kernels write into a

@@ -29,3 +29,31 @@ def mfcc_rel_l2(a, b):
     num = np.linalg.norm(a - b, axis=0)
     den = np.linalg.norm(b, axis=0)
     return num / np.maximum(den, 1e-30)
+
+
+def dense_geometry_sets(plan_fn):
+    """Template-length sets (1-8 templates of 640 .. 48000 samples, remainders mod 160 on both sides of 96 so that
+    windows have 1 and 2 right-edge frames) through K4's planner -> {(DH, threads, CTAs per SM): lengths}, one set per
+    reachable geometry: the one with the fewest templates and samples, so that a device test of every geometry stays
+    cheap.  plan_fn(lengths) -> (DH, threads, CTAs per SM, shared-memory bytes)."""
+    grid = [640, 1001, 4097, 8000, 15503, 16000, 24013, 33406, 40111, 48000]
+    sets = set()
+    for T in range(1, 9):
+        for a in grid:
+            for b in grid:
+                if a <= b:
+                    sets.add(tuple(sorted([a] * (T - 1) + [b])))
+        for i in range(len(grid)):
+            sets.add(tuple(sorted((grid * 2)[i:i + T])))
+    rng = np.random.default_rng(160)
+    for _ in range(400):
+        T = int(rng.integers(1, 9))
+        sets.add(tuple(sorted(int(v) for v in rng.integers(640, 48001, T))))
+    reach = {}
+    for lens in sorted(sets, key=lambda s: (len(s), sum(s), s)):
+        try:
+            g = tuple(plan_fn(list(lens))[:3])
+        except ValueError:                       # does not fit shared memory: ewk_dense_scores refuses it too
+            continue
+        reach.setdefault(g, list(lens))
+    return reach
