@@ -324,6 +324,8 @@ def _declare_stream_protos(lib):
         "ewk_read_segment": (C.c_int, [vp, i32, i64, i64, f32p]),
         "ewk_stream_results": (C.c_int, [vp, vp]),
         "ewk_dense_scores": (C.c_int, [vp, i64, i32, i32, i32, vp, i32]),
+        "ewk_dense_scores_streams": (C.c_int, [vp, _p(C.c_int32), i32, _p(i64), _p(C.c_int32), i32, i32, vp, i64, i32]),
+        "ewk_dense_ready": (C.c_int, [vp, _p(C.c_int32), i32, i32, i32, i32, _p(i64), _p(C.c_int32), vp, i64, i32]),
         "ewk_prepare_segments": (C.c_int, [vp, i32, _p(C.c_int32), _p(i64), _p(i64), _p(i64), f32p, i64, i32]),
         "ewk_results_device_ptr": (C.c_int, [vp, _p(vp)]),
         "ewk_set_results_buffer": (C.c_int, [vp, vp]),
@@ -424,6 +426,20 @@ def _resampled_input(pcm_or_codes, fmt):
     else:
         raise TypeError(f"push_resampled takes float32, int16 or uint8 G.711 input, got {dt}")
     return ptr, ns, n, stride, code, a
+
+
+def _stream_list(streams):
+    """int32 array of stream indices (ValueError for values no int32 holds: the library names the others)."""
+    st = np.asarray(streams, dtype=np.int64).reshape(-1)
+    if st.size and (st.min() < -2**31 or st.max() >= 2**31):
+        raise ValueError("stream index out of range")
+    return np.ascontiguousarray(st, dtype=np.int32)
+
+
+def _unpack_rows(out, n_hops, T):
+    """Packed [sum n_i][T] scores -> list of [n_i, T] views, in list order."""
+    ends = np.cumsum(n_hops, dtype=np.int64)
+    return [out[(e - n) * T:e * T].reshape(n, T) for e, n in zip(ends.tolist(), [int(v) for v in n_hops])]
 
 
 def _bank_methods():
@@ -608,8 +624,57 @@ def _bank_methods():
                                            out.ctypes.data, HOST))
         return out
 
+    def dense_scores_streams(self, streams, hop0, n_hops, template_first=0, template_count=1, out_device_ptr=None,
+                             out_cap=None):
+        """Ragged dense scoring (include/ewk.h: ewk_dense_scores_streams): row i scores stream streams[i] at hops
+        [hop0[i], hop0[i] + n_hops[i]) (0 included).  Returns a list of float32 [n_hops[i], template_count] arrays; with
+        out_device_ptr the rows go there packed back to back in list order (out_cap floats, default exactly what they
+        need) and None is returned."""
+        st = _stream_list(streams)
+        h0 = np.ascontiguousarray(np.asarray(hop0, dtype=np.int64).reshape(-1))
+        nh64 = np.asarray(n_hops, dtype=np.int64).reshape(-1)
+        if len(h0) != len(st) or len(nh64) != len(st):
+            raise ValueError("one hop0 and one n_hops per stream")
+        if nh64.size and (nh64.min() < -2**31 or nh64.max() >= 2**31):
+            raise ValueError("n_hops out of range")
+        nh = np.ascontiguousarray(nh64, dtype=np.int32)
+        T = int(template_count)
+        need = max(0, int(nh64[nh64 > 0].sum()) * T)
+        args = (st.ctypes.data_as(_p(C.c_int32)), len(st), i64ptr(h0), nh.ctypes.data_as(_p(C.c_int32)), template_first, T)
+        if out_device_ptr is not None:
+            self._ck(self.lib.ewk_dense_scores_streams(self.h, *args, C.c_void_p(out_device_ptr),
+                                                       need if out_cap is None else int(out_cap), DEVICE))
+            return None
+        out = np.empty(need, np.float32)
+        self._ck(self.lib.ewk_dense_scores_streams(self.h, *args, out.ctypes.data if need else None,
+                                                   need if out_cap is None else int(out_cap), HOST))
+        return _unpack_rows(out, nh64, T)
+
+    def dense_ready(self, streams=None, max_hops=100, template_first=0, template_count=1, out_device_ptr=None,
+                    out_cap=None):
+        """Dense scores paced by each stream's own audio (include/ewk.h: ewk_dense_ready): each listed stream (None: every
+        stream) is scored from its cursor at every hop its landed audio completes, at most max_hops, and its cursor moves
+        on.  Returns (hop0, scores): int64 [n] first hops and a list of float32 [n_i, template_count] arrays.  With
+        out_device_ptr (out_cap floats, default n * max_hops * template_count) the rows go there packed in list order and
+        (hop0, n_hops) is returned."""
+        st = None if streams is None else _stream_list(streams)
+        n = self.cfg.n_streams if st is None else len(st)
+        T = int(template_count)
+        h0 = np.zeros(n, np.int64)
+        nh = np.zeros(n, np.int32)
+        cap = n * int(max_hops) * T if out_cap is None else int(out_cap)
+        args = (None if st is None else st.ctypes.data_as(_p(C.c_int32)), n, int(max_hops), template_first, T, i64ptr(h0),
+                nh.ctypes.data_as(_p(C.c_int32)))
+        if out_device_ptr is not None:
+            self._ck(self.lib.ewk_dense_ready(self.h, *args, C.c_void_p(out_device_ptr), cap, DEVICE))
+            return h0, nh
+        out = np.empty(max(0, cap), np.float32)
+        self._ck(self.lib.ewk_dense_ready(self.h, *args, out.ctypes.data if out.size else None, cap, HOST))
+        return h0, _unpack_rows(out, nh, T)
+
     def dense_last_plan(self):
-        """(DH, threads, CTAs per SM, shared-memory bytes) of the latest dense_scores launch (zeros before the first)."""
+        """(DH, threads, CTAs per SM, shared-memory bytes) of the latest K4 launch (dense_scores, dense_scores_streams or
+        dense_ready; zeros before the first)."""
         out = (C.c_int32 * 4)()
         self._ck(self.lib.ewk_dense_last_plan(self.h, out))
         return tuple(int(v) for v in out)
@@ -695,7 +760,7 @@ def _bank_methods():
                  "resample_push"]
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
-    for f in (prepare_segments, dense_scores, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
+    for f in (prepare_segments, dense_scores, dense_scores_streams, dense_ready, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
               push_resampled_each, push_streams, tick_ready, reset_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
               set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count):
         setattr(Context, f.__name__, f)

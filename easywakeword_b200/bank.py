@@ -18,6 +18,7 @@ from . import _lib
 from .wakeword import WakeWord, load_wav_16k
 
 TICK_SAMPLES = 1600
+DENSE_ROUND = 500                 # hops per ewk_dense_ready call of WakeWordBank.dense_ready (5 s of audio)
 EV_TIMEOUT, EV_SCORED = _lib.EV_TIMEOUT, _lib.EV_SCORED
 
 
@@ -187,6 +188,23 @@ class WakeWordBank:
         pushed): calculate_similarity of the latest template-length window complete at each hop (K4)."""
         T = len(self.templates) - template_first if template_count is None else template_count
         return self.ctx.dense_scores(hop0, n_hops, template_first, T)
+
+    def dense_ready(self, streams=None, template_first: int = 0, template_count: Optional[int] = None):
+        """Per-hop scores paced by each stream's own audio (include/ewk.h: ewk_dense_ready): every hop of the listed
+        streams (None: all) that their landed audio completes and no earlier call scored, in rounds of DENSE_ROUND hops,
+        so that no due hop is left when it returns.  Returns (hop0, scores): int64 first hop of each listed stream's
+        scores and a list of float32 [n_i, T] arrays.  A stream recycled with reset() starts again at hop 1."""
+        T = len(self.templates) - template_first if template_count is None else template_count
+        hop0, parts = None, None
+        while True:
+            h0, rows = self.ctx.dense_ready(streams, DENSE_ROUND, template_first, T)
+            if hop0 is None:
+                hop0, parts = h0, [[r] for r in rows]
+            else:
+                for p, r in zip(parts, rows):
+                    p.append(r)
+            if not rows or max(len(r) for r in rows) < DENSE_ROUND:
+                return hop0, [p[0] if len(p) == 1 else np.concatenate(p) for p in parts]
 
     def read_segment(self, event) -> np.ndarray:
         """word_audio of a level-2 event as float32 (what level 3 transcribes)."""

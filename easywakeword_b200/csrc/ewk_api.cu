@@ -205,6 +205,10 @@ void ewk_ctx::release() {
         if (h_pos[i]) cudaFreeHost(h_pos[i]);
         ev_pos[i] = nullptr; h_pos[i] = nullptr;
         b_pos[i].free();
+        if (ev_drow[i]) cudaEventDestroy(ev_drow[i]);
+        if (h_drow[i]) cudaFreeHost(h_drow[i]);
+        ev_drow[i] = nullptr; h_drow[i] = nullptr;
+        b_drow[i].free();
     }
     b_reset.free();
     if (own_stream) cudaStreamDestroy(own_stream);
@@ -619,6 +623,7 @@ int ewk_ctx::init_streams() {
     h_written.assign(n, 0);
     h_visible_lb.assign(n, 0);
     h_tick.assign(n, 0);
+    h_dense_next.assign(n, 1);
     h_frame_size.assign(n, 0);
     h_rate.assign(n, 0);
     h_inputs.assign(n, 0);
@@ -1059,21 +1064,28 @@ int ewk_ctx::land_resampled(int stream0, int n_streams, const void* d_src, long 
     return EWK_OK;
 }
 
-int ewk_ctx::upload_rows(const std::vector<RowDesc>& rows, cudaStream_t on, int* slot) {
-    ewk_ctx* ctx = this;
-    const int k = pos_idx;
-    pos_idx ^= 1;
-    const size_t bytes = sizeof(RowDesc) * (size_t)bank.n_streams;
-    if (!h_pos[k]) {
-        CK(cudaHostAlloc((void**)&h_pos[k], bytes, cudaHostAllocDefault));
-        CK(cudaEventCreateWithFlags(&ev_pos[k], cudaEventDisableTiming));
+// descriptors (at most one per stream) -> the next of two pinned + device slots, copied on stream `on`; a slot is reused
+// only once the kernel that read its previous contents has run (ev[k]).  *slot receives its index.
+template <class D>
+static int upload_slot(ewk_ctx* ctx, D* (&h)[2], DevBuf (&b)[2], cudaEvent_t (&ev)[2], const bool (&ev_valid)[2], int& idx,
+                       const std::vector<D>& rows, cudaStream_t on, int* slot) {
+    const int k = idx;
+    idx ^= 1;
+    const size_t bytes = sizeof(D) * (size_t)ctx->bank.n_streams;
+    if (!h[k]) {
+        CK(cudaHostAlloc((void**)&h[k], bytes, cudaHostAllocDefault));
+        CK(cudaEventCreateWithFlags(&ev[k], cudaEventDisableTiming));
     }
-    CK(b_pos[k].ensure(bytes));
-    if (ev_pos_valid[k]) CK(cudaEventSynchronize(ev_pos[k]));
-    std::memcpy(h_pos[k], rows.data(), sizeof(RowDesc) * rows.size());
-    CK(cudaMemcpyAsync(b_pos[k].p, h_pos[k], sizeof(RowDesc) * rows.size(), cudaMemcpyHostToDevice, on));
+    CK(b[k].ensure(bytes));
+    if (ev_valid[k]) CK(cudaEventSynchronize(ev[k]));
+    std::memcpy(h[k], rows.data(), sizeof(D) * rows.size());
+    CK(cudaMemcpyAsync(b[k].p, h[k], sizeof(D) * rows.size(), cudaMemcpyHostToDevice, on));
     *slot = k;
     return EWK_OK;
+}
+
+int ewk_ctx::upload_rows(const std::vector<RowDesc>& rows, cudaStream_t on, int* slot) {
+    return upload_slot(this, h_pos, b_pos, ev_pos, ev_pos_valid, pos_idx, rows, on, slot);
 }
 
 // tails for the widest filter in use; rows of streams already running move with their content
@@ -1420,7 +1432,7 @@ extern "C" int ewk_reset_streams(ewk_ctx* ctx, const int32_t* streams, int n) {
     ctx->launches++;
     for (int i = 0; i < n; i++) {
         const int s = streams[i];
-        ctx->h_written[s] = 0; ctx->h_visible_lb[s] = 0; ctx->h_tick[s] = 0;
+        ctx->h_written[s] = 0; ctx->h_visible_lb[s] = 0; ctx->h_tick[s] = 0; ctx->h_dense_next[s] = 1;
         ctx->h_frame_size[s] = 0; ctx->h_rate[s] = 0; ctx->h_inputs[s] = 0;
     }
     return EWK_OK;
@@ -1805,6 +1817,82 @@ extern "C" int ewk_dense_last_plan(const ewk_ctx* ctx, int32_t out[4]) {
     return EWK_OK;
 }
 
+// What every K4 entry point checks and plans from its template range alone (errors name `who`): the templates, the
+// window geometry (dense_setup), the ring length.
+static int dense_prepare(ewk_ctx* ctx, const char* who, int tmpl_first, int tmpl_count, DenseArgs& A, DensePlan& plan) {
+    if (tmpl_count < 1 || tmpl_count > DENSE_MAX_T || tmpl_first < 0 || tmpl_first + tmpl_count > ctx->cfg.max_templates) {
+        ctx->fail("%s: bad template range [%d, %d) (at most %d per call, %d slots)", who, tmpl_first, tmpl_first + tmpl_count,
+                  DENSE_MAX_T, ctx->cfg.max_templates);
+        return EWK_ERR_ARG;
+    }
+    int64_t lens[DENSE_MAX_T];
+    for (int k = 0; k < tmpl_count; k++) {
+        const TemplateFeat& tf = ctx->h_tmpl[tmpl_first + k];
+        if (!tf.valid) { ctx->fail("No reference word set. Call set_reference() first."); return EWK_ERR_NO_TEMPLATE; }
+        if (tf.n_samples < DENSE_MIN_L || tf.n_samples > DENSE_MAX_L) {
+            ctx->fail("%s: template %d has %lld samples; dense scoring needs %d..%d", who, tmpl_first + k,
+                      (long long)tf.n_samples, DENSE_MIN_L, DENSE_MAX_L);
+            return EWK_ERR_ARG;
+        }
+        lens[k] = tf.n_samples;
+    }
+    if (!dense_setup(lens, tmpl_count, A, plan)) {
+        ctx->fail("%s: this template set does not fit shared memory (%d templates, windows of %d..%d hops)", who,
+                  tmpl_count, (int)((*std::min_element(lens, lens + tmpl_count) + HOP - 1) / HOP),
+                  (int)((*std::max_element(lens, lens + tmpl_count) + HOP - 1) / HOP));
+        return EWK_ERR_ARG;
+    }
+    for (int k = 0; k < tmpl_count; k++) A.t[k].slot = tmpl_first + k;
+    if ((long long)ctx->bank.P < 160LL * (A.n_max + plan.DH + 4) + N_FFT) {        // the kernel wraps ring positions once
+        ctx->fail("%s: ring of %d samples is too short for a template of %d hops", who, ctx->bank.P, A.n_max);
+        return EWK_ERR_ARG;
+    }
+    return EWK_OK;
+}
+
+// the audio of every window of stream s at hops [hop0, hop0 + n_hops) (n_hops >= 1) must be resident
+static int dense_resident(ewk_ctx* ctx, const char* who, int s, long long hop0, long long n_hops, int max_n) {
+    const long long need_hi = 160LL * (hop0 + n_hops - 1);
+    const long long need_lo = std::max<long long>(0, 160LL * (hop0 - max_n) - N_FFT / 2);
+    if (ctx->h_written[s] < need_hi) {
+        ctx->fail("%s: stream %d has %lld samples, hop %lld needs %lld", who, s, ctx->h_written[s], hop0 + n_hops - 1, need_hi);
+        return EWK_ERR_STATE;
+    }
+    if (ctx->h_written[s] - need_lo > ctx->bank.P) {
+        ctx->fail("%s: stream %d no longer holds sample %lld (ring of %d)", who, s, need_lo, ctx->bank.P);
+        return EWK_ERR_STATE;
+    }
+    return EWK_OK;
+}
+
+// K4 over n_ctas CTAs into d_out: the uniform instance, or the per-row one when A.rows is set
+static int dense_launch(ewk_ctx* ctx, DenseArgs& A, const DensePlan& plan, float* d_out, int n_ctas) {
+    BankView& B = ctx->bank;
+    A.out = d_out;
+    if (!ctx->b_keep_rows.p) {
+        CK(ctx->b_keep_rows.ensure(sizeof(float) * (size_t)B.n_streams * DENSE_KEEP * ROW));
+        CK(ctx->b_keep_end.ensure(sizeof(long long) * 2 * (size_t)B.n_streams));
+        CK(cudaMemsetAsync(ctx->b_keep_end.p, 0, sizeof(long long) * 2 * (size_t)B.n_streams, ctx->stream));
+    }
+    CK(ctx->b_g2.ensure(sizeof(float) * (size_t)B.n_streams * DENSE_WAYS * A.DG * N_MFCC));
+    A.keep_rows = (float*)ctx->b_keep_rows.p;
+    A.keep_end = (long long*)ctx->b_keep_end.p;
+    A.g2 = (float*)ctx->b_g2.p;
+    const bool pre = ctx->cfg.preemphasis != 0.f;
+    auto k4 = A.rows ? (pre ? dense_score_kernel<true, true> : dense_score_kernel<false, true>)
+                     : (pre ? dense_score_kernel<true, false> : dense_score_kernel<false, false>);
+    CK(cudaFuncSetAttribute(k4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem));
+    CK(cudaFuncSetAttribute(k4, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+    cudaEvent_t pe = ctx->prof_begin(4);
+    k4<<<n_ctas, plan.threads, plan.smem, ctx->stream>>>(ctx->d_tables, B, ctx->d_tmpl, A);
+    ctx->prof_end(pe, 4);
+    CK(cudaGetLastError());
+    ctx->launches++;
+    ctx->dense_plan_info[0] = plan.DH; ctx->dense_plan_info[1] = plan.threads; ctx->dense_plan_info[2] = plan.per_sm;
+    ctx->dense_plan_info[3] = (int)plan.smem;
+    return EWK_OK;
+}
+
 extern "C" int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int tmpl_first, int tmpl_count, float* out, int where) {
     if (!ctx) return EWK_ERR_ARG;
     int rc = need_streams(ctx, "ewk_dense_scores");
@@ -1826,73 +1914,153 @@ extern "C" int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int tmpl
                   n_hops, tmpl_first, tmpl_first + tmpl_count, DENSE_MAX_T);
         return EWK_ERR_ARG;
     }
-    int64_t lens[DENSE_MAX_T];
-    for (int k = 0; k < tmpl_count; k++) {
-        const TemplateFeat& tf = ctx->h_tmpl[tmpl_first + k];
-        if (!tf.valid) { ctx->fail("No reference word set. Call set_reference() first."); return EWK_ERR_NO_TEMPLATE; }
-        if (tf.n_samples < DENSE_MIN_L || tf.n_samples > DENSE_MAX_L) {
-            ctx->fail("ewk_dense_scores: template %d has %lld samples; dense scoring needs %d..%d", tmpl_first + k,
-                      (long long)tf.n_samples, DENSE_MIN_L, DENSE_MAX_L);
-            return EWK_ERR_ARG;
-        }
-        lens[k] = tf.n_samples;
-    }
     DenseArgs A{};
     DensePlan plan;
-    if (!dense_setup(lens, tmpl_count, A, plan)) {
-        ctx->fail("ewk_dense_scores: this template set does not fit shared memory (%d templates, windows of %d..%d hops)",
-                  tmpl_count, (int)((*std::min_element(lens, lens + tmpl_count) + HOP - 1) / HOP),
-                  (int)((*std::max_element(lens, lens + tmpl_count) + HOP - 1) / HOP));
-        return EWK_ERR_ARG;
-    }
+    rc = dense_prepare(ctx, "ewk_dense_scores", tmpl_first, tmpl_count, A, plan);
+    if (rc) return rc;
     A.hop0 = hop0; A.n_hops = n_hops;
-    for (int k = 0; k < tmpl_count; k++) A.t[k].slot = tmpl_first + k;
-    const int max_n = A.n_max;
-    if ((long long)B.P < 160LL * (max_n + plan.DH + 4) + N_FFT) {        // the kernel wraps ring positions once
-        ctx->fail("ewk_dense_scores: ring of %d samples is too short for a template of %d hops", B.P, max_n);
-        return EWK_ERR_ARG;
-    }
-    // the audio of every requested window must be resident
-    const long long need_hi = 160LL * (hop0 + n_hops - 1);
-    const long long need_lo = std::max<long long>(0, 160LL * (hop0 - max_n) - N_FFT / 2);
     for (int s = 0; s < B.n_streams; s++) {
-        if (ctx->h_written[s] < need_hi) {
-            ctx->fail("ewk_dense_scores: stream %d has %lld samples, hop %lld needs %lld", s, ctx->h_written[s],
-                      (long long)(hop0 + n_hops - 1), need_hi);
-            return EWK_ERR_STATE;
-        }
-        if (ctx->h_written[s] - need_lo > B.P) {
-            ctx->fail("ewk_dense_scores: stream %d no longer holds sample %lld (ring of %d)", s, need_lo, B.P);
-            return EWK_ERR_STATE;
-        }
+        rc = dense_resident(ctx, "ewk_dense_scores", s, hop0, n_hops, A.n_max);
+        if (rc) return rc;
     }
     CK(cudaSetDevice(ctx->device));
     const size_t n_out = (size_t)B.n_streams * n_hops * tmpl_count;
     float* d_out = out;
     if (where == EWK_HOST) { CK(ctx->b_dense.ensure(sizeof(float) * n_out)); d_out = (float*)ctx->b_dense.p; }
-    A.out = d_out;
-    if (!ctx->b_keep_rows.p) {
-        CK(ctx->b_keep_rows.ensure(sizeof(float) * (size_t)B.n_streams * DENSE_KEEP * ROW));
-        CK(ctx->b_keep_end.ensure(sizeof(long long) * 2 * (size_t)B.n_streams));
-        CK(cudaMemsetAsync(ctx->b_keep_end.p, 0, sizeof(long long) * 2 * (size_t)B.n_streams, ctx->stream));
-    }
-    CK(ctx->b_g2.ensure(sizeof(float) * (size_t)B.n_streams * DENSE_WAYS * A.DG * N_MFCC));
-    A.keep_rows = (float*)ctx->b_keep_rows.p;
-    A.keep_end = (long long*)ctx->b_keep_end.p;
-    A.g2 = (float*)ctx->b_g2.p;
-    auto k4 = ctx->cfg.preemphasis != 0.f ? dense_score_kernel<true> : dense_score_kernel<false>;
-    CK(cudaFuncSetAttribute(k4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem));
-    CK(cudaFuncSetAttribute(k4, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    cudaEvent_t pe = ctx->prof_begin(4);
-    k4<<<B.n_streams, plan.threads, plan.smem, ctx->stream>>>(ctx->d_tables, B, ctx->d_tmpl, A);
-    ctx->prof_end(pe, 4);
-    CK(cudaGetLastError());
-    ctx->launches++;
-    ctx->dense_plan_info[0] = plan.DH; ctx->dense_plan_info[1] = plan.threads; ctx->dense_plan_info[2] = plan.per_sm;
-    ctx->dense_plan_info[3] = (int)plan.smem;
+    rc = dense_launch(ctx, A, plan, d_out, B.n_streams);
+    if (rc) return rc;
     if (where == EWK_HOST) {
         CK(cudaMemcpyAsync(out, d_out, sizeof(float) * n_out, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
+    }
+    return EWK_OK;
+}
+
+// Rows of ewk_dense_scores_streams and ewk_dense_ready: row i scores stream streams[i] at hops [hop0[i], hop0[i] + n_hops[i]),
+// packed into out in list order.  Every check comes before the first launch or copy, so an error changes no state.
+static int dense_rows(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, const int64_t* hop0, const int32_t* n_hops,
+                      int tmpl_first, int tmpl_count, float* out, int64_t out_cap, int where) {
+    BankView& B = ctx->bank;
+    if (n < 0 || (n > 0 && (!streams || !hop0 || !n_hops))) { ctx->fail("%s: bad row list (n=%d)", who, n); return EWK_ERR_ARG; }
+    if (n == 0) return EWK_OK;
+    std::vector<int> row_of((size_t)B.n_streams, -1);
+    long long hops = 0;
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        if (s < 0 || s >= B.n_streams) { ctx->fail("%s: bad stream %d (context has %d)", who, s, B.n_streams); return EWK_ERR_ARG; }
+        if (row_of[s] >= 0) { ctx->fail("%s: stream %d is listed twice", who, s); return EWK_ERR_ARG; }
+        row_of[s] = i;
+        if (hop0[i] < 0 || n_hops[i] < 0 || hop0[i] > ((int64_t)1 << 48)) {
+            ctx->fail("%s: row %d of stream %d has bad hops (hop0=%lld n_hops=%d)", who, i, s, (long long)hop0[i], n_hops[i]);
+            return EWK_ERR_ARG;
+        }
+        hops += n_hops[i];
+    }
+    DenseArgs A{};
+    DensePlan plan;
+    int rc = dense_prepare(ctx, who, tmpl_first, tmpl_count, A, plan);
+    if (rc) return rc;
+    const long long n_out = hops * tmpl_count;
+    if (n_out > 0 && (!out || out_cap < n_out)) {
+        ctx->fail("%s: out holds %lld floats, the rows need %lld", who, out ? (long long)out_cap : 0LL, n_out);
+        return EWK_ERR_ARG;
+    }
+    CK(cudaSetDevice(ctx->device));
+    if (ctx->pending.valid) {
+        // as in ewk_dense_scores: the in-flight host push lands now only if a listed row reaches into its samples
+        bool need = false;
+        const std::vector<RowDesc>& prow = ctx->pending.rows;
+        for (int j = 0; !need && j < ctx->pending.n_streams; j++) {
+            const int s = prow.empty() ? ctx->pending.stream0 + j : prow[j].stream, i = row_of[s];
+            need = i >= 0 && n_hops[i] > 0 && ctx->h_written[s] < 160LL * (hop0[i] + n_hops[i] - 1);
+        }
+        if (need) { rc = ctx->flush_pending(); if (rc) return rc; }
+    }
+    for (int i = 0; i < n; i++) {
+        if (n_hops[i] == 0) continue;
+        rc = dense_resident(ctx, who, streams[i], hop0[i], n_hops[i], A.n_max);
+        if (rc) return rc;
+    }
+    if (n_out == 0) return EWK_OK;
+    // descriptors of the non-empty rows: outputs in list order, CTAs longest first so that a launch ends with short rows
+    // (EWK_DENSE_LONGEST_FIRST=0 keeps list order, to measure what the order buys)
+    const char* lf = getenv("EWK_DENSE_LONGEST_FIRST");
+    const bool longest_first = !lf || atoi(lf) != 0;
+    std::vector<DenseRow> rows;
+    long long off = 0;
+    for (int i = 0; i < n; i++) {
+        if (n_hops[i] > 0) rows.push_back(DenseRow{hop0[i], off, streams[i], n_hops[i]});
+        off += (long long)n_hops[i] * tmpl_count;
+    }
+    if (longest_first)
+        std::stable_sort(rows.begin(), rows.end(), [](const DenseRow& a, const DenseRow& b) { return a.n_hops > b.n_hops; });
+    int k = -1;
+    rc = upload_slot(ctx, ctx->h_drow, ctx->b_drow, ctx->ev_drow, ctx->ev_drow_valid, ctx->drow_idx, rows, ctx->stream, &k);
+    if (rc) return rc;
+    float* d_out = out;
+    if (where == EWK_HOST) { CK(ctx->b_dense.ensure(sizeof(float) * (size_t)n_out)); d_out = (float*)ctx->b_dense.p; }
+    A.rows = (const DenseRow*)ctx->b_drow[k].p;
+    rc = dense_launch(ctx, A, plan, d_out, (int)rows.size());
+    if (rc) return rc;
+    CK(cudaEventRecord(ctx->ev_drow[k], ctx->stream));        // the slot is free once this K4 has read it
+    ctx->ev_drow_valid[k] = true;
+    if (where == EWK_HOST) {
+        CK(cudaMemcpyAsync(out, d_out, sizeof(float) * (size_t)n_out, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    return EWK_OK;
+}
+
+extern "C" int ewk_dense_scores_streams(ewk_ctx* ctx, const int32_t* streams, int n, const int64_t* hop0, const int32_t* n_hops,
+                                        int template_first, int template_count, float* out, int64_t out_cap, int where) {
+    if (!ctx) return EWK_ERR_ARG;
+    int rc = need_streams(ctx, "ewk_dense_scores_streams");
+    if (rc) return rc;
+    return dense_rows(ctx, "ewk_dense_scores_streams", streams, n, hop0, n_hops, template_first, template_count, out, out_cap,
+                      where);
+}
+
+extern "C" int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first,
+                               int template_count, int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap,
+                               int where) {
+    if (!ctx) return EWK_ERR_ARG;
+    const char* who = "ewk_dense_ready";
+    int rc = need_streams(ctx, who);
+    if (rc) return rc;
+    BankView& B = ctx->bank;
+    if (max_hops < 1 || max_hops > (1 << 20)) { ctx->fail("%s: max_hops must be in [1, %d]", who, 1 << 20); return EWK_ERR_ARG; }
+    std::vector<int32_t> all;
+    if (!streams) {
+        all.resize((size_t)B.n_streams);
+        for (int s = 0; s < B.n_streams; s++) all[s] = s;
+        streams = all.data();
+        n = B.n_streams;
+    }
+    if (n < 0 || (n > 0 && (!hop0_out || !n_hops_out))) { ctx->fail("%s: bad stream list (n=%d)", who, n); return EWK_ERR_ARG; }
+    std::vector<char> seen((size_t)B.n_streams, 0);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        if (s < 0 || s >= B.n_streams) { ctx->fail("%s: bad stream %d (context has %d)", who, s, B.n_streams); return EWK_ERR_ARG; }
+        if (seen[s]) { ctx->fail("%s: stream %d is listed twice", who, s); return EWK_ERR_ARG; }
+        seen[s] = 1;
+    }
+    CK(cudaSetDevice(ctx->device));
+    rc = ctx->flush_pending();                               // the due hops depend on every landed sample
+    if (rc) return rc;
+    // due rule: hop h is due once 160 h samples have landed, from the cursor on, at most max_hops
+    std::vector<int64_t> h0((size_t)n);
+    std::vector<int32_t> nh((size_t)n);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        h0[i] = ctx->h_dense_next[s];
+        nh[i] = (int32_t)std::max<long long>(0, std::min<long long>(h0[i] + max_hops, ctx->h_written[s] / 160 + 1) - h0[i]);
+    }
+    rc = dense_rows(ctx, who, streams, n, h0.data(), nh.data(), template_first, template_count, out, out_cap, where);
+    if (rc) return rc;
+    for (int i = 0; i < n; i++) {
+        hop0_out[i] = h0[i];
+        n_hops_out[i] = nh[i];
+        ctx->h_dense_next[streams[i]] += nh[i];
     }
     return EWK_OK;
 }

@@ -86,6 +86,12 @@ struct ewk_ctx {
     cudaEvent_t ev_pos[2] = {nullptr, nullptr};
     bool ev_pos_valid[2] = {false, false};
     int pos_idx = 0;
+    // per-row descriptors of a ragged K4 call (ewk_dense_scores_streams, ewk_dense_ready): two slots of the same kind
+    ewk::DenseRow* h_drow[2] = {nullptr, nullptr};
+    ewk::DevBuf b_drow[2];
+    cudaEvent_t ev_drow[2] = {nullptr, nullptr};
+    bool ev_drow_valid[2] = {false, false};
+    int drow_idx = 0;
     ewk::DevBuf b_reset;                     // K9's stream list
     int flush_pending();
     ewk::DevBuf b_stage2[2];
@@ -102,7 +108,7 @@ struct ewk_ctx {
     ewk::BankView bank{};
     void* own_results = nullptr;
     ewk::DevBuf b_trace, b_read, b_dense, b_keep_rows, b_keep_end, b_g2;
-    int dense_plan_info[4] = {0, 0, 0, 0};  // K4 geometry of the latest ewk_dense_scores: hops per sub-chunk, threads, CTAs per SM, smem bytes (ewk_dense_last_plan)
+    int dense_plan_info[4] = {0, 0, 0, 0};  // K4 geometry of the latest K4 call: hops per sub-chunk, threads, CTAs per SM, smem bytes (ewk_dense_last_plan)
     int chunk_cap = 0;
     bool all_presummed = false;            // K1's block sums cover every sample pushed since the last tick
     int pushes_since_tick = 0;
@@ -112,6 +118,7 @@ struct ewk_ctx {
     std::vector<long long> h_written;      // host mirror of StreamState.written
     std::vector<long long> h_visible_lb;   // lower bound of StreamState.visible (audio-clock overrun check)
     std::vector<long long> h_tick;
+    std::vector<long long> h_dense_next;   // ewk_dense_ready's cursor: the next hop it scores (1 after create / reset)
     std::vector<int> h_frame_size;         // latched frame size per stream (0: no push yet)
     std::vector<int> h_rate;               // input rate latched by the stream's first push (0: none yet; 16000: ewk_push)
     std::vector<long long> h_inputs;       // input samples the stream received (at its own rate)

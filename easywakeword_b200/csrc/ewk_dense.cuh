@@ -74,8 +74,15 @@ struct DenseTmplDev {
     double inv_f;                      // 1 / F (IEEE double division: the same bits on host and device)
 };
 
+// One row of a ragged call (ewk_dense_scores_streams / ewk_dense_ready): CTA x scores stream `stream` at hops
+// [hop0, hop0 + n_hops) into out[out, out + n_hops T), laid out [n_hops][T]
+struct DenseRow {
+    long long hop0, out;
+    int stream, n_hops;
+};
+
 struct DenseArgs {
-    long long hop0;                    // first hop scored (hop h <-> 160 h samples of the stream)
+    long long hop0;                    // first hop scored (hop h <-> 160 h samples of the stream); uniform instance only
     int n_hops;
     int T;
     int DH;                            // hops per sub-chunk (32 or 64)
@@ -89,7 +96,8 @@ struct DenseArgs {
     // a template and edge index that use it (window view of the generic loader); n_first: the shortest window using it
     int re_goff[DENSE_MAX_RE], re_delta[DENSE_MAX_RE], re_rep[DENSE_MAX_RE], re_rep_e[DENSE_MAX_RE], re_nfirst[DENSE_MAX_RE];
     DenseTmplDev t[DENSE_MAX_T];
-    float* out;                        // [n_streams][n_hops][T]
+    float* out;                        // uniform: [n_streams][n_hops][T]; rows: packed as their descriptors say
+    const DenseRow* rows;              // ROWS instance: one descriptor per CTA
     float* g2;                         // [n_streams][DENSE_WAYS][DG][20]: grid rows floored with a way's floor (tags in shared memory)
     // carry-over between consecutive calls: the newest stream-grid rows of every stream (functions of the PCM only)
     float* keep_rows;                  // [n_streams][DENSE_KEEP][ROW], row of grid frame g at g % DENSE_KEEP
@@ -211,7 +219,9 @@ __device__ __forceinline__ int next_task(int* counter, int lane) {
 
 __device__ __forceinline__ int wrap1(int r, int n) { return r >= n ? r - n : r; }
 
-template <bool PRE>
+// ROWS = false: CTA s scores stream s at the call's hops [A.hop0, A.hop0 + A.n_hops).  ROWS = true: CTA x takes
+// descriptor A.rows[x] (its stream, hop range and output block); the body is the same.
+template <bool PRE, bool ROWS>
 __global__ void __launch_bounds__(1024, 1)
 dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const TemplateFeat* __restrict__ tmpl, DenseArgs A) {
     extern __shared__ __align__(16) float smem[];
@@ -236,7 +246,15 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     int* WAYU = ctl + 32;
     int* WAYMASK = ctl + 40;
     int* COMBO = ctl + 56;
-    const int s = blockIdx.x;
+    const int s = ROWS ? A.rows[blockIdx.x].stream : blockIdx.x;
+    // the row's hops are re-read where they are used: values kept live across the kernel would cost registers
+    auto hop0 = [&]() -> long long { return ROWS ? A.rows[blockIdx.x].hop0 : A.hop0; };
+    auto n_hops = [&]() -> int { return ROWS ? A.rows[blockIdx.x].n_hops : A.n_hops; };
+    // score of hop (hs + hl), template k
+    auto out_at = [&](long long hs, int hl, int k) -> float* {
+        if (ROWS) return A.out + A.rows[blockIdx.x].out + (size_t)(hs - hop0() + hl) * NT + k;
+        return A.out + ((size_t)s * A.n_hops + (size_t)(hs - A.hop0 + hl)) * NT + k;
+    };
     copy_frame_tables(*ft, T, tid, nthr);
     float* scr = scratch + warp * SCR_WARP;
     float* patch = patchb + warp * N_MFCC;
@@ -256,7 +274,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     {
         // rows computed by the previous call are reused when this call continues where it stopped: the history of
         // the first window (up to n_max frames) is loaded instead of recomputed
-        long long need_lo = A.hop0 - A.n_max + 1;
+        long long need_lo = hop0() - A.n_max + 1;
         if (need_lo < 2) need_lo = 2;
         const long long klo = A.keep_rows ? A.keep_end[2 * s] : 0, kend = A.keep_rows ? A.keep_end[2 * s + 1] : 0;
         if (klo <= need_lo && need_lo < kend && kend - need_lo <= DG) {
@@ -343,8 +361,8 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
         return score_from_dots(uvm, uum, vvm, uvs, uus, vvs);
     };
 
-    for (long long hs = A.hop0; hs < A.hop0 + A.n_hops; hs += DH) {
-        const int nh = (int)min((long long)DH, A.hop0 + A.n_hops - hs);
+    for (long long hs = hop0(); hs < hop0() + n_hops(); hs += DH) {
+        const int nh = (int)min((long long)DH, hop0() + n_hops() - hs);
         const int n_half = (nh + 31) >> 5;
         // ================================================================ phase A: frames of this sub-chunk
         // stream-grid rows [g_from, g_hi]: every template's windows of these hops reach back to hs - n + 1 (the row a
@@ -466,7 +484,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
             const int hl = 32 * hh + lane;
             const TemplateFeat& tf = tmpl[tp.slot];
             if (hl >= nh) continue;
-            float* outp = A.out + ((size_t)s * A.n_hops + (size_t)(hs - A.hop0 + hl)) * NT + k;
+            float* outp = out_at(hs, hl, k);
             WAY[k * DH + hl] = -1;
             if (hs + hl - tp.n < 0 || !tf.valid) { *outp = __int_as_float(0x7fc00000); WFL[k * DH + hl] = INFINITY; continue; }
             float wmax = -INFINITY, wmin = INFINITY;
@@ -621,7 +639,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
                 const int hh = job % n_half, k = job / n_half;
                 const int hl = 32 * hh + lane;
                 if (hl >= nh || WAY[k * DH + hl] < 0) continue;
-                A.out[((size_t)s * A.n_hops + (size_t)(hs - A.hop0 + hl)) * NT + k] = score_window(k, hl, tmpl[A.t[k].slot]);
+                *out_at(hs, hl, k) = score_window(k, hl, tmpl[A.t[k].slot]);
             }
             __syncthreads();
         }

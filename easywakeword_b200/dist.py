@@ -135,6 +135,15 @@ class ShardedBank:
                 rows.append(blk)
         return self.bank.step_streams(streams, rows)
 
+    def dense_ready(self, global_streams, template_first: int = 0, template_count=None):
+        """WakeWordBank.dense_ready over global stream ids: every rank may be called with the whole list and scores the
+        streams it owns (dist.local_streams).  Returns {global stream id: (first hop, float32 [n, T] scores)}."""
+        loc = local_streams(global_streams, self.n_total, self.world, self.rank)
+        if not loc:
+            return {}
+        hop0, rows = self.bank.dense_ready(loc, template_first, template_count)
+        return {self.first + s: (int(h), r) for s, h, r in zip(loc, hop0, rows)}
+
     def gather(self):
         ctx = self.bank.ctx
         if self.peer is not None and ctx.publish_seq() > 0:

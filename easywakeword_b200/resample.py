@@ -65,6 +65,14 @@ def due_ticks(written, ticks, max_ticks=None) -> np.ndarray:
     return due if max_ticks is None else np.minimum(due, int(max_ticks))
 
 
+def due_hops(written, next_hop, max_hops=None) -> np.ndarray:
+    """Hops ewk_dense_ready scores: hop h is due once 160 h samples have landed, so a stream that landed `written`
+    16 kHz samples and whose dense cursor is at `next_hop` has max(0, written // 160 + 1 - next_hop) due (hops
+    next_hop, next_hop + 1, ...), at most max_hops."""
+    due = np.maximum(0, np.asarray(written, dtype=np.int64) // 160 + 1 - np.asarray(next_hop, dtype=np.int64))
+    return due if max_hops is None else np.minimum(due, int(max_hops))
+
+
 class StreamResampler:
     """Chunked conversion of [rows, n] feeds to 16 kHz whose concatenated output equals the one-shot result
     sample for sample: every call is given the filter's half-width of history and emits only the outputs whose

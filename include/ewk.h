@@ -311,12 +311,38 @@ int ewk_reset_streams(ewk_ctx* ctx, const int32_t* streams, int n);
  * `where` tells whether `out` is host or device memory. */
 int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int template_first, int template_count,
                      float* out, int where);
+/* Ragged dense scoring: row i scores stream streams[i] at hops [hop0[i], hop0[i] + n_hops[i]) against templates
+ * [template_first, template_first + template_count), each score the value ewk_dense_scores gives for that stream, hop
+ * and template (NaN where the window starts before the stream).  out is packed in list order: row i starts at float
+ * T * (n_hops[0] + .. + n_hops[i - 1]) (T = template_count) and is laid out [n_hops[i]][T]; out_cap is its capacity in
+ * floats, and host output is copied back over the used length only.  n_hops[i] = 0 scores nothing for that row and
+ * costs no CTA; n = 0 is a no-op.  One K4 launch, one CTA per non-empty row, longest rows first.  A pending host push
+ * lands first only if some row reaches into it; overlap mode behaves as for ewk_dense_scores.
+ * EWK_ERR_ARG (naming the stream): a stream out of range or listed twice, hop0 or n_hops negative, out_cap below the
+ * packed length, a template range ewk_dense_scores rejects (EWK_ERR_NO_TEMPLATE for an empty slot).  EWK_ERR_STATE
+ * (naming the stream): a row whose hops are not yet pushed, or whose oldest needed sample has left the ring.  On an
+ * error nothing is scored.  Neither reads nor moves the cursors of ewk_dense_ready. */
+int ewk_dense_scores_streams(ewk_ctx* ctx, const int32_t* streams, int n, const int64_t* hop0, const int32_t* n_hops,
+                             int template_first, int template_count, float* out, int64_t out_cap, int where);
+/* Dense scores paced by each stream's own audio.  The context keeps a cursor next_s per stream, 1 after ewk_create and
+ * after ewk_reset_streams of the stream (hop 0 holds no sample).  Each listed stream (streams = NULL: every stream of the
+ * bank, n ignored) is scored at hops [next_s, min(next_s + max_hops, written_s / 160 + 1)), written_s read after any
+ * pending host push has landed, i.e. hop h is scored once 160 h samples have landed; hop0_out[i] = next_s and
+ * n_hops_out[i] = the count, then next_s moves past them.  Output as ewk_dense_scores_streams, packed in list order;
+ * n * max_hops * template_count floats always suffice.  A stream with nothing due gets 0 hops and costs no CTA.  The same
+ * audio gives the same per-hop scores however it was split into pushes and calls.  max_hops in [1, 1 << 20].
+ * Errors as ewk_dense_scores_streams; on any error no cursor moves (EWK_ERR_STATE for a stream whose cursor's windows
+ * have left the ring: score it more often, or reset it).  ewk_dense_scores and ewk_dense_scores_streams leave the
+ * cursors alone. */
+int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first, int template_count,
+                    int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where);
 /* Launch geometry ewk_dense_scores chooses for templates of these lengths (samples, n <= 8, each 640..48000):
  * out = {hops per sub-chunk (32 or 64), threads per CTA, CTAs per SM, dynamic shared memory bytes}.  Host code only
  * (no context, no device): the function ewk_dense_scores itself plans with.  EWK_ERR_ARG for lengths out of range or a
  * set that does not fit shared memory. */
 int ewk_dense_plan(const int64_t* template_lens, int n, int32_t out[4]);
-/* The geometry (same layout) the context's latest ewk_dense_scores launched; zeros before the first call. */
+/* The geometry (same layout) the context's latest K4 call (ewk_dense_scores, ewk_dense_scores_streams, ewk_dense_ready)
+ * launched; zeros before the first call.  All three plan alike for the same template set. */
 int ewk_dense_last_plan(const ewk_ctx* ctx, int32_t out[4]);
 /* Copy the dense per-stream results [n_streams] to host memory. */
 int ewk_stream_results(ewk_ctx* ctx, ewk_stream_result* out);
