@@ -31,6 +31,66 @@ def mfcc_rel_l2(a, b):
     return num / np.maximum(den, 1e-30)
 
 
+class K3Probe:
+    """tests/k3_probe.cu built with the library's nvcc flags into `out_dir` and loaded with ctypes.  tables() runs on
+    the host only; log_mel / frames / power need a device."""
+
+    def __init__(self, out_dir):
+        import ctypes as C
+        import os
+        import subprocess
+        from easywakeword_b200 import build
+        here = os.path.dirname(os.path.abspath(__file__))
+        so = os.path.join(str(out_dir), "k3_probe.so")
+        cmd = [build._nvcc(), *build.NVCC_FLAGS, "-I", build.CSRC, "-o", so,
+               os.path.join(here, "k3_probe.cu")]
+        r = subprocess.run(cmd, capture_output=True, text=True)
+        if r.returncode != 0:
+            raise RuntimeError("nvcc failed building the K3 probe:\n" + r.stdout + r.stderr)
+        lib = C.CDLL(so)
+        f32p, vp = C.POINTER(C.c_float), C.c_void_p
+        lib.k3p_tables.restype, lib.k3p_tables.argtypes = C.c_longlong, [vp, C.c_longlong, C.POINTER(C.c_longlong)]
+        lib.k3p_log_mel.restype, lib.k3p_log_mel.argtypes = C.c_int, [f32p, f32p, C.c_longlong]
+        lib.k3p_frames.restype, lib.k3p_frames.argtypes = C.c_int, [f32p, C.c_int, C.c_float, f32p, f32p]
+        lib.k3p_power.restype, lib.k3p_power.argtypes = C.c_int, [f32p, C.c_int, f32p]
+        self.lib, self.C = lib, C
+
+    def tables(self):
+        """-> (image bytes, (sizeof(DeviceTables), FRAME_IMAGE_OFFSET, sizeof(FrameTables)))."""
+        C = self.C
+        sizes = (C.c_longlong * 3)()
+        n = self.lib.k3p_tables(None, 0, sizes)
+        buf = (C.c_ubyte * n)()
+        assert self.lib.k3p_tables(buf, n, sizes) == n
+        return bytes(buf), tuple(int(v) for v in sizes)
+
+    def _p(self, a):
+        return a.ctypes.data_as(self.C.POINTER(self.C.c_float))
+
+    def log_mel(self, S):
+        """TEN_LOG10_2 * __log2f(fmaxf(S, 1e-10f)) on the device (the model's log_fn)."""
+        S = np.ascontiguousarray(S, np.float32)
+        out = np.empty_like(S)
+        if S.size:
+            assert self.lib.k3p_log_mel(self._p(S), self._p(out), S.size) == 0
+        return out
+
+    def frames(self, x, floor_db=-np.inf):
+        """warp_frame_mfcc on loaded frames [n, 512] -> (MFCC [n, 20], un-floored log-mel [n, 128])."""
+        x = np.ascontiguousarray(x, np.float32).reshape(-1, 512)
+        m = np.empty((len(x), 20), np.float32)
+        lm = np.empty((len(x), 128), np.float32)
+        assert self.lib.k3p_frames(self._p(x), len(x), float(floor_db), self._p(m), self._p(lm)) == 0
+        return m, lm
+
+    def power(self, x):
+        """warp_power_spectrum on loaded frames [n, 512] -> P [n, 257]."""
+        x = np.ascontiguousarray(x, np.float32).reshape(-1, 512)
+        P = np.empty((len(x), 257), np.float32)
+        assert self.lib.k3p_power(self._p(x), len(x), self._p(P)) == 0
+        return P
+
+
 def dense_geometry_sets(plan_fn):
     """Template-length sets (1-8 templates of 640 .. 48000 samples, remainders mod 160 on both sides of 96 so that
     windows have 1 and 2 right-edge frames) through K4's planner -> {(DH, threads, CTAs per SM): lengths}, one set per
