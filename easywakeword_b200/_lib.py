@@ -298,6 +298,8 @@ class StreamStatus(C.Structure):
 EVENT_DTYPE = np.dtype([("stream", "<i4"), ("kind", "<i4"), ("tick", "<i8"), ("seg_start", "<i8"),
                         ("seg_len", "<i4"), ("template_slot", "<i4"), ("score", "<f4"), ("matched", "<i4")])
 RESULT_DTYPE = np.dtype([("score", "<f4"), ("flags", "<u4")])
+DETECTION_DTYPE = np.dtype([("stream", "<i4"), ("template_slot", "<i4"), ("hop", "<i8"), ("run_start", "<i8"),
+                            ("emit_hop", "<i8"), ("seg_start", "<i8"), ("seg_len", "<i4"), ("score", "<f4")])
 EV_TIMEOUT, EV_SCORED = 1, 2
 
 
@@ -326,6 +328,8 @@ def _declare_stream_protos(lib):
         "ewk_dense_scores": (C.c_int, [vp, i64, i32, i32, i32, vp, i32]),
         "ewk_dense_scores_streams": (C.c_int, [vp, _p(C.c_int32), i32, _p(i64), _p(C.c_int32), i32, i32, vp, i64, i32]),
         "ewk_dense_ready": (C.c_int, [vp, _p(C.c_int32), i32, i32, i32, i32, _p(i64), _p(C.c_int32), vp, i64, i32]),
+        "ewk_dense_detect": (C.c_int, [vp, _p(C.c_int32), i32, i32, i32, i32, i32, i32, vp, i32, _p(i64), _p(C.c_int32),
+                                       vp, i64, i32]),
         "ewk_prepare_segments": (C.c_int, [vp, i32, _p(C.c_int32), _p(i64), _p(i64), _p(i64), f32p, i64, i32]),
         "ewk_results_device_ptr": (C.c_int, [vp, _p(vp)]),
         "ewk_set_results_buffer": (C.c_int, [vp, vp]),
@@ -672,6 +676,44 @@ def _bank_methods():
         self._ck(self.lib.ewk_dense_ready(self.h, *args, out.ctypes.data if out.size else None, cap, HOST))
         return h0, _unpack_rows(out, nh, T)
 
+    def dense_detect(self, streams=None, max_hops=100, template_first=0, template_count=1, hold_hops=20,
+                     refractory_hops=50, scores=False, out_device_ptr=None, det_cap=None, out_cap=None, hops=False):
+        """Detections from per-hop scores on the device (include/ewk.h: ewk_dense_detect): each listed stream (None: every
+        stream) is scored from the detector's own cursor at every hop its landed audio completes, at most max_hops, and
+        those hops go through the stream's peak picker (threshold: its similarity_threshold).  Returns a DETECTION_DTYPE
+        array in list order, then emit_hop order.  det holds n * ceil(max_hops / 2) records unless det_cap is given.
+        scores=True also returns (hop0, list of float32 [n_i, template_count] arrays); with out_device_ptr the scores go
+        there packed in list order (out_cap floats, default n * max_hops * template_count) and (hop0, n_hops) is returned
+        with the detections.  Otherwise the scores stay on the device; hops=True then returns (hop0, n_hops) with them."""
+        st = None if streams is None else _stream_list(streams)
+        n = self.cfg.n_streams if st is None else len(st)
+        T = int(template_count)
+        cap = n * ((min(int(max_hops), 1 << 20) + 1) // 2) if det_cap is None else int(det_cap)
+        det = np.empty(max(0, cap), DETECTION_DTYPE)
+        h0 = np.zeros(n, np.int64)
+        nh = np.zeros(n, np.int32)
+        ocap = n * int(max_hops) * T if out_cap is None else int(out_cap)
+        buf = None
+        if out_device_ptr is not None:
+            out, where = C.c_void_p(out_device_ptr), DEVICE
+        elif scores:
+            buf = np.empty(max(0, ocap), np.float32)
+            out, where = (buf.ctypes.data if buf.size else None), HOST
+        else:
+            out, ocap, where = None, 0, HOST
+        rc = self.lib.ewk_dense_detect(self.h, None if st is None else st.ctypes.data_as(_p(C.c_int32)), n, int(max_hops),
+                                       int(template_first), T, int(hold_hops), int(refractory_hops),
+                                       det.ctypes.data if det.size else None, cap, i64ptr(h0),
+                                       nh.ctypes.data_as(_p(C.c_int32)), out, ocap, where)
+        if rc < 0:
+            self._ck(rc)
+        d = det[:rc].copy()
+        if out_device_ptr is not None:
+            return d, (h0, nh)
+        if scores:
+            return d, (h0, _unpack_rows(buf, nh, T))
+        return (d, (h0, nh)) if hops else d
+
     def dense_last_plan(self):
         """(DH, threads, CTAs per SM, shared-memory bytes) of the latest K4 launch (dense_scores, dense_scores_streams or
         dense_ready; zeros before the first)."""
@@ -760,7 +802,7 @@ def _bank_methods():
                  "resample_push"]
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
-    for f in (prepare_segments, dense_scores, dense_scores_streams, dense_ready, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
+    for f in (prepare_segments, dense_scores, dense_scores_streams, dense_ready, dense_detect, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
               push_resampled_each, push_streams, tick_ready, reset_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
               set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count):
         setattr(Context, f.__name__, f)

@@ -206,6 +206,26 @@ class WakeWordBank:
             if not rows or max(len(r) for r in rows) < DENSE_ROUND:
                 return hop0, [p[0] if len(p) == 1 else np.concatenate(p) for p in parts]
 
+    def dense_detect(self, streams=None, template_first: int = 0, template_count: Optional[int] = None,
+                     hold_hops: int = 20, refractory_hops: int = 50) -> np.ndarray:
+        """Wake-word detections from per-hop scores, without the energy gate (include/ewk.h: ewk_dense_detect): every hop
+        of the listed streams (None: all) that their landed audio completes and no earlier dense_detect took, in rounds of
+        DENSE_ROUND hops, so that no due hop is left when it returns.  A stream detects where its best per-hop score
+        reaches its similarity_threshold; a run reports its first peak once it ends or hold_hops after the peak, and a
+        stream stays quiet for refractory_hops after a run.  Returns a _lib.DETECTION_DTYPE array sorted by
+        (emit_hop, stream); prepare_for_transcription takes it as it is.  The detector has its own cursor (dense_ready's is
+        untouched); reset() restarts it.  Feed hold_hops hops of trailing audio to finish a recording's last run."""
+        T = len(self.templates) - template_first if template_count is None else template_count
+        parts = []
+        while True:
+            d, (_, nh) = self.ctx.dense_detect(streams, DENSE_ROUND, template_first, T, hold_hops, refractory_hops,
+                                               hops=True)
+            parts.append(d)
+            if nh.size == 0 or nh.max() < DENSE_ROUND:
+                break
+        det = np.concatenate(parts)
+        return det[np.lexsort((det["stream"], det["emit_hop"]))]
+
     def read_segment(self, event) -> np.ndarray:
         """word_audio of a level-2 event as float32 (what level 3 transcribes)."""
         return self.ctx.read_segment(int(event["stream"]), int(event["seg_start"]), int(event["seg_len"]))

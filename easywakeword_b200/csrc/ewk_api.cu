@@ -209,7 +209,13 @@ void ewk_ctx::release() {
         if (h_drow[i]) cudaFreeHost(h_drow[i]);
         ev_drow[i] = nullptr; h_drow[i] = nullptr;
         b_drow[i].free();
+        if (ev_ddet[i]) cudaEventDestroy(ev_ddet[i]);
+        if (h_ddet[i]) cudaFreeHost(h_ddet[i]);
+        ev_ddet[i] = nullptr; h_ddet[i] = nullptr;
+        b_ddet[i].free();
     }
+    if (h_det_map) cudaFreeHost(h_det_map);
+    h_det_map = nullptr; det_map_cap = 0;
     b_reset.free();
     if (own_stream) cudaStreamDestroy(own_stream);
     d_tables = nullptr; d_tmpl = nullptr; own_stream = nullptr; copy_stream = nullptr;
@@ -624,6 +630,7 @@ int ewk_ctx::init_streams() {
     h_visible_lb.assign(n, 0);
     h_tick.assign(n, 0);
     h_dense_next.assign(n, 1);
+    h_det_next.assign(n, 1);
     h_frame_size.assign(n, 0);
     h_rate.assign(n, 0);
     h_inputs.assign(n, 0);
@@ -661,7 +668,7 @@ void ewk_ctx::release_streams() {
         if (p) cudaFree(p);
     bank = BankView{};
     own_results = nullptr;
-    b_trace.free(); b_read.free(); b_dense.free(); b_keep_rows.free(); b_keep_end.free(); b_g2.free();
+    b_trace.free(); b_read.free(); b_dense.free(); b_keep_rows.free(); b_keep_end.free(); b_g2.free(); b_det_state.free();
     for (auto& p : prof_pairs) { cudaEventDestroy(p.a); cudaEventDestroy(p.b); }
     for (auto e : prof_free) cudaEventDestroy(e);
     prof_pairs.clear(); prof_free.clear();
@@ -1427,12 +1434,13 @@ extern "C" int ewk_reset_streams(ewk_ctx* ctx, const int32_t* streams, int n) {
     const size_t row_bytes = (size_t)B.P * (B.fmt == 1 ? 2 : 4);
     const dim3 grid((unsigned)((row_bytes + RESET_SLICE - 1) / RESET_SLICE), (unsigned)std::min(n, 65535));
     stream_reset_kernel<<<grid, RESET_THREADS, 0, ctx->stream>>>(B, (const int*)ctx->b_reset.p, n,
-                                                                 (long long*)ctx->b_keep_end.p);
+                                                                 (long long*)ctx->b_keep_end.p,
+                                                                 (DetState*)ctx->b_det_state.p);
     CK(cudaGetLastError());
     ctx->launches++;
     for (int i = 0; i < n; i++) {
         const int s = streams[i];
-        ctx->h_written[s] = 0; ctx->h_visible_lb[s] = 0; ctx->h_tick[s] = 0; ctx->h_dense_next[s] = 1;
+        ctx->h_written[s] = 0; ctx->h_visible_lb[s] = 0; ctx->h_tick[s] = 0; ctx->h_dense_next[s] = 1; ctx->h_det_next[s] = 1;
         ctx->h_frame_size[s] = 0; ctx->h_rate[s] = 0; ctx->h_inputs[s] = 0;
     }
     return EWK_OK;
@@ -1936,10 +1944,14 @@ extern "C" int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int tmpl
     return EWK_OK;
 }
 
-// Rows of ewk_dense_scores_streams and ewk_dense_ready: row i scores stream streams[i] at hops [hop0[i], hop0[i] + n_hops[i]),
-// packed into out in list order.  Every check comes before the first launch or copy, so an error changes no state.
+// Rows of ewk_dense_scores_streams, ewk_dense_ready and ewk_dense_detect: row i scores stream streams[i] at hops
+// [hop0[i], hop0[i] + n_hops[i]), packed into out in list order.  Every check comes before the first launch or copy, so an
+// error changes no state.  d_scores (ewk_dense_detect): the caller reads the scores on the device after K4 and copies
+// host output itself; out may then be NULL (the scores stay in device scratch), and *d_scores receives where K4 wrote
+// them (NULL when no row has hops).
 static int dense_rows(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, const int64_t* hop0, const int32_t* n_hops,
-                      int tmpl_first, int tmpl_count, float* out, int64_t out_cap, int where) {
+                      int tmpl_first, int tmpl_count, float* out, int64_t out_cap, int where, float** d_scores = nullptr) {
+    if (d_scores) *d_scores = nullptr;
     BankView& B = ctx->bank;
     if (n < 0 || (n > 0 && (!streams || !hop0 || !n_hops))) { ctx->fail("%s: bad row list (n=%d)", who, n); return EWK_ERR_ARG; }
     if (n == 0) return EWK_OK;
@@ -1961,7 +1973,7 @@ static int dense_rows(ewk_ctx* ctx, const char* who, const int32_t* streams, int
     int rc = dense_prepare(ctx, who, tmpl_first, tmpl_count, A, plan);
     if (rc) return rc;
     const long long n_out = hops * tmpl_count;
-    if (n_out > 0 && (!out || out_cap < n_out)) {
+    if (n_out > 0 && (out || !d_scores) && (!out || out_cap < n_out)) {
         ctx->fail("%s: out holds %lld floats, the rows need %lld", who, out ? (long long)out_cap : 0LL, n_out);
         return EWK_ERR_ARG;
     }
@@ -1998,12 +2010,13 @@ static int dense_rows(ewk_ctx* ctx, const char* who, const int32_t* streams, int
     rc = upload_slot(ctx, ctx->h_drow, ctx->b_drow, ctx->ev_drow, ctx->ev_drow_valid, ctx->drow_idx, rows, ctx->stream, &k);
     if (rc) return rc;
     float* d_out = out;
-    if (where == EWK_HOST) { CK(ctx->b_dense.ensure(sizeof(float) * (size_t)n_out)); d_out = (float*)ctx->b_dense.p; }
+    if (where == EWK_HOST || !out) { CK(ctx->b_dense.ensure(sizeof(float) * (size_t)n_out)); d_out = (float*)ctx->b_dense.p; }
     A.rows = (const DenseRow*)ctx->b_drow[k].p;
     rc = dense_launch(ctx, A, plan, d_out, (int)rows.size());
     if (rc) return rc;
     CK(cudaEventRecord(ctx->ev_drow[k], ctx->stream));        // the slot is free once this K4 has read it
     ctx->ev_drow_valid[k] = true;
+    if (d_scores) { *d_scores = d_out; return EWK_OK; }
     if (where == EWK_HOST) {
         CK(cudaMemcpyAsync(out, d_out, sizeof(float) * (size_t)n_out, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
@@ -2063,6 +2076,120 @@ extern "C" int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int 
         ctx->h_dense_next[streams[i]] += nh[i];
     }
     return EWK_OK;
+}
+
+static_assert(sizeof(DetRecord) == sizeof(ewk_detection) && sizeof(ewk_detection) == 48, "ewk_detection layout");
+static_assert(offsetof(DetRecord, score) == offsetof(ewk_detection, score), "ewk_detection layout");
+
+// ewk_dense_ready's due rule on the detector's own cursor, then K4 (per-row) and K4D behind it on the context's stream
+extern "C" int ewk_dense_detect(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first,
+                                int template_count, int hold_hops, int refractory_hops, ewk_detection* det, int det_cap,
+                                int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where) {
+    if (!ctx) return EWK_ERR_ARG;
+    const char* who = "ewk_dense_detect";
+    int rc = need_streams(ctx, who);
+    if (rc) return rc;
+    BankView& B = ctx->bank;
+    if (max_hops < 1 || max_hops > (1 << 20)) { ctx->fail("%s: max_hops must be in [1, %d]", who, 1 << 20); return EWK_ERR_ARG; }
+    if (hold_hops < 1 || refractory_hops < 0) {
+        ctx->fail("%s: hold_hops must be >= 1 and refractory_hops >= 0 (got %d, %d)", who, hold_hops, refractory_hops);
+        return EWK_ERR_ARG;
+    }
+    std::vector<int32_t> all;
+    if (!streams) {
+        all.resize((size_t)B.n_streams);
+        for (int s = 0; s < B.n_streams; s++) all[s] = s;
+        streams = all.data();
+        n = B.n_streams;
+    }
+    if (n < 0) { ctx->fail("%s: bad stream list (n=%d)", who, n); return EWK_ERR_ARG; }
+    std::vector<char> seen((size_t)B.n_streams, 0);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        if (s < 0 || s >= B.n_streams) { ctx->fail("%s: bad stream %d (context has %d)", who, s, B.n_streams); return EWK_ERR_ARG; }
+        if (seen[s]) { ctx->fail("%s: stream %d is listed twice", who, s); return EWK_ERR_ARG; }
+        seen[s] = 1;
+    }
+    CK(cudaSetDevice(ctx->device));
+    rc = ctx->flush_pending();                               // the due hops depend on every landed sample
+    if (rc) return rc;
+    std::vector<int64_t> h0((size_t)n);
+    std::vector<int32_t> nh((size_t)n);
+    long long need = 0;                                      // emissions are >= 2 hops apart: ceil(n_i / 2) per row
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        h0[i] = ctx->h_det_next[s];
+        nh[i] = (int32_t)std::max<long long>(0, std::min<long long>(h0[i] + max_hops, ctx->h_written[s] / 160 + 1) - h0[i]);
+        need += (nh[i] + 1) / 2;
+    }
+    if (det_cap < need || (need > 0 && !det)) {
+        ctx->fail("%s: det holds %d records, the due hops need %lld", who, det ? det_cap : 0, need);
+        return EWK_ERR_ARG;
+    }
+    // K4D's output: counts [n_streams], then the records of row i from offset sum_{j < i} ceil(n_j / 2)
+    const size_t rec_off = ((size_t)4 * B.n_streams + 15) / 16 * 16, map_bytes = rec_off + sizeof(DetRecord) * (size_t)need;
+    if (map_bytes > ctx->det_map_cap) {
+        if (ctx->h_det_map) CK(cudaFreeHost(ctx->h_det_map));
+        ctx->h_det_map = nullptr; ctx->det_map_cap = 0;
+        const size_t want = map_bytes + map_bytes / 4 + 256;
+        CK(cudaHostAlloc(&ctx->h_det_map, want, cudaHostAllocMapped | cudaHostAllocPortable));
+        ctx->det_map_cap = want;
+    }
+    float* d_scores = nullptr;
+    rc = dense_rows(ctx, who, streams, n, h0.data(), nh.data(), template_first, template_count, out, out_cap, where,
+                    &d_scores);
+    if (rc) return rc;
+    int n_det = 0;
+    if (d_scores) {
+        if (!ctx->b_det_state.p) {
+            CK(ctx->b_det_state.ensure(sizeof(DetState) * (size_t)B.n_streams));
+            CK(cudaMemsetAsync(ctx->b_det_state.p, 0, sizeof(DetState) * (size_t)B.n_streams, ctx->stream));
+        }
+        std::vector<DetRow> rows;
+        long long off = 0, doff = 0;
+        for (int i = 0; i < n; i++) {
+            if (nh[i] > 0) rows.push_back(DetRow{h0[i], off, doff, streams[i], nh[i], i, 0});
+            off += (long long)nh[i] * template_count;
+            doff += (nh[i] + 1) / 2;
+        }
+        int k = -1;
+        rc = upload_slot(ctx, ctx->h_ddet, ctx->b_ddet, ctx->ev_ddet, ctx->ev_ddet_valid, ctx->ddet_idx, rows, ctx->stream, &k);
+        if (rc) return rc;
+        char* d_map = nullptr;
+        CK(cudaHostGetDevicePointer((void**)&d_map, ctx->h_det_map, 0));
+        DetArgs D{};
+        D.T = template_count; D.slot0 = template_first; D.hold = hold_hops; D.refractory = refractory_hops;
+        for (int t = 0; t < template_count; t++) {
+            const int L = (int)ctx->h_tmpl[template_first + t].n_samples;
+            D.L[t] = L; D.n[t] = (L + HOP - 1) / HOP;
+        }
+        D.rows = (const DetRow*)ctx->b_ddet[k].p; D.n_rows = (int)rows.size();
+        D.scores = d_scores; D.state = (DetState*)ctx->b_det_state.p;
+        D.counts = (int*)d_map; D.rec = (DetRecord*)(d_map + rec_off);
+        cudaEvent_t pe = ctx->prof_begin(4);
+        dense_detect_kernel<<<(D.n_rows + DETECT_WARPS - 1) / DETECT_WARPS, 32 * DETECT_WARPS, 0, ctx->stream>>>(B.prm, D);
+        ctx->prof_end(pe, 4);
+        CK(cudaGetLastError());
+        ctx->launches++;
+        CK(cudaEventRecord(ctx->ev_ddet[k], ctx->stream));
+        ctx->ev_ddet_valid[k] = true;
+        if (out && where == EWK_HOST)
+            CK(cudaMemcpyAsync(out, d_scores, sizeof(float) * (size_t)off, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        // list order, then emit order within a row
+        const int* counts = (const int*)ctx->h_det_map;
+        const DetRecord* rec = (const DetRecord*)((const char*)ctx->h_det_map + rec_off);
+        for (const DetRow& r : rows) {
+            std::memcpy((DetRecord*)det + n_det, rec + r.det, sizeof(DetRecord) * (size_t)counts[r.row]);
+            n_det += counts[r.row];
+        }
+    }
+    for (int i = 0; i < n; i++) {
+        if (hop0_out) hop0_out[i] = h0[i];
+        if (n_hops_out) n_hops_out[i] = nh[i];
+        ctx->h_det_next[streams[i]] += nh[i];
+    }
+    return n_det;
 }
 
 extern "C" int ewk_stream_results(ewk_ctx* ctx, ewk_stream_result* out) {

@@ -92,6 +92,16 @@ struct ewk_ctx {
     cudaEvent_t ev_drow[2] = {nullptr, nullptr};
     bool ev_drow_valid[2] = {false, false};
     int drow_idx = 0;
+    // per-row descriptors of K4D (ewk_dense_detect): two slots of the same kind
+    ewk::DetRow* h_ddet[2] = {nullptr, nullptr};
+    ewk::DevBuf b_ddet[2];
+    cudaEvent_t ev_ddet[2] = {nullptr, nullptr};
+    bool ev_ddet_valid[2] = {false, false};
+    int ddet_idx = 0;
+    ewk::DevBuf b_det_state;                 // K4D's DetState [n_streams], allocated (zeroed) by the first detect call
+    // K4D's output, pinned and mapped into the device: per-row record counts [n_streams], then records (row i at its offset)
+    void* h_det_map = nullptr;
+    size_t det_map_cap = 0;
     ewk::DevBuf b_reset;                     // K9's stream list
     int flush_pending();
     ewk::DevBuf b_stage2[2];
@@ -119,6 +129,7 @@ struct ewk_ctx {
     std::vector<long long> h_visible_lb;   // lower bound of StreamState.visible (audio-clock overrun check)
     std::vector<long long> h_tick;
     std::vector<long long> h_dense_next;   // ewk_dense_ready's cursor: the next hop it scores (1 after create / reset)
+    std::vector<long long> h_det_next;     // ewk_dense_detect's own cursor, independent of ewk_dense_ready's
     std::vector<int> h_frame_size;         // latched frame size per stream (0: no push yet)
     std::vector<int> h_rate;               // input rate latched by the stream's first push (0: none yet; 16000: ewk_push)
     std::vector<long long> h_inputs;       // input samples the stream received (at its own rate)

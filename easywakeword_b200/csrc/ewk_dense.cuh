@@ -657,4 +657,108 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     }
 }
 
+// ---- K4D — dense_detect: a per-stream peak picker over the scores K4 just wrote (ewk_dense_detect) -------------------
+// Per hop h: b = max over the call's templates of score[h][k] ignoring NaN (NaN when all are), k* the lowest k reaching
+// it, above = b >= the stream's similarity_threshold (NaN: never).  State machine per stream (DetState, carried between
+// calls):
+//   IDLE,  above, h >= quiet_until  -> ARMED, pending = peak h, run_start h, score b, slot, window of k*
+//   ARMED, above                    -> peak fields replaced if b > pending score (first maximum wins); then, once
+//                                      h - peak >= hold: emit at h -> SPENT
+//   ARMED, not above                -> emit at h, quiet_until = h + refractory -> IDLE
+//   SPENT, not above                -> quiet_until = h + refractory -> IDLE
+// oracle/dense_detect.py is the same machine on the host.  Only comparisons and integer arithmetic: the result is exact.
+constexpr int DETECT_WARPS = 4;        // rows (one warp each) per CTA
+
+struct DetRecord {                     // mirrors ewk_detection (include/ewk.h)
+    int stream, template_slot;
+    long long hop, run_start, emit_hop, seg_start;
+    int seg_len;
+    float score;
+};
+
+// One non-empty row of a detect call: stream `stream`, hops [hop0, hop0 + n_hops), scores at `scores` ([n_hops][T]
+// floats into the call's packed K4 output); its records go to rec[det, det + ceil(n_hops / 2)) and their count to
+// counts[row] (row: the stream's index in the call's list)
+struct DetRow {
+    long long hop0, scores, det;
+    int stream, n_hops, row, pad;
+};
+
+struct DetArgs {
+    int T, slot0, hold, refractory;    // templates [slot0, slot0 + T) of the call
+    int n[DENSE_MAX_T], L[DENSE_MAX_T]; // per template: window in hops (ceil(L / 160)) and samples
+    const DetRow* rows;
+    int n_rows;
+    const float* scores;
+    DetState* state;                   // [n_streams]
+    DetRecord* rec;                    // host-mapped: only emitted records cross PCIe
+    int* counts;                       // host-mapped [list length]
+};
+
+__global__ void __launch_bounds__(32 * DETECT_WARPS)
+dense_detect_kernel(const StreamParams* __restrict__ prm, DetArgs A) {
+    const int lane = threadIdx.x & 31, w = blockIdx.x * DETECT_WARPS + (threadIdx.x >> 5);
+    if (w >= A.n_rows) return;
+    const DetRow r = A.rows[w];
+    const float thr = prm[r.stream].similarity_threshold;
+    const float* __restrict__ sc = A.scores + r.scores;
+    DetRecord* __restrict__ out = A.rec + r.det;
+    DetState st = A.state[r.stream];
+    int nd = 0;
+    for (int base = 0; base < r.n_hops; base += 32) {
+        // lane j: b and k* of hop base + j
+        float b = __int_as_float(0x7fc00000);
+        int kb = 0;
+        if (base + lane < r.n_hops) {
+            const float* row = sc + (size_t)(base + lane) * A.T;
+            for (int k = 0; k < A.T; k++) {
+                const float v = row[k];
+                if (v > b || (b != b && v == v)) { b = v; kb = k; }
+            }
+        }
+        const int cnt = min(32, r.n_hops - base);
+        for (int i = 0; i < cnt; i++) {                      // the walk, in hop order (warp-uniform)
+            const float bh = __shfl_sync(FULL, b, i);
+            const int kh = __shfl_sync(FULL, kb, i);
+            const long long h = r.hop0 + base + i;
+            int nk = 0, Lk = 0;                                  // window of k* (selects: no local copy of A)
+#pragma unroll
+            for (int t = 0; t < DENSE_MAX_T; t++)
+                if (t == kh) { nk = A.n[t]; Lk = A.L[t]; }
+            const bool above = bh >= thr;
+            bool emit = false;
+            if (st.mode == DET_IDLE) {
+                if (above && h >= st.quiet_until) {
+                    st.mode = DET_ARMED; st.peak = h; st.run_start = h; st.score = bh; st.slot = A.slot0 + kh;
+                    st.seg_start = 160LL * (h - nk); st.seg_len = Lk;
+                }
+            } else if (st.mode == DET_ARMED) {
+                if (above) {
+                    if (bh > st.score) {
+                        st.peak = h; st.score = bh; st.slot = A.slot0 + kh;
+                        st.seg_start = 160LL * (h - nk); st.seg_len = Lk;
+                    }
+                    if (h - st.peak >= A.hold) { emit = true; st.mode = DET_SPENT; }
+                } else {
+                    emit = true; st.quiet_until = h + A.refractory; st.mode = DET_IDLE;
+                }
+            } else if (!above) {
+                st.quiet_until = h + A.refractory; st.mode = DET_IDLE;
+            }
+            if (emit) {
+                if (lane == 0) {
+                    DetRecord* o = out + nd;
+                    o->stream = r.stream; o->template_slot = st.slot; o->hop = st.peak; o->run_start = st.run_start;
+                    o->emit_hop = h; o->seg_start = st.seg_start; o->seg_len = st.seg_len; o->score = st.score;
+                }
+                nd++;
+            }
+        }
+    }
+    if (lane == 0) {
+        A.state[r.stream] = st;
+        A.counts[r.row] = nd;
+    }
+}
+
 }  // namespace ewk

@@ -1501,14 +1501,25 @@ __global__ void peer_wait_kernel(const unsigned long long* __restrict__ sig_row,
 // ------------------------------------------------------------------------------------ K9 (stream recycling)
 // ewk_reset_streams: every listed stream back to the state init_streams gives it.  CTA (x, y) clears byte slice x of the
 // ring row of list[y] with 16-byte stores (rows are P * esz bytes, P a multiple of 64: 16-byte aligned); the CTAs of
-// slice 0 also write the StreamState, the block_ss and chunk_ms rows, the result record and K4's carried-row range.
+// slice 0 also write the StreamState, the block_ss and chunk_ms rows, the result record, K4's carried-row range and
+// K4D's detector state.
 // The K8 input tail needs no clearing: a stream at input position 0 reads none of it and rewrites it on its next push.
 // HBM-bound: P * esz bytes per stream plus a few KB.
 constexpr int RESET_THREADS = 256;
 constexpr int RESET_SLICE = RESET_THREADS * 16 * 8;       // bytes of a ring row per CTA (8 stores per thread)
 
+// Per-stream state of the dense detector (K4D, ewk_dense_detect; ewk_dense.cuh).  All zeros is the initial state:
+// IDLE, quiet_until 0, no pending record.
+enum : int { DET_IDLE = 0, DET_ARMED = 1, DET_SPENT = 2 };
+struct DetState {
+    int mode, slot;                    // slot: template slot of the pending peak
+    long long quiet_until, peak, run_start, seg_start;
+    int seg_len;
+    float score;                       // pending peak score
+};
+
 __global__ void __launch_bounds__(RESET_THREADS)
-stream_reset_kernel(BankView B, const int* __restrict__ list, int n, long long* keep_end) {
+stream_reset_kernel(BankView B, const int* __restrict__ list, int n, long long* keep_end, DetState* det) {
     const size_t row_bytes = (size_t)B.P * (B.fmt == 1 ? 2 : 4);
     for (int y = blockIdx.y; y < n; y += gridDim.y) {
         const int s = list[y];
@@ -1523,6 +1534,7 @@ stream_reset_kernel(BankView B, const int* __restrict__ list, int n, long long* 
             B.st[s] = z;
             store_result(B.results + s, StreamResult{__int_as_float(0x7fc00000), 0u});   // nanf(""), as init_streams
             if (keep_end) { keep_end[2 * s] = 0; keep_end[2 * s + 1] = 0; }
+            if (det) det[s] = DetState{};
         }
         double* ss = B.block_ss + (size_t)s * B.NB;
         for (int i = threadIdx.x; i < B.NB; i += RESET_THREADS) ss[i] = 0.0;

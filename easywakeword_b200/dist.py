@@ -144,6 +144,18 @@ class ShardedBank:
         hop0, rows = self.bank.dense_ready(loc, template_first, template_count)
         return {self.first + s: (int(h), r) for s, h, r in zip(loc, hop0, rows)}
 
+    def dense_detect(self, global_streams, template_first: int = 0, template_count=None, hold_hops: int = 20,
+                     refractory_hops: int = 50):
+        """WakeWordBank.dense_detect over global stream ids: every rank may be called with the whole list and detects on
+        the streams it owns (dist.local_streams).  Returns this rank's detections with global stream ids."""
+        from . import _lib
+        loc = local_streams(global_streams, self.n_total, self.world, self.rank)
+        if not loc:
+            return np.zeros(0, _lib.DETECTION_DTYPE)
+        det = self.bank.dense_detect(loc, template_first, template_count, hold_hops, refractory_hops)
+        det["stream"] += self.first
+        return det
+
     def gather(self):
         ctx = self.bank.ctx
         if self.peer is not None and ctx.publish_seq() > 0:

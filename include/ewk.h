@@ -146,6 +146,16 @@ typedef struct ewk_stream_result {  /* dense per-stream record, 8 bytes: what mu
                                        ewk_tick | bits 8..31 events so far                               */
 } ewk_stream_result;
 
+typedef struct ewk_detection {      /* dense detector decision (ewk_dense_detect), 48 bytes               */
+    int32_t stream, template_slot;  /* slot of the peak score                                             */
+    int64_t hop;                    /* peak hop                                                           */
+    int64_t run_start;              /* first hop of the run                                               */
+    int64_t emit_hop;               /* hop at which it was decided (run end, or peak + hold)              */
+    int64_t seg_start;              /* 160 * (hop - n_k): the peak window, for ewk_read_segment /          */
+    int32_t seg_len;                /*   ewk_prepare_segments (level 3); seg_len = L_k                    */
+    float score;                    /* peak score                                                         */
+} ewk_detection;
+
 typedef struct ewk_vad_result {     /* template voice-activity analysis, 32 bytes                          */
     double duration_s;              /* max((last - first) * 160 / 16000, 0.2); 0 when voiced == 0         */
     float max_rms, threshold;       /* max frame RMS and max_rms * 0.1 (float32)                          */
@@ -289,8 +299,9 @@ int ewk_stream_input(ewk_ctx* ctx, int stream, int32_t* sr_in, int64_t* n_in);
  * state ewk_create gives a stream.  Afterwards stream s behaves exactly like stream s of a new context with the same
  * ewk_config, templates and stream parameters given the same calls: events, result records, tick traces,
  * ewk_stream_status, ewk_stream_input, ewk_read_last (zeros before the ring fills), ewk_read_segment, dense scores.  Its
- * ticks and sample indices count from the reset.  Streams not listed are untouched.  Stream parameters are kept (change
- * them with ewk_set_stream_params); the input-rate latch is cleared, so the next session may come at any rate.  A pending
+ * ticks and sample indices count from the reset; its detector (ewk_dense_detect) is back to cursor 1, IDLE,
+ * quiet_until 0.  Streams not listed are untouched.  Stream parameters are kept (change them with
+ * ewk_set_stream_params); the input-rate latch is cleared, so the next session may come at any rate.  A pending
  * host push lands first (its samples belong to the old session and are cleared with it); in overlap mode the call joins
  * K3 first.  One launch (K9) for the whole list; duplicates are harmless, n = 0 is a no-op.
  * EWK_ERR_STATE while the event queue is not empty ("poll first": events carry no session, so an old session's event
@@ -336,6 +347,35 @@ int ewk_dense_scores_streams(ewk_ctx* ctx, const int32_t* streams, int n, const 
  * cursors alone. */
 int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first, int template_count,
                     int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where);
+/* Wake-word detections from per-hop scores, on the device: a peak picker per stream that needs no gate.  The context
+ * keeps a second cursor per stream for it, 1 after ewk_create and after ewk_reset_streams, independent of
+ * ewk_dense_ready's.  Each listed stream (streams = NULL: every stream, n ignored) is scored at the hops ewk_dense_ready's
+ * due rule gives from this cursor (at most max_hops), and those hops go in order through a state machine whose state
+ * the context keeps per stream between calls:
+ *   b_h = max over the call's templates of score[h][k], ignoring NaN (NaN when all are); k* the lowest k reaching it;
+ *   above_h = b_h >= the stream's similarity_threshold (ewk_stream_params; NaN is never above).
+ *   IDLE,  above_h and h >= quiet_until -> ARMED; pending = {peak h, run_start h, score b_h, slot template_first + k*,
+ *                                          seg_start 160 (h - n_k*), seg_len L_k*}
+ *   ARMED, above_h      -> if b_h > pending score (strictly: the first maximum wins) the peak fields move to h; then if
+ *                          h - peak >= hold_hops the pending record is emitted with emit_hop h -> SPENT
+ *   ARMED, not above_h  -> emit with emit_hop h, quiet_until = h + refractory_hops -> IDLE
+ *   SPENT, not above_h  -> quiet_until = h + refractory_hops -> IDLE
+ * quiet_until is 0 initially.  Any two emissions are >= 2 hops apart, so a call emits at most sum_i ceil(n_hops_i / 2)
+ * records and n * ceil(max_hops / 2) always suffice.  A run still ARMED at the end of a call carries to the next; every
+ * pending run is emitted at most hold_hops hops after its peak, so feed hold_hops more hops of audio (e.g. trailing
+ * silence) to finish a recording.  The same audio gives the same detections however it was split into pushes and calls.
+ * Returns the number of records written to det[0 .. det_cap), in list order and within a stream in emit_hop order, or a
+ * status.  hop0_out / n_hops_out (either may be NULL) receive the hops scored per listed stream.  out may be NULL: the
+ * scores then stay in device scratch and cross no PCIe; otherwise they are packed and laid out as by ewk_dense_ready, in
+ * host or device memory (`where`).  One K4 launch plus one K4D launch (one warp per non-empty row) on the context's
+ * stream; only the emitted records and a count per row cross PCIe.  Synchronises with the context's stream.
+ * Errors as ewk_dense_ready, and EWK_ERR_ARG for hold_hops < 1, refractory_hops < 0 or det_cap below
+ * sum_i ceil(n_hops_i / 2).  Every check comes before the first launch: on any error no cursor, detector state or score
+ * moves.  ewk_dense_scores, ewk_dense_scores_streams and ewk_dense_ready neither read nor move the detector; pending
+ * pushes and overlap mode behave as for ewk_dense_ready. */
+int ewk_dense_detect(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first, int template_count,
+                     int hold_hops, int refractory_hops, ewk_detection* det, int det_cap,
+                     int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where);
 /* Launch geometry ewk_dense_scores chooses for templates of these lengths (samples, n <= 8, each 640..48000):
  * out = {hops per sub-chunk (32 or 64), threads per CTA, CTAs per SM, dynamic shared memory bytes}.  Host code only
  * (no context, no device): the function ewk_dense_scores itself plans with.  EWK_ERR_ARG for lengths out of range or a
