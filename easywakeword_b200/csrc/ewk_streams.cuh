@@ -893,7 +893,9 @@ tick_gate_kernel(BankView B, int n_ticks, TraceView tr, int trace_stride, int tr
                         if (np == GATE_MAXP) { np = 255; break; }
                         plan.pc[j][np++] = (short)c;
                     }
-                    if (np == 1 && fs == TICK && dv == TICK && (q0 % TICK) == 0 && B.R >= TICK) alias = 1;
+                    // the recent window IS chunk pc[0] only when the tick's 1600 new samples sit inside the logical ring:
+                    // with R % 1600 != 0 the tick at q0 = floor(R / 1600) * 1600 lands in the tail and wraps into chunk 0
+                    if (np == 1 && fs == TICK && dv == TICK && (q0 % TICK) == 0 && q0 + TICK <= B.R) alias = 1;
                 }
             }
             plan.V[j] = V;

@@ -116,9 +116,10 @@ class SoundBufferOracle:
     FREQUENCY = FREQUENCY
     MIN_THRESHOLD = MIN_THRESHOLD
 
-    def __init__(self, seconds=10, fast=False):
+    def __init__(self, seconds=10, fast=False, ring_samples=None):
+        # ring_samples: a ring of any integer length (the reference's seconds * 16000 cannot say 20000 samples)
         self.buffer_seconds = seconds
-        self.buffer_length = self.buffer_seconds * self.FREQUENCY
+        self.buffer_length = int(ring_samples) if ring_samples is not None else self.buffer_seconds * self.FREQUENCY
         self.data = np.zeros(self.buffer_length)
         self.pointer = 0
         self.frame_size = 0
@@ -220,13 +221,16 @@ def segment_bounds(sound_start_time, sound_end_time, current_time):
 
 
 def detect_stream(stream, template, *, block=512, buffer_seconds=10, max_ticks=None,
-                  restart_on_timeout=True, fast=False, matcher=None, keep_audio=False, timing=None, **params):
+                  restart_on_timeout=True, fast=False, matcher=None, keep_audio=False, timing=None, ring_samples=None,
+                  **params):
     """SoundBuffer + WordMatcher + WakeWord._wait_for_buffer/_detect_word (wakeword.py:1002-1007,
     1036-1159, listen loop 1202-1211) over one stream under the audio clock.
 
     stream: float32 samples.  template: float32 samples (set_reference).  Level 3 is stubbed to
     "no transcription" (wakeword.py:1152-1155), so a level-2 match only produces an event.
     Returns the same dict layout as oracle.ref_harness.run_reference_stream, plus per-tick state.
+    ring_samples: ring length in samples instead of buffer_seconds * 16000.  template=None with a matcher that is None
+    skips level 2 (events keep their tick and length, score NaN): the gate's own decisions at any ring length.
     """
     p = dict(DEFAULTS)
     p.update(params)
@@ -235,8 +239,8 @@ def detect_stream(stream, template, *, block=512, buffer_seconds=10, max_ticks=N
                              p["speech_duration_max"], p["post_speech_silence"])
     timeout = p["timeout"]
     stream = np.asarray(stream, dtype=np.float32)
-    buf = SoundBufferOracle(seconds=buffer_seconds, fast=fast)
-    if matcher is None:
+    buf = SoundBufferOracle(seconds=buffer_seconds, fast=fast, ring_samples=ring_samples)
+    if matcher is None and template is not None:
         matcher = WordMatcherOracle()
         matcher.set_reference(np.asarray(template, dtype=np.float32))
 
@@ -325,7 +329,8 @@ def detect_stream(stream, template, *, block=512, buffer_seconds=10, max_ticks=N
                                 state = WAITING
                                 t_state.append(state)
                                 continue
-                            ok, sim = matcher.matches(word_audio, threshold=thr)     # :1121
+                            ok, sim = (matcher.matches(word_audio, threshold=thr)    # :1121
+                                       if matcher is not None else (False, float("nan")))
                             ev = {"tick": k, "seg_len": int(len(word_audio)), "score": float(sim),
                                   "matched": bool(ok), "n_back": n_back, "n_drop": n_drop}
                             if keep_audio:

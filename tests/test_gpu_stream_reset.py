@@ -117,7 +117,7 @@ class Log:
                     ring=np.stack([ctx.read_last(s, RING_S * 16000) for s in streams]))
 
 
-def _assert_same(a, b, ring):
+def _assert_same(a, b):
     assert len(a["ev"]) == len(b["ev"])
     for f in a["ev"].dtype.names:
         x, y = a["ev"][f], b["ev"][f]
@@ -135,12 +135,9 @@ def _assert_same(a, b, ring):
     for k in ("thr", "rms"):
         if k not in a["tr"]:
             continue
-        if ring == "f32":
-            # where one context's K1 formed block sums and the other's gate summed the samples itself (a different
-            # history of pushes since the last tick), float sums of squares differ in the last bits of a double
-            np.testing.assert_allclose(a["tr"][k], b["tr"][k], rtol=1e-12, atol=0)
-        else:
-            assert np.array_equal(a["tr"][k], b["tr"][k]), k           # int16: exact integer sums either way
+        # bit for bit on either ring format: whether one context's K1 formed block sums and the other's gate summed the
+        # samples itself, a block's squares add in one order (oracle/gate_model.py)
+        assert np.array_equal(a["tr"][k].view(np.int64), b["tr"][k].view(np.int64)), k
 
 
 PCM, G711 = ("pcm",), ("g711",)
@@ -228,9 +225,9 @@ def _scenario(word, ring, pre, post=None, prm=None, overlap=False, pending=False
                 lg.poll()
             ticks += due
         got = A.state(reset)
-        _assert_same(got, B.state(reset), ring)
+        _assert_same(got, B.state(reset))
         if C:
-            _assert_same(A.state(keep), C.state(keep), ring)
+            _assert_same(A.state(keep), C.state(keep))
         assert len(got["ev"]) >= 2                                     # the new sessions produced events
         if publish:
             recs = []
