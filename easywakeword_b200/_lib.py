@@ -301,6 +301,35 @@ RESULT_DTYPE = np.dtype([("score", "<f4"), ("flags", "<u4")])
 DETECTION_DTYPE = np.dtype([("stream", "<i4"), ("template_slot", "<i4"), ("hop", "<i8"), ("run_start", "<i8"),
                             ("emit_hop", "<i8"), ("seg_start", "<i8"), ("seg_len", "<i4"), ("score", "<f4")])
 EV_TIMEOUT, EV_SCORED = 1, 2
+# ewk_stream_blob: the 96-byte header at offset 0 of a stream blob (ewk_export_streams); the rest of a blob is opaque
+STREAM_BLOB_HEADER_DTYPE = np.dtype([
+    ("magic", "<u4"), ("version", "<u4"), ("n_streams", "<i4"), ("ring_samples", "<i4"), ("slack_samples", "<i4"),
+    ("pcm_format", "<i4"), ("n_mfcc", "<i4"), ("preemphasis_bits", "<u4"), ("meta_bytes", "<i4"),
+    ("n_templates", "<i4"), ("tail_floats", "<i4"), ("reserved", "<i4"), ("ids_offset", "<i8"), ("meta_offset", "<i8"),
+    ("template_offset", "<i8"), ("bulk_offset", "<i8"), ("bulk_row_bytes", "<i8"), ("total_bytes", "<i8")])
+STREAM_BLOB_MAGIC, STREAM_BLOB_VERSION = 0x534B5745, 1
+STREAM_META_BYTES, STREAM_TEMPLATE_BYTES = 304, 176       # per-stream meta record, per-slot template record
+
+
+def stream_blob_layout(ring_samples, slack_samples, pcm_format, n, n_templates, tail_floats):
+    """Section offsets of a version-1 stream blob of n streams (what ewk_export_streams writes and ewk_import_streams
+    recomputes): header | int32 ids | meta records | template records | bulk rows, each 16-byte aligned.  A bulk row is
+    the raw ring (P = ring + slack rounded up to 64 samples), the block sums (P // 1600 doubles), the chunk mean squares
+    (2 * (ring // 160) doubles) and tail_floats K8 input-tail floats.  ewk_stream_blob_bytes is this total with
+    n_templates = max_templates and tail_floats = the context's widest K8 tail, rounded up to 4."""
+    a16 = lambda v: (v + 15) // 16 * 16                                          # noqa: E731
+    P = (ring_samples + slack_samples + 63) // 64 * 64
+    esz = 2 if pcm_format == PCM_I16 else 4
+    ss_off = P * esz
+    ms_off = ss_off + a16(8 * (P // 1600))
+    tail_off = ms_off + 16 * max(1, ring_samples // 160)
+    row = a16(tail_off + 4 * tail_floats)
+    ids = STREAM_BLOB_HEADER_DTYPE.itemsize
+    meta = a16(ids + 4 * n)
+    tmpl = meta + STREAM_META_BYTES * n
+    bulk = tmpl + STREAM_TEMPLATE_BYTES * n_templates
+    return dict(ids_offset=ids, meta_offset=meta, template_offset=tmpl, bulk_offset=bulk, bulk_row_bytes=row,
+                total_bytes=bulk + row * n, ss_off=ss_off, ms_off=ms_off, tail_off=tail_off)
 
 
 def _declare_stream_protos(lib):
@@ -316,6 +345,9 @@ def _declare_stream_protos(lib):
         "ewk_tick_ready": (C.c_int, [vp, i32, _p(C.c_int32), vp, vp, vp, vp]),
         "ewk_stream_input": (C.c_int, [vp, i32, _p(C.c_int32), _p(i64)]),
         "ewk_reset_streams": (C.c_int, [vp, _p(C.c_int32), i32]),
+        "ewk_stream_blob_bytes": (C.c_int64, [vp, i32]),
+        "ewk_export_streams": (C.c_int, [vp, _p(C.c_int32), i32, vp, i64, i32]),
+        "ewk_import_streams": (C.c_int, [vp, _p(C.c_int32), i32, vp, i64, i32]),
         "ewk_tick": (C.c_int, [vp, i32]),
         "ewk_set_overlap": (C.c_int, [vp, i32]),
         "ewk_join": (C.c_int, [vp]),
@@ -572,6 +604,48 @@ def _bank_methods():
         lst = lst.astype(np.int32)
         self._ck(self.lib.ewk_reset_streams(self.h, lst.ctypes.data_as(_p(C.c_int32)), int(lst.size)))
 
+    def stream_blob_bytes(self, n):
+        """Bytes that always hold a blob of n of this context's streams (include/ewk.h: ewk_stream_blob_bytes), for the
+        input rates the context has seen so far."""
+        v = int(self.lib.ewk_stream_blob_bytes(self.h, int(n)))
+        if v < 0:
+            self._ck(v)
+        return v
+
+    def export_streams(self, streams, where=HOST, out=None):
+        """Snapshot the listed streams into a blob (include/ewk.h: ewk_export_streams); the streams go on untouched.
+        where=HOST returns the blob as a np.uint8 array of its exact length (save it with np.save).  where=DEVICE writes
+        it into out = (ptr, cap), 16-byte aligned memory of this context's device, and returns None: the blob's length is
+        its header's total_bytes, and import_streams takes (ptr, cap) as it is."""
+        st = _stream_list(streams)
+        sp = st.ctypes.data_as(_p(C.c_int32))
+        if where == DEVICE:
+            if out is None:
+                raise ValueError("a device export takes out=(ptr, cap)")
+            ptr, cap = out
+            self._ck(self.lib.ewk_export_streams(self.h, sp, len(st), C.c_void_p(int(ptr)), int(cap), DEVICE))
+            return None
+        if out is not None:
+            raise ValueError("out is for where=DEVICE; a host export returns its array")
+        cap = self.stream_blob_bytes(len(st))
+        buf = np.zeros(cap, np.uint8)
+        self._ck(self.lib.ewk_export_streams(self.h, sp, len(st), buf.ctypes.data, cap, HOST))
+        n = int(buf[:STREAM_BLOB_HEADER_DTYPE.itemsize].view(STREAM_BLOB_HEADER_DTYPE)[0]["total_bytes"])
+        return buf[:n]
+
+    def import_streams(self, streams, blob, where=HOST):
+        """Make blob stream i stream streams[i] of this context (include/ewk.h: ewk_import_streams).  blob: a host
+        np.uint8 array (any exported blob, e.g. np.load of a saved one), or with where=DEVICE (ptr, length) in this
+        context's device memory.  The event queue must be empty (poll first)."""
+        st = _stream_list(streams)
+        sp = st.ctypes.data_as(_p(C.c_int32))
+        if where == DEVICE:
+            ptr, length = blob
+            self._ck(self.lib.ewk_import_streams(self.h, sp, len(st), C.c_void_p(int(ptr)), int(length), DEVICE))
+            return
+        b = np.ascontiguousarray(blob).view(np.uint8).reshape(-1)
+        self._ck(self.lib.ewk_import_streams(self.h, sp, len(st), b.ctypes.data if b.size else None, int(b.size), HOST))
+
     def stream_input(self, stream):
         """-> (input rate latched by the stream's first push (0: none yet), input samples received)."""
         sr, n = C.c_int32(), C.c_int64()
@@ -803,7 +877,7 @@ def _bank_methods():
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
     for f in (prepare_segments, dense_scores, dense_scores_streams, dense_ready, dense_detect, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
-              push_resampled_each, push_streams, tick_ready, reset_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
+              push_resampled_each, push_streams, tick_ready, reset_streams, stream_blob_bytes, export_streams, import_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
               set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count):
         setattr(Context, f.__name__, f)
 

@@ -22,6 +22,22 @@ DENSE_ROUND = 500                 # hops per ewk_dense_ready call of WakeWordBan
 EV_TIMEOUT, EV_SCORED = _lib.EV_TIMEOUT, _lib.EV_SCORED
 
 
+def stream_blob_rates(blob) -> np.ndarray:
+    """The input rate each stream of a host blob (export_streams) is latched to (0: none yet), from its meta records."""
+    b = np.ascontiguousarray(blob).view(np.uint8).reshape(-1)
+    hsz = _lib.STREAM_BLOB_HEADER_DTYPE.itemsize
+    if b.size < hsz:
+        raise ValueError("not a stream blob")
+    h = b[:hsz].view(_lib.STREAM_BLOB_HEADER_DTYPE)[0]
+    if int(h["magic"]) != _lib.STREAM_BLOB_MAGIC or int(h["meta_bytes"]) != _lib.STREAM_META_BYTES:
+        raise ValueError("not a stream blob of version 1")
+    n, off = int(h["n_streams"]), int(h["meta_offset"])
+    if n < 0 or off + n * _lib.STREAM_META_BYTES > b.size:
+        raise ValueError("truncated stream blob")
+    rec = b[off:off + n * _lib.STREAM_META_BYTES].reshape(n, _lib.STREAM_META_BYTES)
+    return np.ascontiguousarray(rec[:, 52:56]).view("<i4").reshape(-1)      # StreamMeta.rate
+
+
 class WakeWordBank:
     """N independent audio streams, one GPU.
 
@@ -121,6 +137,58 @@ class WakeWordBank:
             for s in dict.fromkeys(lst):
                 self.set_stream(s, **overrides)
         return events
+
+    # ---- migration
+    def export_streams(self, streams) -> np.ndarray:
+        """A host blob (np.uint8) holding the listed streams' whole live state (include/ewk.h: ewk_export_streams): ring,
+        gate, timing, dense cursors, detector and K8 input tails.  The streams go on untouched and their queued events
+        stay here.  Save it with np.save for a checkpoint; import_streams on any bank with the same buffer_seconds,
+        max_push_seconds / frame_size (the slack), pcm_dtype, n_mfcc and preemphasis takes it."""
+        return self.ctx.export_streams(streams)
+
+    def import_streams(self, streams, blob) -> np.ndarray:
+        """Blob stream i becomes stream streams[i] of this bank and goes on exactly as it would have where it was
+        exported (include/ewk.h: ewk_import_streams); its parameters come with it.  Drains the event queue first and
+        returns those events (handle them as poll()'s), as reset does.  ValueError for a stream latched to an input rate
+        other than this bank's sample_rate (a later push would fail).  Moved streams sit at their own positions: feed
+        them with push_streams / step_streams, as after staggered resets."""
+        lst = [int(s) for s in np.asarray(streams, dtype=np.int64).reshape(-1)]
+        for i, rate in enumerate(stream_blob_rates(blob)):
+            if rate not in (0, self.sample_rate):
+                raise ValueError(f"blob stream {i} takes {rate} Hz input; this bank takes {self.sample_rate} Hz")
+        events = self.poll()
+        self.ctx.import_streams(lst, blob)
+        return events
+
+    def move_streams(self, streams, dst: "WakeWordBank", dst_streams):
+        """Move live calls: streams of this bank become dst_streams of dst (dst may be this bank).  In order: drain dst's
+        queue, export, import, drain this bank's queue, reset the source slots that did not receive a stream.  Returns
+        (source_events, destination_events): the drained events, with the ids of the bank that raised them.  A stream
+        latched to another rate than dst's sample_rate is refused before anything is drained; if the import itself fails
+        (e.g. banks of another geometry), the exception carries dst's drained events as `drained_events` and the source
+        is untouched."""
+        src = [int(s) for s in np.asarray(streams, dtype=np.int64).reshape(-1)]
+        dst_l = [int(s) for s in np.asarray(dst_streams, dtype=np.int64).reshape(-1)]
+        if len(src) != len(dst_l):
+            raise ValueError("one destination stream per source stream")
+        for s in src:                                  # refused before anything is drained
+            rate = self.ctx.stream_input(s)[0]
+            if rate not in (0, dst.sample_rate):
+                raise ValueError(f"stream {s} takes {rate} Hz input; the destination bank takes {dst.sample_rate} Hz")
+        dst_events = dst.poll()
+        blob = self.export_streams(src)
+        try:
+            more = dst.import_streams(dst_l, blob)
+        except Exception as e:                         # the caller still gets what was drained
+            e.drained_events = dst_events
+            raise
+        if len(more):
+            dst_events = np.concatenate([dst_events, more])
+        src_events = self.poll()
+        free = [s for s in src if dst is not self or s not in dst_l]
+        if free:
+            self.ctx.reset_streams(free)
+        return src_events, dst_events
 
     # ---- data plane
     def push(self, pcm, where=_lib.HOST):

@@ -217,6 +217,8 @@ void ewk_ctx::release() {
     if (h_det_map) cudaFreeHost(h_det_map);
     h_det_map = nullptr; det_map_cap = 0;
     b_reset.free();
+    b_blob.free();
+    b_mig.free();
     if (own_stream) cudaStreamDestroy(own_stream);
     d_tables = nullptr; d_tmpl = nullptr; own_stream = nullptr; copy_stream = nullptr;
 }
@@ -1443,6 +1445,355 @@ extern "C" int ewk_reset_streams(ewk_ctx* ctx, const int32_t* streams, int n) {
         ctx->h_written[s] = 0; ctx->h_visible_lb[s] = 0; ctx->h_tick[s] = 0; ctx->h_dense_next[s] = 1; ctx->h_det_next[s] = 1;
         ctx->h_frame_size[s] = 0; ctx->h_rate[s] = 0; ctx->h_inputs[s] = 0;
     }
+    return EWK_OK;
+}
+
+// ------------------------------------------------------------------------------------------ K10 (stream migration)
+// Blob version 1: header (ewk_stream_blob) | int32 source ids [n] | StreamMeta [n] | BlobTemplate [n_templates] | bulk
+// rows [n] (MigrateGeom), each section 16-byte aligned.  The layout follows from the fingerprint and three counts, so
+// an importer recomputes it and takes no offset on trust.
+struct BlobTemplate {       // a template slot a stream of the blob is scored against, as the source context holds it
+    int32_t slot, valid;
+    int64_t n_samples;
+    float mean[N_MFCC], std[N_MFCC];
+};
+static_assert(sizeof(BlobTemplate) == 176 && sizeof(ewk_stream_blob) == 96, "blob version 1 layout");
+
+struct BlobLayout { long long ids, meta, tmpl, bulk, total; MigrateGeom g; };
+
+static long long align16(long long v) { return (v + 15) & ~15LL; }
+
+static BlobLayout blob_layout(const BankView& B, int n, int n_tmpl, int tail_floats) {
+    BlobLayout L{};
+    const long long esz = B.fmt == 1 ? 2 : 4;
+    L.g.ss_off = (long long)B.P * esz;
+    L.g.ms_off = L.g.ss_off + align16(8LL * B.NB);
+    L.g.tail_off = L.g.ms_off + 16LL * B.chunk_cap;
+    L.g.tail_floats = tail_floats;
+    L.g.row_bytes = align16(L.g.tail_off + 4LL * tail_floats);
+    L.ids = (long long)sizeof(ewk_stream_blob);
+    L.meta = align16(L.ids + 4LL * n);
+    L.tmpl = L.meta + (long long)sizeof(StreamMeta) * n;
+    L.bulk = L.tmpl + (long long)sizeof(BlobTemplate) * n_tmpl;
+    L.total = L.bulk + L.g.row_bytes * n;
+    return L;
+}
+
+// live K8 input tail of a stream latched to `rate` after `inputs` input samples: inputs [rs_tail_start, inputs), the only
+// part of its tail row a later push reads (0 at rate 0 or 16000: direct pushes keep none); -1 for a rate K8 rejects
+static int tail_len_of(int rate, long long inputs) {
+    if (rate == 0 || rate == RS_TARGET) return 0;
+    ResampleDesign d;
+    if (rate < 1000 || rate > 768000 || !rs_design(rate, d) || inputs < 0) return -1;
+    return (int)(inputs - rs_tail_start(inputs, d));
+}
+
+static int round4(int v) { return (v + 3) & ~3; }
+
+static int n_mfcc_of(const ewk_config& c) { return c.n_mfcc > 0 ? c.n_mfcc : N_MFCC; }
+
+static uint32_t float_bits(float f) { uint32_t u; std::memcpy(&u, &f, 4); return u; }
+
+static int check_stream_list(ewk_ctx* ctx, const char* who, const int32_t* streams, int n) {
+    const int ns = ctx->bank.n_streams;
+    if (n < 0 || (n > 0 && !streams)) { ctx->fail("%s: bad stream list (n=%d)", who, n); return EWK_ERR_ARG; }
+    std::vector<char> seen((size_t)ns, 0);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        if (s < 0 || s >= ns) { ctx->fail("%s: bad stream %d (context has %d)", who, s, ns); return EWK_ERR_ARG; }
+        if (seen[s]) { ctx->fail("%s: stream %d is listed twice", who, s); return EWK_ERR_ARG; }
+        seen[s] = 1;
+    }
+    return EWK_OK;
+}
+
+static int check_blob_ptr(ewk_ctx* ctx, const char* who, const void* blob, int where) {
+    if (!blob) { ctx->fail("%s: blob is NULL", who); return EWK_ERR_ARG; }
+    if (where == EWK_HOST) return EWK_OK;
+    if (where != EWK_DEVICE) { ctx->fail("%s: where must be EWK_HOST or EWK_DEVICE", who); return EWK_ERR_ARG; }
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, blob) != cudaSuccess) {
+        cudaGetLastError();
+        ctx->fail("%s: the device blob is not CUDA memory", who);
+        return EWK_ERR_ARG;
+    }
+    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != ctx->device) {
+        ctx->fail("%s: the device blob is not memory of the context's device %d (copy it there first)", who, ctx->device);
+        return EWK_ERR_ARG;
+    }
+    if ((uintptr_t)blob & 15) { ctx->fail("%s: the device blob must be 16-byte aligned", who); return EWK_ERR_ARG; }
+    return EWK_OK;
+}
+
+static dim3 migrate_grid(const BankView& B, int n) {
+    const size_t ring_bytes = (size_t)B.P * (B.fmt == 1 ? 2 : 4);
+    return dim3((unsigned)((ring_bytes + RESET_SLICE - 1) / RESET_SLICE), (unsigned)std::min(n, 65535));
+}
+
+extern "C" int64_t ewk_stream_blob_bytes(const ewk_ctx* ctx, int n) {
+    if (!ctx || n < 0) return EWK_ERR_ARG;
+    if (ctx->bank.n_streams == 0) return EWK_ERR_STATE;
+    return blob_layout(ctx->bank, n, ctx->cfg.max_templates, round4(ctx->rs_tail_cap)).total;
+}
+
+extern "C" int ewk_export_streams(ewk_ctx* ctx, const int32_t* streams, int n, void* blob, int64_t blob_cap, int where) {
+    if (!ctx) return EWK_ERR_ARG;
+    const char* who = "ewk_export_streams";
+    int rc = need_streams(ctx, who);                          // overlap mode: K3 may still write the result records
+    if (rc) return rc;
+    BankView& B = ctx->bank;
+    rc = check_stream_list(ctx, who, streams, n);
+    if (rc) return rc;
+    rc = check_blob_ptr(ctx, who, blob, where);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    rc = ctx->flush_pending();                                // its samples belong to the streams
+    if (rc) return rc;
+    const int T = ctx->cfg.max_templates;
+    std::vector<char> used((size_t)T, 0);
+    int tail = 0;
+    for (int i = 0; i < n; i++) {
+        const StreamParams& p = ctx->h_prm[streams[i]];
+        for (int k = p.template_first; k < p.template_first + p.template_count; k++) used[k] = 1;
+        tail = std::max(tail, tail_len_of(ctx->h_rate[streams[i]], ctx->h_inputs[streams[i]]));
+    }
+    const int n_tmpl = (int)std::count(used.begin(), used.end(), 1);
+    const BlobLayout L = blob_layout(B, n, n_tmpl, round4(tail));
+    if (blob_cap < L.total) {
+        ctx->fail("%s: blob_cap %lld is below the %lld bytes of this blob", who, (long long)blob_cap, L.total);
+        return EWK_ERR_ARG;
+    }
+    // everything in front of the bulk rows is host knowledge; K10 adds each stream's device state to its meta record
+    std::vector<char> pre((size_t)L.bulk, 0);
+    ewk_stream_blob* h = reinterpret_cast<ewk_stream_blob*>(pre.data());
+    h->magic = EWK_STREAM_BLOB_MAGIC; h->version = EWK_STREAM_BLOB_VERSION; h->n_streams = n;
+    h->ring_samples = ctx->cfg.ring_samples; h->slack_samples = ctx->cfg.slack_samples; h->pcm_format = ctx->cfg.pcm_format;
+    h->n_mfcc = n_mfcc_of(ctx->cfg); h->preemphasis_bits = float_bits(ctx->cfg.preemphasis);
+    h->meta_bytes = (int32_t)sizeof(StreamMeta); h->n_templates = n_tmpl; h->tail_floats = L.g.tail_floats;
+    h->ids_offset = L.ids; h->meta_offset = L.meta; h->template_offset = L.tmpl; h->bulk_offset = L.bulk;
+    h->bulk_row_bytes = L.g.row_bytes; h->total_bytes = L.total;
+    if (n > 0) std::memcpy(pre.data() + L.ids, streams, sizeof(int32_t) * (size_t)n);
+    StreamMeta* meta = reinterpret_cast<StreamMeta*>(pre.data() + L.meta);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        StreamMeta& m = meta[i];
+        m.written = ctx->h_written[s]; m.visible_lb = ctx->h_visible_lb[s]; m.tick = ctx->h_tick[s];
+        m.dense_next = ctx->h_dense_next[s]; m.det_next = ctx->h_det_next[s]; m.inputs = ctx->h_inputs[s];
+        m.frame_size = ctx->h_frame_size[s]; m.rate = ctx->h_rate[s]; m.tail_len = tail_len_of(ctx->h_rate[s], ctx->h_inputs[s]);
+        m.prm = ctx->h_prm[s];
+    }
+    BlobTemplate* tp = reinterpret_cast<BlobTemplate*>(pre.data() + L.tmpl);
+    for (int k = 0, j = 0; k < T; k++) {
+        if (!used[k]) continue;
+        const TemplateFeat& tf = ctx->h_tmpl[k];
+        tp[j].slot = k; tp[j].valid = tf.valid; tp[j].n_samples = tf.n_samples;
+        std::memcpy(tp[j].mean, tf.mean, sizeof(tf.mean));
+        std::memcpy(tp[j].std, tf.std, sizeof(tf.std));
+        j++;
+    }
+    char* target = (char*)blob;
+    if (where == EWK_HOST) {                                  // the blob forms in scratch and crosses PCIe in one copy
+        CK(ctx->b_blob.ensure((size_t)L.total));
+        target = (char*)ctx->b_blob.p;
+    }
+    CK(cudaMemcpyAsync(target, pre.data(), (size_t)L.bulk, cudaMemcpyHostToDevice, ctx->stream));
+    if (n > 0) {
+        stream_export_kernel<<<migrate_grid(B, n), RESET_THREADS, 0, ctx->stream>>>(
+            B, (const int*)(target + L.ids), n, (const DetState*)ctx->b_det_state.p, ctx->d_rs_tail, ctx->rs_tail_cap,
+            (StreamMeta*)(target + L.meta), target + L.bulk, L.g);
+        CK(cudaGetLastError());
+        ctx->launches++;
+    }
+    if (where == EWK_HOST) CK(cudaMemcpyAsync(blob, target, (size_t)L.total, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return EWK_OK;
+}
+
+// the name of the first field of a meta record that no sequence of calls produces in a context of this geometry
+static const char* bad_meta_field(const ewk_ctx* ctx, const StreamMeta& m, int tail_floats) {
+    const BankView& B = ctx->bank;
+    auto frame_ok = [&](int fs) { return fs == 0 || (fs >= MIN_FRAME_SIZE && fs <= B.R); };
+    if (m.written < 0 || m.st.written != m.written) return "written";
+    if (m.st.ss_from < 0 || m.st.ss_from > m.written) return "ss_from";
+    if (m.st.visible < 0 || m.st.visible > m.written || m.visible_lb < 0 || m.visible_lb > m.written) return "visible";
+    if (m.tick < 0 || m.st.tick < 0) return "tick";
+    if (!frame_ok(m.frame_size) || !frame_ok(m.st.frame_size)) return "frame_size";
+    if (m.st.state < ST_WAITING || m.st.state > ST_AFTER_SOUND) return "state";
+    const long long last_hop = m.written / HOP + 1;
+    if (m.dense_next < 1 || m.dense_next > last_hop) return "dense cursor";
+    if (m.det_next < 1 || m.det_next > last_hop) return "detect cursor";
+    const int tl = tail_len_of(m.rate, m.inputs);
+    if (tl < 0) return m.inputs < 0 ? "inputs" : "rate";
+    if (m.rate == 0 ? (m.inputs != 0 || m.written != 0) : m.rate == RS_TARGET ? m.inputs != m.written : false) return "inputs";
+    if (m.rate != 0 && m.rate != RS_TARGET) {
+        ResampleDesign d;
+        rs_design(m.rate, d);
+        if (m.inputs < 0 || rs_ready(m.inputs, d) != m.written) return "inputs";
+    }
+    if (m.tail_len != tl || tl > tail_floats) return "tail_len";
+    if (m.det.mode < DET_IDLE || m.det.mode > DET_SPENT) return "detector mode";
+    const StreamParams& p = m.prm;
+    if (!(p.pre_speech_silence > 0) || !(p.speech_duration_min > 0) || !(p.speech_duration_max > 0) ||
+        !(p.speech_duration_min <= p.speech_duration_max) || !(p.post_speech_silence > 0) || !frame_ok(p.frame_size))
+        return "stream parameters";
+    if (p.template_first < 0 || p.template_count < 0 || p.template_first + p.template_count > ctx->cfg.max_templates)
+        return "template range";
+    return nullptr;
+}
+
+extern "C" int ewk_import_streams(ewk_ctx* ctx, const int32_t* streams, int n, const void* blob, int64_t blob_len,
+                                  int where) {
+    if (!ctx) return EWK_ERR_ARG;
+    const char* who = "ewk_import_streams";
+    int rc = need_streams(ctx, who);                          // overlap mode: K3 still reads the rings
+    if (rc) return rc;
+    BankView& B = ctx->bank;
+    rc = check_stream_list(ctx, who, streams, n);
+    if (rc) return rc;
+    rc = check_blob_ptr(ctx, who, blob, where);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    ewk_stream_blob h;
+    if (blob_len < (int64_t)sizeof(h)) { ctx->fail("%s: blob_len %lld holds no blob header", who, (long long)blob_len); return EWK_ERR_ARG; }
+    if (where == EWK_HOST) std::memcpy(&h, blob, sizeof(h));
+    else {
+        CK(cudaMemcpyAsync(&h, blob, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    if (h.magic != EWK_STREAM_BLOB_MAGIC || h.version != EWK_STREAM_BLOB_VERSION) {
+        ctx->fail("%s: not a stream blob of version %d (magic 0x%08x, version %u)", who, EWK_STREAM_BLOB_VERSION, h.magic, h.version);
+        return EWK_ERR_ARG;
+    }
+    if (h.n_streams != n) { ctx->fail("%s: the blob holds %d streams, the list %d", who, h.n_streams, n); return EWK_ERR_ARG; }
+    const struct { const char* name; long long blob, mine; } fp[] = {
+        {"ring_samples", h.ring_samples, ctx->cfg.ring_samples}, {"slack_samples", h.slack_samples, ctx->cfg.slack_samples},
+        {"pcm_format", h.pcm_format, ctx->cfg.pcm_format}, {"n_mfcc", h.n_mfcc, n_mfcc_of(ctx->cfg)},
+        {"preemphasis", h.preemphasis_bits, float_bits(ctx->cfg.preemphasis)}};
+    for (const auto& f : fp)
+        if (f.blob != f.mine) {
+            ctx->fail("%s: the blob's %s (%lld) differs from the context's (%lld)", who, f.name, f.blob, f.mine);
+            return EWK_ERR_ARG;
+        }
+    if (h.meta_bytes != (int32_t)sizeof(StreamMeta) || h.n_templates < 0 || h.n_templates > EWK_MAX_TEMPLATES ||
+        h.tail_floats < 0 || (h.tail_floats & 3) || h.tail_floats > 1 << 20) {
+        ctx->fail("%s: bad blob header (meta_bytes %d, n_templates %d, tail_floats %d)", who, h.meta_bytes, h.n_templates,
+                  h.tail_floats);
+        return EWK_ERR_ARG;
+    }
+    const BlobLayout L = blob_layout(B, n, h.n_templates, h.tail_floats);
+    if (h.ids_offset != L.ids || h.meta_offset != L.meta || h.template_offset != L.tmpl || h.bulk_offset != L.bulk ||
+        h.bulk_row_bytes != L.g.row_bytes || h.total_bytes != L.total) {
+        ctx->fail("%s: the blob's section offsets are not those of its header's counts", who);
+        return EWK_ERR_ARG;
+    }
+    if (blob_len < L.total) {
+        ctx->fail("%s: blob_len %lld is below the blob's %lld bytes", who, (long long)blob_len, L.total);
+        return EWK_ERR_ARG;
+    }
+    std::vector<char> dev_pre;
+    const char* pre = (const char*)blob;
+    if (where == EWK_DEVICE) {
+        dev_pre.resize((size_t)L.bulk);
+        CK(cudaMemcpyAsync(dev_pre.data(), blob, (size_t)L.bulk, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        pre = dev_pre.data();
+    }
+    // a private copy of the meta records: what is checked is what the kernel gets
+    std::vector<StreamMeta> meta((size_t)n);
+    if (n > 0) std::memcpy(meta.data(), pre + L.meta, sizeof(StreamMeta) * (size_t)n);
+    const BlobTemplate* tp = reinterpret_cast<const BlobTemplate*>(pre + L.tmpl);
+    std::vector<int> tmpl_of((size_t)ctx->cfg.max_templates, -1);       // slot -> its record
+    for (int j = 0; j < h.n_templates; j++) {
+        if (tp[j].slot < 0 || tp[j].slot >= ctx->cfg.max_templates || tmpl_of[tp[j].slot] >= 0) {
+            ctx->fail("%s: template record %d names slot %d (the context has %d slots)", who, j, tp[j].slot, ctx->cfg.max_templates);
+            return EWK_ERR_ARG;
+        }
+        tmpl_of[tp[j].slot] = j;
+    }
+    bool need_det = false;
+    int need_tail = 0;
+    for (int i = 0; i < n; i++) {
+        const StreamMeta& m = meta[i];
+        if (const char* f = bad_meta_field(ctx, m, h.tail_floats)) {
+            ctx->fail("%s: blob stream %d: %s is outside what the entry points produce", who, i, f);
+            return EWK_ERR_ARG;
+        }
+        for (int k = m.prm.template_first; k < m.prm.template_first + m.prm.template_count; k++)
+            if (tmpl_of[k] < 0) { ctx->fail("%s: blob stream %d: template slot %d has no record", who, i, k); return EWK_ERR_ARG; }
+        const DetState z{};
+        need_det |= std::memcmp(&m.det, &z, sizeof(z)) != 0;
+        need_tail = std::max(need_tail, m.tail_len);
+    }
+    for (int i = 0; i < n; i++) {
+        const StreamParams& p = meta[i].prm;
+        for (int k = p.template_first; k < p.template_first + p.template_count; k++) {
+            const BlobTemplate& t = tp[tmpl_of[k]];
+            const TemplateFeat& mine = ctx->h_tmpl[k];
+            if (t.valid != mine.valid || t.n_samples != mine.n_samples || std::memcmp(t.mean, mine.mean, sizeof(t.mean)) ||
+                std::memcmp(t.std, mine.std, sizeof(t.std))) {
+                ctx->fail("%s: blob stream %d (source stream %d) is scored against template slot %d, which differs in "
+                          "this context", who, i, reinterpret_cast<const int32_t*>(pre + L.ids)[i], k);
+                return EWK_ERR_STATE;
+            }
+        }
+    }
+    rc = ctx->flush_pending();                                // a pending host push belongs to the slots' old sessions
+    if (rc) return rc;
+    int cnt[2] = {0, 0};
+    CK(cudaMemcpyAsync(cnt, B.ev_count, sizeof(cnt), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    if (cnt[0] != 0 || cnt[1] != 0) {
+        ctx->fail("%s: %d events are queued; poll first", who, cnt[0]);
+        return EWK_ERR_STATE;
+    }
+    if (n == 0) return EWK_OK;
+    if (need_det && !ctx->b_det_state.p) {
+        CK(ctx->b_det_state.ensure(sizeof(DetState) * (size_t)B.n_streams));
+        CK(cudaMemsetAsync(ctx->b_det_state.p, 0, sizeof(DetState) * (size_t)B.n_streams, ctx->stream));
+    }
+    if (need_tail > 0) {
+        rc = ctx->ensure_rs_tail(need_tail);
+        if (rc) return rc;
+    }
+    // one upload: the destination list, then the checked small state
+    const size_t list_bytes = (size_t)align16(4LL * n);
+    std::vector<char> up(list_bytes + sizeof(MigrateSmall) * (size_t)n, 0);
+    std::memcpy(up.data(), streams, sizeof(int32_t) * (size_t)n);
+    MigrateSmall* sm = reinterpret_cast<MigrateSmall*>(up.data() + list_bytes);
+    for (int i = 0; i < n; i++) {
+        sm[i].prm = meta[i].prm;
+        sm[i].st = meta[i].st;
+        sm[i].st.last_ev = -1;                                // a queue index of another context means nothing here
+        sm[i].res = meta[i].res;
+        sm[i].det = meta[i].det;
+        sm[i].tail_len = meta[i].tail_len;
+    }
+    CK(ctx->b_mig.ensure(up.size()));
+    CK(cudaMemcpyAsync(ctx->b_mig.p, up.data(), up.size(), cudaMemcpyHostToDevice, ctx->stream));
+    const char* bulk = (const char*)blob + L.bulk;
+    if (where == EWK_HOST) {
+        CK(ctx->b_blob.ensure((size_t)(L.total - L.bulk)));
+        CK(cudaMemcpyAsync(ctx->b_blob.p, bulk, (size_t)(L.total - L.bulk), cudaMemcpyHostToDevice, ctx->stream));
+        bulk = (const char*)ctx->b_blob.p;
+    }
+    stream_import_kernel<<<migrate_grid(B, n), RESET_THREADS, 0, ctx->stream>>>(
+        B, (const int*)ctx->b_mig.p, (const MigrateSmall*)((const char*)ctx->b_mig.p + list_bytes), n, bulk, L.g,
+        (long long*)ctx->b_keep_end.p, (DetState*)ctx->b_det_state.p, ctx->d_rs_tail, ctx->rs_tail_cap);
+    CK(cudaGetLastError());
+    ctx->launches++;
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        const StreamMeta& m = meta[i];
+        ctx->h_written[s] = m.written; ctx->h_visible_lb[s] = m.visible_lb; ctx->h_tick[s] = m.tick;
+        ctx->h_dense_next[s] = m.dense_next; ctx->h_det_next[s] = m.det_next; ctx->h_frame_size[s] = m.frame_size;
+        ctx->h_rate[s] = m.rate; ctx->h_inputs[s] = m.inputs; ctx->h_prm[s] = m.prm;
+    }
+    ctx->max_post = 0.0;
+    for (int s = 0; s < B.n_streams; s++) ctx->max_post = std::max(ctx->max_post, ctx->h_prm[s].post_speech_silence);
+    // K2 takes block sums of ticks at or past a stream's ss_from only when every push since the last tick formed them;
+    // an imported stream's sums came from another context's pushes, so K2 reads its samples on the next tick
+    ctx->all_presummed = false;
+    CK(cudaStreamSynchronize(ctx->stream));
     return EWK_OK;
 }
 

@@ -103,6 +103,8 @@ struct ewk_ctx {
     void* h_det_map = nullptr;
     size_t det_map_cap = 0;
     ewk::DevBuf b_reset;                     // K9's stream list
+    ewk::DevBuf b_blob;                      // K10: a host blob's device copy (export: the whole blob; import: its bulk rows)
+    ewk::DevBuf b_mig;                       // K10 import: the destination list and the checked small state, one upload
     int flush_pending();
     ewk::DevBuf b_stage2[2];
     ewk::DevBuf b_raw[2];                    // compact host input: G.711 codes (ewk_push_g711, decoded into b_stage2) or a native-rate feed

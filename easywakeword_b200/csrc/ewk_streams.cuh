@@ -1545,4 +1545,107 @@ stream_reset_kernel(BankView B, const int* __restrict__ list, int n, long long* 
     }
 }
 
+// ------------------------------------------------------------------------------------ K10 (stream migration)
+// ewk_export_streams / ewk_import_streams (include/ewk.h): a stream's whole device state to and from row y of a blob's
+// bulk section, in K9's grid shape.  CTA (x, y) copies 32 KB slice x of the ring row with 16-byte loads and stores;
+// the CTAs of slice 0 also copy the block_ss, chunk_ms and K8 tail rows and the small state (StreamState, result record, DetState).  One read and one
+// write per byte: HBM-bound.  Rings hold absolute sample a at a % P in every context with the same ring_samples and
+// slack_samples, and block_ss holds block b at b % NB, so every row moves verbatim.
+// A bulk row (all parts 16-byte aligned): ring [P * esz] | block_ss [NB] doubles, zero-padded | chunk_ms [2 chunk_cap]
+// doubles | K8 input tail [tail_floats] floats: the stream's live inputs [t0, c) (StreamMeta.tail_len of them), zeros
+// beyond, so a blob carries nothing an earlier occupant of the slot left in its tail row.
+struct MigrateGeom { long long row_bytes, ss_off, ms_off, tail_off; int tail_floats, pad; };
+
+// One record per stream of a blob's meta section.  The host fills the mirrors and the parameters; on export K10 fills
+// st, res and det.  Import reads it on the host only: the kernel takes the checked copy (MigrateSmall).
+struct StreamMeta {
+    long long written, visible_lb, tick, dense_next, det_next, inputs;   // host mirrors of the context
+    int frame_size, rate, tail_len, pad;                                 // tail_len: live K8 tail inputs c - t0 (0 at 16 kHz)
+    StreamParams prm;
+    StreamState st;
+    StreamResult res;
+    DetState det;                                                        // zeros when the source had no detector state
+};
+static_assert(sizeof(StreamMeta) == 304, "StreamMeta is part of blob version 1");
+
+// the small state is copied by the CTA's threads in 8-byte words (every struct here is a multiple of 8 bytes)
+template <class T> __device__ __forceinline__ void copy_words(T* dst, const T* src) {
+    static_assert(sizeof(T) % 8 == 0, "8-byte words");
+    const long long* a = reinterpret_cast<const long long*>(src);
+    long long* b = reinterpret_cast<long long*>(dst);
+    for (int i = threadIdx.x; i < (int)(sizeof(T) / 8); i += blockDim.x) b[i] = a[i];
+}
+
+struct MigrateSmall {       // import: the checked small state of one stream (last_ev already -1)
+    StreamParams prm;
+    StreamState st;
+    StreamResult res;
+    DetState det;
+    int tail_len, pad;
+};
+
+__global__ void __launch_bounds__(RESET_THREADS)
+stream_export_kernel(BankView B, const int* __restrict__ list, int n, const DetState* __restrict__ det,
+                     const float* __restrict__ tail, int tail_cap, StreamMeta* meta, char* bulk, MigrateGeom g) {
+    const size_t ring_bytes = (size_t)B.P * (B.fmt == 1 ? 2 : 4);
+    for (int y = blockIdx.y; y < n; y += gridDim.y) {
+        const int s = list[y];
+        const int4* src = reinterpret_cast<const int4*>(reinterpret_cast<const char*>(B.ring) + (size_t)s * ring_bytes);
+        char* row = bulk + (size_t)y * g.row_bytes;
+        int4* dst = reinterpret_cast<int4*>(row);
+        const size_t w0 = (size_t)blockIdx.x * (RESET_SLICE / 16), w1 = min(w0 + RESET_SLICE / 16, ring_bytes / 16);
+        for (size_t w = w0 + threadIdx.x; w < w1; w += RESET_THREADS) dst[w] = src[w];
+        if (blockIdx.x != 0) continue;
+        copy_words(&meta[y].st, B.st + s);
+        copy_words(&meta[y].res, B.results + s);
+        if (det) copy_words(&meta[y].det, det + s);
+        else if (threadIdx.x == 0) meta[y].det = DetState{};
+        const double* ss = B.block_ss + (size_t)s * B.NB;
+        double* oss = reinterpret_cast<double*>(row + g.ss_off);
+        const int n_ss = (int)((g.ms_off - g.ss_off) / 8);
+        for (int i = threadIdx.x; i < n_ss; i += RESET_THREADS) oss[i] = i < B.NB ? ss[i] : 0.0;
+        const double* ms = B.chunk_ms + (size_t)s * 2 * B.chunk_cap;
+        double* oms = reinterpret_cast<double*>(row + g.ms_off);
+        for (int i = threadIdx.x; i < 2 * B.chunk_cap; i += RESET_THREADS) oms[i] = ms[i];
+        float* ot = reinterpret_cast<float*>(row + g.tail_off);
+        for (int i = threadIdx.x; i < g.tail_floats; i += RESET_THREADS)
+            ot[i] = (tail && i < meta[y].tail_len) ? tail[(size_t)s * tail_cap + i] : 0.f;   // tail_len <= tail_cap (host)
+    }
+}
+
+// list and small: the host's checked copy (one upload); bulk values are copied, never used as an index or a length
+__global__ void __launch_bounds__(RESET_THREADS)
+stream_import_kernel(BankView B, const int* __restrict__ list, const MigrateSmall* __restrict__ small, int n,
+                     const char* __restrict__ bulk, MigrateGeom g, long long* keep_end, DetState* det, float* tail,
+                     int tail_cap) {
+    const size_t ring_bytes = (size_t)B.P * (B.fmt == 1 ? 2 : 4);
+    for (int y = blockIdx.y; y < n; y += gridDim.y) {
+        const int s = list[y];
+        const char* row = bulk + (size_t)y * g.row_bytes;
+        const int4* src = reinterpret_cast<const int4*>(row);
+        int4* dst = reinterpret_cast<int4*>(reinterpret_cast<char*>(B.ring) + (size_t)s * ring_bytes);
+        const size_t w0 = (size_t)blockIdx.x * (RESET_SLICE / 16), w1 = min(w0 + RESET_SLICE / 16, ring_bytes / 16);
+        for (size_t w = w0 + threadIdx.x; w < w1; w += RESET_THREADS) dst[w] = src[w];
+        if (blockIdx.x != 0) continue;
+        const MigrateSmall& m = small[y];
+        copy_words(B.prm + s, &m.prm);
+        copy_words(B.st + s, &m.st);
+        if (det) copy_words(det + s, &m.det);
+        if (threadIdx.x == 0) {
+            store_result(B.results + s, m.res);
+            if (keep_end) { keep_end[2 * s] = 0; keep_end[2 * s + 1] = 0; }    // K4 rebuilds its carried rows
+        }
+        const double* ss = reinterpret_cast<const double*>(row + g.ss_off);
+        double* oss = B.block_ss + (size_t)s * B.NB;
+        for (int i = threadIdx.x; i < B.NB; i += RESET_THREADS) oss[i] = ss[i];
+        const double* ms = reinterpret_cast<const double*>(row + g.ms_off);
+        double* oms = B.chunk_ms + (size_t)s * 2 * B.chunk_cap;
+        for (int i = threadIdx.x; i < 2 * B.chunk_cap; i += RESET_THREADS) oms[i] = ms[i];
+        if (tail) {
+            const float* t = reinterpret_cast<const float*>(row + g.tail_off);
+            for (int i = threadIdx.x; i < m.tail_len; i += RESET_THREADS) tail[(size_t)s * tail_cap + i] = t[i];
+        }
+    }
+}
+
 }  // namespace ewk

@@ -308,6 +308,60 @@ int ewk_stream_input(ewk_ctx* ctx, int stream, int32_t* sr_in, int64_t* n_in);
  * polled afterwards would point ewk_read_segment at the new session's audio) and for a context with n_streams = 0;
  * EWK_ERR_ARG for a stream out of range or streams = NULL with n > 0.  Synchronises with the context's stream. */
 int ewk_reset_streams(ewk_ctx* ctx, const int32_t* streams, int n);
+/* Stream migration: move live sessions between slots, contexts and GPUs (rebalancing, draining a GPU, checkpoints).
+ * ewk_export_streams snapshots streams[0..n) into a blob; ewk_import_streams makes blob stream i stream streams[i] of a
+ * context.  Afterwards stream streams[i] behaves exactly like the exported stream would have in its source context
+ * given the same calls from then on: events (with the destination's stream id), result records, tick traces,
+ * ewk_stream_status, ewk_stream_input, ewk_read_last, ewk_read_segment / ewk_prepare_segments of segments still in the
+ * ring, dense scores, the cursors of ewk_dense_ready and ewk_dense_detect, and the detector's state with a pending
+ * ARMED run.  Stream parameters travel with the stream (the destination's overlap-mode ring reserve follows them, as
+ * with ewk_set_stream_params).  Streams not listed are untouched.
+ * A blob may be imported into the same context (other slots, any permutation: exporting [a, b] and importing into
+ * [b, a] swaps two live calls) or into another context with the same ring_samples, slack_samples, pcm_format, n_mfcc
+ * and preemphasis, of any n_streams, max_events or max_templates, on the same GPU or another.  `where` says whether
+ * the blob is host memory (pinned or pageable) or device memory of the context's device (16-byte aligned; copy it
+ * across GPUs with your own copy, e.g. torch .to()).  A device blob must be complete when ewk_import_streams is called:
+ * the call reads it on the context's stream and does not wait for copies queued on other streams, so synchronise with
+ * the copy first (e.g. torch.cuda.synchronize(device), or make the context's stream wait for an event recorded behind
+ * it).  A blob is position-independent and may be saved to a file.  A host blob goes through a device scratch buffer of
+ * its size (export: the whole blob; import: its bulk rows), which the context keeps for later calls until it is
+ * destroyed: about 360 KB per stream of a 10 s int16 ring; device blobs need none.
+ * ewk_export_streams is read-only: the source goes on exactly as without it.  It lands a pending host push first (its
+ * samples belong to the stream) and in overlap mode joins K3 first; events already raised stay in the source's queue
+ * with the source's ids, so it needs no poll.
+ * ewk_import_streams lands a pending push first (its samples belong to the slots' old sessions) and joins K3.  The
+ * imported streams' newest-event link is cleared, K4 rebuilds their carried rows, and the detector state and K8 input
+ * tails are allocated or grown as needed.
+ * Both are one launch (K10) plus plain copies, and synchronise with the context's stream.  Every check comes before the
+ * first launch: on any error no stream of the context changes.
+ * EWK_ERR_ARG: a stream out of range or listed twice, n different from the blob's count, blob_cap / blob_len too small,
+ * bad magic or version, a fingerprint field different from the context's (named), a device blob that is not 16-byte
+ * aligned memory of the context's device, and a meta field outside what the entry points produce (named).
+ * EWK_ERR_STATE: import while the context's event queue holds events ("poll first", as ewk_reset_streams), a context
+ * with n_streams = 0, and a template slot a stream is scored against whose features or n_samples in the context are not
+ * bit-identical to the blob's (named): a moved call never scores silently against another word. */
+#define EWK_STREAM_BLOB_MAGIC 0x534B5745u      /* "EWKS" */
+#define EWK_STREAM_BLOB_VERSION 1
+typedef struct ewk_stream_blob {               /* at offset 0 of every blob, 96 bytes; the rest of a blob is opaque    */
+    uint32_t magic, version;
+    int32_t n_streams;                         /* streams in the blob                                                  */
+    int32_t ring_samples, slack_samples;       /* fingerprint: the importing context's ewk_config must have the same   */
+    int32_t pcm_format, n_mfcc;                /*   values (n_mfcc 0 is stored as 20)                                  */
+    uint32_t preemphasis_bits;                 /*   and the same float32 bit pattern of preemphasis                    */
+    int32_t meta_bytes;                        /* per-stream record of the meta section                                */
+    int32_t n_templates;                       /* records of the template section: every slot a stream is scored on    */
+    int32_t tail_floats;                       /* K8 input tail floats per bulk row                                     */
+    int32_t reserved;
+    int64_t ids_offset;                        /* int32 source stream ids [n_streams]                                  */
+    int64_t meta_offset, template_offset, bulk_offset;   /* sections, 16-byte aligned                                  */
+    int64_t bulk_row_bytes;                    /* one row per stream: ring, block sums, chunk mean squares, K8 tail    */
+    int64_t total_bytes;                       /* length of the blob                                                   */
+} ewk_stream_blob;
+/* An upper bound of the bytes ewk_export_streams(ctx, .., n, ..) writes, for the input rates the context has seen so
+ * far (host code: no device work). */
+int64_t ewk_stream_blob_bytes(const ewk_ctx* ctx, int n);
+int ewk_export_streams(ewk_ctx* ctx, const int32_t* streams, int n, void* blob, int64_t blob_cap, int where);
+int ewk_import_streams(ewk_ctx* ctx, const int32_t* streams, int n, const void* blob, int64_t blob_len, int where);
 /* Dense per-hop scoring (SURVEY §8(a) A9; usage shape of examples/tune_threshold.py:86-116 at hop
  * granularity): for every stream, every hop h in [hop0, hop0 + n_hops) (hop h <-> 160*h samples pushed)
  * and every template slot k in [template_first, template_first + template_count), the value
