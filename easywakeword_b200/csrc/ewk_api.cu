@@ -2099,7 +2099,16 @@ extern "C" int ewk_prepare_segments(ewk_ctx* ctx, int n_seg, const int32_t* stre
     CK(cudaGetLastError());
     ctx->launches++;
     if (where == EWK_HOST) {
-        CK(cudaMemcpyAsync(out, d_out, sizeof(float) * (size_t)out_len, cudaMemcpyDeviceToHost, ctx->stream));
+        // copy back only the segments' ranges (merged where they touch): the scratch holds stale data elsewhere, and
+        // floats of `out` between or after the segments are the caller's
+        std::vector<std::pair<int64_t, int64_t>> iv(n_seg);
+        for (int i = 0; i < n_seg; i++) iv[i] = {out_offsets[i], out_offsets[i] + lens[i]};
+        std::sort(iv.begin(), iv.end());
+        for (size_t i = 0; i < iv.size();) {
+            int64_t a = iv[i].first, b = iv[i].second;
+            for (++i; i < iv.size() && iv[i].first <= b; ++i) b = std::max(b, iv[i].second);
+            CK(cudaMemcpyAsync(out + a, d_out + a, sizeof(float) * (size_t)(b - a), cudaMemcpyDeviceToHost, ctx->stream));
+        }
     }
     CK(cudaStreamSynchronize(ctx->stream));
     return EWK_OK;

@@ -4,6 +4,12 @@
 //            (librosa.feature.rms(frame_length=400, hop_length=160, center=True, pad_mode='constant'))
 //   threshold = max(rms) * 0.1 (float32), voiced = rms > threshold, duration = (last - first) * 160 / 16000,
 //   returned as max(duration, 0.2); "not voiced" (all-zero input) is reported through `voiced = 0`.
+// The frame RMS is librosa's float32 arithmetic bit for bit (oracle/vad_model.py): its np.mean over a contiguous frame
+// is numpy's pairwise sum, which for 400 samples is four blocks [0,96) [96,200) [200,296) [296,400) of 8 sequential
+// accumulators each, combined ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) per block and (B0+B1)+(B2+B3) across blocks, then
+// a float32 divide by 400 and a float32 sqrt.  One warp per frame: lane l runs block l/8's accumulator l%8 (12 or 13
+// squares), and a xor butterfly over offsets 1, 2, 4, 8, 16 is exactly that grouping (float addition commutes).  The
+// _rn intrinsics keep every square and sum a separate rounding: nothing contracts into an FMA.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -36,19 +42,23 @@ template_vad_kernel(const VadDesc* __restrict__ descs, VadResult* __restrict__ o
     float* rms = rms_ws + d.rms_off;
     __shared__ float red_f[NW];
     __shared__ long long red_lo[NW], red_hi[NW];
-    // frame RMS, one warp per frame; double accumulation, rounded once to float32
+    // frame RMS, one warp per frame: lane = (block, accumulator) of numpy's pairwise float32 sum
+    const int blk = lane >> 3, acc = lane & 7;
+    const int b0 = blk == 0 ? 0 : blk == 1 ? 96 : blk == 2 ? 200 : 296;
+    const int nterm = (blk & 1) ? 13 : 12;                   // blocks of 96 and 104 samples
     float vmax = 0.f;
     for (long long t = warp; t < F; t += NW) {
-        const long long i0 = t * VAD_HOP - VAD_FRAME / 2;
-        double ss = 0.0;
-        for (int i = lane; i < VAD_FRAME; i += 32) {
-            const long long p = i0 + i;
+        const long long i0 = t * VAD_HOP - VAD_FRAME / 2 + b0 + acc;
+        float r = 0.f;
+        for (int k = 0; k < nterm; k++) {
+            const long long p = i0 + 8 * k;
             const float v = (p >= 0 && p < d.len) ? __ldg(x + p) : 0.f;
-            ss += (double)v * (double)v;
+            const float sq = __fmul_rn(v, v);
+            r = k ? __fadd_rn(r, sq) : sq;
         }
 #pragma unroll
-        for (int o = 16; o; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
-        const float r = sqrtf((float)(ss / (double)VAD_FRAME));
+        for (int o = 1; o < 32; o <<= 1) r = __fadd_rn(r, __shfl_xor_sync(0xffffffffu, r, o));
+        r = __fsqrt_rn(__fdiv_rn(r, (float)VAD_FRAME));
         if (lane == 0) rms[t] = r;
         vmax = fmaxf(vmax, r);
     }

@@ -241,17 +241,23 @@ class SoundBuffer:
         return self.samples_collected >= self.buffer_length
 
 
-def analyze_reference_audio_duration(audio: np.ndarray) -> Optional[float]:
-    """Speech duration of a template by the reference's RMS voice-activity rule (wakeword.py:872-893):
-    25 ms frames every 10 ms (zero-padded centring), frames above 0.1 * max RMS, first-to-last span."""
+def template_frame_rms(audio: np.ndarray) -> np.ndarray:
+    """Frame RMS of the reference's voice-activity rule: 25 ms frames every 10 ms, zero-padded centring.
+    The audio is taken as float32, as librosa.load returns it.  Each frame is a contiguous row, so its mean square is
+    numpy's pairwise float32 sum over the row: the arithmetic of librosa.feature.rms, and of K6."""
     frame_length = int(0.025 * SoundBuffer.FREQUENCY)
     hop_length = int(0.010 * SoundBuffer.FREQUENCY)
-    y = np.pad(np.asarray(audio), frame_length // 2)
+    y = np.pad(np.asarray(audio, dtype=np.float32).reshape(-1), frame_length // 2)
     n_frames = 1 + (len(y) - frame_length) // hop_length
-    if n_frames < 1:
-        return None
     idx = np.arange(frame_length)[None, :] + hop_length * np.arange(n_frames)[:, None]
-    rms = np.sqrt(np.mean(np.abs(y[idx]) ** 2, axis=1))
+    return np.sqrt(np.mean(np.abs(y[idx]) ** 2, axis=1))
+
+
+def analyze_reference_audio_duration(audio: np.ndarray) -> Optional[float]:
+    """Speech duration of a template by the reference's RMS voice-activity rule (wakeword.py:872-893):
+    frames above 0.1 * max RMS (template_frame_rms), first-to-last span."""
+    hop_length = int(0.010 * SoundBuffer.FREQUENCY)
+    rms = template_frame_rms(audio)
     voiced = np.where(rms > np.max(rms) * VOICE_ACTIVITY_THRESHOLD)[0]
     if len(voiced) == 0:
         return None

@@ -198,8 +198,8 @@ int ewk_read_segment(ewk_ctx* ctx, int stream, int64_t seg_start, int64_t seg_le
  * speech-to-text call (wakeword.py:1020-1025): x - mean(x), / max|.| when > 0, * 1.5, clip to [-1, 1] — for
  * n_seg segments of the rings at once (typically the matched events of one ewk_poll).  Segment i is
  * streams[i], absolute samples [starts[i], starts[i] + lens[i]); its float32 result is written at
- * out + out_offsets[i].  `where` tells whether `out` is host or device memory.  EWK_ERR_STATE if a segment was
- * already overwritten in its ring. */
+ * out + out_offsets[i]; no other float of `out` is written.  `where` tells whether `out` is host or device memory.
+ * EWK_ERR_STATE if a segment was already overwritten in its ring.  A failed call writes nothing to `out`. */
 int ewk_prepare_segments(ewk_ctx* ctx, int n_seg, const int32_t* streams, const int64_t* starts, const int64_t* lens,
                          const int64_t* out_offsets, float* out, int64_t out_len, int where);
 /* Overlap of level-2 matching with the next push (off by default).  When enabled, ewk_tick launches K3 on a second

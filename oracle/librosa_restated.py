@@ -175,11 +175,20 @@ def preemphasis(y, coef=0.97):
 
 
 def rms(y, frame_length=2048, hop_length=512):
-    """librosa.feature.rms(center=True, pad_mode='constant') -> [1, n_frames]."""
+    """librosa.feature.rms(center=True, pad_mode='constant', dtype=float32) -> [1, n_frames].
+
+    Framed the way librosa.util.frame frames: a strided view [frame_length, n_frames] whose frame-sample axis (-2)
+    is contiguous, squared in float32 (util.abs2) and averaged with np.mean over that axis.  Because the reduced axis
+    is contiguous, numpy runs its pairwise float32 sum once per frame; oracle/vad_model.py states that sum's shape
+    and tests/test_vad_model.py pins the two together.  (frame_signal's fancy-indexed [frame_length, n_frames] copy
+    would reduce row by row instead and differs from librosa in the last bit of about half of all frames.)"""
     y = np.asarray(y)
     ypad = np.pad(y, frame_length // 2, mode="constant")
-    x = frame_signal(ypad, frame_length, hop_length)
-    power = np.mean(np.abs(x) ** 2, axis=0, keepdims=True)
+    n_frames = 1 + (len(ypad) - frame_length) // hop_length
+    s = ypad.strides[-1]
+    x = np.lib.stride_tricks.as_strided(ypad, shape=(frame_length, n_frames), strides=(s, hop_length * s),
+                                        writeable=False)
+    power = np.mean(np.square(x, dtype=np.float32), axis=-2, keepdims=True)
     return np.sqrt(power)
 
 

@@ -192,10 +192,10 @@ def test_bank_level3_handoff_and_multi_template(word):
         assert abs(float(e["score"]) - max(sc)) <= 0.01
         if abs(sc[0] - sc[1]) > 0.02:
             assert int(e["template_slot"]) == int(np.argmax(sc))
-    # N1: device pre-processing == the reference formula (float64) rounded to float32
+    # N1: device pre-processing == the reference formula (float64) rounded to float32, bit for bit on an int16 ring
     last = [e for e in ev if e["matched"]][-2:]
     got = bank.prepare_for_transcription(last)
     for e, g in zip(last, got):
         seg = synth.from_int16(q[e["stream"], e["seg_start"]:e["seg_start"] + e["seg_len"]]).astype(np.float64)
-        np.testing.assert_allclose(g, O.prepare_for_level3(seg).astype(np.float32), atol=2e-7, rtol=0)
+        assert np.array_equal(g.view(np.uint32), O.prepare_for_level3(seg).astype(np.float32).view(np.uint32))
     bank.close()
