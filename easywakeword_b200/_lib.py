@@ -362,6 +362,12 @@ def _declare_stream_protos(lib):
         "ewk_dense_ready": (C.c_int, [vp, _p(C.c_int32), i32, i32, i32, i32, _p(i64), _p(C.c_int32), vp, i64, i32]),
         "ewk_dense_detect": (C.c_int, [vp, _p(C.c_int32), i32, i32, i32, i32, i32, i32, vp, i32, _p(i64), _p(C.c_int32),
                                        vp, i64, i32]),
+        "ewk_dense_scores_sets": (C.c_int, [vp, _p(C.c_int32), i32, _p(i64), _p(C.c_int32), _p(C.c_int32),
+                                            _p(C.c_int32), vp, i64, i32]),
+        "ewk_dense_ready_sets": (C.c_int, [vp, _p(C.c_int32), i32, i32, _p(C.c_int32), _p(C.c_int32), _p(i64),
+                                           _p(C.c_int32), vp, i64, i32]),
+        "ewk_dense_detect_sets": (C.c_int, [vp, _p(C.c_int32), i32, i32, _p(C.c_int32), _p(C.c_int32), i32, i32, vp, i32,
+                                            _p(i64), _p(C.c_int32), vp, i64, i32]),
         "ewk_prepare_segments": (C.c_int, [vp, i32, _p(C.c_int32), _p(i64), _p(i64), _p(i64), f32p, i64, i32]),
         "ewk_results_device_ptr": (C.c_int, [vp, _p(vp)]),
         "ewk_set_results_buffer": (C.c_int, [vp, vp]),
@@ -478,10 +484,142 @@ def _unpack_rows(out, n_hops, T):
     return [out[(e - n) * T:e * T].reshape(n, T) for e, n in zip(ends.tolist(), [int(v) for v in n_hops])]
 
 
+def sets_offsets(n_hops, T):
+    """Float offset of each row of a per-row-set call (include/ewk.h: ewk_dense_scores_sets): row i starts at
+    sum_{j < i} n_hops[j] T[j].  Returns (offsets int64 [n], total floats)."""
+    sizes = np.asarray(n_hops, np.int64).reshape(-1) * np.asarray(T, np.int64).reshape(-1)
+    ends = np.cumsum(sizes)
+    return ends - sizes, int(ends[-1]) if sizes.size else 0
+
+
+def _unpack_rows_sets(out, n_hops, T):
+    """Packed rows of a per-row-set call -> list of [n_i, T_i] views, in list order."""
+    off, _ = sets_offsets(n_hops, T)
+    return [out[o:o + int(n) * int(t)].reshape(int(n), int(t)) for o, n, t in zip(off.tolist(), n_hops, T)]
+
+
+def sets_launches(set_lens):
+    """The K4 launches of a per-row-set call whose rows have template sets of these lengths: {(DH, threads, CTAs per
+    SM): row indices}, one launch per geometry each set has alone (dense_plan), in order of first appearance."""
+    groups = {}
+    for i, lens in enumerate(set_lens):
+        groups.setdefault(dense_plan(lens)[:3], []).append(i)
+    return groups
+
+
 def _bank_methods():
     def set_stream_params(self, stream=-1, params=None, **over):
         p = params if params is not None else default_stream_params(**over)
         self._ck(self.lib.ewk_set_stream_params(self.h, stream, C.byref(p)))
+        ranges = self._template_ranges()
+        ranges[slice(None) if stream < 0 else stream] = (p.template_first, p.template_count)
+
+    def _template_ranges(self):
+        """[n_streams, 2] (template_first, template_count) of each stream as set through set_stream_params; -1: not
+        known here (never set, or the stream was imported)."""
+        if getattr(self, "_ranges", None) is None:
+            self._ranges = np.full((self.cfg.n_streams, 2), -1, np.int32)
+        return self._ranges
+
+    def _row_sets(self, st, n, template_first, template_count):
+        """-> (first int32 [n] or None, count int32 [n] or None, T int64 [n]) of a per-row-set call's rows (st None:
+        every stream).  Both None: each stream's own range, NULL to the library, T from set_stream_params."""
+        if (template_first is None) != (template_count is None):
+            raise ValueError("give both template_first and template_count, or neither")
+        if template_first is None:
+            idx = np.arange(n) if st is None else st
+            r = self._template_ranges()[idx]
+            if n and r[:, 1].min() < 0:
+                raise ValueError(f"stream {int(idx[np.argmax(r[:, 1] < 0)])} has a template range this Context did not "
+                                 "set (imported stream): pass template_first / template_count")
+            return None, None, r[:, 1].astype(np.int64)
+        tf = np.ascontiguousarray(np.broadcast_to(np.asarray(template_first, np.int64), (n,)), np.int32)
+        tc = np.ascontiguousarray(np.broadcast_to(np.asarray(template_count, np.int64), (n,)), np.int32)
+        return tf, tc, tc.astype(np.int64)
+
+    def dense_scores_sets(self, streams, hop0, n_hops, template_first=None, template_count=None, out_device_ptr=None,
+                          out_cap=None):
+        """dense_scores_streams with a template set per row (include/ewk.h: ewk_dense_scores_sets): row i is scored
+        against slots [template_first[i], template_first[i] + template_count[i]) (both None: its stream's own range).
+        Returns a list of float32 [n_hops[i], T_i] arrays; with out_device_ptr the rows go there packed as the header
+        says (out_cap floats, default exactly what they need) and None is returned."""
+        st = _stream_list(streams)
+        h0 = np.ascontiguousarray(np.asarray(hop0, dtype=np.int64).reshape(-1))
+        nh64 = np.asarray(n_hops, dtype=np.int64).reshape(-1)
+        if len(h0) != len(st) or len(nh64) != len(st):
+            raise ValueError("one hop0 and one n_hops per stream")
+        if nh64.size and (nh64.min() < -2**31 or nh64.max() >= 2**31):
+            raise ValueError("n_hops out of range")
+        nh = np.ascontiguousarray(nh64, dtype=np.int32)
+        tf, tc, T = self._row_sets(st, len(st), template_first, template_count)
+        need = max(0, sets_offsets(np.maximum(nh64, 0), T)[1])
+        args = (st.ctypes.data_as(_p(C.c_int32)), len(st), i64ptr(h0), nh.ctypes.data_as(_p(C.c_int32)),
+                None if tf is None else tf.ctypes.data_as(_p(C.c_int32)),
+                None if tc is None else tc.ctypes.data_as(_p(C.c_int32)))
+        if out_device_ptr is not None:
+            self._ck(self.lib.ewk_dense_scores_sets(self.h, *args, C.c_void_p(out_device_ptr),
+                                                    need if out_cap is None else int(out_cap), DEVICE))
+            return None
+        out = np.empty(need, np.float32)
+        self._ck(self.lib.ewk_dense_scores_sets(self.h, *args, out.ctypes.data if need else None,
+                                                need if out_cap is None else int(out_cap), HOST))
+        return _unpack_rows_sets(out, nh64, T)
+
+    def dense_ready_sets(self, streams=None, max_hops=100, template_first=None, template_count=None,
+                         out_device_ptr=None, out_cap=None):
+        """dense_ready with a template set per row (include/ewk.h: ewk_dense_ready_sets; arguments as dense_scores_sets,
+        one entry per listed stream, or per stream when streams is None).  Moves dense_ready's cursor.  Returns (hop0,
+        list of float32 [n_i, T_i] arrays), or (hop0, n_hops) with out_device_ptr (out_cap floats, default
+        n * max_hops * max T_i)."""
+        st = None if streams is None else _stream_list(streams)
+        n = self.cfg.n_streams if st is None else len(st)
+        tf, tc, T = self._row_sets(st, n, template_first, template_count)
+        h0 = np.zeros(n, np.int64)
+        nh = np.zeros(n, np.int32)
+        cap = n * int(max_hops) * (int(T.max()) if n else 0) if out_cap is None else int(out_cap)
+        args = (None if st is None else st.ctypes.data_as(_p(C.c_int32)), n, int(max_hops),
+                None if tf is None else tf.ctypes.data_as(_p(C.c_int32)),
+                None if tc is None else tc.ctypes.data_as(_p(C.c_int32)), i64ptr(h0), nh.ctypes.data_as(_p(C.c_int32)))
+        if out_device_ptr is not None:
+            self._ck(self.lib.ewk_dense_ready_sets(self.h, *args, C.c_void_p(out_device_ptr), cap, DEVICE))
+            return h0, nh
+        out = np.empty(max(0, cap), np.float32)
+        self._ck(self.lib.ewk_dense_ready_sets(self.h, *args, out.ctypes.data if out.size else None, cap, HOST))
+        return h0, _unpack_rows_sets(out, nh, T)
+
+    def dense_detect_sets(self, streams=None, max_hops=100, template_first=None, template_count=None, hold_hops=20,
+                          refractory_hops=50, scores=False, out_device_ptr=None, det_cap=None, out_cap=None, hops=False):
+        """dense_detect with a template set per row (include/ewk.h: ewk_dense_detect_sets; sets as dense_ready_sets).
+        Moves dense_detect's cursor and detector state; returns what dense_detect returns, score rows [n_i, T_i]."""
+        st = None if streams is None else _stream_list(streams)
+        n = self.cfg.n_streams if st is None else len(st)
+        tf, tc, T = self._row_sets(st, n, template_first, template_count)
+        cap = n * ((min(int(max_hops), 1 << 20) + 1) // 2) if det_cap is None else int(det_cap)
+        det = np.empty(max(0, cap), DETECTION_DTYPE)
+        h0 = np.zeros(n, np.int64)
+        nh = np.zeros(n, np.int32)
+        ocap = n * int(max_hops) * (int(T.max()) if n else 0) if out_cap is None else int(out_cap)
+        buf = None
+        if out_device_ptr is not None:
+            out, where = C.c_void_p(out_device_ptr), DEVICE
+        elif scores:
+            buf = np.empty(max(0, ocap), np.float32)
+            out, where = (buf.ctypes.data if buf.size else None), HOST
+        else:
+            out, ocap, where = None, 0, HOST
+        rc = self.lib.ewk_dense_detect_sets(self.h, None if st is None else st.ctypes.data_as(_p(C.c_int32)), n,
+                                            int(max_hops), None if tf is None else tf.ctypes.data_as(_p(C.c_int32)),
+                                            None if tc is None else tc.ctypes.data_as(_p(C.c_int32)), int(hold_hops),
+                                            int(refractory_hops), det.ctypes.data if det.size else None, cap, i64ptr(h0),
+                                            nh.ctypes.data_as(_p(C.c_int32)), out, ocap, where)
+        if rc < 0:
+            self._ck(rc)
+        d = det[:rc].copy()
+        if out_device_ptr is not None:
+            return d, (h0, nh)
+        if scores:
+            return d, (h0, _unpack_rows_sets(buf, nh, T))
+        return (d, (h0, nh)) if hops else d
 
     def push(self, pcm, stream0=0, where=HOST):
         """pcm: [n_streams, n] array in the ring's dtype (rows may be strided), or (ptr, n_streams, n, stride)."""
@@ -642,9 +780,11 @@ def _bank_methods():
         if where == DEVICE:
             ptr, length = blob
             self._ck(self.lib.ewk_import_streams(self.h, sp, len(st), C.c_void_p(int(ptr)), int(length), DEVICE))
+            self._template_ranges()[st] = -1
             return
         b = np.ascontiguousarray(blob).view(np.uint8).reshape(-1)
         self._ck(self.lib.ewk_import_streams(self.h, sp, len(st), b.ctypes.data if b.size else None, int(b.size), HOST))
+        self._template_ranges()[st] = -1                  # parameters travel with the streams
 
     def stream_input(self, stream):
         """-> (input rate latched by the stream's first push (0: none yet), input samples received)."""
@@ -876,6 +1016,8 @@ def _bank_methods():
                  "resample_push"]
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
+    for f in (_template_ranges, _row_sets, dense_scores_sets, dense_ready_sets, dense_detect_sets):
+        setattr(Context, f.__name__, f)
     for f in (prepare_segments, dense_scores, dense_scores_streams, dense_ready, dense_detect, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
               push_resampled_each, push_streams, tick_ready, reset_streams, stream_blob_bytes, export_streams, import_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
               set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count):

@@ -257,15 +257,21 @@ class WakeWordBank:
         T = len(self.templates) - template_first if template_count is None else template_count
         return self.ctx.dense_scores(hop0, n_hops, template_first, T)
 
-    def dense_ready(self, streams=None, template_first: int = 0, template_count: Optional[int] = None):
+    def dense_ready(self, streams=None, template_first: int = 0, template_count: Optional[int] = None,
+                    own_templates: bool = False):
         """Per-hop scores paced by each stream's own audio (include/ewk.h: ewk_dense_ready): every hop of the listed
         streams (None: all) that their landed audio completes and no earlier call scored, in rounds of DENSE_ROUND hops,
         so that no due hop is left when it returns.  Returns (hop0, scores): int64 first hop of each listed stream's
-        scores and a list of float32 [n_i, T] arrays.  A stream recycled with reset() starts again at hop 1."""
+        scores and a list of float32 [n_i, T] arrays.  A stream recycled with reset() starts again at hop 1.
+        own_templates=True scores each stream against its own set_stream(..., template_first=, template_count=) range
+        in the same calls (ewk_dense_ready_sets); its arrays are then [n_i, T_i]."""
         T = len(self.templates) - template_first if template_count is None else template_count
         hop0, parts = None, None
         while True:
-            h0, rows = self.ctx.dense_ready(streams, DENSE_ROUND, template_first, T)
+            if own_templates:
+                h0, rows = self.ctx.dense_ready_sets(streams, DENSE_ROUND)
+            else:
+                h0, rows = self.ctx.dense_ready(streams, DENSE_ROUND, template_first, T)
             if hop0 is None:
                 hop0, parts = h0, [[r] for r in rows]
             else:
@@ -275,19 +281,25 @@ class WakeWordBank:
                 return hop0, [p[0] if len(p) == 1 else np.concatenate(p) for p in parts]
 
     def dense_detect(self, streams=None, template_first: int = 0, template_count: Optional[int] = None,
-                     hold_hops: int = 20, refractory_hops: int = 50) -> np.ndarray:
+                     hold_hops: int = 20, refractory_hops: int = 50, own_templates: bool = False) -> np.ndarray:
         """Wake-word detections from per-hop scores, without the energy gate (include/ewk.h: ewk_dense_detect): every hop
         of the listed streams (None: all) that their landed audio completes and no earlier dense_detect took, in rounds of
         DENSE_ROUND hops, so that no due hop is left when it returns.  A stream detects where its best per-hop score
         reaches its similarity_threshold; a run reports its first peak once it ends or hold_hops after the peak, and a
         stream stays quiet for refractory_hops after a run.  Returns a _lib.DETECTION_DTYPE array sorted by
         (emit_hop, stream); prepare_for_transcription takes it as it is.  The detector has its own cursor (dense_ready's is
-        untouched); reset() restarts it.  Feed hold_hops hops of trailing audio to finish a recording's last run."""
+        untouched); reset() restarts it.  Feed hold_hops hops of trailing audio to finish a recording's last run.
+        own_templates=True detects each stream against its own set_stream(..., template_first=, template_count=) range
+        in the same calls (ewk_dense_detect_sets): personal wake words, one launch per geometry."""
         T = len(self.templates) - template_first if template_count is None else template_count
         parts = []
         while True:
-            d, (_, nh) = self.ctx.dense_detect(streams, DENSE_ROUND, template_first, T, hold_hops, refractory_hops,
-                                               hops=True)
+            if own_templates:
+                d, (_, nh) = self.ctx.dense_detect_sets(streams, DENSE_ROUND, hold_hops=hold_hops,
+                                                        refractory_hops=refractory_hops, hops=True)
+            else:
+                d, (_, nh) = self.ctx.dense_detect(streams, DENSE_ROUND, template_first, T, hold_hops, refractory_hops,
+                                                   hops=True)
             parts.append(d)
             if nh.size == 0 or nh.max() < DENSE_ROUND:
                 break

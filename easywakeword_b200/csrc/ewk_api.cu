@@ -214,6 +214,8 @@ void ewk_ctx::release() {
         ev_ddet[i] = nullptr; h_ddet[i] = nullptr;
         b_ddet[i].free();
     }
+    dset_stage.free(); drow_sets.free(); ddet_sets.free(); b_dset.free();
+    h_dset.clear();
     if (h_det_map) cudaFreeHost(h_det_map);
     h_det_map = nullptr; det_map_cap = 0;
     b_reset.free();
@@ -321,6 +323,7 @@ static int install_template(ewk_ctx* ctx, int slot, const float* mean20, const f
     tf.n_samples = n_samples;
     tf.valid = 1;
     ctx->h_tmpl[slot] = tf;
+    ctx->dense_sets_forget(slot);
     CK(cudaMemcpyAsync(ctx->d_tmpl + slot, &ctx->h_tmpl[slot], sizeof(tf), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return EWK_OK;
@@ -362,6 +365,7 @@ extern "C" int ewk_clear_template(ewk_ctx* ctx, int slot) {
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
     ctx->h_tmpl[slot] = TemplateFeat{};
+    ctx->dense_sets_forget(slot);
     CK(cudaMemcpyAsync(ctx->d_tmpl + slot, &ctx->h_tmpl[slot], sizeof(TemplateFeat), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     return EWK_OK;
@@ -2233,8 +2237,9 @@ static int dense_resident(ewk_ctx* ctx, const char* who, int s, long long hop0, 
     return EWK_OK;
 }
 
-// K4 over n_ctas CTAs into d_out: the uniform instance, or the per-row one when A.rows is set
-static int dense_launch(ewk_ctx* ctx, DenseArgs& A, const DensePlan& plan, float* d_out, int n_ctas) {
+// K4 over n_ctas CTAs into d_out: the uniform instance, or the per-row one when A.rows is set (sets: its per-row-set
+// form, A.rows holding DenseRowSet descriptors)
+static int dense_launch(ewk_ctx* ctx, DenseArgs& A, const DensePlan& plan, float* d_out, int n_ctas, bool sets = false) {
     BankView& B = ctx->bank;
     A.out = d_out;
     if (!ctx->b_keep_rows.p) {
@@ -2247,7 +2252,8 @@ static int dense_launch(ewk_ctx* ctx, DenseArgs& A, const DensePlan& plan, float
     A.keep_end = (long long*)ctx->b_keep_end.p;
     A.g2 = (float*)ctx->b_g2.p;
     const bool pre = ctx->cfg.preemphasis != 0.f;
-    auto k4 = A.rows ? (pre ? dense_score_kernel<true, true> : dense_score_kernel<false, true>)
+    auto k4 = sets     ? (pre ? dense_score_kernel<true, true, true> : dense_score_kernel<false, true, true>)
+            : A.rows ? (pre ? dense_score_kernel<true, true> : dense_score_kernel<false, true>)
                      : (pre ? dense_score_kernel<true, false> : dense_score_kernel<false, false>);
     CK(cudaFuncSetAttribute(k4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem));
     CK(cudaFuncSetAttribute(k4, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
@@ -2384,6 +2390,217 @@ static int dense_rows(ewk_ctx* ctx, const char* who, const int32_t* streams, int
     return EWK_OK;
 }
 
+// ---- per-row template sets: ewk_dense_scores_sets, ewk_dense_ready_sets, ewk_dense_detect_sets ----------------------
+static inline int dset_key(int first, int count) { return first * DENSE_MAX_T + count - 1; }
+
+void ewk_ctx::dense_sets_forget(int slot) {
+    for (int c = 1; c <= DENSE_MAX_T; c++)
+        for (int f = std::max(0, slot - c + 1); f <= slot; f++)
+            if ((size_t)dset_key(f, c) < h_dset.size()) h_dset[dset_key(f, c)].valid = false;
+}
+
+struct RowSets { const int32_t* first; const int32_t* count; };   // row i: [first[i], first[i] + count[i]); NULL: own range
+
+// Row i's set -> key[i] (its index in the context's table), with every check of the set; sets not cached yet are built
+// into `fresh`, which dense_sets_commit uploads once the call has passed every check.  Messages name the row and stream.
+static int dense_sets_resolve(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, const RowSets& rs,
+                              std::vector<int>& key, std::map<int, DenseSetHost>& fresh) {
+    if (!rs.first != !rs.count) {
+        ctx->fail("%s: template_first and template_count must both be given or both be NULL", who);
+        return EWK_ERR_ARG;
+    }
+    if (ctx->h_dset.empty()) ctx->h_dset.resize((size_t)ctx->cfg.max_templates * DENSE_MAX_T);
+    key.assign((size_t)n, -1);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        const int f = rs.first ? rs.first[i] : ctx->h_prm[s].template_first;
+        const int c = rs.count ? rs.count[i] : ctx->h_prm[s].template_count;
+        if (c < 1 || c > DENSE_MAX_T || f < 0 || f > ctx->cfg.max_templates - c) {
+            ctx->fail("%s: row %d (stream %d) has a bad template range [%d, %d) (1..%d templates of %d slots)", who, i, s, f,
+                      f + c, DENSE_MAX_T, ctx->cfg.max_templates);
+            return EWK_ERR_ARG;
+        }
+        key[i] = dset_key(f, c);
+        if (ctx->h_dset[key[i]].valid || fresh.count(key[i])) continue;
+        for (int k = f; k < f + c; k++) {
+            const TemplateFeat& tf = ctx->h_tmpl[k];
+            if (!tf.valid) {
+                ctx->fail("%s: row %d (stream %d): template slot %d is empty. No reference word set. Call set_reference() first.",
+                          who, i, s, k);
+                return EWK_ERR_NO_TEMPLATE;
+            }
+            if (tf.n_samples < DENSE_MIN_L || tf.n_samples > DENSE_MAX_L) {
+                ctx->fail("%s: row %d (stream %d): template %d has %lld samples; dense scoring needs %d..%d", who, i, s, k,
+                          (long long)tf.n_samples, DENSE_MIN_L, DENSE_MAX_L);
+                return EWK_ERR_ARG;
+            }
+        }
+        char w[192];
+        snprintf(w, sizeof w, "%s: row %d (stream %d)", who, i, s);
+        DenseArgs A{};
+        DensePlan plan;
+        const int rc = dense_prepare(ctx, w, f, c, A, plan);
+        if (rc) return rc;
+        DenseSetHost& e = fresh[key[i]];
+        e.DH = plan.DH; e.threads = plan.threads; e.per_sm = plan.per_sm; e.smem = plan.smem;
+        DenseSetDev& d = e.dev;
+        d.T = A.T; d.DG = A.DG; d.DLE = A.DLE; d.n_re_u = A.n_re_u; d.n_min = A.n_min; d.n_max = A.n_max;
+        d.g_back = A.g_back; d.slot0 = f;
+        std::memcpy(d.re_goff, A.re_goff, sizeof d.re_goff); std::memcpy(d.re_delta, A.re_delta, sizeof d.re_delta);
+        std::memcpy(d.re_rep, A.re_rep, sizeof d.re_rep); std::memcpy(d.re_rep_e, A.re_rep_e, sizeof d.re_rep_e);
+        std::memcpy(d.re_nfirst, A.re_nfirst, sizeof d.re_nfirst);
+        std::memcpy(d.t, A.t, sizeof d.t);
+    }
+    return EWK_OK;
+}
+
+// the new descriptors -> a staging slot -> their places in the table (one copy per run of consecutive keys), in stream
+// order behind every K4 / K4D that read an older descriptor at those places
+static int dense_sets_commit(ewk_ctx* ctx, const std::map<int, DenseSetHost>& fresh) {
+    if (!ctx->b_dset.p) CK(ctx->b_dset.ensure(sizeof(DenseSetDev) * ctx->h_dset.size()));
+    if (fresh.empty()) return EWK_OK;
+    std::vector<DenseSetDev> up;
+    std::vector<int> keys;
+    for (const auto& kv : fresh) { keys.push_back(kv.first); up.push_back(kv.second.dev); }
+    SlotPair<DenseSetDev>& st = ctx->dset_stage;
+    int k = -1;
+    int rc = upload_slot(ctx, st.h, st.b, st.ev, st.ev_valid, st.idx, up, ctx->stream, &k);
+    if (rc) return rc;
+    DenseSetDev* tab = (DenseSetDev*)ctx->b_dset.p;
+    const DenseSetDev* stage = (const DenseSetDev*)st.b[k].p;
+    for (size_t a = 0; a < keys.size();) {
+        size_t b = a + 1;
+        while (b < keys.size() && keys[b] == keys[b - 1] + 1) b++;
+        CK(cudaMemcpyAsync(tab + keys[a], stage + a, sizeof(DenseSetDev) * (b - a), cudaMemcpyDeviceToDevice, ctx->stream));
+        a = b;
+    }
+    CK(cudaEventRecord(st.ev[k], ctx->stream));
+    st.ev_valid[k] = true;
+    for (const auto& kv : fresh) { ctx->h_dset[kv.first] = kv.second; ctx->h_dset[kv.first].valid = true; }
+    return EWK_OK;
+}
+
+// dense_rows with a template set per row: row i is packed from float sum_{j < i} n_hops[j] T_j, laid out [n_hops[i]][T_i].
+// One K4 launch per launch geometry (DH, threads, CTAs per SM) among the rows' sets, each set at the geometry it has
+// alone; the launch gets its group's largest shared memory and g2 stride.  *keys (when given) receives each row's key.
+static int dense_rows_sets(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, const int64_t* hop0,
+                           const int32_t* n_hops, const RowSets& rs, float* out, int64_t out_cap, int where,
+                           float** d_scores = nullptr, std::vector<int>* keys = nullptr) {
+    if (d_scores) *d_scores = nullptr;
+    BankView& B = ctx->bank;
+    if (n < 0 || (n > 0 && (!streams || !hop0 || !n_hops))) { ctx->fail("%s: bad row list (n=%d)", who, n); return EWK_ERR_ARG; }
+    if (n == 0) return EWK_OK;
+    std::vector<int> row_of((size_t)B.n_streams, -1);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        if (s < 0 || s >= B.n_streams) { ctx->fail("%s: bad stream %d (context has %d)", who, s, B.n_streams); return EWK_ERR_ARG; }
+        if (row_of[s] >= 0) { ctx->fail("%s: stream %d is listed twice", who, s); return EWK_ERR_ARG; }
+        row_of[s] = i;
+        if (hop0[i] < 0 || n_hops[i] < 0 || hop0[i] > ((int64_t)1 << 48)) {
+            ctx->fail("%s: row %d of stream %d has bad hops (hop0=%lld n_hops=%d)", who, i, s, (long long)hop0[i], n_hops[i]);
+            return EWK_ERR_ARG;
+        }
+    }
+    std::vector<int> key;
+    std::map<int, DenseSetHost> fresh;
+    int rc = dense_sets_resolve(ctx, who, streams, n, rs, key, fresh);
+    if (rc) return rc;
+    auto set_of = [&](int i) -> const DenseSetHost& {
+        const auto it = fresh.find(key[i]);
+        return it != fresh.end() ? it->second : ctx->h_dset[key[i]];
+    };
+    long long n_out = 0;
+    for (int i = 0; i < n; i++) n_out += (long long)n_hops[i] * set_of(i).dev.T;
+    if (n_out > 0 && (out || !d_scores) && (!out || out_cap < n_out)) {
+        ctx->fail("%s: out holds %lld floats, the rows need %lld", who, out ? (long long)out_cap : 0LL, n_out);
+        return EWK_ERR_ARG;
+    }
+    CK(cudaSetDevice(ctx->device));
+    if (ctx->pending.valid) {
+        // as in ewk_dense_scores: the in-flight host push lands now only if a listed row reaches into its samples
+        bool need = false;
+        const std::vector<RowDesc>& prow = ctx->pending.rows;
+        for (int j = 0; !need && j < ctx->pending.n_streams; j++) {
+            const int s = prow.empty() ? ctx->pending.stream0 + j : prow[j].stream, i = row_of[s];
+            need = i >= 0 && n_hops[i] > 0 && ctx->h_written[s] < 160LL * (hop0[i] + n_hops[i] - 1);
+        }
+        if (need) { rc = ctx->flush_pending(); if (rc) return rc; }
+    }
+    for (int i = 0; i < n; i++) {
+        if (n_hops[i] == 0) continue;
+        rc = dense_resident(ctx, who, streams[i], hop0[i], n_hops[i], set_of(i).dev.n_max);
+        if (rc) return rc;
+    }
+    if (keys) *keys = key;
+    if (n_out == 0) return EWK_OK;
+    rc = dense_sets_commit(ctx, fresh);
+    if (rc) return rc;
+    // geometry groups in order of first appearance; within a group the longest rows first, as in dense_rows
+    struct Group { DensePlan plan; int DG; std::vector<DenseRowSet> rows; };
+    std::vector<Group> groups;
+    const DenseSetDev* tab = (const DenseSetDev*)ctx->b_dset.p;
+    long long off = 0;
+    int max_dg = 0;
+    for (int i = 0; i < n; i++) {
+        const DenseSetHost& e = ctx->h_dset[key[i]];
+        if (n_hops[i] > 0) {
+            size_t g = 0;
+            while (g < groups.size() && !(groups[g].plan.DH == e.DH && groups[g].plan.threads == e.threads &&
+                                          groups[g].plan.per_sm == e.per_sm)) g++;
+            if (g == groups.size()) groups.push_back(Group{DensePlan{e.DH, e.threads, e.per_sm, 0}, 0, {}});
+            groups[g].plan.smem = std::max(groups[g].plan.smem, e.smem);
+            groups[g].DG = std::max(groups[g].DG, e.dev.DG);
+            groups[g].rows.push_back(DenseRowSet{DenseRow{hop0[i], off, streams[i], n_hops[i]}, tab + key[i]});
+            max_dg = std::max(max_dg, e.dev.DG);
+        }
+        off += (long long)n_hops[i] * e.dev.T;
+    }
+    const char* lf = getenv("EWK_DENSE_LONGEST_FIRST");
+    const bool longest_first = !lf || atoi(lf) != 0;
+    std::vector<DenseRowSet> rows;
+    for (Group& g : groups) {
+        if (longest_first)
+            std::stable_sort(g.rows.begin(), g.rows.end(),
+                             [](const DenseRowSet& a, const DenseRowSet& b) { return a.r.n_hops > b.r.n_hops; });
+        rows.insert(rows.end(), g.rows.begin(), g.rows.end());
+    }
+    SlotPair<DenseRowSet>& sp = ctx->drow_sets;
+    int k = -1;
+    rc = upload_slot(ctx, sp.h, sp.b, sp.ev, sp.ev_valid, sp.idx, rows, ctx->stream, &k);
+    if (rc) return rc;
+    float* d_out = out;
+    if (where == EWK_HOST || !out) { CK(ctx->b_dense.ensure(sizeof(float) * (size_t)n_out)); d_out = (float*)ctx->b_dense.p; }
+    CK(ctx->b_g2.ensure(sizeof(float) * (size_t)B.n_streams * DENSE_WAYS * max_dg * N_MFCC));
+    size_t base = 0;
+    for (const Group& g : groups) {
+        DenseArgs A{};
+        A.DH = g.plan.DH;
+        A.DG = g.DG;
+        A.rows = (const DenseRow*)((const DenseRowSet*)sp.b[k].p + base);
+        rc = dense_launch(ctx, A, g.plan, d_out, (int)g.rows.size(), true);
+        if (rc) return rc;
+        base += g.rows.size();
+    }
+    CK(cudaEventRecord(sp.ev[k], ctx->stream));               // the slot is free once these K4 launches have read it
+    sp.ev_valid[k] = true;
+    if (d_scores) { *d_scores = d_out; return EWK_OK; }
+    if (where == EWK_HOST) {
+        CK(cudaMemcpyAsync(out, d_out, sizeof(float) * (size_t)n_out, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    return EWK_OK;
+}
+
+extern "C" int ewk_dense_scores_sets(ewk_ctx* ctx, const int32_t* streams, int n, const int64_t* hop0, const int32_t* n_hops,
+                                     const int32_t* template_first, const int32_t* template_count, float* out, int64_t out_cap,
+                                     int where) {
+    if (!ctx) return EWK_ERR_ARG;
+    int rc = need_streams(ctx, "ewk_dense_scores_sets");
+    if (rc) return rc;
+    return dense_rows_sets(ctx, "ewk_dense_scores_sets", streams, n, hop0, n_hops, RowSets{template_first, template_count},
+                           out, out_cap, where);
+}
+
 extern "C" int ewk_dense_scores_streams(ewk_ctx* ctx, const int32_t* streams, int n, const int64_t* hop0, const int32_t* n_hops,
                                         int template_first, int template_count, float* out, int64_t out_cap, int where) {
     if (!ctx) return EWK_ERR_ARG;
@@ -2393,11 +2610,12 @@ extern "C" int ewk_dense_scores_streams(ewk_ctx* ctx, const int32_t* streams, in
                       where);
 }
 
-extern "C" int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first,
-                               int template_count, int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap,
-                               int where) {
+// ewk_dense_ready (rs = NULL: the call's one set [template_first, template_first + template_count)) and
+// ewk_dense_ready_sets (rs: a set per row)
+static int dense_ready_impl(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, int max_hops, int template_first,
+                            int template_count, const RowSets* rs, int64_t* hop0_out, int32_t* n_hops_out, float* out,
+                            int64_t out_cap, int where) {
     if (!ctx) return EWK_ERR_ARG;
-    const char* who = "ewk_dense_ready";
     int rc = need_streams(ctx, who);
     if (rc) return rc;
     BankView& B = ctx->bank;
@@ -2428,7 +2646,8 @@ extern "C" int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int 
         h0[i] = ctx->h_dense_next[s];
         nh[i] = (int32_t)std::max<long long>(0, std::min<long long>(h0[i] + max_hops, ctx->h_written[s] / 160 + 1) - h0[i]);
     }
-    rc = dense_rows(ctx, who, streams, n, h0.data(), nh.data(), template_first, template_count, out, out_cap, where);
+    rc = rs ? dense_rows_sets(ctx, who, streams, n, h0.data(), nh.data(), *rs, out, out_cap, where)
+            : dense_rows(ctx, who, streams, n, h0.data(), nh.data(), template_first, template_count, out, out_cap, where);
     if (rc) return rc;
     for (int i = 0; i < n; i++) {
         hop0_out[i] = h0[i];
@@ -2438,15 +2657,30 @@ extern "C" int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int 
     return EWK_OK;
 }
 
+extern "C" int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first,
+                               int template_count, int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap,
+                               int where) {
+    return dense_ready_impl(ctx, "ewk_dense_ready", streams, n, max_hops, template_first, template_count, nullptr, hop0_out,
+                            n_hops_out, out, out_cap, where);
+}
+
+extern "C" int ewk_dense_ready_sets(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, const int32_t* template_first,
+                                    const int32_t* template_count, int64_t* hop0_out, int32_t* n_hops_out, float* out,
+                                    int64_t out_cap, int where) {
+    const RowSets rs{template_first, template_count};
+    return dense_ready_impl(ctx, "ewk_dense_ready_sets", streams, n, max_hops, 0, 0, &rs, hop0_out, n_hops_out, out, out_cap,
+                            where);
+}
+
 static_assert(sizeof(DetRecord) == sizeof(ewk_detection) && sizeof(ewk_detection) == 48, "ewk_detection layout");
 static_assert(offsetof(DetRecord, score) == offsetof(ewk_detection, score), "ewk_detection layout");
 
-// ewk_dense_ready's due rule on the detector's own cursor, then K4 (per-row) and K4D behind it on the context's stream
-extern "C" int ewk_dense_detect(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first,
-                                int template_count, int hold_hops, int refractory_hops, ewk_detection* det, int det_cap,
-                                int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where) {
+// ewk_dense_ready's due rule on the detector's own cursor, then K4 (per-row) and K4D behind it on the context's stream.
+// rs = NULL: ewk_dense_detect's one set; rs: ewk_dense_detect_sets, a set per row (K4 per geometry, K4D's set form)
+static int dense_detect_impl(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, int max_hops, int template_first,
+                             int template_count, const RowSets* rs, int hold_hops, int refractory_hops, ewk_detection* det,
+                             int det_cap, int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where) {
     if (!ctx) return EWK_ERR_ARG;
-    const char* who = "ewk_dense_detect";
     int rc = need_streams(ctx, who);
     if (rc) return rc;
     BankView& B = ctx->bank;
@@ -2496,8 +2730,10 @@ extern "C" int ewk_dense_detect(ewk_ctx* ctx, const int32_t* streams, int n, int
         ctx->det_map_cap = want;
     }
     float* d_scores = nullptr;
-    rc = dense_rows(ctx, who, streams, n, h0.data(), nh.data(), template_first, template_count, out, out_cap, where,
-                    &d_scores);
+    std::vector<int> keys;
+    rc = rs ? dense_rows_sets(ctx, who, streams, n, h0.data(), nh.data(), *rs, out, out_cap, where, &d_scores, &keys)
+            : dense_rows(ctx, who, streams, n, h0.data(), nh.data(), template_first, template_count, out, out_cap, where,
+                         &d_scores);
     if (rc) return rc;
     int n_det = 0;
     if (d_scores) {
@@ -2506,33 +2742,43 @@ extern "C" int ewk_dense_detect(ewk_ctx* ctx, const int32_t* streams, int n, int
             CK(cudaMemsetAsync(ctx->b_det_state.p, 0, sizeof(DetState) * (size_t)B.n_streams, ctx->stream));
         }
         std::vector<DetRow> rows;
+        std::vector<DetRowSet> srows;                         // rs: the same rows with their sets
         long long off = 0, doff = 0;
         for (int i = 0; i < n; i++) {
-            if (nh[i] > 0) rows.push_back(DetRow{h0[i], off, doff, streams[i], nh[i], i, 0});
-            off += (long long)nh[i] * template_count;
+            if (nh[i] > 0) {
+                rows.push_back(DetRow{h0[i], off, doff, streams[i], nh[i], i, 0});
+                if (rs) srows.push_back(DetRowSet{rows.back(), (const DenseSetDev*)ctx->b_dset.p + keys[i]});
+            }
+            off += (long long)nh[i] * (rs ? ctx->h_dset[keys[i]].dev.T : template_count);
             doff += (nh[i] + 1) / 2;
         }
         int k = -1;
-        rc = upload_slot(ctx, ctx->h_ddet, ctx->b_ddet, ctx->ev_ddet, ctx->ev_ddet_valid, ctx->ddet_idx, rows, ctx->stream, &k);
+        SlotPair<DetRowSet>& sp = ctx->ddet_sets;
+        rc = rs ? upload_slot(ctx, sp.h, sp.b, sp.ev, sp.ev_valid, sp.idx, srows, ctx->stream, &k)
+                : upload_slot(ctx, ctx->h_ddet, ctx->b_ddet, ctx->ev_ddet, ctx->ev_ddet_valid, ctx->ddet_idx, rows, ctx->stream, &k);
         if (rc) return rc;
         char* d_map = nullptr;
         CK(cudaHostGetDevicePointer((void**)&d_map, ctx->h_det_map, 0));
         DetArgs D{};
-        D.T = template_count; D.slot0 = template_first; D.hold = hold_hops; D.refractory = refractory_hops;
-        for (int t = 0; t < template_count; t++) {
-            const int L = (int)ctx->h_tmpl[template_first + t].n_samples;
-            D.L[t] = L; D.n[t] = (L + HOP - 1) / HOP;
+        D.hold = hold_hops; D.refractory = refractory_hops;
+        if (!rs) {
+            D.T = template_count; D.slot0 = template_first;
+            for (int t = 0; t < template_count; t++) {
+                const int L = (int)ctx->h_tmpl[template_first + t].n_samples;
+                D.L[t] = L; D.n[t] = (L + HOP - 1) / HOP;
+            }
         }
-        D.rows = (const DetRow*)ctx->b_ddet[k].p; D.n_rows = (int)rows.size();
+        D.rows = (const DetRow*)(rs ? sp.b[k].p : ctx->b_ddet[k].p); D.n_rows = (int)rows.size();
         D.scores = d_scores; D.state = (DetState*)ctx->b_det_state.p;
         D.counts = (int*)d_map; D.rec = (DetRecord*)(d_map + rec_off);
         cudaEvent_t pe = ctx->prof_begin(4);
-        dense_detect_kernel<<<(D.n_rows + DETECT_WARPS - 1) / DETECT_WARPS, 32 * DETECT_WARPS, 0, ctx->stream>>>(B.prm, D);
+        (rs ? dense_detect_kernel<true> : dense_detect_kernel<false>)
+            <<<(D.n_rows + DETECT_WARPS - 1) / DETECT_WARPS, 32 * DETECT_WARPS, 0, ctx->stream>>>(B.prm, D);
         ctx->prof_end(pe, 4);
         CK(cudaGetLastError());
         ctx->launches++;
-        CK(cudaEventRecord(ctx->ev_ddet[k], ctx->stream));
-        ctx->ev_ddet_valid[k] = true;
+        CK(cudaEventRecord(rs ? sp.ev[k] : ctx->ev_ddet[k], ctx->stream));
+        (rs ? sp.ev_valid[k] : ctx->ev_ddet_valid[k]) = true;
         if (out && where == EWK_HOST)
             CK(cudaMemcpyAsync(out, d_scores, sizeof(float) * (size_t)off, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
@@ -2550,6 +2796,22 @@ extern "C" int ewk_dense_detect(ewk_ctx* ctx, const int32_t* streams, int n, int
         ctx->h_det_next[streams[i]] += nh[i];
     }
     return n_det;
+}
+
+extern "C" int ewk_dense_detect(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first,
+                                int template_count, int hold_hops, int refractory_hops, ewk_detection* det, int det_cap,
+                                int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where) {
+    return dense_detect_impl(ctx, "ewk_dense_detect", streams, n, max_hops, template_first, template_count, nullptr,
+                             hold_hops, refractory_hops, det, det_cap, hop0_out, n_hops_out, out, out_cap, where);
+}
+
+extern "C" int ewk_dense_detect_sets(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, const int32_t* template_first,
+                                     const int32_t* template_count, int hold_hops, int refractory_hops, ewk_detection* det,
+                                     int det_cap, int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap,
+                                     int where) {
+    const RowSets rs{template_first, template_count};
+    return dense_detect_impl(ctx, "ewk_dense_detect_sets", streams, n, max_hops, 0, 0, &rs, hold_hops, refractory_hops, det,
+                             det_cap, hop0_out, n_hops_out, out, out_cap, where);
 }
 
 extern "C" int ewk_stream_results(ewk_ctx* ctx, ewk_stream_result* out) {

@@ -34,6 +34,32 @@ struct DevBuf {
     void free() { if (p) cudaFree(p); p = nullptr; cap = 0; }
 };
 
+// two slots of pinned host + device memory for descriptors (upload_slot), each reused only once its reader has run (ev)
+template <class D>
+struct SlotPair {
+    D* h[2] = {nullptr, nullptr};
+    DevBuf b[2];
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    bool ev_valid[2] = {false, false};
+    int idx = 0;
+    void free() {
+        for (int i = 0; i < 2; i++) {
+            if (ev[i]) cudaEventDestroy(ev[i]);
+            if (h[i]) cudaFreeHost(h[i]);
+            ev[i] = nullptr; h[i] = nullptr; ev_valid[i] = false;
+            b[i].free();
+        }
+    }
+};
+
+// A template set's descriptor for K4 / K4D (valid: built and on the device) and the launch geometry it has alone
+struct DenseSetHost {
+    bool valid = false;
+    int DH = 0, threads = 0, per_sm = 0;
+    size_t smem = 0;
+    DenseSetDev dev{};
+};
+
 }  // namespace ewk
 
 struct ewk_ctx {
@@ -99,6 +125,15 @@ struct ewk_ctx {
     bool ev_ddet_valid[2] = {false, false};
     int ddet_idx = 0;
     ewk::DevBuf b_det_state;                 // K4D's DetState [n_streams], allocated (zeroed) by the first detect call
+    // per-row template sets (ewk_dense_*_sets): the descriptor of set [first, first + count) sits at index
+    // first * DENSE_MAX_T + count - 1 of a device table; h_dset mirrors it.  A set is built and uploaded on first use and
+    // kept until a template slot of its range changes (dense_sets_forget).  New descriptors go through dset_stage.
+    std::vector<ewk::DenseSetHost> h_dset;
+    ewk::DevBuf b_dset;
+    ewk::SlotPair<ewk::DenseSetDev> dset_stage;
+    ewk::SlotPair<ewk::DenseRowSet> drow_sets;   // K4 row descriptors of a per-row-set call
+    ewk::SlotPair<ewk::DetRowSet> ddet_sets;     // K4D row descriptors of ewk_dense_detect_sets
+    void dense_sets_forget(int slot);
     // K4D's output, pinned and mapped into the device: per-row record counts [n_streams], then records (row i at its offset)
     void* h_det_map = nullptr;
     size_t det_map_cap = 0;

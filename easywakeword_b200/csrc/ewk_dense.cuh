@@ -81,6 +81,20 @@ struct DenseRow {
     int stream, n_hops;
 };
 
+// The template-dependent part of DenseArgs for one template set [slot0, slot0 + T) (fields as there).  The context
+// keeps a table of them (ewk_dense_*_sets); a SETS-instance CTA takes its set from its row descriptor.
+struct DenseSetDev {
+    int T, DG, DLE, n_re_u, n_min, n_max, g_back, slot0;
+    int re_goff[DENSE_MAX_RE], re_delta[DENSE_MAX_RE], re_rep[DENSE_MAX_RE], re_rep_e[DENSE_MAX_RE], re_nfirst[DENSE_MAX_RE];
+    DenseTmplDev t[DENSE_MAX_T];
+};
+
+// A row of a per-row-set call: the row and its set in the context's table
+struct DenseRowSet {
+    DenseRow r;
+    const DenseSetDev* set;
+};
+
 struct DenseArgs {
     long long hop0;                    // first hop scored (hop h <-> 160 h samples of the stream); uniform instance only
     int n_hops;
@@ -97,8 +111,9 @@ struct DenseArgs {
     int re_goff[DENSE_MAX_RE], re_delta[DENSE_MAX_RE], re_rep[DENSE_MAX_RE], re_rep_e[DENSE_MAX_RE], re_nfirst[DENSE_MAX_RE];
     DenseTmplDev t[DENSE_MAX_T];
     float* out;                        // uniform: [n_streams][n_hops][T]; rows: packed as their descriptors say
-    const DenseRow* rows;              // ROWS instance: one descriptor per CTA
-    float* g2;                         // [n_streams][DENSE_WAYS][DG][20]: grid rows floored with a way's floor (tags in shared memory)
+    const DenseRow* rows;              // ROWS instance: one descriptor per CTA (SETS instance: DenseRowSet descriptors)
+    float* g2;                         // [n_streams][DENSE_WAYS][DG][20]: grid rows floored with a way's floor (tags in shared memory);
+                                       // SETS instance: streams DG (the launch's largest) apart, a set's own DG within
     // carry-over between consecutive calls: the newest stream-grid rows of every stream (functions of the PCM only)
     float* keep_rows;                  // [n_streams][DENSE_KEEP][ROW], row of grid frame g at g % DENSE_KEEP
     long long* keep_end;               // [n_streams][2]: grid frames [keep_end[2s], keep_end[2s+1]) are stored (0, 0: nothing)
@@ -220,13 +235,23 @@ __device__ __forceinline__ int next_task(int* counter, int lane) {
 __device__ __forceinline__ int wrap1(int r, int n) { return r >= n ? r - n : r; }
 
 // ROWS = false: CTA s scores stream s at the call's hops [A.hop0, A.hop0 + A.n_hops).  ROWS = true: CTA x takes
-// descriptor A.rows[x] (its stream, hop range and output block); the body is the same.
-template <bool PRE, bool ROWS>
+// descriptor A.rows[x] (its stream, hop range and output block); the body is the same.  SETS = true (with ROWS): the
+// descriptors are DenseRowSet, and each CTA takes the template-dependent fields (T, DG, DLE, n_re_u, n_min, n_max,
+// g_back, re_*, t[]) from its row's set instead of A; A.DH is the launch's, A.DG the g2 stride.
+template <bool PRE, bool ROWS, bool SETS = false>
 __global__ void __launch_bounds__(1024, 1)
 dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const TemplateFeat* __restrict__ tmpl, DenseArgs A) {
+    static_assert(ROWS || !SETS, "per-row sets need row descriptors");
     extern __shared__ __align__(16) float smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5, nthr = blockDim.x;
-    const int DH = A.DH, DG = A.DG, DLE = A.DLE, NT = A.T;
+    // the row's set is re-read where it is used, as the row's hops are
+    auto row = [&]() -> const DenseRow& {
+        if constexpr (SETS) return reinterpret_cast<const DenseRowSet*>(A.rows)[blockIdx.x].r;
+        else return A.rows[blockIdx.x];
+    };
+    auto set = [&]() -> const DenseSetDev& { return *reinterpret_cast<const DenseRowSet*>(A.rows)[blockIdx.x].set; };
+#define DSET(f) (SETS ? set().f : A.f)
+    const int DH = A.DH, DG = DSET(DG), DLE = DSET(DLE), NT = DSET(T);
     FrameTables* ft = reinterpret_cast<FrameTables*>(smem);
     float* scratch = smem + sizeof(FrameTables) / sizeof(float);
     float2* MS = reinterpret_cast<float2*>(scratch + (size_t)nwarps * SCR_WARP);   // [T][20][DH] (mean, std) of a coefficient
@@ -234,7 +259,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     float* LE0 = G + (size_t)DG * ROW;                           // [DLE][ROW], start j at j % DLE: frame t = 0
     float* LE1 = LE0 + (size_t)DLE * ROW;                        //                                  frame t = 1
     float* RE = LE1 + (size_t)DLE * ROW;                         // [n_re_u][DH][ROW]
-    float* PM = RE + (size_t)A.n_re_u * DH * ROW;                // [T][B0_PARTS][2][DH] partial (max over all frames, min over grid frames)
+    float* PM = RE + (size_t)DSET(n_re_u) * DH * ROW;                // [T][B0_PARTS][2][DH] partial (max over all frames, min over grid frames)
     float* WFL = PM + (size_t)2 * NT * DH * B0_PARTS;            // [T][DH] floor of a floored window, +INF otherwise
     float* EMN = WFL + (size_t)NT * DH;                          // [T][DH] min over the window's edge frames
     float* patchb = EMN + (size_t)NT * DH;                       // [nwarps][20]
@@ -246,13 +271,13 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     int* WAYU = ctl + 32;
     int* WAYMASK = ctl + 40;
     int* COMBO = ctl + 56;
-    const int s = ROWS ? A.rows[blockIdx.x].stream : blockIdx.x;
+    const int s = ROWS ? row().stream : blockIdx.x;
     // the row's hops are re-read where they are used: values kept live across the kernel would cost registers
-    auto hop0 = [&]() -> long long { return ROWS ? A.rows[blockIdx.x].hop0 : A.hop0; };
-    auto n_hops = [&]() -> int { return ROWS ? A.rows[blockIdx.x].n_hops : A.n_hops; };
+    auto hop0 = [&]() -> long long { return ROWS ? row().hop0 : A.hop0; };
+    auto n_hops = [&]() -> int { return ROWS ? row().n_hops : A.n_hops; };
     // score of hop (hs + hl), template k
     auto out_at = [&](long long hs, int hl, int k) -> float* {
-        if (ROWS) return A.out + A.rows[blockIdx.x].out + (size_t)(hs - hop0() + hl) * NT + k;
+        if (ROWS) return A.out + row().out + (size_t)(hs - hop0() + hl) * NT + k;
         return A.out + ((size_t)s * A.n_hops + (size_t)(hs - A.hop0 + hl)) * NT + k;
     };
     copy_frame_tables(*ft, T, tid, nthr);
@@ -264,7 +289,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     const size_t esz = B.fmt == 1 ? 2 : 4;
     const void* ring_s = (const char*)B.ring + (size_t)s * B.P * esz;
     const int fmt = B.fmt, P = B.P;
-    float* G2 = A.g2 + (size_t)s * DENSE_WAYS * DG * N_MFCC;
+    float* G2 = A.g2 + (size_t)s * DENSE_WAYS * (SETS ? A.DG : DG) * N_MFCC;
     __syncthreads();
     const float pre = PRE ? ft->preemph : 0.f;
     const int n_mfcc = ft->n_mfcc;
@@ -274,7 +299,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     {
         // rows computed by the previous call are reused when this call continues where it stopped: the history of
         // the first window (up to n_max frames) is loaded instead of recomputed
-        long long need_lo = hop0() - A.n_max + 1;
+        long long need_lo = hop0() - DSET(n_max) + 1;
         if (need_lo < 2) need_lo = 2;
         const long long klo = A.keep_rows ? A.keep_end[2 * s] : 0, kend = A.keep_rows ? A.keep_end[2 * s + 1] : 0;
         if (klo <= need_lo && need_lo < kend && kend - need_lo <= DG) {
@@ -298,7 +323,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     // (mean, std) of coefficient c for the 32 hops of half hh of template k from exact integer window sums over the
     // stream-grid rows as way w sees them (w < 0: un-floored) plus the window's un-floored edge rows; lanes = hops
     auto window_sums = [&](int k, int c, int hh, int nh, long long hs, int w, float f, bool& valid_o, float& mean_o, float& sd_o) {
-        const DenseTmplDev& tp = A.t[k];
+        const DenseTmplDev& tp = DSET(t[k]);
         const int hl = 32 * hh + lane;
         const bool valid = hl < nh && hs + hl - tp.n >= 0;
         valid_o = valid;
@@ -367,19 +392,19 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
         // ================================================================ phase A: frames of this sub-chunk
         // stream-grid rows [g_from, g_hi]: every template's windows of these hops reach back to hs - n + 1 (the row a
         // sliding difference removes) and forward to hop - (n - t_hi)
-        long long g_lo = hs - A.n_max + 1;
+        long long g_lo = hs - DSET(n_max) + 1;
         if (g_lo < 2) g_lo = 2;                                   // grid frame g needs samples from 160 g - 256 >= 0
-        const long long g_hi = hs + nh - 1 - A.g_back;
+        const long long g_hi = hs + nh - 1 - DSET(g_back);
         const long long g_from = max(g_lo, g_done);
         if (g_valid_lo == LLONG_MAX) g_valid_lo = g_from;
         const int n_g = (int)max(0LL, g_hi - g_from + 1);
         // left-edge rows of the starts these hops use: [hs - n_max, hs + nh - n_min), those not yet in the rings
-        long long le_lo = hs - A.n_max;
+        long long le_lo = hs - DSET(n_max);
         if (le_lo < 0) le_lo = 0;
-        const long long le_hi = hs + nh - A.n_min;               // exclusive
+        const long long le_hi = hs + nh - DSET(n_min);               // exclusive
         const long long le_from = max(le_lo, le_done);
         const int n_le = (int)max(0LL, le_hi - le_from);
-        const int n_re = A.n_re_u * nh;                          // enumerated as (distinct right-edge frame, hop slot)
+        const int n_re = DSET(n_re_u) * nh;                          // enumerated as (distinct right-edge frame, hop slot)
         // 32-bit bases for this sub-chunk: ring position of sample 160 * hs, ring rows / slots of the first new frames
         const int hs_pos = (int)((160 * hs) % P);
         const int gfrom_row = n_g > 0 ? (int)(g_from % DG) : 0;
@@ -388,7 +413,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
         if (tid == 0) { ctl[1] = 0; ctl[2] = 0; ctl[3] = 0; ctl[4] = 0; ctl[5] = 0; ctl[6] = 0; ctl[7] = 0; }
         if (tid < NT) {
             // per template: ring row of grid frame (hs - n) and LE slot of start (hs - n), both possibly "negative" frames
-            const long long j0 = hs - A.t[tid].n;
+            const long long j0 = hs - DSET(t[tid]).n;
             ctl[8 + tid] = (int)(((j0 % DG) + DG) % DG);
             ctl[16 + tid] = (int)(((j0 % DLE) + DLE) % DLE);
             WAYMASK[2 * tid] = 0; WAYMASK[2 * tid + 1] = 0;
@@ -417,12 +442,12 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
             } else {
                 const int q = job - n_g - 2 * n_le;
                 const int u = q / nh, hl = q - u * nh;
-                if (hs + hl - A.re_nfirst[u] < 0) continue;                     // every window that uses it starts before the stream
+                if (hs + hl - DSET(re_nfirst[u]) < 0) continue;                     // every window that uses it starts before the stream
                 // through the window of a template that uses it (the frame itself depends on (goff, delta) only)
-                const DenseTmplDev& tp = A.t[A.re_rep[u]];
+                const DenseTmplDev& tp = DSET(t[DSET(re_rep[u])]);
                 int pos = hs_pos + 160 * (hl - tp.n);
                 if (pos < 0) pos += P; else if (pos >= P) pos -= P;
-                dense_frame<PRE>(FR_RE, ring_s, fmt, P, pos, tp.t_hi + 1 + A.re_rep_e[u], tp.L, pre, *ft, scr, lane, -INFINITY,
+                dense_frame<PRE>(FR_RE, ring_s, fmt, P, pos, tp.t_hi + 1 + DSET(re_rep_e[u]), tp.L, pre, *ft, scr, lane, -INFINITY,
                                  RE + (u * DH + hl) * ROW, true);
             }
         }
@@ -437,7 +462,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
             if (job < n_b0) {
                 // ---- B0: partial max / min over a quarter of the window's frames, lanes = hops
                 const int p = job % B0_PARTS, kh = job / B0_PARTS, hh = kh % n_half, k = kh / n_half;
-                const DenseTmplDev& tp = A.t[k];
+                const DenseTmplDev& tp = DSET(t[k]);
                 const int hl = 32 * hh + lane;
                 const bool valid = hl < nh && hs + hl - tp.n >= 0;
                 float wmax = -INFINITY, wmin = INFINITY;
@@ -480,7 +505,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
         // ================================================================ phase S: floors, scores of un-floored windows
         for (int job = warp; job < NT * n_half; job += nwarps) {
             const int hh = job % n_half, k = job / n_half;
-            const DenseTmplDev& tp = A.t[k];
+            const DenseTmplDev& tp = DSET(t[k]);
             const int hl = 32 * hh + lane;
             const TemplateFeat& tf = tmpl[tp.slot];
             if (hl >= nh) continue;
@@ -558,7 +583,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
                     continue;
                 }
                 const int e_ = FLIST[job], k = e_ / DH, hl = e_ - k * DH;
-                const DenseTmplDev& tp = A.t[k];
+                const DenseTmplDev& tp = DSET(t[k]);
                 const float f = WFL[k * DH + hl];
                 const int fb = __float_as_int(f);
                 int way = -1;                                                   // the way that holds this floor, if any
@@ -639,7 +664,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
                 const int hh = job % n_half, k = job / n_half;
                 const int hl = 32 * hh + lane;
                 if (hl >= nh || WAY[k * DH + hl] < 0) continue;
-                *out_at(hs, hl, k) = score_window(k, hl, tmpl[A.t[k].slot]);
+                *out_at(hs, hl, k) = score_window(k, hl, tmpl[DSET(t[k]).slot]);
             }
             __syncthreads();
         }
@@ -647,7 +672,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     if (A.keep_rows && g_done > 2) {
         // keep the newest rows for the next call, as many as its first window reaches back
         float* kr = A.keep_rows + (size_t)s * DENSE_KEEP * ROW;
-        const long long lo = max(g_valid_lo, g_done - min(min(DENSE_KEEP, DG), A.n_max + 1));
+        const long long lo = max(g_valid_lo, g_done - min(min(DENSE_KEEP, DG), DSET(n_max) + 1));
         const int cnt = (int)max(0LL, g_done - lo);
         for (int i = tid; i < cnt * ROW; i += nthr) {
             const long long g = lo + i / ROW;
@@ -655,6 +680,7 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
         }
         if (tid == 0) { A.keep_end[2 * s] = lo; A.keep_end[2 * s + 1] = g_done; }
     }
+#undef DSET
 }
 
 // ---- K4D — dense_detect: a per-stream peak picker over the scores K4 just wrote (ewk_dense_detect) -------------------
@@ -684,6 +710,12 @@ struct DetRow {
     int stream, n_hops, row, pad;
 };
 
+// A row of a per-row-set detect call: the row and its set (T, slot0, per-template n and L) in the context's table
+struct DetRowSet {
+    DetRow r;
+    const DenseSetDev* set;
+};
+
 struct DetArgs {
     int T, slot0, hold, refractory;    // templates [slot0, slot0 + T) of the call
     int n[DENSE_MAX_T], L[DENSE_MAX_T]; // per template: window in hops (ceil(L / 160)) and samples
@@ -695,11 +727,15 @@ struct DetArgs {
     int* counts;                       // host-mapped [list length]
 };
 
+// SETS = true: A.rows holds DetRowSet descriptors, and each row takes T, slot0, n and L from its set instead of A
+template <bool SETS = false>
 __global__ void __launch_bounds__(32 * DETECT_WARPS)
 dense_detect_kernel(const StreamParams* __restrict__ prm, DetArgs A) {
     const int lane = threadIdx.x & 31, w = blockIdx.x * DETECT_WARPS + (threadIdx.x >> 5);
     if (w >= A.n_rows) return;
-    const DetRow r = A.rows[w];
+    const DetRow r = SETS ? reinterpret_cast<const DetRowSet*>(A.rows)[w].r : A.rows[w];
+    const DenseSetDev* __restrict__ set = SETS ? reinterpret_cast<const DetRowSet*>(A.rows)[w].set : nullptr;
+    const int T = SETS ? set->T : A.T, slot0 = SETS ? set->slot0 : A.slot0;
     const float thr = prm[r.stream].similarity_threshold;
     const float* __restrict__ sc = A.scores + r.scores;
     DetRecord* __restrict__ out = A.rec + r.det;
@@ -710,8 +746,8 @@ dense_detect_kernel(const StreamParams* __restrict__ prm, DetArgs A) {
         float b = __int_as_float(0x7fc00000);
         int kb = 0;
         if (base + lane < r.n_hops) {
-            const float* row = sc + (size_t)(base + lane) * A.T;
-            for (int k = 0; k < A.T; k++) {
+            const float* row = sc + (size_t)(base + lane) * T;
+            for (int k = 0; k < T; k++) {
                 const float v = row[k];
                 if (v > b || (b != b && v == v)) { b = v; kb = k; }
             }
@@ -722,20 +758,23 @@ dense_detect_kernel(const StreamParams* __restrict__ prm, DetArgs A) {
             const int kh = __shfl_sync(FULL, kb, i);
             const long long h = r.hop0 + base + i;
             int nk = 0, Lk = 0;                                  // window of k* (selects: no local copy of A)
+            if (SETS) { nk = set->t[kh].n; Lk = set->t[kh].L; }
+            else {
 #pragma unroll
-            for (int t = 0; t < DENSE_MAX_T; t++)
-                if (t == kh) { nk = A.n[t]; Lk = A.L[t]; }
+                for (int t = 0; t < DENSE_MAX_T; t++)
+                    if (t == kh) { nk = A.n[t]; Lk = A.L[t]; }
+            }
             const bool above = bh >= thr;
             bool emit = false;
             if (st.mode == DET_IDLE) {
                 if (above && h >= st.quiet_until) {
-                    st.mode = DET_ARMED; st.peak = h; st.run_start = h; st.score = bh; st.slot = A.slot0 + kh;
+                    st.mode = DET_ARMED; st.peak = h; st.run_start = h; st.score = bh; st.slot = slot0 + kh;
                     st.seg_start = 160LL * (h - nk); st.seg_len = Lk;
                 }
             } else if (st.mode == DET_ARMED) {
                 if (above) {
                     if (bh > st.score) {
-                        st.peak = h; st.score = bh; st.slot = A.slot0 + kh;
+                        st.peak = h; st.score = bh; st.slot = slot0 + kh;
                         st.seg_start = 160LL * (h - nk); st.seg_len = Lk;
                     }
                     if (h - st.peak >= A.hold) { emit = true; st.mode = DET_SPENT; }

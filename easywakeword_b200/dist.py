@@ -135,24 +135,26 @@ class ShardedBank:
                 rows.append(blk)
         return self.bank.step_streams(streams, rows)
 
-    def dense_ready(self, global_streams, template_first: int = 0, template_count=None):
+    def dense_ready(self, global_streams, template_first: int = 0, template_count=None, own_templates: bool = False):
         """WakeWordBank.dense_ready over global stream ids: every rank may be called with the whole list and scores the
         streams it owns (dist.local_streams).  Returns {global stream id: (first hop, float32 [n, T] scores)}."""
         loc = local_streams(global_streams, self.n_total, self.world, self.rank)
         if not loc:
             return {}
-        hop0, rows = self.bank.dense_ready(loc, template_first, template_count)
+        kw = {"own_templates": True} if own_templates else {}
+        hop0, rows = self.bank.dense_ready(loc, template_first, template_count, **kw)
         return {self.first + s: (int(h), r) for s, h, r in zip(loc, hop0, rows)}
 
     def dense_detect(self, global_streams, template_first: int = 0, template_count=None, hold_hops: int = 20,
-                     refractory_hops: int = 50):
+                     refractory_hops: int = 50, own_templates: bool = False):
         """WakeWordBank.dense_detect over global stream ids: every rank may be called with the whole list and detects on
         the streams it owns (dist.local_streams).  Returns this rank's detections with global stream ids."""
         from . import _lib
         loc = local_streams(global_streams, self.n_total, self.world, self.rank)
         if not loc:
             return np.zeros(0, _lib.DETECTION_DTYPE)
-        det = self.bank.dense_detect(loc, template_first, template_count, hold_hops, refractory_hops)
+        kw = {"own_templates": True} if own_templates else {}
+        det = self.bank.dense_detect(loc, template_first, template_count, hold_hops, refractory_hops, **kw)
         det["stream"] += self.first
         return det
 

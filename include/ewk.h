@@ -430,6 +430,39 @@ int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, i
 int ewk_dense_detect(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first, int template_count,
                      int hold_hops, int refractory_hops, ewk_detection* det, int det_cap,
                      int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where);
+/* Per-row template sets: the forms above with a template set of its own for every row, in one call.  Row i is scored
+ * against slots [template_first[i], template_first[i] + template_count[i]); with both arrays NULL, row i takes its
+ * stream's own range (ewk_stream_params.template_first / template_count, the gate's range).  streams = NULL in the ready
+ * and detect forms means every stream, as there (the arrays then have n_streams entries).
+ *   Results: every score of row i is bit-identical to what ewk_dense_scores_streams gives for that stream and those hops
+ *   with row i's set (NaN where the window starts before the stream); every detection equals what ewk_dense_detect emits
+ *   for that stream with that set (template_slot is the absolute slot; within a set the lowest k wins ties).
+ *   Packing: rows in list order; row i starts at float sum_{j < i} n_hops[j] T_j and is laid out [n_hops[i]][T_i],
+ *   T_i = template_count[i].  n * max_hops * max_i T_i floats always suffice for the ready and detect forms; the
+ *   detection bound stays sum_i ceil(n_hops_i / 2).
+ *   Cursors and state: ewk_dense_ready_sets reads and moves ewk_dense_ready's cursor, ewk_dense_detect_sets the
+ *   detector's cursor and state of ewk_dense_detect, so a stream may switch between the forms, and between sets, from one
+ *   call to the next.  ewk_reset_streams and ewk_export_streams / ewk_import_streams treat them as before.
+ *   Launches: one K4 launch per distinct launch geometry (ewk_dense_plan of the set alone: hops per sub-chunk, threads,
+ *   CTAs per SM; at most 8) among the rows' sets, each row at the geometry its set has alone, plus one K4D launch for
+ *   ewk_dense_detect_sets.  The number of launches does not grow with the number of distinct sets.
+ *   ewk_dense_last_plan reports the call's last K4 launch.  A set's descriptor is built on its first use and kept on
+ *   the device until ewk_set_template, ewk_set_template_features or ewk_clear_template changes a slot of its range, so
+ *   a steady-state call uploads only its row descriptors.
+ *   Errors, all before the first launch (no cursor, detector state or score moves), naming the row and the stream:
+ *   EWK_ERR_ARG for a set of a count outside 1..8 or a range outside [0, max_templates), a template length outside
+ *   640..48000, a set that does not fit shared memory alone (ewk_dense_plan refuses it), or only one of the two arrays
+ *   given; EWK_ERR_NO_TEMPLATE for an empty slot; otherwise the errors of the single-set form. */
+int ewk_dense_scores_sets(ewk_ctx* ctx, const int32_t* streams, int n, const int64_t* hop0, const int32_t* n_hops,
+                          const int32_t* template_first, const int32_t* template_count,
+                          float* out, int64_t out_cap, int where);
+int ewk_dense_ready_sets(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops,
+                         const int32_t* template_first, const int32_t* template_count,
+                         int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where);
+int ewk_dense_detect_sets(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops,
+                          const int32_t* template_first, const int32_t* template_count,
+                          int hold_hops, int refractory_hops, ewk_detection* det, int det_cap,
+                          int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where);
 /* Launch geometry ewk_dense_scores chooses for templates of these lengths (samples, n <= 8, each 640..48000):
  * out = {hops per sub-chunk (32 or 64), threads per CTA, CTAs per SM, dynamic shared memory bytes}.  Host code only
  * (no context, no device): the function ewk_dense_scores itself plans with.  EWK_ERR_ARG for lengths out of range or a
