@@ -59,6 +59,7 @@ def load():
         "ewk_similarity_batch": (C.c_int, [vp, i32, vp, i32, i32, _p(i64), _p(i64), i32, C.c_float, f32p,
                                            _p(C.c_uint8), f32p]),
         "ewk_analyze_templates": (C.c_int, [vp, f32p, i32, _p(i64), _p(i64), i32, vp, f32p, i64]),
+        "ewk_set_templates": (C.c_int, [vp, _p(C.c_int32), i32, vp, i32, _p(i64), _p(i64), vp]),
         "ewk_resample_info": (C.c_int, [i32, _p(C.c_int32), _p(C.c_int32), _p(C.c_int32)]),
         "ewk_resample_out_len": (i64, [i64, i32]),
         "ewk_resample": (C.c_int, [vp, vp, i32, i32, i32, i64, i64, i32, i64, i64, i64, vp, i64, i32]),
@@ -222,6 +223,30 @@ class Context:
             return out, np.split(rms, cuts)
         return out
 
+    def set_templates(self, slots, audios, want_vad=False):
+        """Batched enrolment (include/ewk.h: ewk_set_templates): template slots[i] <- audios[i], each slot bit-identical
+        to set_template(slots[i], audios[i]), in one K3 launch.  audios: a sequence of float32 16 kHz arrays, or a
+        device input (ptr, offsets, lens): template i is the float32 device samples ptr[offsets[i] : offsets[i] +
+        lens[i]].  want_vad: also return analyze_templates of the same audio (VAD_DTYPE [n])."""
+        sl = _int32_list(slots, "template slot")
+        if isinstance(audios, tuple):
+            ptr, offs, lens = audios
+            offs = np.ascontiguousarray(np.asarray(offs, dtype=np.int64).reshape(-1))
+            lens = np.ascontiguousarray(np.asarray(lens, dtype=np.int64).reshape(-1))
+            pcm, where = C.c_void_p(ptr), DEVICE
+        else:
+            audios = [np.ascontiguousarray(a, dtype=np.float32).reshape(-1) for a in audios]
+            lens = np.array([len(a) for a in audios], np.int64)
+            offs = np.concatenate([[0], np.cumsum(lens)[:-1]]).astype(np.int64) if len(lens) else lens
+            host = np.concatenate(audios) if lens.sum() else np.zeros(1, np.float32)
+            pcm, where = host.ctypes.data, HOST
+        if len(offs) != len(sl) or len(lens) != len(sl):
+            raise ValueError("one audio per template slot")
+        vad = np.zeros(len(sl), dtype=VAD_DTYPE) if want_vad else None
+        self._ck(self.lib.ewk_set_templates(self.h, sl.ctypes.data_as(_p(C.c_int32)), len(sl), pcm, where, i64ptr(offs),
+                                            i64ptr(lens), vad.ctypes.data if want_vad else None))
+        return vad
+
     def resample(self, y, sr_in, *, in_first=0, out_first=0, n_out=None, out_device_ptr=None):
         """K7: y[rows, n] or y[n] (float32 / int16, host) at sr_in -> float32 at 16 kHz (absolute output samples
         [out_first, out_first + n_out); default: the one-shot length ceil(n * 16000 / sr_in)).  A device input is
@@ -356,6 +381,7 @@ def _declare_stream_protos(lib):
         "ewk_stream_status_get": (C.c_int, [vp, i32, _p(StreamStatus)]),
         "ewk_read_last": (C.c_int, [vp, i32, i64, f32p]),
         "ewk_read_segment": (C.c_int, [vp, i32, i64, i64, f32p]),
+        "ewk_set_templates_from_streams": (C.c_int, [vp, _p(C.c_int32), i32, _p(C.c_int32), _p(i64), _p(i64), vp]),
         "ewk_stream_results": (C.c_int, [vp, vp]),
         "ewk_dense_scores": (C.c_int, [vp, i64, i32, i32, i32, vp, i32]),
         "ewk_dense_scores_streams": (C.c_int, [vp, _p(C.c_int32), i32, _p(i64), _p(C.c_int32), i32, i32, vp, i64, i32]),
@@ -470,12 +496,17 @@ def _resampled_input(pcm_or_codes, fmt):
     return ptr, ns, n, stride, code, a
 
 
+def _int32_list(values, what):
+    """int32 array of indices (ValueError for values no int32 holds: the library names the others)."""
+    v = np.asarray(values, dtype=np.int64).reshape(-1)
+    if v.size and (v.min() < -2**31 or v.max() >= 2**31):
+        raise ValueError(f"{what} out of range")
+    return np.ascontiguousarray(v, dtype=np.int32)
+
+
 def _stream_list(streams):
     """int32 array of stream indices (ValueError for values no int32 holds: the library names the others)."""
-    st = np.asarray(streams, dtype=np.int64).reshape(-1)
-    if st.size and (st.min() < -2**31 or st.max() >= 2**31):
-        raise ValueError("stream index out of range")
-    return np.ascontiguousarray(st, dtype=np.int32)
+    return _int32_list(streams, "stream index")
 
 
 def _unpack_rows(out, n_hops, T):
@@ -831,6 +862,23 @@ def _bank_methods():
         self._ck(self.lib.ewk_read_segment(self.h, stream, int(seg_start), int(seg_len), f32ptr(out)))
         return out
 
+    def set_templates_from_streams(self, slots, streams, starts, lens, want_vad=False):
+        """Enrolment from the rings (include/ewk.h: ewk_set_templates_from_streams): template slots[i] <- stream
+        streams[i]'s absolute samples [starts[i], starts[i] + lens[i]) (an event's or a detection's seg_start /
+        seg_len), bit-identical to set_templates of what read_segment returns.  want_vad: also return the VAD analysis
+        of each segment (VAD_DTYPE [n])."""
+        sl = _int32_list(slots, "template slot")
+        st = _stream_list(streams)
+        a0 = np.ascontiguousarray(np.asarray(starts, dtype=np.int64).reshape(-1))
+        ln = np.ascontiguousarray(np.asarray(lens, dtype=np.int64).reshape(-1))
+        if not (len(st) == len(a0) == len(ln) == len(sl)):
+            raise ValueError("one stream, start and length per template slot")
+        vad = np.zeros(len(sl), dtype=VAD_DTYPE) if want_vad else None
+        self._ck(self.lib.ewk_set_templates_from_streams(self.h, sl.ctypes.data_as(_p(C.c_int32)), len(sl),
+                                                         st.ctypes.data_as(_p(C.c_int32)), i64ptr(a0), i64ptr(ln),
+                                                         vad.ctypes.data if want_vad else None))
+        return vad
+
     def dense_scores(self, hop0, n_hops, template_first=0, template_count=1, out_device_ptr=None):
         """[n_streams, n_hops, template_count] float32 scores for hops [hop0, hop0 + n_hops)."""
         if out_device_ptr is not None:
@@ -1016,7 +1064,7 @@ def _bank_methods():
                  "resample_push"]
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
-    for f in (_template_ranges, _row_sets, dense_scores_sets, dense_ready_sets, dense_detect_sets):
+    for f in (_template_ranges, _row_sets, dense_scores_sets, dense_ready_sets, dense_detect_sets, set_templates_from_streams):
         setattr(Context, f.__name__, f)
     for f in (prepare_segments, dense_scores, dense_scores_streams, dense_ready, dense_detect, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
               push_resampled_each, push_streams, tick_ready, reset_streams, stream_blob_bytes, export_streams, import_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,

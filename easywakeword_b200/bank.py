@@ -38,6 +38,31 @@ def stream_blob_rates(blob) -> np.ndarray:
     return np.ascontiguousarray(rec[:, 52:56]).view("<i4").reshape(-1)      # StreamMeta.rate
 
 
+def enroll_ranges(streams, starts, lens, slots) -> dict:
+    """{stream: (first slot, slot count, row of its first segment)} of an enrolment (WakeWordBank.enroll), in order of
+    first appearance; ValueError unless the lists have one entry per segment and every stream's slots, in list order,
+    are consecutive (at most 64 of them: include/ewk.h EWK_MAX_STREAM_TEMPLATES)."""
+    n = len(slots)
+    if not (len(streams) == len(starts) == len(lens) == n):
+        raise ValueError(f"enroll: {len(streams)} streams, {len(starts)} starts, {len(lens)} lengths and {n} slots; "
+                         "give one of each per segment")
+    ranges, last = {}, {}
+    for i in range(n):
+        s, k = int(streams[i]), int(slots[i])
+        if s not in ranges:
+            ranges[s] = (k, 1, i)
+        elif k != last[s] + 1:
+            raise ValueError(f"enroll: stream {s} is listed again at segment {i} with slot {k}; its segments must take "
+                             f"consecutive slots (expected {last[s] + 1})")
+        else:
+            first, count, row = ranges[s]
+            if count == 64:
+                raise ValueError(f"enroll: stream {s} takes more than 64 slots (EWK_MAX_STREAM_TEMPLATES)")
+            ranges[s] = (first, count + 1, row)
+        last[s] = k
+    return ranges
+
+
 class WakeWordBank:
     """N independent audio streams, one GPU.
 
@@ -60,7 +85,11 @@ class WakeWordBank:
     templates: list of float32 arrays or WAV paths (slot i = templates[i]); every stream is scored
     against all of them (best score wins) unless set_stream(..., template_first=, template_count=).
     Timing defaults are the reference's (wakeword.py:38-41); speech_duration_min/max default to the
-    auto-calculated values of the first template (tests/test_wakeword_simulated.py:687-775)."""
+    auto-calculated values of the first template (tests/test_wakeword_simulated.py:687-775).
+
+    template_slots: the context's template slots (default len(templates), at most 4096 = include/ewk.h
+    EWK_MAX_TEMPLATE_SLOTS); slots past the constructor's templates are filled later with enroll(), e.g. one personal
+    word per stream spoken by its own user."""
 
     def __init__(self, n_streams: int, templates: Sequence, *, device: int = 0, buffer_seconds: int = 10,
                  pcm_dtype=np.int16, frame_size: int = TICK_SAMPLES, similarity_threshold: float = 75.0,
@@ -68,7 +97,7 @@ class WakeWordBank:
                  speech_duration_max: Optional[float] = None, post_speech_silence: float = 0.4,
                  timeout: float = 30.0, max_push_seconds: float = 1.0, max_events: int = 0,
                  cuda_stream: Optional[int] = None, overlap: bool = False, preemphasis: float = 0.0, n_mfcc: int = 20,
-                 sample_rate: int = 16000):
+                 sample_rate: int = 16000, template_slots: Optional[int] = None):
         if n_streams < 1:
             raise ValueError("n_streams must be at least 1")
         if buffer_seconds <= 0:
@@ -83,9 +112,12 @@ class WakeWordBank:
         if self.pcm_dtype not in (np.dtype(np.int16), np.dtype(np.float32)):
             raise ValueError("pcm_dtype must be int16 or float32")
         fmt = _lib.PCM_I16 if self.pcm_dtype == np.int16 else _lib.PCM_F32
+        n_slots = len(templates) if template_slots is None else int(template_slots)
+        if n_slots < len(templates):
+            raise ValueError(f"template_slots {n_slots} is below the {len(templates)} templates given")
         slack = int(max_push_seconds * 16000) + 2 * max(frame_size, TICK_SAMPLES)
         self.ctx = _lib.Context(device=device, n_streams=n_streams, ring_samples=buffer_seconds * 16000,
-                                slack_samples=slack, pcm_format=fmt, max_templates=max(1, len(templates)),
+                                slack_samples=slack, pcm_format=fmt, max_templates=max(1, n_slots),
                                 max_events=max_events or max(4096, 2 * n_streams), preemphasis=preemphasis,
                                 n_mfcc=n_mfcc)
         if cuda_stream is not None:
@@ -137,6 +169,38 @@ class WakeWordBank:
             for s in dict.fromkeys(lst):
                 self.set_stream(s, **overrides)
         return events
+
+    # ---- enrolment
+    def enroll(self, segments, slots, set_durations: bool = True) -> np.ndarray:
+        """Personal wake words from audio the bank has heard: template slots[i] <- segment i, for all segments in one
+        call on the device (include/ewk.h: ewk_set_templates_from_streams), and each listed stream scored against its
+        own slots from then on (gate, and dense_ready / dense_detect with own_templates=True).
+        segments: structured rows with stream / seg_start / seg_len (poll()'s events, a dense_detect result, as
+        prepare_for_transcription takes them) or a (streams, starts, lens) tuple; the ranges must still be in the rings.
+        A stream listed k times takes k consecutive slots, in list order, and its range becomes those k slots (several
+        recordings of one word, best score wins); ValueError before anything is installed otherwise.  Each listed stream
+        is set through set_stream (the bank's parameters plus its new range); with set_durations its
+        speech_duration_min / max also follow the first of its recordings, by the rule the constructor applies to the
+        first template.  self.templates stays the constructor's list.  Returns the VAD analysis of every segment
+        (_lib.VAD_DTYPE, or None without set_durations)."""
+        if isinstance(segments, tuple):
+            streams, starts, lens = (np.asarray(a, dtype=np.int64).reshape(-1) for a in segments)
+        else:
+            rows = [e for e in segments]
+            streams = np.array([int(e["stream"]) for e in rows], np.int64)
+            starts = np.array([int(e["seg_start"]) for e in rows], np.int64)
+            lens = np.array([int(e["seg_len"]) for e in rows], np.int64)
+        sl = np.asarray(slots, dtype=np.int64).reshape(-1)
+        ranges = enroll_ranges(streams, starts, lens, sl)
+        vad = self.ctx.set_templates_from_streams(sl, streams, starts, lens, want_vad=set_durations)
+        for s, (first, count, row) in ranges.items():
+            over = dict(template_first=first, template_count=count)
+            if set_durations:
+                d = float(vad["duration_s"][row]) if vad["voiced"][row] else None
+                over["speech_duration_min"] = d if d is not None else 0.3
+                over["speech_duration_max"] = 2.0 * d if d is not None else 2.0
+            self.set_stream(s, **over)
+        return vad
 
     # ---- migration
     def export_streams(self, streams) -> np.ndarray:

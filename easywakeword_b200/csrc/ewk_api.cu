@@ -66,7 +66,7 @@ extern "C" int ewk_host_table(int which, float* out, int cap) {
 extern "C" int ewk_create(int device, const ewk_config* cfg, ewk_ctx** out) {
     if (!cfg || !out) { g_create_error = "ewk_create: null argument"; return EWK_ERR_ARG; }
     *out = nullptr;
-    if (cfg->n_streams < 0 || cfg->max_templates < 1 || cfg->max_templates > EWK_MAX_TEMPLATES ||
+    if (cfg->n_streams < 0 || cfg->max_templates < 1 || cfg->max_templates > EWK_MAX_TEMPLATE_SLOTS ||
         (cfg->pcm_format != EWK_PCM_F32 && cfg->pcm_format != EWK_PCM_I16) ||
         (cfg->n_streams > 0 && (cfg->ring_samples < EWK_TICK_SAMPLES || cfg->slack_samples < 0))) {
         g_create_error = "ewk_create: invalid ewk_config";
@@ -467,6 +467,151 @@ extern "C" int ewk_analyze_templates(ewk_ctx* ctx, const float* pcm, int where, 
     return EWK_OK;
 }
 
+// ---- batched enrolment: ewk_set_templates, ewk_set_templates_from_streams ----------------------------------------------
+// The checks both entry points share; entry i is template i (rows of the ring form).
+static int check_enrol(ewk_ctx* ctx, const char* who, const int32_t* slots, int n, const int64_t* offsets,
+                       const int64_t* lens) {
+    if (n < 0 || (n > 0 && (!slots || !offsets || !lens))) {
+        ctx->fail("%s: bad arguments (n=%d, slots, offsets / starts and lens must not be NULL)", who, n);
+        return EWK_ERR_ARG;
+    }
+    std::vector<char> seen((size_t)ctx->cfg.max_templates, 0);
+    for (int i = 0; i < n; i++) {
+        if (slots[i] < 0 || slots[i] >= ctx->cfg.max_templates) {
+            ctx->fail("%s: entry %d: template slot %d out of range [0, %d)", who, i, slots[i], ctx->cfg.max_templates);
+            return EWK_ERR_ARG;
+        }
+        if (seen[slots[i]]) { ctx->fail("%s: entry %d: template slot %d is listed twice", who, i, slots[i]); return EWK_ERR_ARG; }
+        seen[slots[i]] = 1;
+        if (offsets[i] < 0 || lens[i] < 1 || lens[i] > (int64_t)1 << 30) {
+            ctx->fail("%s: entry %d (slot %d): offset %lld len %lld (need offset >= 0, 1 <= len <= 2^30)", who, i, slots[i],
+                      (long long)offsets[i], (long long)lens[i]);
+            return EWK_ERR_ARG;
+        }
+    }
+    return EWK_OK;
+}
+
+// Where the templates' float32 audio comes from: host memory (copied to b_pcm first), device memory, or the rings
+// (gather rows, packed into b_pcm by one gather launch; offsets are then the packed offsets).
+struct EnrolSource { const float* pcm; int where; const std::vector<PrepDesc>* gather; };
+
+// Templates slots[i] <- audio [offsets[i], offsets[i] + lens[i]) of the source, after check_enrol.  Launches: the gather
+// (ring source), one K3 over all templates, one dense_template_install_kernel, one K6 when vad is given; one upload of
+// every descriptor, one copy back of the features (and VAD results), one synchronisation.
+static int enrol_impl(ewk_ctx* ctx, const char* who, const int32_t* slots, int n, const EnrolSource& src,
+                      const int64_t* offsets, const int64_t* lens, ewk_vad_result* vad) {
+    int64_t extent = 0, spill = 0, frames = 0;
+    int max_frames = 1;
+    for (int i = 0; i < n; i++) {
+        extent = std::max(extent, offsets[i] + lens[i]);
+        const int64_t F = 1 + lens[i] / HOP;
+        max_frames = (int)std::max<int64_t>(max_frames, F);
+        if (F > SEG_SMEM_FRAMES) spill += F;
+        frames += F;
+    }
+    // K3 keeps every frame's log-mel row (the top_db floor's input) only up to LM_WS_MAX_BYTES; ewk_set_template always
+    // does for one template, so a batch beyond it would take the other path
+    if (ctx->use_lm && sizeof(float) * (size_t)frames * LM_ROW > ewk_ctx::LM_WS_MAX_BYTES) {
+        ctx->fail("%s: the templates hold %lld frames together; one call takes at most %lld (split the batch)", who,
+                  (long long)frames, (long long)(ewk_ctx::LM_WS_MAX_BYTES / (sizeof(float) * LM_ROW)));
+        return EWK_ERR_ARG;
+    }
+    CK(cudaSetDevice(ctx->device));
+    int rc = ctx->join_match();                              // overlap mode: K3 of the last tick still reads the table
+    if (rc) return rc;
+    const float* d_pcm = src.pcm;
+    if (src.where == EWK_HOST || src.gather) {
+        CK(ctx->b_pcm.ensure(sizeof(float) * (size_t)extent));
+        if (!src.gather) CK(cudaMemcpyAsync(ctx->b_pcm.p, src.pcm, sizeof(float) * (size_t)extent, cudaMemcpyHostToDevice, ctx->stream));
+        d_pcm = (const float*)ctx->b_pcm.p;
+    }
+    // descriptors, one upload: SegDesc [n] | VadDesc [n] | int32 slots [n] | PrepDesc [gather rows]
+    const size_t o_vad = sizeof(SegDesc) * (size_t)n, o_slot = o_vad + sizeof(VadDesc) * (size_t)n;
+    const size_t o_gat = (o_slot + sizeof(int32_t) * (size_t)n + 15) & ~(size_t)15;
+    const size_t n_gat = src.gather ? src.gather->size() : 0;
+    std::vector<char> desc(o_gat + sizeof(PrepDesc) * n_gat);
+    SegDesc* sd = reinterpret_cast<SegDesc*>(desc.data());
+    VadDesc* vd = reinterpret_cast<VadDesc*>(desc.data() + o_vad);
+    int64_t ws_off = 0, f_off = 0;
+    for (int i = 0; i < n; i++) {
+        const int64_t F = 1 + lens[i] / HOP;
+        sd[i] = SegDesc{};
+        sd[i].base = d_pcm; sd[i].start = offsets[i]; sd[i].ring = 0; sd[i].len = (int)lens[i]; sd[i].fmt = 0;
+        sd[i].ws_frame_off = (int)ws_off; sd[i].frames_off = f_off; sd[i].lm_off = f_off;
+        if (F > SEG_SMEM_FRAMES) ws_off += F;
+        vd[i] = VadDesc{d_pcm, offsets[i], lens[i], f_off};
+        f_off += F;
+    }
+    std::memcpy(desc.data() + o_slot, slots, sizeof(int32_t) * (size_t)n);
+    if (n_gat) std::memcpy(desc.data() + o_gat, src.gather->data(), sizeof(PrepDesc) * n_gat);
+    CK(ctx->b_desc.ensure(desc.size()));
+    char* d_desc = (char*)ctx->b_desc.p;
+    CK(cudaMemcpyAsync(d_desc, desc.data(), desc.size(), cudaMemcpyHostToDevice, ctx->stream));
+    if (n_gat) {
+        int64_t longest = 0;
+        for (const PrepDesc& g : *src.gather) longest = std::max<int64_t>(longest, g.len);
+        const dim3 grid((unsigned)std::min<int64_t>(64, (longest + 1023) / 1024), (unsigned)n_gat);
+        ring_gather_kernel<<<grid, 256, 0, ctx->stream>>>(ctx->bank, (const PrepDesc*)(d_desc + o_gat), (float*)ctx->b_pcm.p);
+        CK(cudaGetLastError());
+        ctx->launches++;
+    }
+    // b_feat: K3 features [n][40] | dense features [n][40] | VadResult [n], copied back in one piece
+    const size_t feat_bytes = sizeof(float) * 2 * FEAT * (size_t)n, back = feat_bytes + (vad ? sizeof(VadResult) * (size_t)n : 0);
+    CK(ctx->b_feat.ensure(feat_bytes + sizeof(VadResult) * (size_t)n));
+    CK(ctx->b_frames.ensure(sizeof(float) * (size_t)frames * N_MFCC));
+    float* d_feat = (float*)ctx->b_feat.p;
+    rc = ctx->launch_segments((const SegDesc*)d_desc, n, max_frames, spill, frames, 0, 0, 0.f, d_feat,
+                              (float*)ctx->b_frames.p, nullptr, nullptr);
+    if (rc != EWK_OK) return rc;
+    dense_template_install_kernel<<<(n + ENROL_WARPS - 1) / ENROL_WARPS, ENROL_WARPS * 32, 0, ctx->stream>>>(
+        (const SegDesc*)d_desc, (const int*)(d_desc + o_slot), n, ctx->cfg.n_mfcc > 0 ? ctx->cfg.n_mfcc : N_MFCC, (const float*)ctx->b_frames.p, d_feat,
+        d_feat + (size_t)FEAT * n, ctx->d_tmpl);
+    CK(cudaGetLastError());
+    ctx->launches++;
+    if (vad) {
+        CK(ctx->b_scores.ensure(sizeof(float) * (size_t)frames));      // K6's frame RMS workspace
+        cudaEvent_t pe = ctx->prof_begin(3);
+        template_vad_kernel<<<n, VAD_THREADS, 0, ctx->stream>>>((const VadDesc*)(d_desc + o_vad),
+                                                                (VadResult*)((char*)d_feat + feat_bytes), (float*)ctx->b_scores.p);
+        ctx->prof_end(pe, 3);
+        CK(cudaGetLastError());
+        ctx->launches++;
+    }
+    std::vector<char> h(back);
+    CK(cudaMemcpyAsync(h.data(), d_feat, back, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    // the host mirror of what the install kernel wrote (install_template's fields)
+    const float* hf = reinterpret_cast<const float*>(h.data());
+    for (int i = 0; i < n; i++) {
+        TemplateFeat tf{};
+        std::memcpy(tf.mean, hf + (size_t)i * FEAT, sizeof(tf.mean));
+        std::memcpy(tf.std, hf + (size_t)i * FEAT + N_MFCC, sizeof(tf.std));
+        std::memcpy(tf.dmean, hf + (size_t)(n + i) * FEAT, sizeof(tf.dmean));
+        std::memcpy(tf.dstd, hf + (size_t)(n + i) * FEAT + N_MFCC, sizeof(tf.dstd));
+        tf.n_samples = lens[i];
+        tf.valid = 1;
+        ctx->h_tmpl[slots[i]] = tf;
+        ctx->dense_sets_forget(slots[i]);
+    }
+    if (vad) std::memcpy(vad, h.data() + feat_bytes, sizeof(VadResult) * (size_t)n);
+    return EWK_OK;
+}
+
+extern "C" int ewk_set_templates(ewk_ctx* ctx, const int32_t* slots, int n, const float* pcm, int where,
+                                 const int64_t* offsets, const int64_t* lens, ewk_vad_result* vad) {
+    if (!ctx) return EWK_ERR_ARG;
+    const char* who = "ewk_set_templates";
+    int rc = check_enrol(ctx, who, slots, n, offsets, lens);
+    if (rc) return rc;
+    if (n == 0) return EWK_OK;
+    if (!pcm || (where != EWK_HOST && where != EWK_DEVICE)) {
+        ctx->fail("%s: pcm must not be NULL and where must be EWK_HOST or EWK_DEVICE", who);
+        return EWK_ERR_ARG;
+    }
+    return enrol_impl(ctx, who, slots, n, EnrolSource{pcm, where, nullptr}, offsets, lens, vad);
+}
+
 // ------------------------------------------------------------------------------------------ K7 resampling
 extern "C" int ewk_resample_info(int sr_in, int32_t* half_width, int32_t* up, int32_t* down) {
     ResampleDesign d;
@@ -745,6 +890,11 @@ extern "C" int ewk_set_stream_params(ewk_ctx* ctx, int stream, const ewk_stream_
     }
     if (p->template_first < 0 || p->template_count < 0 || p->template_first + p->template_count > ctx->cfg.max_templates) {
         ctx->fail("template range [%d, %d) outside [0, %d)", p->template_first, p->template_first + p->template_count, ctx->cfg.max_templates);
+        return EWK_ERR_ARG;
+    }
+    if (p->template_count > EWK_MAX_STREAM_TEMPLATES) {
+        ctx->fail("template_count %d above EWK_MAX_STREAM_TEMPLATES (%d): a stream is scored against at most %d slots",
+                  p->template_count, EWK_MAX_STREAM_TEMPLATES, EWK_MAX_STREAM_TEMPLATES);
         return EWK_ERR_ARG;
     }
     CK(cudaSetDevice(ctx->device));
@@ -1640,7 +1790,8 @@ static const char* bad_meta_field(const ewk_ctx* ctx, const StreamMeta& m, int t
     if (!(p.pre_speech_silence > 0) || !(p.speech_duration_min > 0) || !(p.speech_duration_max > 0) ||
         !(p.speech_duration_min <= p.speech_duration_max) || !(p.post_speech_silence > 0) || !frame_ok(p.frame_size))
         return "stream parameters";
-    if (p.template_first < 0 || p.template_count < 0 || p.template_first + p.template_count > ctx->cfg.max_templates)
+    if (p.template_first < 0 || p.template_count < 0 || p.template_count > EWK_MAX_STREAM_TEMPLATES ||
+        p.template_first + p.template_count > ctx->cfg.max_templates)
         return "template range";
     return nullptr;
 }
@@ -1678,7 +1829,7 @@ extern "C" int ewk_import_streams(ewk_ctx* ctx, const int32_t* streams, int n, c
             ctx->fail("%s: the blob's %s (%lld) differs from the context's (%lld)", who, f.name, f.blob, f.mine);
             return EWK_ERR_ARG;
         }
-    if (h.meta_bytes != (int32_t)sizeof(StreamMeta) || h.n_templates < 0 || h.n_templates > EWK_MAX_TEMPLATES ||
+    if (h.meta_bytes != (int32_t)sizeof(StreamMeta) || h.n_templates < 0 || h.n_templates > EWK_MAX_TEMPLATE_SLOTS ||
         h.tail_floats < 0 || (h.tail_floats & 3) || h.tail_floats > 1 << 20) {
         ctx->fail("%s: bad blob header (meta_bytes %d, n_templates %d, tail_floats %d)", who, h.meta_bytes, h.n_templates,
                   h.tail_floats);
@@ -2116,6 +2267,45 @@ extern "C" int ewk_prepare_segments(ewk_ctx* ctx, int n_seg, const int32_t* stre
     }
     CK(cudaStreamSynchronize(ctx->stream));
     return EWK_OK;
+}
+
+extern "C" int ewk_set_templates_from_streams(ewk_ctx* ctx, const int32_t* slots, int n, const int32_t* streams,
+                                              const int64_t* starts, const int64_t* lens, ewk_vad_result* vad) {
+    if (!ctx) return EWK_ERR_ARG;
+    const char* who = "ewk_set_templates_from_streams";
+    int rc = need_streams(ctx, who);                         // overlap mode: K3 of the last tick still reads the table
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    rc = ctx->flush_pending();                               // the ranges may reach into a pending push
+    if (rc) return rc;
+    rc = check_enrol(ctx, who, slots, n, starts, lens);
+    if (rc) return rc;
+    if (n == 0) return EWK_OK;
+    if (!streams) { ctx->fail("%s: streams is NULL", who); return EWK_ERR_ARG; }
+    const BankView& B = ctx->bank;
+    std::vector<PrepDesc> g((size_t)n);
+    std::vector<int64_t> off((size_t)n);
+    int64_t packed = 0;
+    for (int i = 0; i < n; i++) {                            // ewk_read_segment's checks, row by row
+        const int s = streams[i];
+        if (s < 0 || s >= B.n_streams || lens[i] > B.P) {
+            ctx->fail("%s: row %d (stream %d): stream out of range [0, %d) or len %lld above the ring's %d samples", who, i,
+                      s, B.n_streams, (long long)lens[i], B.P);
+            return EWK_ERR_ARG;
+        }
+        if (starts[i] + lens[i] > ctx->h_written[s]) {
+            ctx->fail("%s: row %d (stream %d): segment not pushed yet", who, i, s);
+            return EWK_ERR_STATE;
+        }
+        if (ctx->h_written[s] - starts[i] > B.P) {
+            ctx->fail("%s: row %d (stream %d): segment already overwritten in the ring", who, i, s);
+            return EWK_ERR_STATE;
+        }
+        g[i] = PrepDesc{s, (int)lens[i], starts[i], packed};
+        off[i] = packed;
+        packed += lens[i];
+    }
+    return enrol_impl(ctx, who, slots, n, EnrolSource{nullptr, EWK_DEVICE, &g}, off.data(), lens, vad);
 }
 
 // Launch geometry of K4 for a template set: hops per sub-chunk, threads per CTA and CTAs per SM that fit shared memory.

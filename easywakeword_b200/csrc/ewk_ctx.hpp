@@ -15,8 +15,6 @@
 #include "ewk_resample_push.cuh"
 #include "ewk_tables.hpp"
 
-#define EWK_MAX_TEMPLATES 64
-
 namespace ewk {
 
 struct DevBuf {

@@ -143,9 +143,10 @@ __device__ __forceinline__ void dense_stats(long long S1, long long S2, int F, d
     sd = flat ? 0.f : sqrtf(fmaxf((float)var, 0.f));
 }
 
-// Template features for this kernel: the integer statistics of the template's own MFCC frames (K3's frames_out).
-__global__ void dense_template_features_kernel(const float* __restrict__ frames, int F, int n_mfcc, float* __restrict__ out40) {
-    const int lane = threadIdx.x;
+// Template features for this kernel: the integer statistics of the template's own MFCC frames (K3's frames_out), by one
+// warp (lane < 20: coefficient `lane`).
+__device__ __forceinline__ void dense_template_features(const float* __restrict__ frames, int F, int n_mfcc, int lane,
+                                                       float* __restrict__ out40) {
     long long S1 = 0, S2 = 0;
     if (lane < N_MFCC)
         for (int t = 0; t < F; t++) {
@@ -159,6 +160,34 @@ __global__ void dense_template_features_kernel(const float* __restrict__ frames,
         out40[lane] = lane < n_mfcc ? mean : 0.f;
         out40[N_MFCC + lane] = lane < n_mfcc ? sd : 0.f;
     }
+}
+
+__global__ void dense_template_features_kernel(const float* __restrict__ frames, int F, int n_mfcc, float* __restrict__ out40) {
+    dense_template_features(frames, F, n_mfcc, threadIdx.x, out40);
+}
+
+// Batched enrolment (ewk_set_templates): one warp per template i, over its frames [segs[i].frames_off, + 1 + len / 160)
+// of K3's frames_out; writes dense40[i] and the whole table entry tmpl[slots[i]] from K3's features feat[i] — what
+// ewk_set_template installs for the same audio, field for field.
+constexpr int ENROL_WARPS = 4;
+__global__ void __launch_bounds__(ENROL_WARPS * 32)
+dense_template_install_kernel(const SegDesc* __restrict__ segs, const int* __restrict__ slots, int n, int n_mfcc,
+                              const float* __restrict__ frames, const float* __restrict__ feat,
+                              float* __restrict__ dense40, TemplateFeat* __restrict__ tmpl) {
+    const int i = blockIdx.x * ENROL_WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (i >= n) return;
+    const SegDesc sd = segs[i];
+    float* d = dense40 + (size_t)i * FEAT;
+    dense_template_features(frames + (size_t)sd.frames_off * N_MFCC, 1 + sd.len / HOP, n_mfcc, lane, d);
+    __syncwarp();
+    TemplateFeat* t = tmpl + slots[i];
+    if (lane < N_MFCC) {
+        t->mean[lane] = feat[(size_t)i * FEAT + lane];
+        t->std[lane] = feat[(size_t)i * FEAT + N_MFCC + lane];
+        t->dmean[lane] = d[lane];
+        t->dstd[lane] = d[N_MFCC + lane];
+    }
+    if (lane == 0) { t->n_samples = sd.len; t->valid = 1; t->pad = 0; }
 }
 
 // ---- frame loaders for ring views (no pre-emphasis): frame sample m = 2 lane + 64 a, pairs from one aligned word -----

@@ -17,8 +17,8 @@
 #include "ewk_frame.cuh"
 #include "ewk_segment.cuh"
 
-#ifndef EWK_MAX_TEMPLATES
-#define EWK_MAX_TEMPLATES 64
+#ifndef EWK_MAX_STREAM_TEMPLATES
+#define EWK_MAX_STREAM_TEMPLATES 64      // include/ewk.h: one stream's template_count
 #endif
 
 namespace ewk {
@@ -1123,6 +1123,21 @@ segment_prepare_kernel(BankView B, const PrepDesc* __restrict__ d, float* __rest
     }
 }
 
+// Enrolment from the rings (ewk_set_templates_from_streams): segment blockIdx.y as float32 to out + out_off, converted
+// as ewk_read_segment converts it (int16: q * 2^-15, exact).
+__global__ void __launch_bounds__(256)
+ring_gather_kernel(BankView B, const PrepDesc* __restrict__ d, float* __restrict__ out) {
+    const PrepDesc pd = d[blockIdx.y];
+    const short* q = B.fmt == 1 ? (const short*)B.ring + (size_t)pd.stream * B.P : nullptr;
+    const float* f = B.fmt == 0 ? (const float*)B.ring + (size_t)pd.stream * B.P : nullptr;
+    const int p0 = (int)(pd.start % B.P);
+    for (int i = blockIdx.x * 256 + threadIdx.x; i < pd.len; i += gridDim.x * 256) {
+        int p = p0 + i;
+        if (p >= B.P) p -= B.P;
+        out[pd.out_off + i] = q ? (float)q[p] * (1.0f / 32768.0f) : f[p];
+    }
+}
+
 // ------------------------------------------------------------------------------------ K3 (queue form)
 // Persistent CTAs drain the segments K2 queued: PCM straight from the stream's device ring ->
 // fused MFCC + template match -> score written back into the event record and the per-stream result.
@@ -1146,7 +1161,7 @@ __global__ void __launch_bounds__(512, 2)
 segment_queue_kernel(const DeviceTables* __restrict__ T, BankView B, const TemplateFeat* __restrict__ tmpl, int n_tmpl_slots) {
     extern __shared__ __align__(16) float smem[];
     const SegSmem m = seg_carve(smem, SEG_SMEM_FRAMES);
-    __shared__ float sc_s[EWK_MAX_TEMPLATES];
+    __shared__ float sc_s[EWK_MAX_STREAM_TEMPLATES];
     __shared__ int next_s;
     __shared__ int cum_s[SEG_NB + 1];
     const int tid = threadIdx.x;

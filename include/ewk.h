@@ -40,12 +40,18 @@ typedef enum ewk_mem { EWK_HOST = 0, EWK_DEVICE = 1 } ewk_mem;
 enum { EWK_N_MFCC = 20, EWK_N_MELS = 128, EWK_N_FFT = 512, EWK_HOP = 160, EWK_SAMPLE_RATE = 16000,
        EWK_TICK_SAMPLES = 1600 };
 
+/* Template slots: a context holds up to EWK_MAX_TEMPLATE_SLOTS (ewk_config.max_templates), enough for one personal
+ * word per stream of a full B200 bank; one stream is scored against at most EWK_MAX_STREAM_TEMPLATES consecutive slots
+ * (ewk_stream_params.template_count). */
+#define EWK_MAX_TEMPLATE_SLOTS 4096
+#define EWK_MAX_STREAM_TEMPLATES 64
+
 typedef struct ewk_config {
     int32_t n_streams;      /* independent audio streams resident on this GPU (0: matcher only)       */
     int32_t ring_samples;   /* SoundBuffer.buffer_length = seconds * 16000       wakeword.py:426-428  */
     int32_t slack_samples;  /* extra physical ring so that one ewk_push may run ahead of ewk_tick      */
     int32_t pcm_format;     /* ewk_pcm_format of the device rings                                     */
-    int32_t max_templates;  /* template slots (reference: one WordMatcher holds one template)         */
+    int32_t max_templates;  /* template slots, 1..EWK_MAX_TEMPLATE_SLOTS (reference: one WordMatcher) */
     int32_t max_events;     /* capacity of the device event queue between two ewk_poll calls          */
     /* --- ABI 2: front-end parameters the reference hard-codes (wakeword.py:561-563; exposing them is on its own
      * wish list, LEARNINGS.md:87, README-CODE-ALIGNMENT.md:84-107).  0 selects the reference's value. */
@@ -108,7 +114,8 @@ typedef struct ewk_stream_params {
                                        it (:1061-1062, 1205-1211); <= 0: never                          */
     double min_threshold;           /* SoundBuffer.MIN_THRESHOLD = 0.005                  :409           */
     int32_t template_first;         /* the stream is scored against template slots                      */
-    int32_t template_count;         /*   [template_first, template_first + template_count), best wins   */
+    int32_t template_count;         /*   [template_first, template_first + template_count), best wins;  
+                                       at most EWK_MAX_STREAM_TEMPLATES                                  */
     int32_t live;                   /* 1: a tick sees every pushed sample (SoundBuffer facade driven by
                                        wall-clock polls); 0: audio clock, tick k sees
                                        floor(1600 k / frame_size) * frame_size samples                  */
@@ -221,6 +228,29 @@ int ewk_join(ewk_ctx* ctx);
  * (tests/test_wakeword_simulated.py:687-775: min = duration or 0.3, max = 2 * min or 2.0). */
 int ewk_analyze_templates(ewk_ctx* ctx, const float* pcm, int where, const int64_t* offsets, const int64_t* lens,
                           int n, ewk_vad_result* out, float* rms_out, int64_t rms_cap);
+/* Template enrolment, batched: template slots[i] gets the float32 16 kHz samples pcm[offsets[i] : offsets[i] + lens[i]]
+ * (`where` says host or device), for n templates in one call.  Every field each slot receives (K3's mean / std, the
+ * dense kernel's dmean / dstd, n_samples) is bit-identical to what ewk_set_template(ctx, slots[i], that audio) installs,
+ * and vad (nullable, host) receives vad[i] bit-identical to ewk_analyze_templates of the same audio.  One K3 launch over
+ * all n templates (templates over 48 000 samples take K3's workspace path, as in ewk_set_template), one dense-feature
+ * launch that also writes the table entries, one K6 launch when vad is given, one copy of the features back and one
+ * synchronisation: the number of launches does not grow with n.  Dense sets (ewk_dense_*_sets) covering a written slot
+ * are rebuilt on their next use.  In overlap mode the call joins K3 first.  n = 0 is a no-op.
+ * EWK_ERR_ARG, naming the entry, for a slot out of [0, max_templates) or listed twice, lens[i] < 1 or > 2^30, a negative
+ * offset, or a NULL array with n > 0.  Every check comes before the first launch: a failed call changes no slot. */
+int ewk_set_templates(ewk_ctx* ctx, const int32_t* slots, int n, const float* pcm, int where,
+                      const int64_t* offsets, const int64_t* lens, ewk_vad_result* vad);
+/* Template enrolment from the rings: template slots[i] gets stream streams[i]'s absolute samples
+ * [starts[i], starts[i] + lens[i]) — the coordinates of ewk_event.seg_start / seg_len, ewk_detection.seg_start / seg_len
+ * and ewk_read_segment.  The result equals ewk_set_templates of what ewk_read_segment returns for those ranges, bit for
+ * bit (int16 rings convert as q / 32768).  One gather launch copies the ranges into a float32 device scratch, then the
+ * call runs as ewk_set_templates on it.  Streams may repeat (one stream enrolling several utterances).  A pending host
+ * push lands first; in overlap mode the call joins K3 first.  Errors, named by row and stream, all before the first
+ * launch (a failed call changes no slot): those of ewk_set_templates, EWK_ERR_ARG for a stream out of range or
+ * lens[i] > the physical ring, EWK_ERR_STATE for a range not yet pushed or already overwritten in its ring and for a
+ * context with n_streams = 0. */
+int ewk_set_templates_from_streams(ewk_ctx* ctx, const int32_t* slots, int n, const int32_t* streams,
+                                   const int64_t* starts, const int64_t* lens, ewk_vad_result* vad);
 /* Ingest at other sample rates (SURVEY §8(f) N3): conversion to 16 kHz on the device, the step the reference
  * delegates to librosa.load(sr=16000) / librosa.resample (wakeword.py:588, 866-870; examples/tune_threshold.py:
  * 33-47; soxr HQ).  The filter meets soxr HQ's published specification (linear phase, pass-band to 0.913 of the
