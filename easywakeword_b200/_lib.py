@@ -406,6 +406,7 @@ def _declare_stream_protos(lib):
         "ewk_host_alloc": (C.c_int, [_p(vp), i64]),
         "ewk_host_free": (C.c_int, [vp]),
         "ewk_launch_count": (C.c_int64, [vp]),
+        "ewk_debug_check": (C.c_int, [vp]),
         "ewk_profile": (C.c_int, [vp, i32]),
         "ewk_profile_read": (C.c_int, [vp, _p(C.c_double), _p(C.c_int64)]),
     }
@@ -1053,6 +1054,10 @@ def _bank_methods():
     def launch_count(self):
         return int(self.lib.ewk_launch_count(self.h))
 
+    def debug_check(self):
+        """Poison mode (EWK_POISON set at creation): raise unless every guard band of the context is intact."""
+        self._ck(self.lib.ewk_debug_check(self.h))
+
     def profile(self, enable=True):
         self._ck(self.lib.ewk_profile(self.h, 1 if enable else 0))
 
@@ -1068,7 +1073,8 @@ def _bank_methods():
         setattr(Context, f.__name__, f)
     for f in (prepare_segments, dense_scores, dense_scores_streams, dense_ready, dense_detect, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
               push_resampled_each, push_streams, tick_ready, reset_streams, stream_blob_bytes, export_streams, import_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,
-              set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count):
+              set_results_buffer, set_results_peers, publish_parity, publish_seq, wait_published, published_seq, match_stream, set_cuda_stream, launch_count,
+              debug_check):
         setattr(Context, f.__name__, f)
 
 

@@ -63,6 +63,93 @@ extern "C" int ewk_host_table(int which, float* out, int cap) {
         }                                                                                           \
     } while (0)
 
+// ------------------------------------------------------------------------------------------
+// Pool (ewk_ctx.hpp): every allocation of a context; poison mode fills, guards and checks them.
+cudaError_t Pool::fill(void* p, size_t bytes, bool host) {
+    cudaError_t e = cudaDeviceSynchronize();             // nothing in flight still reads or writes the block
+    if (e != cudaSuccess) return e;
+    if (host) { std::memset(p, poison, bytes); return cudaSuccess; }
+    if (!stream && (e = cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking)) != cudaSuccess) return e;
+    if ((e = cudaMemsetAsync(p, poison, bytes, stream)) != cudaSuccess) return e;
+    return cudaStreamSynchronize(stream);
+}
+
+cudaError_t Pool::alloc(void** p, size_t bytes, const char* name) {
+    if (poison < 0) return cudaMalloc(p, bytes);
+    cudaError_t e = cudaMalloc(p, bytes + GUARD);
+    if (e != cudaSuccess) return e;
+    blocks[*p] = Block{name, bytes, false};
+    return fill(*p, bytes + GUARD, false);
+}
+
+cudaError_t Pool::alloc_host(void** p, size_t bytes, unsigned flags, const char* name) {
+    if (poison < 0) return cudaHostAlloc(p, bytes, flags);
+    cudaError_t e = cudaHostAlloc(p, bytes + GUARD, flags);
+    if (e != cudaSuccess) return e;
+    blocks[*p] = Block{name, bytes, true};
+    return fill(*p, bytes + GUARD, true);
+}
+
+cudaError_t Pool::refill(void* p) {
+    auto it = blocks.find(p);
+    return it == blocks.end() ? cudaSuccess : fill(p, it->second.bytes, it->second.host);
+}
+
+cudaError_t Pool::check_block(void* p, const Block& b, std::string* report) {
+    unsigned char g[GUARD];
+    const unsigned char* q = (const unsigned char*)p + b.bytes;
+    cudaError_t e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) return e;
+    if (b.host) {
+        std::memcpy(g, q, GUARD);
+    } else {
+        if ((e = cudaMemcpyAsync(g, q, GUARD, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return e;
+        if ((e = cudaStreamSynchronize(stream)) != cudaSuccess) return e;
+    }
+    for (size_t i = 0; i < GUARD; i++)
+        if (g[i] != (unsigned char)poison) {
+            char buf[256];
+            snprintf(buf, sizeof(buf), "%s%s (%zu bytes): guard damaged from byte %zu", report->empty() ? "" : "; ", b.name,
+                     b.bytes, b.bytes + i);
+            *report += buf;
+            break;
+        }
+    return cudaSuccess;
+}
+
+cudaError_t Pool::free(void* p, bool host) {
+    cudaError_t e = cudaSuccess;
+    auto it = blocks.find(p);
+    if (it != blocks.end()) {
+        e = check_block(p, it->second, &damage);
+        blocks.erase(it);
+    }
+    const cudaError_t f = host ? cudaFreeHost(p) : cudaFree(p);    // freed even when the guard could not be read
+    return e != cudaSuccess ? e : f;
+}
+
+cudaError_t Pool::check(std::string* report) {
+    *report = damage;
+    for (auto& kv : blocks) {
+        cudaError_t e = check_block(kv.first, kv.second, report);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
+extern "C" int ewk_debug_check(ewk_ctx* ctx) {
+    if (!ctx) return EWK_ERR_ARG;
+    if (ctx->pool.poison < 0) {
+        ctx->fail("ewk_debug_check: poison mode is off (set EWK_POISON before ewk_create)");
+        return EWK_ERR_STATE;
+    }
+    CK(cudaSetDevice(ctx->device));
+    std::string report;
+    CK(ctx->pool.check(&report));
+    if (!report.empty()) { ctx->fail("ewk_debug_check: %s", report.c_str()); return EWK_ERR_STATE; }
+    return EWK_OK;
+}
+
 extern "C" int ewk_create(int device, const ewk_config* cfg, ewk_ctx** out) {
     if (!cfg || !out) { g_create_error = "ewk_create: null argument"; return EWK_ERR_ARG; }
     *out = nullptr;
@@ -135,6 +222,12 @@ extern "C" int ewk_synchronize(ewk_ctx* ctx) {
 int ewk_ctx::init() {
     ewk_ctx* ctx = this;
     CK(cudaSetDevice(device));
+    if (const char* e = getenv("EWK_POISON"); e && *e) {     // test mode (ewk::Pool): the fill byte, decimal or 0x..
+        char* end = nullptr;
+        const long v = strtol(e, &end, 0);
+        if (*end || v < 0 || v > 255) { fail("ewk_create: EWK_POISON=%s is not a byte (0..255)", e); return EWK_ERR_ARG; }
+        pool.poison = (int)v;
+    }
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, device));
     sm_count = prop.multiProcessorCount;
@@ -159,13 +252,13 @@ int ewk_ctx::init() {
     img->preemph = cfg.preemphasis;
     img->n_mfcc = cfg.n_mfcc > 0 ? cfg.n_mfcc : N_MFCC;
     img->pad_[0] = img->pad_[1] = 0;
-    CK(cudaMalloc((void**)&d_tables, FRAME_IMAGE_OFFSET + sizeof(FrameTables)));
+    CK(pool.alloc(&d_tables, FRAME_IMAGE_OFFSET + sizeof(FrameTables), "d_tables"));
     CK(cudaMemcpy(d_tables, h, sizeof(DeviceTables), cudaMemcpyHostToDevice));
     CK(cudaMemcpy(reinterpret_cast<char*>(d_tables) + FRAME_IMAGE_OFFSET, img, sizeof(FrameTables), cudaMemcpyHostToDevice));
     delete img;
     delete h;
     h_tmpl.assign(cfg.max_templates, TemplateFeat{});
-    CK(cudaMalloc(&d_tmpl, sizeof(TemplateFeat) * cfg.max_templates));
+    CK(pool.alloc(&d_tmpl, sizeof(TemplateFeat) * cfg.max_templates, "d_tmpl"));
     CK(cudaMemset(d_tmpl, 0, sizeof(TemplateFeat) * cfg.max_templates));
     CK(cudaFuncSetAttribute(segment_mfcc_match_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                             (int)seg_smem_bytes(SEG_SMEM_FRAMES)));
@@ -181,16 +274,16 @@ void ewk_ctx::release() {
     if (own_stream) cudaStreamSynchronize(own_stream);
     release_streams();
     for (DevBuf* b : {&b_pcm, &b_desc, &b_ws, &b_lm, &b_feat, &b_scores, &b_matched, &b_frames, &b_off}) b->free();
-    for (auto& kv : rs_tables) if (kv.second.H) cudaFree(kv.second.H);
+    for (auto& kv : rs_tables) if (kv.second.H) pool.free(kv.second.H);
     rs_tables.clear();
     b_rs_in.free(); b_rs_out.free();
-    if (d_wait_flag) { cudaFree(d_wait_flag); d_wait_flag = nullptr; }
+    if (d_wait_flag) { pool.free(d_wait_flag); d_wait_flag = nullptr; }
     if (pub_stream) { cudaStreamSynchronize(pub_stream); cudaStreamDestroy(pub_stream); pub_stream = nullptr; }
     if (ev_k3) { cudaEventDestroy(ev_k3); ev_k3 = nullptr; }
     for (int i = 0; i < 2; i++) if (ev_pub[i]) { cudaEventDestroy(ev_pub[i]); ev_pub[i] = nullptr; }
-    if (d_pub_snap) { cudaFree(d_pub_snap); d_pub_snap = nullptr; }
-    if (d_tables) cudaFree(d_tables);
-    if (d_tmpl) cudaFree(d_tmpl);
+    if (d_pub_snap) { pool.free(d_pub_snap); d_pub_snap = nullptr; }
+    if (d_tables) pool.free(d_tables);
+    if (d_tmpl) pool.free(d_tmpl);
     if (copy_stream) { cudaStreamSynchronize(copy_stream); cudaStreamDestroy(copy_stream); }
     if (match_stream) { cudaStreamSynchronize(match_stream); cudaStreamDestroy(match_stream); match_stream = nullptr; }
     if (ev_gate) { cudaEventDestroy(ev_gate); ev_gate = nullptr; }
@@ -202,26 +295,28 @@ void ewk_ctx::release() {
         b_stage2[i].free();
         b_raw[i].free();
         if (ev_pos[i]) cudaEventDestroy(ev_pos[i]);
-        if (h_pos[i]) cudaFreeHost(h_pos[i]);
+        if (h_pos[i]) pool.free(h_pos[i], true);
         ev_pos[i] = nullptr; h_pos[i] = nullptr;
         b_pos[i].free();
         if (ev_drow[i]) cudaEventDestroy(ev_drow[i]);
-        if (h_drow[i]) cudaFreeHost(h_drow[i]);
+        if (h_drow[i]) pool.free(h_drow[i], true);
         ev_drow[i] = nullptr; h_drow[i] = nullptr;
         b_drow[i].free();
         if (ev_ddet[i]) cudaEventDestroy(ev_ddet[i]);
-        if (h_ddet[i]) cudaFreeHost(h_ddet[i]);
+        if (h_ddet[i]) pool.free(h_ddet[i], true);
         ev_ddet[i] = nullptr; h_ddet[i] = nullptr;
         b_ddet[i].free();
     }
     dset_stage.free(); drow_sets.free(); ddet_sets.free(); b_dset.free();
     h_dset.clear();
-    if (h_det_map) cudaFreeHost(h_det_map);
+    if (h_det_map) pool.free(h_det_map, true);
     h_det_map = nullptr; det_map_cap = 0;
     b_reset.free();
     b_blob.free();
     b_mig.free();
     if (own_stream) cudaStreamDestroy(own_stream);
+    if (pool.stream) cudaStreamDestroy(pool.stream);
+    pool.stream = nullptr;
     d_tables = nullptr; d_tmpl = nullptr; own_stream = nullptr; copy_stream = nullptr;
 }
 
@@ -638,7 +733,7 @@ int ewk_ctx::resample_table(int sr_in, const ResampleTable** out) {
         }
         std::vector<float> H;
         rs_build_table(t.d, H);
-        CK(cudaMalloc(&t.H, sizeof(float) * H.size()));
+        CK(pool.alloc(&t.H, sizeof(float) * H.size(), "rs_table"));
         CK(cudaMemcpyAsync(t.H, H.data(), sizeof(float) * H.size(), cudaMemcpyHostToDevice, stream));
         CK(cudaStreamSynchronize(stream));
         it = rs_tables.emplace(sr_in, t).first;
@@ -729,38 +824,42 @@ int ewk_ctx::init_streams() {
     chunk_cap = std::max(1, cfg.ring_samples / MIN_FRAME_SIZE);
     bank.chunk_cap = chunk_cap;
     bank.max_events = std::max(16, cfg.max_events);
-    CK(cudaMalloc(&bank.ring, esz * (size_t)n * bank.P));
+    CK(pool.alloc(&bank.ring, esz * (size_t)n * bank.P, "bank.ring"));
     CK(cudaMemsetAsync(bank.ring, 0, esz * (size_t)n * bank.P, stream));          // np.zeros   wakeword.py:428
-    CK(cudaMalloc(&bank.st, sizeof(StreamState) * (size_t)n));
-    CK(cudaMalloc(&bank.prm, sizeof(StreamParams) * (size_t)n));
-    CK(cudaMalloc(&bank.chunk_ms, sizeof(double) * (size_t)n * 2 * chunk_cap));   // per stream: ms[cap] ++ sorted[cap]
-    CK(cudaMalloc(&bank.events, sizeof(EventRec) * (size_t)bank.max_events));
-    CK(cudaMalloc(&bank.ev_count, sizeof(int) * 8));
+    CK(pool.alloc(&bank.st, sizeof(StreamState) * (size_t)n, "bank.st"));
+    CK(pool.alloc(&bank.prm, sizeof(StreamParams) * (size_t)n, "bank.prm"));
+    CK(pool.alloc(&bank.chunk_ms, sizeof(double) * (size_t)n * 2 * chunk_cap, "bank.chunk_ms"));   // per stream: ms[cap] ++ sorted[cap]
+    // K2 reads only chunks below chunks_valid, but K10 copies whole rows into blobs: zeros keep a blob's bytes a function of
+    // the stream's history
+    CK(cudaMemsetAsync(bank.chunk_ms, 0, sizeof(double) * (size_t)n * 2 * chunk_cap, stream));
+    CK(pool.alloc(&bank.events, sizeof(EventRec) * (size_t)bank.max_events, "bank.events"));
+    CK(pool.alloc(&bank.ev_count, sizeof(int) * 8, "bank.ev_count"));
     CK(cudaMemsetAsync(bank.ev_count, 0, sizeof(int) * 8, stream));
-    CK(cudaMalloc(&bank.bk_count, sizeof(int) * SEG_NB));
+    CK(pool.alloc(&bank.bk_count, sizeof(int) * SEG_NB, "bank.bk_count"));
     CK(cudaMemsetAsync(bank.bk_count, 0, sizeof(int) * SEG_NB, stream));
-    CK(cudaMalloc(&bank.bk_list, sizeof(int) * (size_t)SEG_NB * bank.max_events));
+    CK(pool.alloc(&bank.bk_list, sizeof(int) * (size_t)SEG_NB * bank.max_events, "bank.bk_list"));
 #ifdef EWK_K3_TRACE
     if (getenv("EWK_K3_TRACE")) {
-        CK(cudaMalloc(&bank.k3_trace, sizeof(long long) * K3_TRACE_WORDS * (size_t)queue_grid()));
+        CK(pool.alloc(&bank.k3_trace, sizeof(long long) * K3_TRACE_WORDS * (size_t)queue_grid(), "bank.k3_trace"));
         CK(cudaMemsetAsync(bank.k3_trace, 0, sizeof(long long) * K3_TRACE_WORDS * (size_t)queue_grid(), stream));
     }
 #endif
 
     bank.NB = bank.P / TICK;
-    CK(cudaMalloc(&bank.block_ss, sizeof(double) * (size_t)n * std::max(1, bank.NB)));
-    CK(cudaMalloc(&own_results, sizeof(StreamResult) * (size_t)n));
+    CK(pool.alloc(&bank.block_ss, sizeof(double) * (size_t)n * std::max(1, bank.NB), "bank.block_ss"));
+    CK(cudaMemsetAsync(bank.block_ss, 0, sizeof(double) * (size_t)n * std::max(1, bank.NB), stream));   // as chunk_ms
+    CK(pool.alloc(&own_results, sizeof(StreamResult) * (size_t)n, "own_results"));
     bank.results = (StreamResult*)own_results;
     if (const char* e = getenv("EWK_K3")) k3_frames = atoi(e) == 2;      // EWK_K3=2: the frame-parallel form (measured, not the default)
     if (!k3_frames) {
-        if (use_lm) CK(cudaMalloc(&bank.lm_ws, sizeof(float) * (size_t)queue_grid() * SEG_SMEM_FRAMES * LM_ROW));
+        if (use_lm) CK(pool.alloc(&bank.lm_ws, sizeof(float) * (size_t)queue_grid() * SEG_SMEM_FRAMES * LM_ROW, "bank.lm_ws"));
     } else {
         // frame-parallel K3: a frame table for the candidates of ONE ewk_tick call (it restarts after every K3 launch)
         const size_t cap = std::min<size_t>((size_t)bank.max_events * SEG_SMEM_FRAMES, ((size_t)2 << 30) / (FROW * sizeof(float)));
         bank.frow_cap = (int)cap;
-        CK(cudaMalloc(&bank.frow, sizeof(float) * FROW * cap));
-        CK(cudaMalloc(&bank.frame_ev, sizeof(int) * cap));
-        CK(cudaMalloc(&bank.ev_done, sizeof(int) * (size_t)bank.max_events));
+        CK(pool.alloc(&bank.frow, sizeof(float) * FROW * cap, "bank.frow"));
+        CK(pool.alloc(&bank.frame_ev, sizeof(int) * cap, "bank.frame_ev"));
+        CK(pool.alloc(&bank.ev_done, sizeof(int) * (size_t)bank.max_events, "bank.ev_done"));
     }
     std::vector<StreamState> st(n);
     std::memset(st.data(), 0, sizeof(StreamState) * n);
@@ -809,14 +908,14 @@ void ewk_ctx::release_streams() {
         std::vector<long long> h((size_t)K3_TRACE_WORDS * queue_grid());
         cudaMemcpy(h.data(), bank.k3_trace, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
         if (FILE* f = fopen(getenv("EWK_K3_TRACE"), "wb")) { fwrite(h.data(), sizeof(long long), h.size(), f); fclose(f); }
-        cudaFree(bank.k3_trace);
+        pool.free(bank.k3_trace);
     }
 #endif
-    if (d_rs_tail) { cudaFree(d_rs_tail); d_rs_tail = nullptr; rs_tail_cap = 0; }
+    if (d_rs_tail) { pool.free(d_rs_tail); d_rs_tail = nullptr; rs_tail_cap = 0; }
     for (void* p : {bank.ring, (void*)bank.st, (void*)bank.prm, (void*)bank.chunk_ms, (void*)bank.events,
                     (void*)bank.ev_count, (void*)bank.block_ss, (void*)bank.lm_ws, own_results, (void*)bank.frow,
                     (void*)bank.frame_ev, (void*)bank.ev_done, (void*)bank.bk_count, (void*)bank.bk_list})
-        if (p) cudaFree(p);
+        if (p) pool.free(p);
     bank = BankView{};
     own_results = nullptr;
     b_trace.free(); b_read.free(); b_dense.free(); b_keep_rows.free(); b_keep_end.free(); b_g2.free(); b_det_state.free();
@@ -1236,7 +1335,7 @@ static int upload_slot(ewk_ctx* ctx, D* (&h)[2], DevBuf (&b)[2], cudaEvent_t (&e
     idx ^= 1;
     const size_t bytes = sizeof(D) * (size_t)ctx->bank.n_streams;
     if (!h[k]) {
-        CK(cudaHostAlloc((void**)&h[k], bytes, cudaHostAllocDefault));
+        CK(ctx->pool.alloc_host(&h[k], bytes, cudaHostAllocDefault, "upload_slot host"));
         CK(cudaEventCreateWithFlags(&ev[k], cudaEventDisableTiming));
     }
     CK(b[k].ensure(bytes));
@@ -1256,12 +1355,12 @@ int ewk_ctx::ensure_rs_tail(int cap) {
     ewk_ctx* ctx = this;
     if (rs_tail_cap >= cap) return EWK_OK;
     float* nt = nullptr;
-    CK(cudaMalloc(&nt, sizeof(float) * (size_t)bank.n_streams * cap));
+    CK(pool.alloc(&nt, sizeof(float) * (size_t)bank.n_streams * cap, "d_rs_tail"));
     if (d_rs_tail) {
         CK(cudaMemcpy2DAsync(nt, sizeof(float) * cap, d_rs_tail, sizeof(float) * rs_tail_cap, sizeof(float) * rs_tail_cap,
                              bank.n_streams, cudaMemcpyDeviceToDevice, stream));
         CK(cudaStreamSynchronize(stream));
-        CK(cudaFree(d_rs_tail));
+        CK(pool.free(d_rs_tail));
     }
     d_rs_tail = nt;
     rs_tail_cap = cap;
@@ -2913,11 +3012,13 @@ static int dense_detect_impl(ewk_ctx* ctx, const char* who, const int32_t* strea
     // K4D's output: counts [n_streams], then the records of row i from offset sum_{j < i} ceil(n_j / 2)
     const size_t rec_off = ((size_t)4 * B.n_streams + 15) / 16 * 16, map_bytes = rec_off + sizeof(DetRecord) * (size_t)need;
     if (map_bytes > ctx->det_map_cap) {
-        if (ctx->h_det_map) CK(cudaFreeHost(ctx->h_det_map));
+        if (ctx->h_det_map) CK(ctx->pool.free(ctx->h_det_map, true));
         ctx->h_det_map = nullptr; ctx->det_map_cap = 0;
-        const size_t want = map_bytes + map_bytes / 4 + 256;
-        CK(cudaHostAlloc(&ctx->h_det_map, want, cudaHostAllocMapped | cudaHostAllocPortable));
+        const size_t want = ctx->pool.poison >= 0 ? map_bytes : map_bytes + map_bytes / 4 + 256;
+        CK(ctx->pool.alloc_host(&ctx->h_det_map, want, cudaHostAllocMapped | cudaHostAllocPortable, "h_det_map"));
         ctx->det_map_cap = want;
+    } else if (ctx->pool.poison >= 0) {
+        CK(ctx->pool.refill(ctx->h_det_map));                // the previous call's records are dead
     }
     float* d_scores = nullptr;
     std::vector<int> keys;
@@ -3084,11 +3185,11 @@ extern "C" int ewk_set_results_peers(ewk_ctx* ctx, void* const* bases, int n_bas
         CK(cudaStreamCreateWithPriority(&ctx->pub_stream, cudaStreamNonBlocking, prio_hi));
         CK(cudaEventCreateWithFlags(&ctx->ev_k3, cudaEventDisableTiming));
         for (int i = 0; i < 2; i++) CK(cudaEventCreateWithFlags(&ctx->ev_pub[i], cudaEventDisableTiming));
-        CK(cudaMalloc(&ctx->d_pub_snap, sizeof(StreamResult) * 2 * (size_t)B.n_streams));
+        CK(ctx->pool.alloc(&ctx->d_pub_snap, sizeof(StreamResult) * 2 * (size_t)B.n_streams, "d_pub_snap"));
     }
     B.pub_snap = (StreamResult*)ctx->d_pub_snap;
     if (n_bases && signals && !ctx->d_wait_flag) {
-        CK(cudaMalloc(&ctx->d_wait_flag, sizeof(int)));
+        CK(ctx->pool.alloc(&ctx->d_wait_flag, sizeof(int), "d_wait_flag"));
         CK(cudaMemsetAsync(ctx->d_wait_flag, 0, sizeof(int), ctx->stream));
     }
     return EWK_OK;

@@ -17,19 +17,53 @@
 
 namespace ewk {
 
+// Every device allocation of a context, and every pinned host buffer it owns, comes from its Pool.  EWK_POISON=<byte>
+// (read per context by ewk_create) is a test mode: each allocation is filled with the byte before anything initialises
+// it and is followed by a guard band of GUARD bytes of it, per-call scratch is refilled at every ensure, and
+// ewk_debug_check reports guard bands that changed.  So a read of memory nobody wrote sees the byte instead of the zeros a
+// fresh cudaMalloc usually holds, and a write past a buffer's end is found.  Unset, an allocation is a plain cudaMalloc /
+// cudaHostAlloc of the size asked for.  Poison mode synchronises the device around every fill and check.
+struct Pool {
+    static constexpr size_t GUARD = 256;
+    int poison = -1;                           // the fill byte; -1: off
+    struct Block { const char* name; size_t bytes; bool host; };
+    std::map<void*, Block> blocks;             // poison mode: every live allocation and its requested size
+    std::string damage;                        // guard damage found when a block was freed, kept for ewk_debug_check
+    cudaStream_t stream = nullptr;             // poison mode: fills and guard read-backs (created by the first fill)
+    cudaError_t alloc(void** p, size_t bytes, const char* name);
+    cudaError_t alloc_host(void** p, size_t bytes, unsigned flags, const char* name);
+    template <class T> cudaError_t alloc(T** p, size_t bytes, const char* name) { return alloc((void**)p, bytes, name); }
+    template <class T> cudaError_t alloc_host(T** p, size_t bytes, unsigned flags, const char* name) {
+        return alloc_host((void**)p, bytes, flags, name);
+    }
+    cudaError_t refill(void* p);               // poison mode: the whole block (not its guard) holds the byte again
+    cudaError_t free(void* p, bool host = false);   // cudaFree / cudaFreeHost, after checking the guard in poison mode
+    cudaError_t check(std::string* report);    // every live guard; damage found at free time included
+    cudaError_t check_block(void* p, const Block& b, std::string* report);
+    cudaError_t fill(void* p, size_t bytes, bool host);
+};
+
+// scratch: the content is dead whenever ensure is called (per-call workspaces), so poison mode refills it every time;
+// otherwise (staging slots that may hold a pending push, descriptor slots, state kept across calls) only at allocation
 struct DevBuf {
+    Pool* pool;
+    const char* name;
+    bool scratch;
     void* p = nullptr;
     size_t cap = 0;
+    DevBuf(Pool* pool_, const char* name_, bool scratch_) : pool(pool_), name(name_), scratch(scratch_) {}
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
     cudaError_t ensure(size_t bytes) {
-        if (bytes <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
-        size_t want = bytes + bytes / 4 + 256;
-        cudaError_t e = cudaMalloc(&p, want);
+        if (bytes <= cap) return scratch && pool->poison >= 0 && p ? pool->refill(p) : cudaSuccess;
+        free();
+        // poison mode: exactly the bytes asked for, so that a read past them lands in the guard band
+        size_t want = pool->poison >= 0 ? bytes : bytes + bytes / 4 + 256;
+        cudaError_t e = pool->alloc(&p, want, name);
         if (e == cudaSuccess) cap = want;
         return e;
     }
-    void free() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+    void free() { if (p) pool->free(p); p = nullptr; cap = 0; }
 };
 
 // two slots of pinned host + device memory for descriptors (upload_slot), each reused only once its reader has run (ev)
@@ -40,10 +74,11 @@ struct SlotPair {
     cudaEvent_t ev[2] = {nullptr, nullptr};
     bool ev_valid[2] = {false, false};
     int idx = 0;
+    SlotPair(Pool* pool, const char* name) : b{{pool, name, false}, {pool, name, false}} {}
     void free() {
         for (int i = 0; i < 2; i++) {
             if (ev[i]) cudaEventDestroy(ev[i]);
-            if (h[i]) cudaFreeHost(h[i]);
+            if (h[i]) b[i].pool->free(h[i], true);
             ev[i] = nullptr; h[i] = nullptr; ev_valid[i] = false;
             b[i].free();
         }
@@ -61,6 +96,7 @@ struct DenseSetHost {
 }  // namespace ewk
 
 struct ewk_ctx {
+    ewk::Pool pool;              // declared first: the buffers below allocate from it
     int device = 0;
     int sm_count = 0;
     bool use_lm = true;          // keep log-mel rows of K3 frames in a global workspace (EWK_SEG_LM=0 disables)
@@ -106,45 +142,45 @@ struct ewk_ctx {
     // (ewk_push_resampled_each): two slots of pinned host + device memory for n_streams rows, each reused only once the
     // kernel that read it has finished (ev_pos)
     ewk::RowDesc* h_pos[2] = {nullptr, nullptr};
-    ewk::DevBuf b_pos[2];
+    ewk::DevBuf b_pos[2]{{&pool, "b_pos", false}, {&pool, "b_pos", false}};
     cudaEvent_t ev_pos[2] = {nullptr, nullptr};
     bool ev_pos_valid[2] = {false, false};
     int pos_idx = 0;
     // per-row descriptors of a ragged K4 call (ewk_dense_scores_streams, ewk_dense_ready): two slots of the same kind
     ewk::DenseRow* h_drow[2] = {nullptr, nullptr};
-    ewk::DevBuf b_drow[2];
+    ewk::DevBuf b_drow[2]{{&pool, "b_drow", false}, {&pool, "b_drow", false}};
     cudaEvent_t ev_drow[2] = {nullptr, nullptr};
     bool ev_drow_valid[2] = {false, false};
     int drow_idx = 0;
     // per-row descriptors of K4D (ewk_dense_detect): two slots of the same kind
     ewk::DetRow* h_ddet[2] = {nullptr, nullptr};
-    ewk::DevBuf b_ddet[2];
+    ewk::DevBuf b_ddet[2]{{&pool, "b_ddet", false}, {&pool, "b_ddet", false}};
     cudaEvent_t ev_ddet[2] = {nullptr, nullptr};
     bool ev_ddet_valid[2] = {false, false};
     int ddet_idx = 0;
-    ewk::DevBuf b_det_state;                 // K4D's DetState [n_streams], allocated (zeroed) by the first detect call
+    ewk::DevBuf b_det_state{&pool, "b_det_state", false};                 // K4D's DetState [n_streams], allocated (zeroed) by the first detect call
     // per-row template sets (ewk_dense_*_sets): the descriptor of set [first, first + count) sits at index
     // first * DENSE_MAX_T + count - 1 of a device table; h_dset mirrors it.  A set is built and uploaded on first use and
     // kept until a template slot of its range changes (dense_sets_forget).  New descriptors go through dset_stage.
     std::vector<ewk::DenseSetHost> h_dset;
-    ewk::DevBuf b_dset;
-    ewk::SlotPair<ewk::DenseSetDev> dset_stage;
-    ewk::SlotPair<ewk::DenseRowSet> drow_sets;   // K4 row descriptors of a per-row-set call
-    ewk::SlotPair<ewk::DetRowSet> ddet_sets;     // K4D row descriptors of ewk_dense_detect_sets
+    ewk::DevBuf b_dset{&pool, "b_dset", false};
+    ewk::SlotPair<ewk::DenseSetDev> dset_stage{&pool, "dset_stage"};
+    ewk::SlotPair<ewk::DenseRowSet> drow_sets{&pool, "drow_sets"};   // K4 row descriptors of a per-row-set call
+    ewk::SlotPair<ewk::DetRowSet> ddet_sets{&pool, "ddet_sets"};     // K4D row descriptors of ewk_dense_detect_sets
     void dense_sets_forget(int slot);
     // K4D's output, pinned and mapped into the device: per-row record counts [n_streams], then records (row i at its offset)
     void* h_det_map = nullptr;
     size_t det_map_cap = 0;
-    ewk::DevBuf b_reset;                     // K9's stream list
-    ewk::DevBuf b_blob;                      // K10: a host blob's device copy (export: the whole blob; import: its bulk rows)
-    ewk::DevBuf b_mig;                       // K10 import: the destination list and the checked small state, one upload
+    ewk::DevBuf b_reset{&pool, "b_reset", true};                     // K9's stream list
+    ewk::DevBuf b_blob{&pool, "b_blob", true};                      // K10: a host blob's device copy (export: the whole blob; import: its bulk rows)
+    ewk::DevBuf b_mig{&pool, "b_mig", true};                       // K10 import: the destination list and the checked small state, one upload
     int flush_pending();
-    ewk::DevBuf b_stage2[2];
-    ewk::DevBuf b_raw[2];                    // compact host input: G.711 codes (ewk_push_g711, decoded into b_stage2) or a native-rate feed
+    ewk::DevBuf b_stage2[2]{{&pool, "b_stage2", false}, {&pool, "b_stage2", false}};
+    ewk::DevBuf b_raw[2]{{&pool, "b_raw", false}, {&pool, "b_raw", false}};                    // compact host input: G.711 codes (ewk_push_g711, decoded into b_stage2) or a native-rate feed
     ewk::DeviceTables* d_tables = nullptr;
     ewk::TemplateFeat* d_tmpl = nullptr;
     std::vector<ewk::TemplateFeat> h_tmpl;
-    ewk::DevBuf b_pcm, b_desc, b_ws, b_lm, b_feat, b_scores, b_matched, b_frames, b_off;
+    ewk::DevBuf b_pcm{&pool, "b_pcm", true}, b_desc{&pool, "b_desc", true}, b_ws{&pool, "b_ws", true}, b_lm{&pool, "b_lm", true}, b_feat{&pool, "b_feat", true}, b_scores{&pool, "b_scores", true}, b_matched{&pool, "b_matched", true}, b_frames{&pool, "b_frames", true}, b_off{&pool, "b_off", true};
 
     void fail(const char* fmt, ...);
     int init();
@@ -152,7 +188,7 @@ struct ewk_ctx {
     // stream bank
     ewk::BankView bank{};
     void* own_results = nullptr;
-    ewk::DevBuf b_trace, b_read, b_dense, b_keep_rows, b_keep_end, b_g2;
+    ewk::DevBuf b_trace{&pool, "b_trace", true}, b_read{&pool, "b_read", true}, b_dense{&pool, "b_dense", true}, b_keep_rows{&pool, "b_keep_rows", false}, b_keep_end{&pool, "b_keep_end", false}, b_g2{&pool, "b_g2", true};
     int dense_plan_info[4] = {0, 0, 0, 0};  // K4 geometry of the latest K4 call: hops per sub-chunk, threads, CTAs per SM, smem bytes (ewk_dense_last_plan)
     int chunk_cap = 0;
     bool all_presummed = false;            // K1's block sums cover every sample pushed since the last tick
@@ -192,7 +228,7 @@ struct ewk_ctx {
     // K7 filter tables, one per input rate seen
     struct ResampleTable { ewk::ResampleDesign d; float* H = nullptr; };
     std::map<int, ResampleTable> rs_tables;
-    ewk::DevBuf b_rs_in, b_rs_out;
+    ewk::DevBuf b_rs_in{&pool, "b_rs_in", true}, b_rs_out{&pool, "b_rs_out", true};
     int resample_table(int sr_in, const ResampleTable** out);
     // A.rows set: the grid is the descriptors' n_items flat output tiles (fir_tiles per row)
     int launch_fir(const ResampleTable& t, ewk::RsPushArgs& A, int n_rows, int prof_cls, const char* who,

@@ -542,6 +542,14 @@ int ewk_host_alloc(void** out, int64_t bytes);
 int ewk_host_free(void* p);
 /* Kernel launches issued by this context so far (for bench accounting). */
 int64_t ewk_launch_count(const ewk_ctx* ctx);
+/* Memory check of the poison test mode.  With EWK_POISON=<byte> (0..255, decimal or 0x..) set when the context is
+ * created, every device allocation of the context and every pinned host buffer it owns is filled with the byte before
+ * the library initialises it and is followed by a guard band of the byte; per-call workspaces are refilled at every call
+ * and allocated at exactly the size the call needs.  ewk_debug_check synchronises the device and reads every guard band
+ * back: EWK_OK if none changed, else EWK_ERR_STATE with ewk_last_error naming each damaged buffer and the first damaged
+ * byte (damage found when a buffer was freed or regrown is kept and reported here).  EWK_ERR_STATE also when poison mode
+ * is off.  Poison mode synchronises the device at every allocation; it is for tests, not for serving. */
+int ewk_debug_check(ewk_ctx* ctx);
 /* Per-kernel device timing with CUDA events on the context's stream.  ewk_profile(ctx, 1) starts
  * bracketing every kernel launch with an event pair; ewk_profile_read synchronises and returns, per
  * kernel class (0 ring_push, 1 tick_gate, 2 segment_queue, 3 segment_batch, 4 dense_score, 5 segment_prepare, 6 publish,

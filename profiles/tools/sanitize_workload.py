@@ -1,83 +1,26 @@
-"""A small run of every kernel of libewk.so for compute-sanitizer (memcheck / racecheck; one tool per gpurun call):
+"""A small run of every kernel of libewk.so:
 
-    compute-sanitizer --tool memcheck  python profiles/tools/sanitize_workload.py
-    compute-sanitizer --tool racecheck python profiles/tools/sanitize_workload.py
+    python profiles/tools/sanitize_workload.py [group ...]
 
-K0 G.711 decode, K1 in its three forms (fused sums, cp.async.bulk beside K3, unaligned), K2 (presummed, bulk-staged and
-generic paths), K3 (queue form with overlap, frame-parallel form, batch form with spill), K4 (dense scores, several
-templates, floored windows), K5, K6, K7 and the peer publication on local destinations.  Sizes are tiny: the tools slow
-kernels down 10-100x."""
+The workloads are the groups of tests/test_gpu_poison.py (WORKLOADS), which together launch every __global__ kernel and
+template instance of csrc/; each group's docstring names what it reaches.  The memory check itself is
+`pytest -m gpu tests/test_gpu_poison.py tests/test_gpu_buffer_edges.py` (DESIGN.md §7: compute-sanitizer is closed on
+the GPUs this project is measured on)."""
 import os
 import sys
 
-import numpy as np
-
 REPO = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, REPO)
+sys.path.insert(0, os.path.join(REPO, "tests"))
 
 
-def main():
-    import torch
-    from easywakeword_b200 import _lib, synth
-    from easywakeword_b200.bank import WakeWordBank
-    word = np.load(os.path.join(REPO, "tests", "golden", "reference_word.npz"))["pcm_i16"].astype(np.float32) / np.float32(32768)
-    # level 2 alone: batch K3 incl. a long input that spills to the global workspace, K6, K7
-    ctx = _lib.Context(device=0, n_streams=0, max_templates=2)
-    ctx.set_template(0, word)
-    x, _ = synth.stream(5, 4.0, word, gain=(2.0, 3.0), inserts_per_10s=(1, 1), zero_gaps=1)
-    x = synth.from_int16(synth.to_int16(x))
-    ctx.similarity_batch(0, x, [0, 8001], [len(x), 20000])
-    ctx.analyze_templates([word, x[:9000]])
-    ctx.resample(np.random.default_rng(0).standard_normal(4410).astype(np.float32), 44100)
-    ctx.close()
-    # the stream bank: host pushes, G.711 pushes, device pushes (fused and bulk forms), overlap, publication, K5
-    n = 160
-    pcm = synth.stream_batch(7000, n, 8.0, word, distractor_prob=0.2, zero_gaps=1)
-    for k3 in ("1", "2"):
-        os.environ["EWK_K3"] = k3
-        bank = WakeWordBank(n, [word, word[::-1].copy()], device=0, buffer_seconds=3, speech_duration_min=0.5, speech_duration_max=1.6,
-                            max_push_seconds=1.0)
-        c = bank.ctx
-        dests = [torch.zeros((2, 256, 2), dtype=torch.int32, device="cuda:0") for _ in range(2)]
-        sigs = [torch.zeros(2, 16, dtype=torch.int64, device="cuda:0") for _ in range(2)]
-        c.set_results_peers([d.data_ptr() for d in dests], stride_records=256, offset_records=3, signals=[g.data_ptr() for g in sigs], slot=0)
-        c.set_overlap(True)
-        ev = []
-        for i, b in enumerate(range(0, pcm.shape[1], 16000)):
-            blk = np.ascontiguousarray(pcm[:, b:b + 16000])
-            if i % 3 == 0:
-                bank.step(blk)                                    # host push: staging + lazy landing
-            elif i % 3 == 1:
-                t = torch.from_numpy(blk).cuda()
-                torch.cuda.synchronize()
-                bank.step((t.data_ptr(), n, 16000, 16000), where=_lib.DEVICE)   # device push beside K3: bulk form
-            else:
-                bank.push(np.ascontiguousarray(blk[:, :8001]))    # unaligned: scalar ring_push, generic gate path
-                bank.push(np.ascontiguousarray(blk[:, 8001:]))
-                bank.tick(10)
-            c.wait_published(1, c.publish_seq())
-            ev.append(bank.poll())
-            hits = ev[-1][ev[-1]["kind"] == 2][:2]
-            if len(hits):
-                bank.prepare_for_transcription(hits)              # K5 on segments that are still in the rings
-        ev = np.concatenate(ev)
-        c.set_results_peers([])
-        bank.close()
-        print(f"EWK_K3={k3}: {int((ev['kind'] == 2).sum())} level-2 events")
-    os.environ.pop("EWK_K3")
-    # G.711 feed and the dense kernel (3 templates, floored windows from the zero gaps)
-    from easywakeword_b200.resample import ULAW_TABLE
-    bank = WakeWordBank(4, [word, synth.synthetic_word(seed=9, duration=0.5), synth.sine(440.0, 1.0, 0.3)], device=0, buffer_seconds=6,
-                        max_push_seconds=2.0)
-    codes = np.random.default_rng(1).integers(0, 256, size=(4, 16000), dtype=np.uint8)
-    bank.push_g711(codes, law="ulaw")
-    bank.tick(10)
-    q = synth.stream_batch(8100, 4, 4.0, word, zero_gaps=2, gain=(2.0, 4.0))
-    for hop0, sc in bank.dense_sweep(np.ascontiguousarray(q[:, p:p + 32000]) for p in range(0, q.shape[1], 32000)):
-        assert sc.shape[0] == 4
-    bank.close()
+def main(groups):
+    from test_gpu_poison import WORKLOADS, run_workload
+    for g in groups or list(WORKLOADS):
+        run_workload(g, None)
+        print(f"{g}: done")
     print("sanitize workload done")
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1:])
