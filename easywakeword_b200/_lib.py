@@ -23,7 +23,7 @@ class EwkError(RuntimeError):
 class Config(C.Structure):
     _fields_ = [("n_streams", C.c_int32), ("ring_samples", C.c_int32), ("slack_samples", C.c_int32),
                 ("pcm_format", C.c_int32), ("max_templates", C.c_int32), ("max_events", C.c_int32),
-                ("preemphasis", C.c_float), ("n_mfcc", C.c_int32), ("reserved0", C.c_int32), ("reserved1", C.c_int32)]
+                ("preemphasis", C.c_float), ("n_mfcc", C.c_int32), ("template_frames", C.c_int32), ("reserved1", C.c_int32)]
 
 
 _lib = None
@@ -65,6 +65,11 @@ def load():
         "ewk_resample": (C.c_int, [vp, vp, i32, i32, i32, i64, i64, i32, i64, i64, i64, vp, i64, i32]),
         "ewk_dense_plan": (C.c_int, [_p(i64), i32, _p(C.c_int32)]),
         "ewk_dense_last_plan": (C.c_int, [vp, _p(C.c_int32)]),
+        "ewk_get_template_frames": (C.c_int, [vp, i32, f32p, i64, _p(C.c_int32)]),
+        "ewk_align_segments": (C.c_int, [vp, i32, _p(C.c_int32), _p(i64), _p(i64), _p(C.c_int32), _p(C.c_int32), f32p, i64,
+                                         _p(C.c_int32), f32p, i32]),
+        "ewk_align_buffers": (C.c_int, [vp, i32, vp, i32, i32, _p(i64), _p(i64), _p(C.c_int32), _p(C.c_int32), f32p, i64,
+                                        _p(C.c_int32), f32p, i32]),
     }
     for name, (res, args) in protos.items():
         fn = getattr(lib, name)
@@ -123,10 +128,13 @@ class Context:
     """Owns one ewk_ctx (one GPU)."""
 
     def __init__(self, device=0, n_streams=0, ring_samples=160000, slack_samples=16000, pcm_format=PCM_I16,
-                 max_templates=4, max_events=0, preemphasis=0.0, n_mfcc=0):
+                 max_templates=4, max_events=0, preemphasis=0.0, n_mfcc=0, template_frames=False):
+        """template_frames=True keeps every template slot's MFCC frames for frame alignment (align_segments /
+        align_buffers): 24 KB of device memory per slot."""
         self.lib = load()
         self.cfg = Config(n_streams, ring_samples, slack_samples, pcm_format, max_templates,
-                          max_events or max(1024, 4 * n_streams), float(preemphasis), int(n_mfcc), 0, 0)
+                          max_events or max(1024, 4 * n_streams), float(preemphasis), int(n_mfcc),
+                          1 if template_frames else 0, 0)
         h = C.c_void_p()
         rc = self.lib.ewk_create(device, C.byref(self.cfg), C.byref(h))
         if rc != EWK_OK:
@@ -246,6 +254,58 @@ class Context:
         self._ck(self.lib.ewk_set_templates(self.h, sl.ctypes.data_as(_p(C.c_int32)), len(sl), pcm, where, i64ptr(offs),
                                             i64ptr(lens), vad.ctypes.data if want_vad else None))
         return vad
+
+    def template_frames(self, slot):
+        """The frames stored for a template slot (include/ewk.h: ewk_get_template_frames): float32 [n_frames, 20],
+        bit-identical to extract_mfcc(audio, want_frames=True)[2]; 0 rows for a slot without frames (features only,
+        cleared, or over 48 000 samples).  Needs Context(template_frames=True)."""
+        nf = C.c_int32()
+        self._ck(self.lib.ewk_get_template_frames(self.h, int(slot), None, 0, C.byref(nf)))
+        out = np.empty((nf.value, 20), np.float32)
+        if nf.value:
+            self._ck(self.lib.ewk_get_template_frames(self.h, int(slot), f32ptr(out), nf.value, C.byref(nf)))
+        return out
+
+    def _align(self, fn, n, head, template_first, template_count, T, out_device_ptrs, dist_cap):
+        """Shared tail of align_segments / align_buffers: the set arrays, outputs and unpacking."""
+        need = int(T.sum())
+        if out_device_ptrs is not None:
+            d, bs, bd = out_device_ptrs
+            self._ck(fn(self.h, n, *head, template_first, template_count, C.cast(C.c_void_p(d), _p(C.c_float)),
+                        need if dist_cap is None else int(dist_cap),
+                        None if bs is None else C.cast(C.c_void_p(bs), _p(C.c_int32)),
+                        None if bd is None else C.cast(C.c_void_p(bd), _p(C.c_float)), DEVICE))
+            return None
+        dist = np.empty(max(1, need), np.float32)
+        best_slot = np.empty(n, np.int32)
+        best_dist = np.empty(n, np.float32)
+        self._ck(fn(self.h, n, *head, template_first, template_count, f32ptr(dist), need if dist_cap is None else int(dist_cap),
+                    best_slot.ctypes.data_as(_p(C.c_int32)), f32ptr(best_dist), HOST))
+        off, _ = sets_offsets(np.ones(n, np.int64), T)
+        return [dist[o:o + int(t)] for o, t in zip(off.tolist(), T)], best_slot, best_dist
+
+    def align_buffers(self, pcm, offsets, lens, template_first, template_count, out_device_ptrs=None, dist_cap=None):
+        """Frame-alignment distances of caller audio (include/ewk.h: ewk_align_buffers): row i is pcm[offsets[i] :
+        offsets[i] + lens[i]] (float32 or int16, host) against slots [template_first[i], template_first[i] +
+        template_count[i]) (scalars broadcast).  Returns (list of float32 [T_i] distances, best_slot int32 [n], best_dist
+        float32 [n]); with out_device_ptrs = (dist, best_slot or None, best_dist or None) device pointers the outputs go
+        there packed and None is returned."""
+        pcm = np.ascontiguousarray(pcm).reshape(-1)
+        if pcm.dtype == np.int16:
+            fmt = PCM_I16
+        else:
+            pcm = pcm.astype(np.float32, copy=False)
+            fmt = PCM_F32
+        off = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64).reshape(-1))
+        ln = np.ascontiguousarray(np.asarray(lens, dtype=np.int64).reshape(-1))
+        n = len(off)
+        if len(ln) != n:
+            raise ValueError("one offset and one length per row")
+        tf = _int32_list(np.broadcast_to(np.asarray(template_first, np.int64), (n,)), "template_first")
+        tc = _int32_list(np.broadcast_to(np.asarray(template_count, np.int64), (n,)), "template_count")
+        return self._align(self.lib.ewk_align_buffers, n, (pcm.ctypes.data, fmt, HOST, i64ptr(off), i64ptr(ln)),
+                           tf.ctypes.data_as(_p(C.c_int32)), tc.ctypes.data_as(_p(C.c_int32)), tc.astype(np.int64),
+                           out_device_ptrs, dist_cap)
 
     def resample(self, y, sr_in, *, in_first=0, out_first=0, n_out=None, out_device_ptr=None):
         """K7: y[rows, n] or y[n] (float32 / int16, host) at sr_in -> float32 at 16 kHz (absolute output samples
@@ -880,6 +940,24 @@ def _bank_methods():
                                                          vad.ctypes.data if want_vad else None))
         return vad
 
+    def align_segments(self, streams, starts, lens, template_first=None, template_count=None, out_device_ptrs=None,
+                       dist_cap=None):
+        """Frame-alignment distances of ring segments (include/ewk.h: ewk_align_segments): row i is stream streams[i]'s
+        absolute samples [starts[i], starts[i] + lens[i]) (an event's or a detection's seg_start / seg_len) against slots
+        [template_first[i], template_first[i] + template_count[i]) (both None: its stream's own range).  Returns (list of
+        float32 [T_i] distances, best_slot int32 [n], best_dist float32 [n]); with out_device_ptrs = (dist, best_slot or
+        None, best_dist or None) device pointers the outputs go there packed and None is returned."""
+        st = _stream_list(streams)
+        a0 = np.ascontiguousarray(np.asarray(starts, dtype=np.int64).reshape(-1))
+        ln = np.ascontiguousarray(np.asarray(lens, dtype=np.int64).reshape(-1))
+        n = len(st)
+        if len(a0) != n or len(ln) != n:
+            raise ValueError("one stream, start and length per row")
+        tf, tc, T = self._row_sets(st, n, template_first, template_count)
+        return self._align(self.lib.ewk_align_segments, n, (st.ctypes.data_as(_p(C.c_int32)), i64ptr(a0), i64ptr(ln)),
+                           None if tf is None else tf.ctypes.data_as(_p(C.c_int32)),
+                           None if tc is None else tc.ctypes.data_as(_p(C.c_int32)), T, out_device_ptrs, dist_cap)
+
     def dense_scores(self, hop0, n_hops, template_first=0, template_count=1, out_device_ptr=None):
         """[n_streams, n_hops, template_count] float32 scores for hops [hop0, hop0 + n_hops)."""
         if out_device_ptr is not None:
@@ -1069,7 +1147,7 @@ def _bank_methods():
                  "resample_push"]
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
-    for f in (_template_ranges, _row_sets, dense_scores_sets, dense_ready_sets, dense_detect_sets, set_templates_from_streams):
+    for f in (align_segments, _template_ranges, _row_sets, dense_scores_sets, dense_ready_sets, dense_detect_sets, set_templates_from_streams):
         setattr(Context, f.__name__, f)
     for f in (prepare_segments, dense_scores, dense_scores_streams, dense_ready, dense_detect, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
               push_resampled_each, push_streams, tick_ready, reset_streams, stream_blob_bytes, export_streams, import_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,

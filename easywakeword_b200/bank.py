@@ -20,6 +20,17 @@ from .wakeword import WakeWord, load_wav_16k
 TICK_SAMPLES = 1600
 DENSE_ROUND = 500                 # hops per ewk_dense_ready call of WakeWordBank.dense_ready (5 s of audio)
 EV_TIMEOUT, EV_SCORED = _lib.EV_TIMEOUT, _lib.EV_SCORED
+VERIFY_DTYPE = np.dtype([("stream", "<i4"), ("seg_start", "<i8"), ("seg_len", "<i4"), ("best_slot", "<i4"),
+                         ("distance", "<f4")])
+
+
+def _segment_rows(segments):
+    """(streams, starts, lens) int64 arrays of structured rows with stream / seg_start / seg_len or of a tuple."""
+    if isinstance(segments, tuple):
+        return tuple(np.asarray(a, dtype=np.int64).reshape(-1) for a in segments)
+    rows = [e for e in segments]
+    return (np.array([int(e["stream"]) for e in rows], np.int64), np.array([int(e["seg_start"]) for e in rows], np.int64),
+            np.array([int(e["seg_len"]) for e in rows], np.int64))
 
 
 def stream_blob_rates(blob) -> np.ndarray:
@@ -89,7 +100,11 @@ class WakeWordBank:
 
     template_slots: the context's template slots (default len(templates), at most 4096 = include/ewk.h
     EWK_MAX_TEMPLATE_SLOTS); slots past the constructor's templates are filled later with enroll(), e.g. one personal
-    word per stream spoken by its own user."""
+    word per stream spoken by its own user.
+
+    alignment: keep every template's MFCC frames (24 KB of device memory per slot) so that verify() can check level-2
+    candidates by frame alignment (DTW) before level 3: pooled level-2 features match the right sounds in the wrong
+    order, an alignment does not."""
 
     def __init__(self, n_streams: int, templates: Sequence, *, device: int = 0, buffer_seconds: int = 10,
                  pcm_dtype=np.int16, frame_size: int = TICK_SAMPLES, similarity_threshold: float = 75.0,
@@ -97,7 +112,7 @@ class WakeWordBank:
                  speech_duration_max: Optional[float] = None, post_speech_silence: float = 0.4,
                  timeout: float = 30.0, max_push_seconds: float = 1.0, max_events: int = 0,
                  cuda_stream: Optional[int] = None, overlap: bool = False, preemphasis: float = 0.0, n_mfcc: int = 20,
-                 sample_rate: int = 16000, template_slots: Optional[int] = None):
+                 sample_rate: int = 16000, template_slots: Optional[int] = None, alignment: bool = False):
         if n_streams < 1:
             raise ValueError("n_streams must be at least 1")
         if buffer_seconds <= 0:
@@ -119,7 +134,8 @@ class WakeWordBank:
         self.ctx = _lib.Context(device=device, n_streams=n_streams, ring_samples=buffer_seconds * 16000,
                                 slack_samples=slack, pcm_format=fmt, max_templates=max(1, n_slots),
                                 max_events=max_events or max(4096, 2 * n_streams), preemphasis=preemphasis,
-                                n_mfcc=n_mfcc)
+                                n_mfcc=n_mfcc, template_frames=alignment)
+        self.alignment = bool(alignment)
         if cuda_stream is not None:
             self.ctx.set_cuda_stream(cuda_stream)
         if overlap:
@@ -183,13 +199,7 @@ class WakeWordBank:
         speech_duration_min / max also follow the first of its recordings, by the rule the constructor applies to the
         first template.  self.templates stays the constructor's list.  Returns the VAD analysis of every segment
         (_lib.VAD_DTYPE, or None without set_durations)."""
-        if isinstance(segments, tuple):
-            streams, starts, lens = (np.asarray(a, dtype=np.int64).reshape(-1) for a in segments)
-        else:
-            rows = [e for e in segments]
-            streams = np.array([int(e["stream"]) for e in rows], np.int64)
-            starts = np.array([int(e["seg_start"]) for e in rows], np.int64)
-            lens = np.array([int(e["seg_len"]) for e in rows], np.int64)
+        streams, starts, lens = _segment_rows(segments)
         sl = np.asarray(slots, dtype=np.int64).reshape(-1)
         ranges = enroll_ranges(streams, starts, lens, sl)
         vad = self.ctx.set_templates_from_streams(sl, streams, starts, lens, want_vad=set_durations)
@@ -398,15 +408,36 @@ class WakeWordBank:
         return self.ctx.prepare_segments([int(e["stream"]) for e in ev], [int(e["seg_start"]) for e in ev],
                                          [int(e["seg_len"]) for e in ev])
 
+    def verify(self, segments, own_templates: bool = True, template_first=None, template_count=None):
+        """Frame-alignment distances of ring segments (include/ewk.h: ewk_align_segments; needs alignment=True): a second
+        stage for level-2 candidates before level 3.  segments: poll()'s events, a dense_detect result or a (streams,
+        starts, lens) tuple; the ranges must still be in the rings.  Each segment is aligned against its stream's own
+        template range (own_templates=True), or against [template_first, template_first + template_count) (scalars or
+        one per segment).  Returns (VERIFY_DTYPE array: stream, seg_start, seg_len, best_slot and its distance; list of
+        float32 [T_i] distances per template of each segment's set).  0 is a perfect match; the distance is not on the
+        score's 0-100 scale, so pick a threshold from your own recordings."""
+        streams, starts, lens = _segment_rows(segments)
+        if own_templates and template_first is None and template_count is None:
+            dist, slot, best = self.ctx.align_segments(streams, starts, lens)
+        else:
+            if template_first is None or template_count is None:
+                raise ValueError("give template_first and template_count, or neither with own_templates=True")
+            dist, slot, best = self.ctx.align_segments(streams, starts, lens, template_first, template_count)
+        out = np.zeros(len(streams), VERIFY_DTYPE)
+        out["stream"], out["seg_start"], out["seg_len"] = streams, starts, lens
+        out["best_slot"], out["distance"] = slot, best
+        return out, dist
+
     def status(self, stream: int):
         return self.ctx.status(stream)
 
     # ---- convenience: the reference's callback surface over the whole bank
     def run(self, blocks: Iterable[np.ndarray], on_match: Optional[Callable] = None, transcriber=None,
-            textword: str = "", numberofwords: int = 1):
+            textword: str = "", numberofwords: int = 1, max_distance: Optional[float] = None):
         """Feed an iterable of [n_streams, n] blocks; for every level-2 match call
         on_match(stream, tick, score, text) where text is the level-3 confirmation (None without a
-        transcriber).  Returns the list of all events."""
+        transcriber).  Returns the list of all events.  max_distance (needs alignment=True): level-2 matches whose
+        verify() distance against their stream's own templates exceeds it are dropped before level 3 and on_match."""
         log = []
         for blk in blocks:
             self.step(blk)
@@ -415,6 +446,9 @@ class WakeWordBank:
             hits = [e for e in ev if e["kind"] == EV_SCORED and e["matched"]]
             if not hits or on_match is None:
                 continue
+            if max_distance is not None:
+                d = self.verify(hits)[0]["distance"]
+                hits = [e for e, x in zip(hits, d) if x <= max_distance]
             audio = self.prepare_for_transcription(hits) if transcriber is not None else [None] * len(hits)
             for e, a in zip(hits, audio):
                 text = transcriber.transcribe(a) if transcriber is not None else None

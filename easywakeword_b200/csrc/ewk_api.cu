@@ -163,8 +163,9 @@ extern "C" int ewk_create(int device, const ewk_config* cfg, ewk_ctx** out) {
         g_create_error = "ewk_create: preemphasis must be in [0, 1)";
         return EWK_ERR_ARG;
     }
-    if (cfg->n_mfcc < 0 || cfg->n_mfcc > EWK_N_MFCC || cfg->reserved0 != 0 || cfg->reserved1 != 0) {
-        g_create_error = "ewk_create: n_mfcc must be 0 (= 20) or in [1, 20]; reserved fields must be 0";
+    if (cfg->n_mfcc < 0 || cfg->n_mfcc > EWK_N_MFCC || (cfg->template_frames != 0 && cfg->template_frames != 1) ||
+        cfg->reserved1 != 0) {
+        g_create_error = "ewk_create: n_mfcc must be 0 (= 20) or in [1, 20], template_frames 0 or 1; reserved1 must be 0";
         return EWK_ERR_ARG;
     }
     int ndev = 0;
@@ -260,6 +261,9 @@ int ewk_ctx::init() {
     h_tmpl.assign(cfg.max_templates, TemplateFeat{});
     CK(pool.alloc(&d_tmpl, sizeof(TemplateFeat) * cfg.max_templates, "d_tmpl"));
     CK(cudaMemset(d_tmpl, 0, sizeof(TemplateFeat) * cfg.max_templates));
+    h_tfr_n.assign(cfg.max_templates, 0);
+    if (cfg.template_frames)      // written per slot by the template writers; K11 reads only a slot's stored frames
+        CK(pool.alloc(&d_tfr, sizeof(float) * ALIGN_MAX_FRAMES * N_MFCC * (size_t)cfg.max_templates, "d_tfr"));
     CK(cudaFuncSetAttribute(segment_mfcc_match_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                             (int)seg_smem_bytes(SEG_SMEM_FRAMES)));
     CK(cudaFuncSetAttribute(segment_mfcc_match_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -284,6 +288,8 @@ void ewk_ctx::release() {
     if (d_pub_snap) { pool.free(d_pub_snap); d_pub_snap = nullptr; }
     if (d_tables) pool.free(d_tables);
     if (d_tmpl) pool.free(d_tmpl);
+    if (d_tfr) pool.free(d_tfr);
+    d_tfr = nullptr;
     if (copy_stream) { cudaStreamSynchronize(copy_stream); cudaStreamDestroy(copy_stream); }
     if (match_stream) { cudaStreamSynchronize(match_stream); cudaStreamDestroy(match_stream); match_stream = nullptr; }
     if (ev_gate) { cudaEventDestroy(ev_gate); ev_gate = nullptr; }
@@ -424,11 +430,23 @@ static int install_template(ewk_ctx* ctx, int slot, const float* mean20, const f
     return EWK_OK;
 }
 
+// Template frame store: slot <- the 1 + n / HOP frames of a template of n samples, K3's frames_out at d_src (device), on
+// the context's stream; a template over ALIGN_MAX_SAMPLES samples (the segments K11 takes) keeps none.
+void ewk_ctx::store_frames(int slot, const float* d_src, long long n) {
+    h_tfr_n[slot] = 0;
+    if (!d_tfr || n > ALIGN_MAX_SAMPLES) return;
+    const long long F = 1 + n / HOP;
+    h_tfr_n[slot] = (int)F;
+    cudaMemcpyAsync(d_tfr + (size_t)slot * ALIGN_MAX_FRAMES * N_MFCC, d_src, sizeof(float) * N_MFCC * (size_t)F,
+                    cudaMemcpyDeviceToDevice, stream);
+}
+
 extern "C" int ewk_set_template_features(ewk_ctx* ctx, int slot, const float* mean20, const float* std20, int64_t n_samples) {
     if (!ctx) return EWK_ERR_ARG;
     int rc = check_slot(ctx, slot, "ewk_set_template_features");
     if (rc) return rc;
     if (!mean20 || !std20 || n_samples < 1) { ctx->fail("ewk_set_template_features: null features or n_samples < 1"); return EWK_ERR_ARG; }
+    ctx->h_tfr_n[slot] = 0;                                  // features without audio: no frames to align against
     return install_template(ctx, slot, mean20, std20, nullptr, n_samples);
 }
 
@@ -439,6 +457,8 @@ extern "C" int ewk_set_template(ewk_ctx* ctx, int slot, const float* pcm, int64_
     float mean[N_MFCC], sd[N_MFCC], dense[FEAT];
     rc = extract_impl(ctx, pcm, n, EWK_HOST, mean, sd, nullptr, 0, dense);
     if (rc) return rc;
+    ctx->store_frames(slot, (const float*)ctx->b_frames.p, n);             // extract_impl left the frames there
+    CK(cudaGetLastError());
     return install_template(ctx, slot, mean, sd, dense, n);
 }
 
@@ -460,6 +480,7 @@ extern "C" int ewk_clear_template(ewk_ctx* ctx, int slot) {
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
     ctx->h_tmpl[slot] = TemplateFeat{};
+    ctx->h_tfr_n[slot] = 0;
     ctx->dense_sets_forget(slot);
     CK(cudaMemcpyAsync(ctx->d_tmpl + slot, &ctx->h_tmpl[slot], sizeof(TemplateFeat), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
@@ -673,6 +694,10 @@ static int enrol_impl(ewk_ctx* ctx, const char* who, const int32_t* slots, int n
         CK(cudaGetLastError());
         ctx->launches++;
     }
+    // the template frame store: one device-to-device copy per template (no launch)
+    for (int i = 0; i < n; i++) ctx->store_frames(slots[i], (const float*)ctx->b_frames.p + (size_t)sd[i].frames_off * N_MFCC,
+                                                  lens[i]);
+    CK(cudaGetLastError());
     std::vector<char> h(back);
     CK(cudaMemcpyAsync(h.data(), d_feat, back, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
@@ -2405,6 +2430,212 @@ extern "C" int ewk_set_templates_from_streams(ewk_ctx* ctx, const int32_t* slots
         packed += lens[i];
     }
     return enrol_impl(ctx, who, slots, n, EnrolSource{nullptr, EWK_DEVICE, &g}, off.data(), lens, vad);
+}
+
+// ---- frame alignment: ewk_get_template_frames, ewk_align_segments, ewk_align_buffers (K3 + K11) ---------------------------
+extern "C" int ewk_get_template_frames(ewk_ctx* ctx, int slot, float* out, int64_t cap, int32_t* n_frames) {
+    if (!ctx) return EWK_ERR_ARG;
+    const char* who = "ewk_get_template_frames";
+    int rc = check_slot(ctx, slot, who);
+    if (rc) return rc;
+    if (!ctx->d_tfr) { ctx->fail("%s: the context keeps no template frames (ewk_config.template_frames = 0)", who); return EWK_ERR_STATE; }
+    if (!ctx->h_tmpl[slot].valid) { ctx->fail("%s: template slot %d is empty. No reference word set. Call set_reference() first.", who, slot); return EWK_ERR_NO_TEMPLATE; }
+    const int F = ctx->h_tfr_n[slot];
+    if (out && cap < F) { ctx->fail("%s: cap %lld < %d frames", who, (long long)cap, F); return EWK_ERR_ARG; }
+    if (n_frames) *n_frames = F;
+    if (out && F) {
+        CK(cudaSetDevice(ctx->device));
+        CK(cudaMemcpyAsync(out, ctx->d_tfr + (size_t)slot * ALIGN_MAX_FRAMES * N_MFCC, sizeof(float) * N_MFCC * (size_t)F,
+                           cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    return EWK_OK;
+}
+
+// Row i: segment descriptor seg[i] (base, start, ring, fmt set by the caller), set [first[i], first[i] + count[i]).  Checks
+// the sets and the output capacity, then runs K3 over every segment (frames and features into workspaces) and K11, and
+// copies the outputs back when where == EWK_HOST.  Every check comes before the first launch.
+static int align_run(ewk_ctx* ctx, const char* who, int n, std::vector<SegDesc>& seg, const std::vector<int>& stream_of,
+                     const int32_t* first, const int32_t* count, float* dist, int64_t dist_cap, int32_t* best_slot,
+                     float* best_dist, int where, const void* h_pcm, size_t pcm_bytes) {
+    std::vector<AlignRow> rows((size_t)n);
+    long long frames = 0, packed = 0;
+    int max_frames = 1;
+    for (int i = 0; i < n; i++) {
+        const int s = stream_of[i];
+        const int f = first[i], c = count[i];
+        if (c < 1 || c > ALIGN_MAX_T || f < 0 || f > ctx->cfg.max_templates - c) {
+            ctx->fail("%s: row %d (stream %d) has a bad template range [%d, %d) (1..%d templates of %d slots)", who, i, s, f,
+                      f + c, ALIGN_MAX_T, ctx->cfg.max_templates);
+            return EWK_ERR_ARG;
+        }
+        for (int k = f; k < f + c; k++) {
+            if (!ctx->h_tmpl[k].valid) {
+                ctx->fail("%s: row %d (stream %d): template slot %d is empty. No reference word set. Call set_reference() first.",
+                          who, i, s, k);
+                return EWK_ERR_NO_TEMPLATE;
+            }
+            if (!ctx->h_tfr_n[k]) {
+                ctx->fail("%s: row %d (stream %d): template slot %d has no frames (cleared, features only, or %lld samples: "
+                          "over %d)", who, i, s, k, (long long)ctx->h_tmpl[k].n_samples, ALIGN_MAX_SAMPLES);
+                return EWK_ERR_ARG;
+            }
+        }
+        const int F = 1 + seg[i].len / HOP;
+        seg[i].ws_frame_off = 0; seg[i].frames_off = frames; seg[i].lm_off = frames;
+        rows[i] = AlignRow{frames, packed, F, f, c, 0};
+        frames += F;
+        packed += c;
+        max_frames = std::max(max_frames, F);
+    }
+    if (dist_cap < packed) {
+        ctx->fail("%s: dist_cap %lld is below the %lld distances of the rows", who, (long long)dist_cap, (long long)packed);
+        return EWK_ERR_ARG;
+    }
+    // K3 keeps every frame's log-mel row (the top_db floor's input) only up to LM_WS_MAX_BYTES, as ewk_extract_mfcc does
+    if (ctx->use_lm && sizeof(float) * (size_t)frames * LM_ROW > ewk_ctx::LM_WS_MAX_BYTES) {
+        ctx->fail("%s: the segments hold %lld frames together; one call takes at most %lld (split the batch)", who,
+                  (long long)frames, (long long)(ewk_ctx::LM_WS_MAX_BYTES / (sizeof(float) * LM_ROW)));
+        return EWK_ERR_ARG;
+    }
+    CK(cudaSetDevice(ctx->device));
+    if (h_pcm) {                                            // host input: one copy, then the segments point into it
+        CK(ctx->b_pcm.ensure(pcm_bytes));
+        CK(cudaMemcpyAsync(ctx->b_pcm.p, h_pcm, pcm_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        for (int i = 0; i < n; i++) seg[i].base = ctx->b_pcm.p;
+    }
+    // descriptors, one upload: SegDesc [n] | AlignRow [n]
+    const size_t o_row = sizeof(SegDesc) * (size_t)n;
+    std::vector<char> desc(o_row + sizeof(AlignRow) * (size_t)n);
+    std::memcpy(desc.data(), seg.data(), o_row);
+    std::memcpy(desc.data() + o_row, rows.data(), sizeof(AlignRow) * (size_t)n);
+    CK(ctx->b_desc.ensure(desc.size()));
+    char* d_desc = (char*)ctx->b_desc.p;
+    CK(cudaMemcpyAsync(d_desc, desc.data(), desc.size(), cudaMemcpyHostToDevice, ctx->stream));
+    CK(ctx->b_feat.ensure(sizeof(float) * FEAT * (size_t)n));
+    CK(ctx->b_frames.ensure(sizeof(float) * N_MFCC * (size_t)frames));
+    int rc = ctx->launch_segments((const SegDesc*)d_desc, n, max_frames, 0, frames, 0, 0, 0.f, (float*)ctx->b_feat.p,
+                                  (float*)ctx->b_frames.p, nullptr, nullptr);
+    if (rc != EWK_OK) return rc;
+    // outputs: the caller's device memory, or scratch dist [packed] | best_dist [n] | best_slot [n] copied back
+    float *o_dist = dist, *o_best = best_dist;
+    int32_t* o_slot = best_slot;
+    if (where == EWK_HOST) {
+        CK(ctx->b_scores.ensure(sizeof(float) * (size_t)(packed + 2 * n)));
+        o_dist = (float*)ctx->b_scores.p;
+        o_best = best_dist ? o_dist + packed : nullptr;
+        o_slot = best_slot ? (int32_t*)(o_dist + packed + n) : nullptr;
+    }
+    cudaEvent_t pe = ctx->prof_begin(3);
+    segment_align_kernel<<<n, ALIGN_THREADS, 0, ctx->stream>>>((const AlignRow*)(d_desc + o_row), (const float*)ctx->b_frames.p,
+                                                               (const float*)ctx->b_feat.p, ctx->d_tfr, ctx->d_tmpl,
+                                                               ctx->cfg.n_mfcc > 0 ? ctx->cfg.n_mfcc : N_MFCC, o_dist,
+                                                               o_best, o_slot);
+    ctx->prof_end(pe, 3);
+    CK(cudaGetLastError());
+    ctx->launches++;
+    if (where == EWK_HOST) {
+        CK(cudaMemcpyAsync(dist, o_dist, sizeof(float) * (size_t)packed, cudaMemcpyDeviceToHost, ctx->stream));
+        if (best_dist) CK(cudaMemcpyAsync(best_dist, o_best, sizeof(float) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+        if (best_slot) CK(cudaMemcpyAsync(best_slot, o_slot, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    CK(cudaStreamSynchronize(ctx->stream));
+    return EWK_OK;
+}
+
+static int align_common_args(ewk_ctx* ctx, const char* who, int n, const int32_t* first, const int32_t* count,
+                             const float* dist, int where) {
+    if (!ctx->d_tfr) { ctx->fail("%s: the context keeps no template frames (ewk_config.template_frames = 0)", who); return EWK_ERR_STATE; }
+    if (n < 0) { ctx->fail("%s: n = %d", who, n); return EWK_ERR_ARG; }
+    if (!first != !count) {
+        ctx->fail("%s: template_first and template_count must both be given or both be NULL", who);
+        return EWK_ERR_ARG;
+    }
+    if (n > 0 && !dist) { ctx->fail("%s: dist must not be NULL", who); return EWK_ERR_ARG; }
+    if (where != EWK_HOST && where != EWK_DEVICE) { ctx->fail("%s: where must be EWK_HOST or EWK_DEVICE", who); return EWK_ERR_ARG; }
+    return EWK_OK;
+}
+
+extern "C" int ewk_align_segments(ewk_ctx* ctx, int n, const int32_t* streams, const int64_t* starts, const int64_t* lens,
+                                  const int32_t* template_first, const int32_t* template_count, float* dist,
+                                  int64_t dist_cap, int32_t* best_slot, float* best_dist, int where) {
+    if (!ctx) return EWK_ERR_ARG;
+    const char* who = "ewk_align_segments";
+    int rc = align_common_args(ctx, who, n, template_first, template_count, dist, where);
+    if (rc) return rc;
+    rc = need_streams(ctx, who);                             // overlap mode: joins K3 of the last tick
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    rc = ctx->flush_pending();                               // the ranges may reach into a pending push
+    if (rc) return rc;
+    if (n == 0) return EWK_OK;
+    if (!streams || !starts || !lens) { ctx->fail("%s: streams, starts and lens must not be NULL", who); return EWK_ERR_ARG; }
+    const BankView& B = ctx->bank;
+    const size_t esz = B.fmt == 1 ? 2 : 4;
+    std::vector<SegDesc> seg((size_t)n);
+    std::vector<int> st((size_t)n), f((size_t)n), c((size_t)n);
+    for (int i = 0; i < n; i++) {                            // ewk_read_segment's checks, row by row
+        const int s = streams[i];
+        st[i] = s;
+        if (s < 0 || s >= B.n_streams) {
+            ctx->fail("%s: row %d (stream %d): stream out of range [0, %d)", who, i, s, B.n_streams);
+            return EWK_ERR_ARG;
+        }
+        if (lens[i] < 1 || lens[i] > ALIGN_MAX_SAMPLES || starts[i] < 0) {
+            ctx->fail("%s: row %d (stream %d): start %lld len %lld (need start >= 0, 1 <= len <= %d)", who, i, s,
+                      (long long)starts[i], (long long)lens[i], ALIGN_MAX_SAMPLES);
+            return EWK_ERR_ARG;
+        }
+        f[i] = template_first ? template_first[i] : ctx->h_prm[s].template_first;
+        c[i] = template_count ? template_count[i] : ctx->h_prm[s].template_count;
+    }
+    for (int i = 0; i < n; i++) {
+        const int s = st[i];
+        if (starts[i] + lens[i] > ctx->h_written[s]) { ctx->fail("%s: row %d (stream %d): segment not pushed yet", who, i, s); return EWK_ERR_STATE; }
+        if (ctx->h_written[s] - starts[i] > B.P) {
+            ctx->fail("%s: row %d (stream %d): segment already overwritten in the ring", who, i, s);
+            return EWK_ERR_STATE;
+        }
+        seg[i] = SegDesc{};
+        seg[i].base = (const char*)B.ring + (size_t)s * B.P * esz;
+        seg[i].start = starts[i] % B.P; seg[i].ring = B.P; seg[i].len = (int)lens[i]; seg[i].fmt = B.fmt;
+    }
+    return align_run(ctx, who, n, seg, st, f.data(), c.data(), dist, dist_cap, best_slot, best_dist, where, nullptr, 0);
+}
+
+extern "C" int ewk_align_buffers(ewk_ctx* ctx, int n, const void* pcm, int pcm_format, int where_in, const int64_t* offsets,
+                                 const int64_t* lens, const int32_t* template_first, const int32_t* template_count,
+                                 float* dist, int64_t dist_cap, int32_t* best_slot, float* best_dist, int where) {
+    if (!ctx) return EWK_ERR_ARG;
+    const char* who = "ewk_align_buffers";
+    int rc = align_common_args(ctx, who, n, template_first, template_count, dist, where);
+    if (rc) return rc;
+    if (n == 0) return EWK_OK;
+    if (!pcm || !offsets || !lens || !template_first || (pcm_format != EWK_PCM_F32 && pcm_format != EWK_PCM_I16) ||
+        (where_in != EWK_HOST && where_in != EWK_DEVICE)) {
+        ctx->fail("%s: need pcm, offsets, lens, template_first / template_count, pcm_format EWK_PCM_F32 or EWK_PCM_I16 and "
+                  "where_in EWK_HOST or EWK_DEVICE", who);
+        return EWK_ERR_ARG;
+    }
+    const size_t esz = pcm_format == EWK_PCM_I16 ? 2 : 4;
+    std::vector<SegDesc> seg((size_t)n);
+    std::vector<int> st((size_t)n, -1);
+    int64_t extent = 0;
+    for (int i = 0; i < n; i++) {
+        if (offsets[i] < 0 || lens[i] < 1 || lens[i] > ALIGN_MAX_SAMPLES) {
+            ctx->fail("%s: row %d (stream -1): offset %lld len %lld (need offset >= 0, 1 <= len <= %d)", who, i,
+                      (long long)offsets[i], (long long)lens[i], ALIGN_MAX_SAMPLES);
+            return EWK_ERR_ARG;
+        }
+        extent = std::max(extent, offsets[i] + lens[i]);
+        seg[i] = SegDesc{};
+        seg[i].base = pcm; seg[i].start = offsets[i]; seg[i].ring = 0; seg[i].len = (int)lens[i];
+        seg[i].fmt = pcm_format == EWK_PCM_I16 ? 1 : 0;
+    }
+    rc = ctx->join_match();                                  // overlap mode: K3 of the last tick shares the K3 workspaces
+    if (rc) return rc;
+    return align_run(ctx, who, n, seg, st, template_first, template_count, dist, dist_cap, best_slot, best_dist, where,
+                     where_in == EWK_HOST ? pcm : nullptr, esz * (size_t)extent);
 }
 
 // Launch geometry of K4 for a template set: hops per sub-chunk, threads per CTA and CTAs per SM that fit shared memory.

@@ -13,6 +13,7 @@
 #include "ewk_vad.cuh"
 #include "ewk_resample.cuh"
 #include "ewk_resample_push.cuh"
+#include "ewk_align.cuh"
 #include "ewk_tables.hpp"
 
 namespace ewk {
@@ -180,6 +181,11 @@ struct ewk_ctx {
     ewk::DeviceTables* d_tables = nullptr;
     ewk::TemplateFeat* d_tmpl = nullptr;
     std::vector<ewk::TemplateFeat> h_tmpl;
+    // template frame store (ewk_config.template_frames = 1): slot k's K3 frames at d_tfr + k * ALIGN_MAX_FRAMES * N_MFCC;
+    // h_tfr_n[k] frames (0: none: an empty slot, features only, or a template over ALIGN_MAX_SAMPLES samples)
+    float* d_tfr = nullptr;
+    std::vector<int> h_tfr_n;
+    void store_frames(int slot, const float* d_src, long long n_samples);   // the frames of a template of n_samples
     ewk::DevBuf b_pcm{&pool, "b_pcm", true}, b_desc{&pool, "b_desc", true}, b_ws{&pool, "b_ws", true}, b_lm{&pool, "b_lm", true}, b_feat{&pool, "b_feat", true}, b_scores{&pool, "b_scores", true}, b_matched{&pool, "b_matched", true}, b_frames{&pool, "b_frames", true}, b_off{&pool, "b_off", true};
 
     void fail(const char* fmt, ...);

@@ -60,7 +60,8 @@ typedef struct ewk_config {
                                its zi = 2 x[0] - x[1] initial state).  The reference applies none: 0 = identity
                                is the parity default and leaves every result bit-identical                    */
     int32_t n_mfcc;         /* MFCC coefficients kept, 1..20; 0 = 20                      wakeword.py:562     */
-    int32_t reserved0;
+    int32_t template_frames;/* 1: keep every template slot's MFCC frame matrix for frame alignment (ewk_align_*);
+                               max_templates x 301 x 20 floats of device memory (24 KB per slot).  0: none        */
     int32_t reserved1;
 } ewk_config;
 
@@ -251,6 +252,50 @@ int ewk_set_templates(ewk_ctx* ctx, const int32_t* slots, int n, const float* pc
  * context with n_streams = 0. */
 int ewk_set_templates_from_streams(ewk_ctx* ctx, const int32_t* slots, int n, const int32_t* streams,
                                    const int64_t* starts, const int64_t* lens, ewk_vad_result* vad);
+/* Frame alignment (second stage after level 2, before level 3): dynamic time warping of a segment's MFCC frames against
+ * a template's, which tells the word from the same sounds in another order (pooled mean / std cannot).  Needs a context
+ * created with ewk_config.template_frames = 1: ewk_set_template, ewk_set_templates and ewk_set_templates_from_streams then
+ * also keep each slot's frame matrix (the K3 frames of its audio, at no extra launch); a template over 48 000 samples
+ * (the longest segment alignment takes: 301 frames), ewk_set_template_features and ewk_clear_template leave the slot without frames.
+ * ewk_get_template_frames: *n_frames (nullable) receives the slot's frame count (0: none) and out[cap frames][20] (nullable)
+ * the frames, bit-identical to ewk_extract_mfcc's `frames` for the slot's audio.  EWK_ERR_STATE with template_frames = 0,
+ * EWK_ERR_NO_TEMPLATE for an empty slot, EWK_ERR_ARG for cap below the count. */
+int ewk_get_template_frames(ewk_ctx* ctx, int slot, float* out, int64_t cap, int32_t* n_frames);
+/* ewk_align_segments: row i is stream streams[i]'s absolute samples [starts[i], starts[i] + lens[i]) (the coordinates of
+ * ewk_event and ewk_detection, with ewk_read_segment's checks), aligned against slots [template_first[i], template_first[i]
+ * + template_count[i]); with both arrays NULL, row i takes its stream's own range (ewk_stream_params).  For a segment with
+ * frames f_0..f_{n-1} (exactly ewk_extract_mfcc's frames of that audio) and mean `mean` (its ewk_extract_mfcc mean), a
+ * template with stored frames g_0..g_{m-1} and its mean, and C = the context's n_mfcc (coefficients c < C only):
+ *   u_i = f_i - mean, v_j = g_j - template mean;  r_i = 1 / sqrt(sum_c u_i[c]^2) (0 when the sum is 0), s_j alike;
+ *   cost_ij = 1 - (dot(u_i, v_j) * r_i) * s_j  (cosine distance; an all-constant segment costs 1 everywhere);
+ *   D_00 = cost_00, D_i0 = D_{i-1,0} + cost_i0, D_0j = D_{0,j-1} + cost_0j,
+ *   D_ij = cost_ij + min(D_{i-1,j-1}, D_{i-1,j}, D_{i,j-1});   distance = D_{n-1,m-1} / (n + m),
+ * in float32 with every dot product and sum of squares a serial fma chain over c from +0 and every other operation rounded
+ * once (oracle/align_model.py is the bit-exact model).  0 is a perfect match; the word against itself gives 0.  There
+ * is no default threshold: a distance is not on the 0-100 score scale.
+ * dist is packed as the _sets forms pack rows: row i starts at sum_{j < i} T_j and holds T_i = template_count[i] values,
+ * in slot order; dist_cap is its capacity in floats.  best_slot[i] (nullable) receives the absolute slot of the lowest
+ * distance (the lowest slot on ties) and best_dist[i] (nullable) that distance.  `where` says whether the three outputs
+ * are host or device memory.  The call reads the rings and changes no stream, cursor, detector or event.  A pending host
+ * push lands first; in overlap mode the call joins K3 first.  One K3 launch (frames and means of every segment) and one
+ * K11 launch (one CTA per row), whatever n; synchronises with the context's stream.  n = 0 is a no-op.
+ * Errors, all before the first launch (a failed call writes no output), naming the row and the stream:
+ *   EWK_ERR_STATE: template_frames = 0; a range not yet pushed or already overwritten; a context with n_streams = 0.
+ *   EWK_ERR_ARG: a stream out of range; lens[i] outside 1..48000 or a negative start; T_i outside 1..64; a slot range
+ *   outside [0, max_templates); one of the two set arrays without the other; dist NULL or dist_cap below the packed
+ *   length; a slot without frames (cleared, features only, or over 48 000 samples).
+ *   EWK_ERR_NO_TEMPLATE: an empty slot. */
+int ewk_align_segments(ewk_ctx* ctx, int n, const int32_t* streams, const int64_t* starts, const int64_t* lens,
+                       const int32_t* template_first, const int32_t* template_count,
+                       float* dist, int64_t dist_cap, int32_t* best_slot, float* best_dist, int where);
+/* The same for caller audio (offline evaluation, threshold tuning): row i is pcm[offsets[i] : offsets[i] + lens[i]] in
+ * pcm_format (EWK_PCM_F32, or EWK_PCM_I16 read as q / 32768), host or device memory according to where_in; host input
+ * crosses in one copy.  The set arrays are required.  Works on any context (n_streams may be 0); the errors are those of
+ * ewk_align_segments that apply, rows named with stream -1. */
+int ewk_align_buffers(ewk_ctx* ctx, int n, const void* pcm, int pcm_format, int where_in,
+                      const int64_t* offsets, const int64_t* lens,
+                      const int32_t* template_first, const int32_t* template_count,
+                      float* dist, int64_t dist_cap, int32_t* best_slot, float* best_dist, int where);
 /* Ingest at other sample rates (SURVEY §8(f) N3): conversion to 16 kHz on the device, the step the reference
  * delegates to librosa.load(sr=16000) / librosa.resample (wakeword.py:588, 866-870; examples/tune_threshold.py:
  * 33-47; soxr HQ).  The filter meets soxr HQ's published specification (linear phase, pass-band to 0.913 of the
@@ -552,8 +597,8 @@ int64_t ewk_launch_count(const ewk_ctx* ctx);
 int ewk_debug_check(ewk_ctx* ctx);
 /* Per-kernel device timing with CUDA events on the context's stream.  ewk_profile(ctx, 1) starts
  * bracketing every kernel launch with an event pair; ewk_profile_read synchronises and returns, per
- * kernel class (0 ring_push, 1 tick_gate, 2 segment_queue, 3 segment_batch, 4 dense_score, 5 segment_prepare, 6 publish,
- * 7 resample_push), the summed
+ * kernel class (0 ring_push, 1 tick_gate, 2 segment_queue, 3 segment_batch (K3 of explicit segments, K6 and K11),
+ * 4 dense_score, 5 segment_prepare, 6 publish, 7 resample_push), the summed
  * milliseconds and the number of launches since profiling was enabled, then resets the sums. */
 enum { EWK_PROF_CLASSES = 8 };
 int ewk_profile(ewk_ctx* ctx, int enable);
