@@ -570,12 +570,6 @@ def _stream_list(streams):
     return _int32_list(streams, "stream index")
 
 
-def _unpack_rows(out, n_hops, T):
-    """Packed [sum n_i][T] scores -> list of [n_i, T] views, in list order."""
-    ends = np.cumsum(n_hops, dtype=np.int64)
-    return [out[(e - n) * T:e * T].reshape(n, T) for e, n in zip(ends.tolist(), [int(v) for v in n_hops])]
-
-
 def sets_offsets(n_hops, T):
     """Float offset of each row of a per-row-set call (include/ewk.h: ewk_dense_scores_sets): row i starts at
     sum_{j < i} n_hops[j] T[j].  Returns (offsets int64 [n], total floats)."""
@@ -588,6 +582,11 @@ def _unpack_rows_sets(out, n_hops, T):
     """Packed rows of a per-row-set call -> list of [n_i, T_i] views, in list order."""
     off, _ = sets_offsets(n_hops, T)
     return [out[o:o + int(n) * int(t)].reshape(int(n), int(t)) for o, n, t in zip(off.tolist(), n_hops, T)]
+
+
+def _one_set(n, template_first, template_count):
+    """-> the (template_first, template_count) arguments of a single-set entry point and T int64 [n]: every row's"""
+    return int(template_first), int(template_count), np.full(n, int(template_count), np.int64)
 
 
 def sets_launches(set_lens):
@@ -628,90 +627,6 @@ def _bank_methods():
         tf = np.ascontiguousarray(np.broadcast_to(np.asarray(template_first, np.int64), (n,)), np.int32)
         tc = np.ascontiguousarray(np.broadcast_to(np.asarray(template_count, np.int64), (n,)), np.int32)
         return tf, tc, tc.astype(np.int64)
-
-    def dense_scores_sets(self, streams, hop0, n_hops, template_first=None, template_count=None, out_device_ptr=None,
-                          out_cap=None):
-        """dense_scores_streams with a template set per row (include/ewk.h: ewk_dense_scores_sets): row i is scored
-        against slots [template_first[i], template_first[i] + template_count[i]) (both None: its stream's own range).
-        Returns a list of float32 [n_hops[i], T_i] arrays; with out_device_ptr the rows go there packed as the header
-        says (out_cap floats, default exactly what they need) and None is returned."""
-        st = _stream_list(streams)
-        h0 = np.ascontiguousarray(np.asarray(hop0, dtype=np.int64).reshape(-1))
-        nh64 = np.asarray(n_hops, dtype=np.int64).reshape(-1)
-        if len(h0) != len(st) or len(nh64) != len(st):
-            raise ValueError("one hop0 and one n_hops per stream")
-        if nh64.size and (nh64.min() < -2**31 or nh64.max() >= 2**31):
-            raise ValueError("n_hops out of range")
-        nh = np.ascontiguousarray(nh64, dtype=np.int32)
-        tf, tc, T = self._row_sets(st, len(st), template_first, template_count)
-        need = max(0, sets_offsets(np.maximum(nh64, 0), T)[1])
-        args = (st.ctypes.data_as(_p(C.c_int32)), len(st), i64ptr(h0), nh.ctypes.data_as(_p(C.c_int32)),
-                None if tf is None else tf.ctypes.data_as(_p(C.c_int32)),
-                None if tc is None else tc.ctypes.data_as(_p(C.c_int32)))
-        if out_device_ptr is not None:
-            self._ck(self.lib.ewk_dense_scores_sets(self.h, *args, C.c_void_p(out_device_ptr),
-                                                    need if out_cap is None else int(out_cap), DEVICE))
-            return None
-        out = np.empty(need, np.float32)
-        self._ck(self.lib.ewk_dense_scores_sets(self.h, *args, out.ctypes.data if need else None,
-                                                need if out_cap is None else int(out_cap), HOST))
-        return _unpack_rows_sets(out, nh64, T)
-
-    def dense_ready_sets(self, streams=None, max_hops=100, template_first=None, template_count=None,
-                         out_device_ptr=None, out_cap=None):
-        """dense_ready with a template set per row (include/ewk.h: ewk_dense_ready_sets; arguments as dense_scores_sets,
-        one entry per listed stream, or per stream when streams is None).  Moves dense_ready's cursor.  Returns (hop0,
-        list of float32 [n_i, T_i] arrays), or (hop0, n_hops) with out_device_ptr (out_cap floats, default
-        n * max_hops * max T_i)."""
-        st = None if streams is None else _stream_list(streams)
-        n = self.cfg.n_streams if st is None else len(st)
-        tf, tc, T = self._row_sets(st, n, template_first, template_count)
-        h0 = np.zeros(n, np.int64)
-        nh = np.zeros(n, np.int32)
-        cap = n * int(max_hops) * (int(T.max()) if n else 0) if out_cap is None else int(out_cap)
-        args = (None if st is None else st.ctypes.data_as(_p(C.c_int32)), n, int(max_hops),
-                None if tf is None else tf.ctypes.data_as(_p(C.c_int32)),
-                None if tc is None else tc.ctypes.data_as(_p(C.c_int32)), i64ptr(h0), nh.ctypes.data_as(_p(C.c_int32)))
-        if out_device_ptr is not None:
-            self._ck(self.lib.ewk_dense_ready_sets(self.h, *args, C.c_void_p(out_device_ptr), cap, DEVICE))
-            return h0, nh
-        out = np.empty(max(0, cap), np.float32)
-        self._ck(self.lib.ewk_dense_ready_sets(self.h, *args, out.ctypes.data if out.size else None, cap, HOST))
-        return h0, _unpack_rows_sets(out, nh, T)
-
-    def dense_detect_sets(self, streams=None, max_hops=100, template_first=None, template_count=None, hold_hops=20,
-                          refractory_hops=50, scores=False, out_device_ptr=None, det_cap=None, out_cap=None, hops=False):
-        """dense_detect with a template set per row (include/ewk.h: ewk_dense_detect_sets; sets as dense_ready_sets).
-        Moves dense_detect's cursor and detector state; returns what dense_detect returns, score rows [n_i, T_i]."""
-        st = None if streams is None else _stream_list(streams)
-        n = self.cfg.n_streams if st is None else len(st)
-        tf, tc, T = self._row_sets(st, n, template_first, template_count)
-        cap = n * ((min(int(max_hops), 1 << 20) + 1) // 2) if det_cap is None else int(det_cap)
-        det = np.empty(max(0, cap), DETECTION_DTYPE)
-        h0 = np.zeros(n, np.int64)
-        nh = np.zeros(n, np.int32)
-        ocap = n * int(max_hops) * (int(T.max()) if n else 0) if out_cap is None else int(out_cap)
-        buf = None
-        if out_device_ptr is not None:
-            out, where = C.c_void_p(out_device_ptr), DEVICE
-        elif scores:
-            buf = np.empty(max(0, ocap), np.float32)
-            out, where = (buf.ctypes.data if buf.size else None), HOST
-        else:
-            out, ocap, where = None, 0, HOST
-        rc = self.lib.ewk_dense_detect_sets(self.h, None if st is None else st.ctypes.data_as(_p(C.c_int32)), n,
-                                            int(max_hops), None if tf is None else tf.ctypes.data_as(_p(C.c_int32)),
-                                            None if tc is None else tc.ctypes.data_as(_p(C.c_int32)), int(hold_hops),
-                                            int(refractory_hops), det.ctypes.data if det.size else None, cap, i64ptr(h0),
-                                            nh.ctypes.data_as(_p(C.c_int32)), out, ocap, where)
-        if rc < 0:
-            self._ck(rc)
-        d = det[:rc].copy()
-        if out_device_ptr is not None:
-            return d, (h0, nh)
-        if scores:
-            return d, (h0, _unpack_rows_sets(buf, nh, T))
-        return (d, (h0, nh)) if hops else d
 
     def push(self, pcm, stream0=0, where=HOST):
         """pcm: [n_streams, n] array in the ring's dtype (rows may be strided), or (ptr, n_streams, n, stride)."""
@@ -969,12 +884,15 @@ def _bank_methods():
                                            out.ctypes.data, HOST))
         return out
 
-    def dense_scores_streams(self, streams, hop0, n_hops, template_first=0, template_count=1, out_device_ptr=None,
-                             out_cap=None):
-        """Ragged dense scoring (include/ewk.h: ewk_dense_scores_streams): row i scores stream streams[i] at hops
-        [hop0[i], hop0[i] + n_hops[i]) (0 included).  Returns a list of float32 [n_hops[i], template_count] arrays; with
-        out_device_ptr the rows go there packed back to back in list order (out_cap floats, default exactly what they
-        need) and None is returned."""
+    def _sets_args(self, st, n, template_first, template_count):
+        """-> the (template_first, template_count) arguments of a *_sets entry point and T int64 [n] (see _row_sets)"""
+        tf, tc, T = self._row_sets(st, n, template_first, template_count)
+        return (None if tf is None else tf.ctypes.data_as(_p(C.c_int32)),
+                None if tc is None else tc.ctypes.data_as(_p(C.c_int32)), T)
+
+    def _scores_rows(self, fn, sets, streams, hop0, n_hops, out_device_ptr, out_cap):
+        """dense_scores_streams / dense_scores_sets through entry point fn; sets(st, n) -> its two template arguments
+        and each row's T"""
         st = _stream_list(streams)
         h0 = np.ascontiguousarray(np.asarray(hop0, dtype=np.int64).reshape(-1))
         nh64 = np.asarray(n_hops, dtype=np.int64).reshape(-1)
@@ -983,17 +901,84 @@ def _bank_methods():
         if nh64.size and (nh64.min() < -2**31 or nh64.max() >= 2**31):
             raise ValueError("n_hops out of range")
         nh = np.ascontiguousarray(nh64, dtype=np.int32)
-        T = int(template_count)
-        need = max(0, int(nh64[nh64 > 0].sum()) * T)
-        args = (st.ctypes.data_as(_p(C.c_int32)), len(st), i64ptr(h0), nh.ctypes.data_as(_p(C.c_int32)), template_first, T)
+        tf, tc, T = sets(st, len(st))
+        need = max(0, int(np.maximum(nh64, 0) @ T))
+        cap = need if out_cap is None else int(out_cap)
+        args = (st.ctypes.data_as(_p(C.c_int32)), len(st), i64ptr(h0), nh.ctypes.data_as(_p(C.c_int32)), tf, tc)
         if out_device_ptr is not None:
-            self._ck(self.lib.ewk_dense_scores_streams(self.h, *args, C.c_void_p(out_device_ptr),
-                                                       need if out_cap is None else int(out_cap), DEVICE))
+            self._ck(fn(self.h, *args, C.c_void_p(out_device_ptr), cap, DEVICE))
             return None
         out = np.empty(need, np.float32)
-        self._ck(self.lib.ewk_dense_scores_streams(self.h, *args, out.ctypes.data if need else None,
-                                                   need if out_cap is None else int(out_cap), HOST))
-        return _unpack_rows(out, nh64, T)
+        self._ck(fn(self.h, *args, out.ctypes.data if need else None, cap, HOST))
+        return _unpack_rows_sets(out, nh64, T)
+
+    def _ready(self, fn, sets, streams, max_hops, out_device_ptr, out_cap):
+        """dense_ready / dense_ready_sets through entry point fn (sets as in _scores_rows)"""
+        st = None if streams is None else _stream_list(streams)
+        n = self.cfg.n_streams if st is None else len(st)
+        tf, tc, T = sets(st, n)
+        h0 = np.zeros(n, np.int64)
+        nh = np.zeros(n, np.int32)
+        cap = n * int(max_hops) * (int(T.max()) if n else 0) if out_cap is None else int(out_cap)
+        args = (None if st is None else st.ctypes.data_as(_p(C.c_int32)), n, int(max_hops), tf, tc, i64ptr(h0),
+                nh.ctypes.data_as(_p(C.c_int32)))
+        if out_device_ptr is not None:
+            self._ck(fn(self.h, *args, C.c_void_p(out_device_ptr), cap, DEVICE))
+            return h0, nh
+        out = np.empty(max(0, cap), np.float32)
+        self._ck(fn(self.h, *args, out.ctypes.data if out.size else None, cap, HOST))
+        return h0, _unpack_rows_sets(out, nh, T)
+
+    def _detect(self, fn, sets, streams, max_hops, hold_hops, refractory_hops, scores, out_device_ptr, det_cap, out_cap,
+                hops):
+        """dense_detect / dense_detect_sets through entry point fn (sets as in _scores_rows)"""
+        st = None if streams is None else _stream_list(streams)
+        n = self.cfg.n_streams if st is None else len(st)
+        tf, tc, T = sets(st, n)
+        cap = n * ((min(int(max_hops), 1 << 20) + 1) // 2) if det_cap is None else int(det_cap)
+        det = np.empty(max(0, cap), DETECTION_DTYPE)
+        h0 = np.zeros(n, np.int64)
+        nh = np.zeros(n, np.int32)
+        ocap = n * int(max_hops) * (int(T.max()) if n else 0) if out_cap is None else int(out_cap)
+        buf = None
+        if out_device_ptr is not None:
+            out, where = C.c_void_p(out_device_ptr), DEVICE
+        elif scores:
+            buf = np.empty(max(0, ocap), np.float32)
+            out, where = (buf.ctypes.data if buf.size else None), HOST
+        else:
+            out, ocap, where = None, 0, HOST
+        rc = fn(self.h, None if st is None else st.ctypes.data_as(_p(C.c_int32)), n, int(max_hops), tf, tc, int(hold_hops),
+                int(refractory_hops), det.ctypes.data if det.size else None, cap, i64ptr(h0), nh.ctypes.data_as(_p(C.c_int32)),
+                out, ocap, where)
+        if rc < 0:
+            self._ck(rc)
+        d = det[:rc].copy()
+        if out_device_ptr is not None:
+            return d, (h0, nh)
+        if scores:
+            return d, (h0, _unpack_rows_sets(buf, nh, T))
+        return (d, (h0, nh)) if hops else d
+
+    def dense_scores_streams(self, streams, hop0, n_hops, template_first=0, template_count=1, out_device_ptr=None,
+                             out_cap=None):
+        """Ragged dense scoring (include/ewk.h: ewk_dense_scores_streams): row i scores stream streams[i] at hops
+        [hop0[i], hop0[i] + n_hops[i]) (0 included).  Returns a list of float32 [n_hops[i], template_count] arrays; with
+        out_device_ptr the rows go there packed back to back in list order (out_cap floats, default exactly what they
+        need) and None is returned."""
+        return self._scores_rows(self.lib.ewk_dense_scores_streams,
+                                 lambda st, n: _one_set(n, template_first, template_count), streams, hop0, n_hops,
+                                 out_device_ptr, out_cap)
+
+    def dense_scores_sets(self, streams, hop0, n_hops, template_first=None, template_count=None, out_device_ptr=None,
+                          out_cap=None):
+        """dense_scores_streams with a template set per row (include/ewk.h: ewk_dense_scores_sets): row i is scored
+        against slots [template_first[i], template_first[i] + template_count[i]) (both None: its stream's own range).
+        Returns a list of float32 [n_hops[i], T_i] arrays; with out_device_ptr the rows go there packed as the header
+        says (out_cap floats, default exactly what they need) and None is returned."""
+        return self._scores_rows(self.lib.ewk_dense_scores_sets,
+                                 lambda st, n: self._sets_args(st, n, template_first, template_count), streams, hop0, n_hops,
+                                 out_device_ptr, out_cap)
 
     def dense_ready(self, streams=None, max_hops=100, template_first=0, template_count=1, out_device_ptr=None,
                     out_cap=None):
@@ -1002,20 +987,18 @@ def _bank_methods():
         on.  Returns (hop0, scores): int64 [n] first hops and a list of float32 [n_i, template_count] arrays.  With
         out_device_ptr (out_cap floats, default n * max_hops * template_count) the rows go there packed in list order and
         (hop0, n_hops) is returned."""
-        st = None if streams is None else _stream_list(streams)
-        n = self.cfg.n_streams if st is None else len(st)
-        T = int(template_count)
-        h0 = np.zeros(n, np.int64)
-        nh = np.zeros(n, np.int32)
-        cap = n * int(max_hops) * T if out_cap is None else int(out_cap)
-        args = (None if st is None else st.ctypes.data_as(_p(C.c_int32)), n, int(max_hops), template_first, T, i64ptr(h0),
-                nh.ctypes.data_as(_p(C.c_int32)))
-        if out_device_ptr is not None:
-            self._ck(self.lib.ewk_dense_ready(self.h, *args, C.c_void_p(out_device_ptr), cap, DEVICE))
-            return h0, nh
-        out = np.empty(max(0, cap), np.float32)
-        self._ck(self.lib.ewk_dense_ready(self.h, *args, out.ctypes.data if out.size else None, cap, HOST))
-        return h0, _unpack_rows(out, nh, T)
+        return self._ready(self.lib.ewk_dense_ready, lambda st, n: _one_set(n, template_first, template_count),
+                           streams, max_hops, out_device_ptr, out_cap)
+
+    def dense_ready_sets(self, streams=None, max_hops=100, template_first=None, template_count=None,
+                         out_device_ptr=None, out_cap=None):
+        """dense_ready with a template set per row (include/ewk.h: ewk_dense_ready_sets; arguments as dense_scores_sets,
+        one entry per listed stream, or per stream when streams is None).  Moves dense_ready's cursor.  Returns (hop0,
+        list of float32 [n_i, T_i] arrays), or (hop0, n_hops) with out_device_ptr (out_cap floats, default
+        n * max_hops * max T_i)."""
+        return self._ready(self.lib.ewk_dense_ready_sets,
+                           lambda st, n: self._sets_args(st, n, template_first, template_count), streams, max_hops,
+                           out_device_ptr, out_cap)
 
     def dense_detect(self, streams=None, max_hops=100, template_first=0, template_count=1, hold_hops=20,
                      refractory_hops=50, scores=False, out_device_ptr=None, det_cap=None, out_cap=None, hops=False):
@@ -1026,34 +1009,16 @@ def _bank_methods():
         scores=True also returns (hop0, list of float32 [n_i, template_count] arrays); with out_device_ptr the scores go
         there packed in list order (out_cap floats, default n * max_hops * template_count) and (hop0, n_hops) is returned
         with the detections.  Otherwise the scores stay on the device; hops=True then returns (hop0, n_hops) with them."""
-        st = None if streams is None else _stream_list(streams)
-        n = self.cfg.n_streams if st is None else len(st)
-        T = int(template_count)
-        cap = n * ((min(int(max_hops), 1 << 20) + 1) // 2) if det_cap is None else int(det_cap)
-        det = np.empty(max(0, cap), DETECTION_DTYPE)
-        h0 = np.zeros(n, np.int64)
-        nh = np.zeros(n, np.int32)
-        ocap = n * int(max_hops) * T if out_cap is None else int(out_cap)
-        buf = None
-        if out_device_ptr is not None:
-            out, where = C.c_void_p(out_device_ptr), DEVICE
-        elif scores:
-            buf = np.empty(max(0, ocap), np.float32)
-            out, where = (buf.ctypes.data if buf.size else None), HOST
-        else:
-            out, ocap, where = None, 0, HOST
-        rc = self.lib.ewk_dense_detect(self.h, None if st is None else st.ctypes.data_as(_p(C.c_int32)), n, int(max_hops),
-                                       int(template_first), T, int(hold_hops), int(refractory_hops),
-                                       det.ctypes.data if det.size else None, cap, i64ptr(h0),
-                                       nh.ctypes.data_as(_p(C.c_int32)), out, ocap, where)
-        if rc < 0:
-            self._ck(rc)
-        d = det[:rc].copy()
-        if out_device_ptr is not None:
-            return d, (h0, nh)
-        if scores:
-            return d, (h0, _unpack_rows(buf, nh, T))
-        return (d, (h0, nh)) if hops else d
+        return self._detect(self.lib.ewk_dense_detect, lambda st, n: _one_set(n, template_first, template_count),
+                            streams, max_hops, hold_hops, refractory_hops, scores, out_device_ptr, det_cap, out_cap, hops)
+
+    def dense_detect_sets(self, streams=None, max_hops=100, template_first=None, template_count=None, hold_hops=20,
+                          refractory_hops=50, scores=False, out_device_ptr=None, det_cap=None, out_cap=None, hops=False):
+        """dense_detect with a template set per row (include/ewk.h: ewk_dense_detect_sets; sets as dense_ready_sets).
+        Moves dense_detect's cursor and detector state; returns what dense_detect returns, score rows [n_i, T_i]."""
+        return self._detect(self.lib.ewk_dense_detect_sets,
+                            lambda st, n: self._sets_args(st, n, template_first, template_count), streams, max_hops,
+                            hold_hops, refractory_hops, scores, out_device_ptr, det_cap, out_cap, hops)
 
     def dense_last_plan(self):
         """(DH, threads, CTAs per SM, shared-memory bytes) of the latest K4 launch (dense_scores, dense_scores_streams or
@@ -1147,7 +1112,8 @@ def _bank_methods():
                  "resample_push"]
         return {names[i]: {"ms": ms[i], "launches": int(n[i])} for i in range(len(names))}
 
-    for f in (align_segments, _template_ranges, _row_sets, dense_scores_sets, dense_ready_sets, dense_detect_sets, set_templates_from_streams):
+    for f in (align_segments, _template_ranges, _row_sets, _sets_args, _scores_rows, _ready, _detect, dense_scores_sets,
+              dense_ready_sets, dense_detect_sets, set_templates_from_streams):
         setattr(Context, f.__name__, f)
     for f in (prepare_segments, dense_scores, dense_scores_streams, dense_ready, dense_detect, dense_last_plan, profile, profile_read, set_stream_params, push, push_g711, push_resampled,
               push_resampled_each, push_streams, tick_ready, reset_streams, stream_blob_bytes, export_streams, import_streams, stream_input, tick, poll, status, read_last, read_segment, results, results_device_ptr,

@@ -304,16 +304,8 @@ void ewk_ctx::release() {
         if (h_pos[i]) pool.free(h_pos[i], true);
         ev_pos[i] = nullptr; h_pos[i] = nullptr;
         b_pos[i].free();
-        if (ev_drow[i]) cudaEventDestroy(ev_drow[i]);
-        if (h_drow[i]) pool.free(h_drow[i], true);
-        ev_drow[i] = nullptr; h_drow[i] = nullptr;
-        b_drow[i].free();
-        if (ev_ddet[i]) cudaEventDestroy(ev_ddet[i]);
-        if (h_ddet[i]) pool.free(h_ddet[i], true);
-        ev_ddet[i] = nullptr; h_ddet[i] = nullptr;
-        b_ddet[i].free();
     }
-    dset_stage.free(); drow_sets.free(); ddet_sets.free(); b_dset.free();
+    dset_stage.free(); drows.free(); ddets.free(); b_dset.free();
     h_dset.clear();
     if (h_det_map) pool.free(h_det_map, true);
     h_det_map = nullptr; det_map_cap = 0;
@@ -2638,13 +2630,10 @@ extern "C" int ewk_align_buffers(ewk_ctx* ctx, int n, const void* pcm, int pcm_f
                      where_in == EWK_HOST ? pcm : nullptr, esz * (size_t)extent);
 }
 
-// Launch geometry of K4 for a template set: hops per sub-chunk, threads per CTA and CTAs per SM that fit shared memory.
-struct DensePlan { int DH, threads, per_sm; size_t smem; };
-
-static bool dense_plan(const DenseArgs& A0, int n_min, int n_max, int n_re_u, DensePlan& out) {
+static bool dense_plan(int T, int n_min, int n_max, int n_re_u, DensePlan& out) {
     const size_t SM_TOTAL = 233472, CTA_MAX = 232448, RESERVED = 1024;     // sm_100: 228 KB per SM, 227 KB per CTA
     auto bytes = [&](int DH, int threads) {
-        return dense_smem_bytes(threads / 32, A0.T, DH, DH + n_max + 2, DH + n_max - n_min, n_re_u);
+        return dense_smem_bytes(threads / 32, T, DH, DH + n_max + 2, DH + n_max - n_min, n_re_u);
     };
     for (int DH : {64, 32})
         for (int threads : {512, 448}) {
@@ -2661,13 +2650,13 @@ static bool dense_plan(const DenseArgs& A0, int n_min, int n_max, int n_re_u, De
 
 // Everything of a K4 call that follows from the template lengths alone (each in [DENSE_MIN_L, DENSE_MAX_L]): window
 // geometry per template, the right-edge frames templates share, and the launch geometry.  ewk_dense_plan reports what
-// ewk_dense_scores launches because both go through here.  False: the set does not fit shared memory.
-static bool dense_setup(const int64_t* lens, int n, DenseArgs& A, DensePlan& plan) {
-    A.T = n;
+// the entry points launch because all go through here.  False: the set does not fit shared memory.
+static bool dense_setup(const int64_t* lens, int n, DenseSetDev& S, DensePlan& plan) {
+    S.T = n;
     int max_n = 0, min_n = 1 << 30, g_back = 1 << 30, n_re_u = 0;
     for (int k = 0; k < n; k++) {
         const int L = (int)lens[k];
-        DenseTmplDev& t = A.t[k];
+        DenseTmplDev& t = S.t[k];
         t.L = L; t.n = (L + HOP - 1) / HOP; t.F = 1 + L / HOP; t.t_hi = (L - N_FFT / 2) / HOP; t.r = t.F - 1 - t.t_hi;
         t.inv_f = 1.0 / (double)t.F;
         max_n = std::max(max_n, t.n); min_n = std::min(min_n, t.n);
@@ -2678,17 +2667,17 @@ static bool dense_setup(const int64_t* lens, int n, DenseArgs& A, DensePlan& pla
         for (int e = 0; e < t.r; e++) {
             const int goff = t.n - (t.t_hi + 1 + e);
             int u = 0;
-            while (u < n_re_u && !(A.re_goff[u] == goff && A.re_delta[u] == delta)) u++;
+            while (u < n_re_u && !(S.re_goff[u] == goff && S.re_delta[u] == delta)) u++;
             if (u == n_re_u) {
-                A.re_goff[u] = goff; A.re_delta[u] = delta; A.re_rep[u] = k; A.re_rep_e[u] = e; A.re_nfirst[u] = t.n;
+                S.re_goff[u] = goff; S.re_delta[u] = delta; S.re_rep[u] = k; S.re_rep_e[u] = e; S.re_nfirst[u] = t.n;
                 n_re_u++;
-            } else if (t.n < A.re_nfirst[u]) { A.re_rep[u] = k; A.re_rep_e[u] = e; A.re_nfirst[u] = t.n; }
+            } else if (t.n < S.re_nfirst[u]) { S.re_rep[u] = k; S.re_rep_e[u] = e; S.re_nfirst[u] = t.n; }
             t.re_u[e] = u;
         }
     }
-    if (!dense_plan(A, min_n, max_n, n_re_u, plan)) return false;
-    A.DH = plan.DH; A.DG = plan.DH + max_n + 2; A.DLE = plan.DH + max_n - min_n; A.n_re_u = n_re_u;
-    A.n_min = min_n; A.n_max = max_n; A.g_back = g_back;
+    if (!dense_plan(n, min_n, max_n, n_re_u, plan)) return false;
+    S.DH = plan.DH; S.DG = plan.DH + max_n + 2; S.DLE = plan.DH + max_n - min_n; S.n_re_u = n_re_u;
+    S.n_min = min_n; S.n_max = max_n; S.g_back = g_back;
     return true;
 }
 
@@ -2696,9 +2685,9 @@ extern "C" int ewk_dense_plan(const int64_t* template_lens, int n, int32_t out[4
     if (!template_lens || !out || n < 1 || n > DENSE_MAX_T) return EWK_ERR_ARG;
     for (int k = 0; k < n; k++)
         if (template_lens[k] < DENSE_MIN_L || template_lens[k] > DENSE_MAX_L) return EWK_ERR_ARG;
-    DenseArgs A{};
+    DenseSetDev S{};
     DensePlan plan;
-    if (!dense_setup(template_lens, n, A, plan)) return EWK_ERR_ARG;
+    if (!dense_setup(template_lens, n, S, plan)) return EWK_ERR_ARG;
     out[0] = plan.DH; out[1] = plan.threads; out[2] = plan.per_sm; out[3] = (int32_t)plan.smem;
     return EWK_OK;
 }
@@ -2709,34 +2698,44 @@ extern "C" int ewk_dense_last_plan(const ewk_ctx* ctx, int32_t out[4]) {
     return EWK_OK;
 }
 
-// What every K4 entry point checks and plans from its template range alone (errors name `who`): the templates, the
-// window geometry (dense_setup), the ring length.
-static int dense_prepare(ewk_ctx* ctx, const char* who, int tmpl_first, int tmpl_count, DenseArgs& A, DensePlan& plan) {
-    if (tmpl_count < 1 || tmpl_count > DENSE_MAX_T || tmpl_first < 0 || tmpl_first + tmpl_count > ctx->cfg.max_templates) {
-        ctx->fail("%s: bad template range [%d, %d) (at most %d per call, %d slots)", who, tmpl_first, tmpl_first + tmpl_count,
-                  DENSE_MAX_T, ctx->cfg.max_templates);
+static bool dense_range_ok(const ewk_ctx* ctx, int first, int count) {
+    return count >= 1 && count <= DENSE_MAX_T && first >= 0 && first <= ctx->cfg.max_templates - count;
+}
+
+// The template set [first, first + count) of a K4 call, with every check of it (errors name `who`): the range, each slot's
+// presence and length, the fit in shared memory (dense_setup) and the ring length.
+static int dense_set_build(ewk_ctx* ctx, const char* who, int first, int count, DenseSetHost& e) {
+    if (!dense_range_ok(ctx, first, count)) {
+        ctx->fail("%s: bad template range [%d, %d) (1..%d templates of %d slots)", who, first, first + count, DENSE_MAX_T,
+                  ctx->cfg.max_templates);
         return EWK_ERR_ARG;
     }
     int64_t lens[DENSE_MAX_T];
-    for (int k = 0; k < tmpl_count; k++) {
-        const TemplateFeat& tf = ctx->h_tmpl[tmpl_first + k];
-        if (!tf.valid) { ctx->fail("No reference word set. Call set_reference() first."); return EWK_ERR_NO_TEMPLATE; }
+    for (int k = first; k < first + count; k++) {
+        const TemplateFeat& tf = ctx->h_tmpl[k];
+        if (!tf.valid) {
+            ctx->fail("%s: template slot %d is empty. No reference word set. Call set_reference() first.", who, k);
+            return EWK_ERR_NO_TEMPLATE;
+        }
         if (tf.n_samples < DENSE_MIN_L || tf.n_samples > DENSE_MAX_L) {
-            ctx->fail("%s: template %d has %lld samples; dense scoring needs %d..%d", who, tmpl_first + k,
-                      (long long)tf.n_samples, DENSE_MIN_L, DENSE_MAX_L);
+            ctx->fail("%s: template %d has %lld samples; dense scoring needs %d..%d", who, k, (long long)tf.n_samples,
+                      DENSE_MIN_L, DENSE_MAX_L);
             return EWK_ERR_ARG;
         }
-        lens[k] = tf.n_samples;
+        lens[k - first] = tf.n_samples;
     }
-    if (!dense_setup(lens, tmpl_count, A, plan)) {
-        ctx->fail("%s: this template set does not fit shared memory (%d templates, windows of %d..%d hops)", who,
-                  tmpl_count, (int)((*std::min_element(lens, lens + tmpl_count) + HOP - 1) / HOP),
-                  (int)((*std::max_element(lens, lens + tmpl_count) + HOP - 1) / HOP));
+    e = DenseSetHost{};
+    DenseSetDev& d = e.dev;
+    if (!dense_setup(lens, count, d, e.plan)) {
+        ctx->fail("%s: this template set does not fit shared memory (%d templates, windows of %d..%d hops)", who, count,
+                  (int)((*std::min_element(lens, lens + count) + HOP - 1) / HOP),
+                  (int)((*std::max_element(lens, lens + count) + HOP - 1) / HOP));
         return EWK_ERR_ARG;
     }
-    for (int k = 0; k < tmpl_count; k++) A.t[k].slot = tmpl_first + k;
-    if ((long long)ctx->bank.P < 160LL * (A.n_max + plan.DH + 4) + N_FFT) {        // the kernel wraps ring positions once
-        ctx->fail("%s: ring of %d samples is too short for a template of %d hops", who, ctx->bank.P, A.n_max);
+    d.slot0 = first;
+    for (int k = 0; k < count; k++) d.t[k].slot = first + k;
+    if ((long long)ctx->bank.P < 160LL * (d.n_max + e.plan.DH + 4) + N_FFT) {        // the kernel wraps ring positions once
+        ctx->fail("%s: ring of %d samples is too short for a template of %d hops", who, ctx->bank.P, d.n_max);
         return EWK_ERR_ARG;
     }
     return EWK_OK;
@@ -2757,9 +2756,24 @@ static int dense_resident(ewk_ctx* ctx, const char* who, int s, long long hop0, 
     return EWK_OK;
 }
 
-// K4 over n_ctas CTAs into d_out: the uniform instance, or the per-row one when A.rows is set (sets: its per-row-set
-// form, A.rows holding DenseRowSet descriptors)
-static int dense_launch(ewk_ctx* ctx, DenseArgs& A, const DensePlan& plan, float* d_out, int n_ctas, bool sets = false) {
+// A host push whose copy is still in flight lands now only if the call's hops reach into its samples: otherwise the copy
+// of the NEXT block keeps overlapping the call's kernel (offline sweeps: push block j + 1, then score block j).
+// last_hop(s): the last hop the call scores on stream s (< 0: none).
+template <class F>
+static int dense_land_if_reached(ewk_ctx* ctx, F last_hop) {
+    if (!ctx->pending.valid) return EWK_OK;
+    const std::vector<RowDesc>& rows = ctx->pending.rows;
+    for (int j = 0; j < ctx->pending.n_streams; j++) {
+        const int s = rows.empty() ? ctx->pending.stream0 + j : rows[j].stream;
+        const long long h = last_hop(s);
+        if (h >= 0 && ctx->h_written[s] < 160LL * h) return ctx->flush_pending();
+    }
+    return EWK_OK;
+}
+
+// K4 over n_ctas CTAs into d_out: the uniform instance, or with A.rows set a row instance: the one-set instance when every
+// row's set is A.set (one_set), else the per-row-set instance
+static int dense_launch(ewk_ctx* ctx, DenseArgs& A, const DensePlan& plan, float* d_out, int n_ctas, bool one_set = true) {
     BankView& B = ctx->bank;
     A.out = d_out;
     if (!ctx->b_keep_rows.p) {
@@ -2767,14 +2781,14 @@ static int dense_launch(ewk_ctx* ctx, DenseArgs& A, const DensePlan& plan, float
         CK(ctx->b_keep_end.ensure(sizeof(long long) * 2 * (size_t)B.n_streams));
         CK(cudaMemsetAsync(ctx->b_keep_end.p, 0, sizeof(long long) * 2 * (size_t)B.n_streams, ctx->stream));
     }
-    CK(ctx->b_g2.ensure(sizeof(float) * (size_t)B.n_streams * DENSE_WAYS * A.DG * N_MFCC));
+    CK(ctx->b_g2.ensure(sizeof(float) * (size_t)B.n_streams * DENSE_WAYS * (one_set ? A.set.DG : A.DG) * N_MFCC));
     A.keep_rows = (float*)ctx->b_keep_rows.p;
     A.keep_end = (long long*)ctx->b_keep_end.p;
     A.g2 = (float*)ctx->b_g2.p;
     const bool pre = ctx->cfg.preemphasis != 0.f;
-    auto k4 = sets     ? (pre ? dense_score_kernel<true, true, true> : dense_score_kernel<false, true, true>)
-            : A.rows ? (pre ? dense_score_kernel<true, true> : dense_score_kernel<false, true>)
-                     : (pre ? dense_score_kernel<true, false> : dense_score_kernel<false, false>);
+    auto k4 = !A.rows ? (pre ? dense_score_kernel<true, false, false> : dense_score_kernel<false, false, false>)
+            : one_set ? (pre ? dense_score_kernel<true, true, false> : dense_score_kernel<false, true, false>)
+                      : (pre ? dense_score_kernel<true, true, true> : dense_score_kernel<false, true, true>);
     CK(cudaFuncSetAttribute(k4, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem));
     CK(cudaFuncSetAttribute(k4, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
     cudaEvent_t pe = ctx->prof_begin(4);
@@ -2793,35 +2807,28 @@ extern "C" int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int tmpl
     if (rc) return rc;
     cudaSetDevice(ctx->device);
     BankView& B = ctx->bank;
-    if (ctx->pending.valid) {
-        // a host push whose copy is still in flight lands now only if these hops reach into its samples: otherwise the copy
-        // of the NEXT block keeps overlapping this call's kernel (offline sweeps: push block j + 1, then score block j)
-        bool need = false;
-        const std::vector<RowDesc>& rows = ctx->pending.rows;
-        for (int i = 0; !need && i < ctx->pending.n_streams; i++)
-            need = ctx->h_written[rows.empty() ? ctx->pending.stream0 + i : rows[i].stream] < 160LL * (hop0 + n_hops - 1);
-        if (need) { rc = ctx->flush_pending(); if (rc) return rc; }
-    }
+    rc = dense_land_if_reached(ctx, [&](int) { return (long long)hop0 + n_hops - 1; });
+    if (rc) return rc;
     if (!out || hop0 < 0 || n_hops < 1 || tmpl_count < 1 || tmpl_count > DENSE_MAX_T || tmpl_first < 0 ||
         tmpl_first + tmpl_count > ctx->cfg.max_templates) {
         ctx->fail("ewk_dense_scores: bad arguments (hop0=%lld n_hops=%d templates [%d, %d), at most %d per call)", (long long)hop0,
                   n_hops, tmpl_first, tmpl_first + tmpl_count, DENSE_MAX_T);
         return EWK_ERR_ARG;
     }
-    DenseArgs A{};
-    DensePlan plan;
-    rc = dense_prepare(ctx, "ewk_dense_scores", tmpl_first, tmpl_count, A, plan);
+    DenseSetHost e;
+    rc = dense_set_build(ctx, "ewk_dense_scores", tmpl_first, tmpl_count, e);
     if (rc) return rc;
-    A.hop0 = hop0; A.n_hops = n_hops;
     for (int s = 0; s < B.n_streams; s++) {
-        rc = dense_resident(ctx, "ewk_dense_scores", s, hop0, n_hops, A.n_max);
+        rc = dense_resident(ctx, "ewk_dense_scores", s, hop0, n_hops, e.dev.n_max);
         if (rc) return rc;
     }
     CK(cudaSetDevice(ctx->device));
     const size_t n_out = (size_t)B.n_streams * n_hops * tmpl_count;
     float* d_out = out;
     if (where == EWK_HOST) { CK(ctx->b_dense.ensure(sizeof(float) * n_out)); d_out = (float*)ctx->b_dense.p; }
-    rc = dense_launch(ctx, A, plan, d_out, B.n_streams);
+    DenseArgs A{};
+    A.hop0 = hop0; A.n_hops = n_hops; A.set = e.dev;
+    rc = dense_launch(ctx, A, e.plan, d_out, B.n_streams);
     if (rc) return rc;
     if (where == EWK_HOST) {
         CK(cudaMemcpyAsync(out, d_out, sizeof(float) * n_out, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2830,87 +2837,7 @@ extern "C" int ewk_dense_scores(ewk_ctx* ctx, int64_t hop0, int n_hops, int tmpl
     return EWK_OK;
 }
 
-// Rows of ewk_dense_scores_streams, ewk_dense_ready and ewk_dense_detect: row i scores stream streams[i] at hops
-// [hop0[i], hop0[i] + n_hops[i]), packed into out in list order.  Every check comes before the first launch or copy, so an
-// error changes no state.  d_scores (ewk_dense_detect): the caller reads the scores on the device after K4 and copies
-// host output itself; out may then be NULL (the scores stay in device scratch), and *d_scores receives where K4 wrote
-// them (NULL when no row has hops).
-static int dense_rows(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, const int64_t* hop0, const int32_t* n_hops,
-                      int tmpl_first, int tmpl_count, float* out, int64_t out_cap, int where, float** d_scores = nullptr) {
-    if (d_scores) *d_scores = nullptr;
-    BankView& B = ctx->bank;
-    if (n < 0 || (n > 0 && (!streams || !hop0 || !n_hops))) { ctx->fail("%s: bad row list (n=%d)", who, n); return EWK_ERR_ARG; }
-    if (n == 0) return EWK_OK;
-    std::vector<int> row_of((size_t)B.n_streams, -1);
-    long long hops = 0;
-    for (int i = 0; i < n; i++) {
-        const int s = streams[i];
-        if (s < 0 || s >= B.n_streams) { ctx->fail("%s: bad stream %d (context has %d)", who, s, B.n_streams); return EWK_ERR_ARG; }
-        if (row_of[s] >= 0) { ctx->fail("%s: stream %d is listed twice", who, s); return EWK_ERR_ARG; }
-        row_of[s] = i;
-        if (hop0[i] < 0 || n_hops[i] < 0 || hop0[i] > ((int64_t)1 << 48)) {
-            ctx->fail("%s: row %d of stream %d has bad hops (hop0=%lld n_hops=%d)", who, i, s, (long long)hop0[i], n_hops[i]);
-            return EWK_ERR_ARG;
-        }
-        hops += n_hops[i];
-    }
-    DenseArgs A{};
-    DensePlan plan;
-    int rc = dense_prepare(ctx, who, tmpl_first, tmpl_count, A, plan);
-    if (rc) return rc;
-    const long long n_out = hops * tmpl_count;
-    if (n_out > 0 && (out || !d_scores) && (!out || out_cap < n_out)) {
-        ctx->fail("%s: out holds %lld floats, the rows need %lld", who, out ? (long long)out_cap : 0LL, n_out);
-        return EWK_ERR_ARG;
-    }
-    CK(cudaSetDevice(ctx->device));
-    if (ctx->pending.valid) {
-        // as in ewk_dense_scores: the in-flight host push lands now only if a listed row reaches into its samples
-        bool need = false;
-        const std::vector<RowDesc>& prow = ctx->pending.rows;
-        for (int j = 0; !need && j < ctx->pending.n_streams; j++) {
-            const int s = prow.empty() ? ctx->pending.stream0 + j : prow[j].stream, i = row_of[s];
-            need = i >= 0 && n_hops[i] > 0 && ctx->h_written[s] < 160LL * (hop0[i] + n_hops[i] - 1);
-        }
-        if (need) { rc = ctx->flush_pending(); if (rc) return rc; }
-    }
-    for (int i = 0; i < n; i++) {
-        if (n_hops[i] == 0) continue;
-        rc = dense_resident(ctx, who, streams[i], hop0[i], n_hops[i], A.n_max);
-        if (rc) return rc;
-    }
-    if (n_out == 0) return EWK_OK;
-    // descriptors of the non-empty rows: outputs in list order, CTAs longest first so that a launch ends with short rows
-    // (EWK_DENSE_LONGEST_FIRST=0 keeps list order, to measure what the order buys)
-    const char* lf = getenv("EWK_DENSE_LONGEST_FIRST");
-    const bool longest_first = !lf || atoi(lf) != 0;
-    std::vector<DenseRow> rows;
-    long long off = 0;
-    for (int i = 0; i < n; i++) {
-        if (n_hops[i] > 0) rows.push_back(DenseRow{hop0[i], off, streams[i], n_hops[i]});
-        off += (long long)n_hops[i] * tmpl_count;
-    }
-    if (longest_first)
-        std::stable_sort(rows.begin(), rows.end(), [](const DenseRow& a, const DenseRow& b) { return a.n_hops > b.n_hops; });
-    int k = -1;
-    rc = upload_slot(ctx, ctx->h_drow, ctx->b_drow, ctx->ev_drow, ctx->ev_drow_valid, ctx->drow_idx, rows, ctx->stream, &k);
-    if (rc) return rc;
-    float* d_out = out;
-    if (where == EWK_HOST || !out) { CK(ctx->b_dense.ensure(sizeof(float) * (size_t)n_out)); d_out = (float*)ctx->b_dense.p; }
-    A.rows = (const DenseRow*)ctx->b_drow[k].p;
-    rc = dense_launch(ctx, A, plan, d_out, (int)rows.size());
-    if (rc) return rc;
-    CK(cudaEventRecord(ctx->ev_drow[k], ctx->stream));        // the slot is free once this K4 has read it
-    ctx->ev_drow_valid[k] = true;
-    if (d_scores) { *d_scores = d_out; return EWK_OK; }
-    if (where == EWK_HOST) {
-        CK(cudaMemcpyAsync(out, d_out, sizeof(float) * (size_t)n_out, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-    }
-    return EWK_OK;
-}
-
-// ---- per-row template sets: ewk_dense_scores_sets, ewk_dense_ready_sets, ewk_dense_detect_sets ----------------------
+// ---- template sets of the row calls: a table of descriptors on the device, built on first use ------------------------
 static inline int dset_key(int first, int count) { return first * DENSE_MAX_T + count - 1; }
 
 void ewk_ctx::dense_sets_forget(int slot) {
@@ -2919,57 +2846,41 @@ void ewk_ctx::dense_sets_forget(int slot) {
             if ((size_t)dset_key(f, c) < h_dset.size()) h_dset[dset_key(f, c)].valid = false;
 }
 
-struct RowSets { const int32_t* first; const int32_t* count; };   // row i: [first[i], first[i] + count[i]); NULL: own range
+// The set of each row of a row call.  uniform (the single-set entry points): [first1, first1 + count1) for every row;
+// otherwise row i's is [first[i], first[i] + count[i]), and with both arrays NULL its stream's own range.
+struct RowSets {
+    const int32_t* first;
+    const int32_t* count;
+    bool uniform;
+    int first1, count1;
+};
 
 // Row i's set -> key[i] (its index in the context's table), with every check of the set; sets not cached yet are built
-// into `fresh`, which dense_sets_commit uploads once the call has passed every check.  Messages name the row and stream.
+// into `fresh`, which dense_sets_commit uploads once the call has passed every check.  A uniform call resolves its one
+// set, and its messages name `who`; otherwise they name the row and the stream.
 static int dense_sets_resolve(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, const RowSets& rs,
                               std::vector<int>& key, std::map<int, DenseSetHost>& fresh) {
-    if (!rs.first != !rs.count) {
+    if (!rs.uniform && !rs.first != !rs.count) {
         ctx->fail("%s: template_first and template_count must both be given or both be NULL", who);
         return EWK_ERR_ARG;
     }
     if (ctx->h_dset.empty()) ctx->h_dset.resize((size_t)ctx->cfg.max_templates * DENSE_MAX_T);
     key.assign((size_t)n, -1);
     for (int i = 0; i < n; i++) {
+        if (rs.uniform && i > 0) { key[i] = key[0]; continue; }
         const int s = streams[i];
-        const int f = rs.first ? rs.first[i] : ctx->h_prm[s].template_first;
-        const int c = rs.count ? rs.count[i] : ctx->h_prm[s].template_count;
-        if (c < 1 || c > DENSE_MAX_T || f < 0 || f > ctx->cfg.max_templates - c) {
-            ctx->fail("%s: row %d (stream %d) has a bad template range [%d, %d) (1..%d templates of %d slots)", who, i, s, f,
-                      f + c, DENSE_MAX_T, ctx->cfg.max_templates);
-            return EWK_ERR_ARG;
-        }
-        key[i] = dset_key(f, c);
-        if (ctx->h_dset[key[i]].valid || fresh.count(key[i])) continue;
-        for (int k = f; k < f + c; k++) {
-            const TemplateFeat& tf = ctx->h_tmpl[k];
-            if (!tf.valid) {
-                ctx->fail("%s: row %d (stream %d): template slot %d is empty. No reference word set. Call set_reference() first.",
-                          who, i, s, k);
-                return EWK_ERR_NO_TEMPLATE;
-            }
-            if (tf.n_samples < DENSE_MIN_L || tf.n_samples > DENSE_MAX_L) {
-                ctx->fail("%s: row %d (stream %d): template %d has %lld samples; dense scoring needs %d..%d", who, i, s, k,
-                          (long long)tf.n_samples, DENSE_MIN_L, DENSE_MAX_L);
-                return EWK_ERR_ARG;
-            }
+        const int f = rs.uniform ? rs.first1 : rs.first ? rs.first[i] : ctx->h_prm[s].template_first;
+        const int c = rs.uniform ? rs.count1 : rs.count ? rs.count[i] : ctx->h_prm[s].template_count;
+        if (dense_range_ok(ctx, f, c)) {
+            key[i] = dset_key(f, c);
+            if (ctx->h_dset[key[i]].valid || fresh.count(key[i])) continue;
         }
         char w[192];
         snprintf(w, sizeof w, "%s: row %d (stream %d)", who, i, s);
-        DenseArgs A{};
-        DensePlan plan;
-        const int rc = dense_prepare(ctx, w, f, c, A, plan);
+        DenseSetHost e;
+        const int rc = dense_set_build(ctx, rs.uniform ? who : w, f, c, e);
         if (rc) return rc;
-        DenseSetHost& e = fresh[key[i]];
-        e.DH = plan.DH; e.threads = plan.threads; e.per_sm = plan.per_sm; e.smem = plan.smem;
-        DenseSetDev& d = e.dev;
-        d.T = A.T; d.DG = A.DG; d.DLE = A.DLE; d.n_re_u = A.n_re_u; d.n_min = A.n_min; d.n_max = A.n_max;
-        d.g_back = A.g_back; d.slot0 = f;
-        std::memcpy(d.re_goff, A.re_goff, sizeof d.re_goff); std::memcpy(d.re_delta, A.re_delta, sizeof d.re_delta);
-        std::memcpy(d.re_rep, A.re_rep, sizeof d.re_rep); std::memcpy(d.re_rep_e, A.re_rep_e, sizeof d.re_rep_e);
-        std::memcpy(d.re_nfirst, A.re_nfirst, sizeof d.re_nfirst);
-        std::memcpy(d.t, A.t, sizeof d.t);
+        fresh[key[i]] = e;
     }
     return EWK_OK;
 }
@@ -3000,12 +2911,18 @@ static int dense_sets_commit(ewk_ctx* ctx, const std::map<int, DenseSetHost>& fr
     return EWK_OK;
 }
 
-// dense_rows with a template set per row: row i is packed from float sum_{j < i} n_hops[j] T_j, laid out [n_hops[i]][T_i].
-// One K4 launch per launch geometry (DH, threads, CTAs per SM) among the rows' sets, each set at the geometry it has
-// alone; the launch gets its group's largest shared memory and g2 stride.  *keys (when given) receives each row's key.
-static int dense_rows_sets(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, const int64_t* hop0,
-                           const int32_t* n_hops, const RowSets& rs, float* out, int64_t out_cap, int where,
-                           float** d_scores = nullptr, std::vector<int>* keys = nullptr) {
+// Rows of ewk_dense_scores_streams, ewk_dense_ready, ewk_dense_detect and their _sets forms: row i scores stream
+// streams[i] at hops [hop0[i], hop0[i] + n_hops[i]) against its set (rs), packed from float sum_{j < i} n_hops[j] T_j and
+// laid out [n_hops[i]][T_i].  One K4 launch per launch geometry (DH, threads, CTAs per SM) among the rows' sets, each set
+// at the geometry it has alone; the launch gets its group's largest shared memory and g2 stride, and runs its rows longest
+// first so that it ends with short ones.  A group whose rows all share one set (every group of a single-set call) runs
+// K4's one-set row instance with that set in its arguments, a group of several sets the per-row-set instance.  Every check comes before the first launch or copy, so an error changes no state.
+// d_scores (the detect calls): the caller reads the scores on the device after K4 and copies host output itself; out may
+// then be NULL (the scores stay in device scratch), and *d_scores receives where K4 wrote them (NULL when no row has
+// hops).  *keys (when given) receives each row's key.
+static int dense_rows(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, const int64_t* hop0,
+                      const int32_t* n_hops, const RowSets& rs, float* out, int64_t out_cap, int where,
+                      float** d_scores = nullptr, std::vector<int>* keys = nullptr) {
     if (d_scores) *d_scores = nullptr;
     BankView& B = ctx->bank;
     if (n < 0 || (n > 0 && (!streams || !hop0 || !n_hops))) { ctx->fail("%s: bad row list (n=%d)", who, n); return EWK_ERR_ARG; }
@@ -3026,6 +2943,7 @@ static int dense_rows_sets(ewk_ctx* ctx, const char* who, const int32_t* streams
     int rc = dense_sets_resolve(ctx, who, streams, n, rs, key, fresh);
     if (rc) return rc;
     auto set_of = [&](int i) -> const DenseSetHost& {
+        if (fresh.empty()) return ctx->h_dset[key[i]];
         const auto it = fresh.find(key[i]);
         return it != fresh.end() ? it->second : ctx->h_dset[key[i]];
     };
@@ -3036,16 +2954,11 @@ static int dense_rows_sets(ewk_ctx* ctx, const char* who, const int32_t* streams
         return EWK_ERR_ARG;
     }
     CK(cudaSetDevice(ctx->device));
-    if (ctx->pending.valid) {
-        // as in ewk_dense_scores: the in-flight host push lands now only if a listed row reaches into its samples
-        bool need = false;
-        const std::vector<RowDesc>& prow = ctx->pending.rows;
-        for (int j = 0; !need && j < ctx->pending.n_streams; j++) {
-            const int s = prow.empty() ? ctx->pending.stream0 + j : prow[j].stream, i = row_of[s];
-            need = i >= 0 && n_hops[i] > 0 && ctx->h_written[s] < 160LL * (hop0[i] + n_hops[i] - 1);
-        }
-        if (need) { rc = ctx->flush_pending(); if (rc) return rc; }
-    }
+    rc = dense_land_if_reached(ctx, [&](int s) {
+        const int i = row_of[s];
+        return i >= 0 && n_hops[i] > 0 ? (long long)hop0[i] + n_hops[i] - 1 : -1LL;
+    });
+    if (rc) return rc;
     for (int i = 0; i < n; i++) {
         if (n_hops[i] == 0) continue;
         rc = dense_resident(ctx, who, streams[i], hop0[i], n_hops[i], set_of(i).dev.n_max);
@@ -3055,36 +2968,43 @@ static int dense_rows_sets(ewk_ctx* ctx, const char* who, const int32_t* streams
     if (n_out == 0) return EWK_OK;
     rc = dense_sets_commit(ctx, fresh);
     if (rc) return rc;
-    // geometry groups in order of first appearance; within a group the longest rows first, as in dense_rows
-    struct Group { DensePlan plan; int DG; std::vector<DenseRowSet> rows; };
+    // geometry groups in order of first appearance
+    struct Group { DensePlan plan; int DG, key; size_t n_rows; };   // key: the rows' one set, -1: several
     std::vector<Group> groups;
-    const DenseSetDev* tab = (const DenseSetDev*)ctx->b_dset.p;
-    long long off = 0;
+    std::vector<unsigned char> group_of((size_t)n);
+    size_t n_rows = 0;
     int max_dg = 0;
     for (int i = 0; i < n; i++) {
+        if (n_hops[i] == 0) continue;
         const DenseSetHost& e = ctx->h_dset[key[i]];
-        if (n_hops[i] > 0) {
-            size_t g = 0;
-            while (g < groups.size() && !(groups[g].plan.DH == e.DH && groups[g].plan.threads == e.threads &&
-                                          groups[g].plan.per_sm == e.per_sm)) g++;
-            if (g == groups.size()) groups.push_back(Group{DensePlan{e.DH, e.threads, e.per_sm, 0}, 0, {}});
-            groups[g].plan.smem = std::max(groups[g].plan.smem, e.smem);
-            groups[g].DG = std::max(groups[g].DG, e.dev.DG);
-            groups[g].rows.push_back(DenseRowSet{DenseRow{hop0[i], off, streams[i], n_hops[i]}, tab + key[i]});
-            max_dg = std::max(max_dg, e.dev.DG);
+        size_t g = 0;
+        while (g < groups.size() && !(groups[g].plan.DH == e.plan.DH && groups[g].plan.threads == e.plan.threads &&
+                                      groups[g].plan.per_sm == e.plan.per_sm)) g++;
+        if (g == groups.size()) groups.push_back(Group{DensePlan{e.plan.DH, e.plan.threads, e.plan.per_sm, 0}, 0, key[i], 0});
+        if (groups[g].key != key[i]) groups[g].key = -1;
+        groups[g].plan.smem = std::max(groups[g].plan.smem, e.plan.smem);
+        groups[g].DG = std::max(groups[g].DG, e.dev.DG);
+        groups[g].n_rows++;
+        group_of[i] = (unsigned char)g;
+        max_dg = std::max(max_dg, e.dev.DG);
+        n_rows++;
+    }
+    // the descriptors group by group, each group's rows longest first
+    const DenseSetDev* tab = (const DenseSetDev*)ctx->b_dset.p;
+    std::vector<DenseRow> rows;
+    rows.reserve(n_rows);
+    for (size_t g = 0; g < groups.size(); g++) {
+        const size_t first = rows.size();
+        long long off = 0;
+        for (int i = 0; i < n; i++) {
+            if (n_hops[i] > 0 && group_of[i] == g) rows.push_back(DenseRow{hop0[i], off, streams[i], n_hops[i], tab + key[i]});
+            off += (long long)n_hops[i] * ctx->h_dset[key[i]].dev.T;
         }
-        off += (long long)n_hops[i] * e.dev.T;
+        auto longer = [](const DenseRow& a, const DenseRow& b) { return a.n_hops > b.n_hops; };
+        if (!std::is_sorted(rows.begin() + first, rows.end(), longer))     // paced calls often give every row max_hops
+            std::stable_sort(rows.begin() + first, rows.end(), longer);
     }
-    const char* lf = getenv("EWK_DENSE_LONGEST_FIRST");
-    const bool longest_first = !lf || atoi(lf) != 0;
-    std::vector<DenseRowSet> rows;
-    for (Group& g : groups) {
-        if (longest_first)
-            std::stable_sort(g.rows.begin(), g.rows.end(),
-                             [](const DenseRowSet& a, const DenseRowSet& b) { return a.r.n_hops > b.r.n_hops; });
-        rows.insert(rows.end(), g.rows.begin(), g.rows.end());
-    }
-    SlotPair<DenseRowSet>& sp = ctx->drow_sets;
+    SlotPair<DenseRow>& sp = ctx->drows;
     int k = -1;
     rc = upload_slot(ctx, sp.h, sp.b, sp.ev, sp.ev_valid, sp.idx, rows, ctx->stream, &k);
     if (rc) return rc;
@@ -3096,10 +3016,11 @@ static int dense_rows_sets(ewk_ctx* ctx, const char* who, const int32_t* streams
         DenseArgs A{};
         A.DH = g.plan.DH;
         A.DG = g.DG;
-        A.rows = (const DenseRow*)((const DenseRowSet*)sp.b[k].p + base);
-        rc = dense_launch(ctx, A, g.plan, d_out, (int)g.rows.size(), true);
+        if (g.key >= 0) A.set = ctx->h_dset[g.key].dev;
+        A.rows = (const DenseRow*)sp.b[k].p + base;
+        rc = dense_launch(ctx, A, g.plan, d_out, (int)g.n_rows, g.key >= 0);
         if (rc) return rc;
-        base += g.rows.size();
+        base += g.n_rows;
     }
     CK(cudaEventRecord(sp.ev[k], ctx->stream));               // the slot is free once these K4 launches have read it
     sp.ev_valid[k] = true;
@@ -3117,8 +3038,8 @@ extern "C" int ewk_dense_scores_sets(ewk_ctx* ctx, const int32_t* streams, int n
     if (!ctx) return EWK_ERR_ARG;
     int rc = need_streams(ctx, "ewk_dense_scores_sets");
     if (rc) return rc;
-    return dense_rows_sets(ctx, "ewk_dense_scores_sets", streams, n, hop0, n_hops, RowSets{template_first, template_count},
-                           out, out_cap, where);
+    return dense_rows(ctx, "ewk_dense_scores_sets", streams, n, hop0, n_hops, RowSets{template_first, template_count, false, 0, 0},
+                      out, out_cap, where);
 }
 
 extern "C" int ewk_dense_scores_streams(ewk_ctx* ctx, const int32_t* streams, int n, const int64_t* hop0, const int32_t* n_hops,
@@ -3126,53 +3047,63 @@ extern "C" int ewk_dense_scores_streams(ewk_ctx* ctx, const int32_t* streams, in
     if (!ctx) return EWK_ERR_ARG;
     int rc = need_streams(ctx, "ewk_dense_scores_streams");
     if (rc) return rc;
-    return dense_rows(ctx, "ewk_dense_scores_streams", streams, n, hop0, n_hops, template_first, template_count, out, out_cap,
-                      where);
+    return dense_rows(ctx, "ewk_dense_scores_streams", streams, n, hop0, n_hops,
+                      RowSets{nullptr, nullptr, true, template_first, template_count}, out, out_cap, where);
 }
 
-// ewk_dense_ready (rs = NULL: the call's one set [template_first, template_first + template_count)) and
-// ewk_dense_ready_sets (rs: a set per row)
-static int dense_ready_impl(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, int max_hops, int template_first,
-                            int template_count, const RowSets* rs, int64_t* hop0_out, int32_t* n_hops_out, float* out,
-                            int64_t out_cap, int where) {
+// The rows a paced call (ewk_dense_ready, ewk_dense_detect and their _sets forms) scores: max_hops is checked, NULL streams
+// means every stream, the list is checked (outs: the caller's per-row outputs are given); then the pending push lands,
+// since the due hops depend on every landed sample, and the due rule runs on `cursor`: hop h is due once 160 h samples
+// have landed, from the cursor on, at most max_hops.
+struct DueRows {
+    std::vector<int32_t> streams;
+    std::vector<int64_t> h0;
+    std::vector<int32_t> nh;
+};
+
+static int dense_due(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, int max_hops, bool outs,
+                     const std::vector<long long>& cursor, DueRows& d) {
+    const int ns = ctx->bank.n_streams;
+    if (max_hops < 1 || max_hops > (1 << 20)) { ctx->fail("%s: max_hops must be in [1, %d]", who, 1 << 20); return EWK_ERR_ARG; }
+    if (!streams) {
+        d.streams.resize((size_t)ns);
+        for (int s = 0; s < ns; s++) d.streams[s] = s;
+        streams = d.streams.data();
+        n = ns;
+    }
+    if (n > 0 && !outs) { ctx->fail("%s: bad stream list (n=%d)", who, n); return EWK_ERR_ARG; }
+    int rc = check_stream_list(ctx, who, streams, n);
+    if (rc) return rc;
+    d.streams.assign(streams, streams + n);
+    CK(cudaSetDevice(ctx->device));
+    rc = ctx->flush_pending();
+    if (rc) return rc;
+    d.h0.resize((size_t)n);
+    d.nh.resize((size_t)n);
+    for (int i = 0; i < n; i++) {
+        const int s = streams[i];
+        d.h0[i] = cursor[s];
+        d.nh[i] = (int32_t)std::max<long long>(0, std::min<long long>(d.h0[i] + max_hops, ctx->h_written[s] / 160 + 1) - d.h0[i]);
+    }
+    return EWK_OK;
+}
+
+// ewk_dense_ready and ewk_dense_ready_sets
+static int dense_ready_impl(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, int max_hops, const RowSets& rs,
+                            int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where) {
     if (!ctx) return EWK_ERR_ARG;
     int rc = need_streams(ctx, who);
     if (rc) return rc;
-    BankView& B = ctx->bank;
-    if (max_hops < 1 || max_hops > (1 << 20)) { ctx->fail("%s: max_hops must be in [1, %d]", who, 1 << 20); return EWK_ERR_ARG; }
-    std::vector<int32_t> all;
-    if (!streams) {
-        all.resize((size_t)B.n_streams);
-        for (int s = 0; s < B.n_streams; s++) all[s] = s;
-        streams = all.data();
-        n = B.n_streams;
-    }
-    if (n < 0 || (n > 0 && (!hop0_out || !n_hops_out))) { ctx->fail("%s: bad stream list (n=%d)", who, n); return EWK_ERR_ARG; }
-    std::vector<char> seen((size_t)B.n_streams, 0);
-    for (int i = 0; i < n; i++) {
-        const int s = streams[i];
-        if (s < 0 || s >= B.n_streams) { ctx->fail("%s: bad stream %d (context has %d)", who, s, B.n_streams); return EWK_ERR_ARG; }
-        if (seen[s]) { ctx->fail("%s: stream %d is listed twice", who, s); return EWK_ERR_ARG; }
-        seen[s] = 1;
-    }
-    CK(cudaSetDevice(ctx->device));
-    rc = ctx->flush_pending();                               // the due hops depend on every landed sample
+    DueRows d;
+    rc = dense_due(ctx, who, streams, n, max_hops, hop0_out && n_hops_out, ctx->h_dense_next, d);
     if (rc) return rc;
-    // due rule: hop h is due once 160 h samples have landed, from the cursor on, at most max_hops
-    std::vector<int64_t> h0((size_t)n);
-    std::vector<int32_t> nh((size_t)n);
-    for (int i = 0; i < n; i++) {
-        const int s = streams[i];
-        h0[i] = ctx->h_dense_next[s];
-        nh[i] = (int32_t)std::max<long long>(0, std::min<long long>(h0[i] + max_hops, ctx->h_written[s] / 160 + 1) - h0[i]);
-    }
-    rc = rs ? dense_rows_sets(ctx, who, streams, n, h0.data(), nh.data(), *rs, out, out_cap, where)
-            : dense_rows(ctx, who, streams, n, h0.data(), nh.data(), template_first, template_count, out, out_cap, where);
+    n = (int)d.streams.size();
+    rc = dense_rows(ctx, who, d.streams.data(), n, d.h0.data(), d.nh.data(), rs, out, out_cap, where);
     if (rc) return rc;
     for (int i = 0; i < n; i++) {
-        hop0_out[i] = h0[i];
-        n_hops_out[i] = nh[i];
-        ctx->h_dense_next[streams[i]] += nh[i];
+        hop0_out[i] = d.h0[i];
+        n_hops_out[i] = d.nh[i];
+        ctx->h_dense_next[d.streams[i]] += d.nh[i];
     }
     return EWK_OK;
 }
@@ -3180,62 +3111,42 @@ static int dense_ready_impl(ewk_ctx* ctx, const char* who, const int32_t* stream
 extern "C" int ewk_dense_ready(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first,
                                int template_count, int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap,
                                int where) {
-    return dense_ready_impl(ctx, "ewk_dense_ready", streams, n, max_hops, template_first, template_count, nullptr, hop0_out,
-                            n_hops_out, out, out_cap, where);
+    return dense_ready_impl(ctx, "ewk_dense_ready", streams, n, max_hops,
+                            RowSets{nullptr, nullptr, true, template_first, template_count}, hop0_out, n_hops_out, out,
+                            out_cap, where);
 }
 
 extern "C" int ewk_dense_ready_sets(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, const int32_t* template_first,
                                     const int32_t* template_count, int64_t* hop0_out, int32_t* n_hops_out, float* out,
                                     int64_t out_cap, int where) {
-    const RowSets rs{template_first, template_count};
-    return dense_ready_impl(ctx, "ewk_dense_ready_sets", streams, n, max_hops, 0, 0, &rs, hop0_out, n_hops_out, out, out_cap,
-                            where);
+    return dense_ready_impl(ctx, "ewk_dense_ready_sets", streams, n, max_hops,
+                            RowSets{template_first, template_count, false, 0, 0}, hop0_out, n_hops_out, out, out_cap, where);
 }
 
 static_assert(sizeof(DetRecord) == sizeof(ewk_detection) && sizeof(ewk_detection) == 48, "ewk_detection layout");
 static_assert(offsetof(DetRecord, score) == offsetof(ewk_detection, score), "ewk_detection layout");
 
-// ewk_dense_ready's due rule on the detector's own cursor, then K4 (per-row) and K4D behind it on the context's stream.
-// rs = NULL: ewk_dense_detect's one set; rs: ewk_dense_detect_sets, a set per row (K4 per geometry, K4D's set form)
-static int dense_detect_impl(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, int max_hops, int template_first,
-                             int template_count, const RowSets* rs, int hold_hops, int refractory_hops, ewk_detection* det,
-                             int det_cap, int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where) {
+// ewk_dense_detect and ewk_dense_detect_sets: ewk_dense_ready's due rule on the detector's own cursor, then K4 (one launch
+// per geometry) and K4D behind it on the context's stream.
+static int dense_detect_impl(ewk_ctx* ctx, const char* who, const int32_t* streams, int n, int max_hops, const RowSets& rs,
+                             int hold_hops, int refractory_hops, ewk_detection* det, int det_cap, int64_t* hop0_out,
+                             int32_t* n_hops_out, float* out, int64_t out_cap, int where) {
     if (!ctx) return EWK_ERR_ARG;
     int rc = need_streams(ctx, who);
     if (rc) return rc;
     BankView& B = ctx->bank;
-    if (max_hops < 1 || max_hops > (1 << 20)) { ctx->fail("%s: max_hops must be in [1, %d]", who, 1 << 20); return EWK_ERR_ARG; }
     if (hold_hops < 1 || refractory_hops < 0) {
         ctx->fail("%s: hold_hops must be >= 1 and refractory_hops >= 0 (got %d, %d)", who, hold_hops, refractory_hops);
         return EWK_ERR_ARG;
     }
-    std::vector<int32_t> all;
-    if (!streams) {
-        all.resize((size_t)B.n_streams);
-        for (int s = 0; s < B.n_streams; s++) all[s] = s;
-        streams = all.data();
-        n = B.n_streams;
-    }
-    if (n < 0) { ctx->fail("%s: bad stream list (n=%d)", who, n); return EWK_ERR_ARG; }
-    std::vector<char> seen((size_t)B.n_streams, 0);
-    for (int i = 0; i < n; i++) {
-        const int s = streams[i];
-        if (s < 0 || s >= B.n_streams) { ctx->fail("%s: bad stream %d (context has %d)", who, s, B.n_streams); return EWK_ERR_ARG; }
-        if (seen[s]) { ctx->fail("%s: stream %d is listed twice", who, s); return EWK_ERR_ARG; }
-        seen[s] = 1;
-    }
-    CK(cudaSetDevice(ctx->device));
-    rc = ctx->flush_pending();                               // the due hops depend on every landed sample
+    DueRows d;
+    rc = dense_due(ctx, who, streams, n, max_hops, true, ctx->h_det_next, d);
     if (rc) return rc;
-    std::vector<int64_t> h0((size_t)n);
-    std::vector<int32_t> nh((size_t)n);
+    n = (int)d.streams.size();
+    const std::vector<int64_t>& h0 = d.h0;
+    const std::vector<int32_t>& nh = d.nh;
     long long need = 0;                                      // emissions are >= 2 hops apart: ceil(n_i / 2) per row
-    for (int i = 0; i < n; i++) {
-        const int s = streams[i];
-        h0[i] = ctx->h_det_next[s];
-        nh[i] = (int32_t)std::max<long long>(0, std::min<long long>(h0[i] + max_hops, ctx->h_written[s] / 160 + 1) - h0[i]);
-        need += (nh[i] + 1) / 2;
-    }
+    for (int i = 0; i < n; i++) need += (nh[i] + 1) / 2;
     if (det_cap < need || (need > 0 && !det)) {
         ctx->fail("%s: det holds %d records, the due hops need %lld", who, det ? det_cap : 0, need);
         return EWK_ERR_ARG;
@@ -3253,9 +3164,7 @@ static int dense_detect_impl(ewk_ctx* ctx, const char* who, const int32_t* strea
     }
     float* d_scores = nullptr;
     std::vector<int> keys;
-    rc = rs ? dense_rows_sets(ctx, who, streams, n, h0.data(), nh.data(), *rs, out, out_cap, where, &d_scores, &keys)
-            : dense_rows(ctx, who, streams, n, h0.data(), nh.data(), template_first, template_count, out, out_cap, where,
-                         &d_scores);
+    rc = dense_rows(ctx, who, d.streams.data(), n, h0.data(), nh.data(), rs, out, out_cap, where, &d_scores, &keys);
     if (rc) return rc;
     int n_det = 0;
     if (d_scores) {
@@ -3264,43 +3173,31 @@ static int dense_detect_impl(ewk_ctx* ctx, const char* who, const int32_t* strea
             CK(cudaMemsetAsync(ctx->b_det_state.p, 0, sizeof(DetState) * (size_t)B.n_streams, ctx->stream));
         }
         std::vector<DetRow> rows;
-        std::vector<DetRowSet> srows;                         // rs: the same rows with their sets
+        rows.reserve((size_t)n);
         long long off = 0, doff = 0;
         for (int i = 0; i < n; i++) {
-            if (nh[i] > 0) {
-                rows.push_back(DetRow{h0[i], off, doff, streams[i], nh[i], i, 0});
-                if (rs) srows.push_back(DetRowSet{rows.back(), (const DenseSetDev*)ctx->b_dset.p + keys[i]});
-            }
-            off += (long long)nh[i] * (rs ? ctx->h_dset[keys[i]].dev.T : template_count);
+            if (nh[i] > 0) rows.push_back(DetRow{h0[i], off, doff, d.streams[i], nh[i], i, 0, (const DenseSetDev*)ctx->b_dset.p + keys[i]});
+            off += (long long)nh[i] * ctx->h_dset[keys[i]].dev.T;
             doff += (nh[i] + 1) / 2;
         }
+        SlotPair<DetRow>& sp = ctx->ddets;
         int k = -1;
-        SlotPair<DetRowSet>& sp = ctx->ddet_sets;
-        rc = rs ? upload_slot(ctx, sp.h, sp.b, sp.ev, sp.ev_valid, sp.idx, srows, ctx->stream, &k)
-                : upload_slot(ctx, ctx->h_ddet, ctx->b_ddet, ctx->ev_ddet, ctx->ev_ddet_valid, ctx->ddet_idx, rows, ctx->stream, &k);
+        rc = upload_slot(ctx, sp.h, sp.b, sp.ev, sp.ev_valid, sp.idx, rows, ctx->stream, &k);
         if (rc) return rc;
         char* d_map = nullptr;
         CK(cudaHostGetDevicePointer((void**)&d_map, ctx->h_det_map, 0));
         DetArgs D{};
         D.hold = hold_hops; D.refractory = refractory_hops;
-        if (!rs) {
-            D.T = template_count; D.slot0 = template_first;
-            for (int t = 0; t < template_count; t++) {
-                const int L = (int)ctx->h_tmpl[template_first + t].n_samples;
-                D.L[t] = L; D.n[t] = (L + HOP - 1) / HOP;
-            }
-        }
-        D.rows = (const DetRow*)(rs ? sp.b[k].p : ctx->b_ddet[k].p); D.n_rows = (int)rows.size();
+        D.rows = (const DetRow*)sp.b[k].p; D.n_rows = (int)rows.size();
         D.scores = d_scores; D.state = (DetState*)ctx->b_det_state.p;
         D.counts = (int*)d_map; D.rec = (DetRecord*)(d_map + rec_off);
         cudaEvent_t pe = ctx->prof_begin(4);
-        (rs ? dense_detect_kernel<true> : dense_detect_kernel<false>)
-            <<<(D.n_rows + DETECT_WARPS - 1) / DETECT_WARPS, 32 * DETECT_WARPS, 0, ctx->stream>>>(B.prm, D);
+        dense_detect_kernel<<<(D.n_rows + DETECT_WARPS - 1) / DETECT_WARPS, 32 * DETECT_WARPS, 0, ctx->stream>>>(B.prm, D);
         ctx->prof_end(pe, 4);
         CK(cudaGetLastError());
         ctx->launches++;
-        CK(cudaEventRecord(rs ? sp.ev[k] : ctx->ev_ddet[k], ctx->stream));
-        (rs ? sp.ev_valid[k] : ctx->ev_ddet_valid[k]) = true;
+        CK(cudaEventRecord(sp.ev[k], ctx->stream));
+        sp.ev_valid[k] = true;
         if (out && where == EWK_HOST)
             CK(cudaMemcpyAsync(out, d_scores, sizeof(float) * (size_t)off, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
@@ -3315,7 +3212,7 @@ static int dense_detect_impl(ewk_ctx* ctx, const char* who, const int32_t* strea
     for (int i = 0; i < n; i++) {
         if (hop0_out) hop0_out[i] = h0[i];
         if (n_hops_out) n_hops_out[i] = nh[i];
-        ctx->h_det_next[streams[i]] += nh[i];
+        ctx->h_det_next[d.streams[i]] += nh[i];
     }
     return n_det;
 }
@@ -3323,17 +3220,18 @@ static int dense_detect_impl(ewk_ctx* ctx, const char* who, const int32_t* strea
 extern "C" int ewk_dense_detect(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, int template_first,
                                 int template_count, int hold_hops, int refractory_hops, ewk_detection* det, int det_cap,
                                 int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap, int where) {
-    return dense_detect_impl(ctx, "ewk_dense_detect", streams, n, max_hops, template_first, template_count, nullptr,
-                             hold_hops, refractory_hops, det, det_cap, hop0_out, n_hops_out, out, out_cap, where);
+    return dense_detect_impl(ctx, "ewk_dense_detect", streams, n, max_hops,
+                             RowSets{nullptr, nullptr, true, template_first, template_count}, hold_hops, refractory_hops,
+                             det, det_cap, hop0_out, n_hops_out, out, out_cap, where);
 }
 
 extern "C" int ewk_dense_detect_sets(ewk_ctx* ctx, const int32_t* streams, int n, int max_hops, const int32_t* template_first,
                                      const int32_t* template_count, int hold_hops, int refractory_hops, ewk_detection* det,
                                      int det_cap, int64_t* hop0_out, int32_t* n_hops_out, float* out, int64_t out_cap,
                                      int where) {
-    const RowSets rs{template_first, template_count};
-    return dense_detect_impl(ctx, "ewk_dense_detect_sets", streams, n, max_hops, 0, 0, &rs, hold_hops, refractory_hops, det,
-                             det_cap, hop0_out, n_hops_out, out, out_cap, where);
+    return dense_detect_impl(ctx, "ewk_dense_detect_sets", streams, n, max_hops,
+                             RowSets{template_first, template_count, false, 0, 0}, hold_hops, refractory_hops, det, det_cap,
+                             hop0_out, n_hops_out, out, out_cap, where);
 }
 
 extern "C" int ewk_stream_results(ewk_ctx* ctx, ewk_stream_result* out) {

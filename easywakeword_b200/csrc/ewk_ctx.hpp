@@ -86,11 +86,13 @@ struct SlotPair {
     }
 };
 
+// Launch geometry of K4 for a template set: hops per sub-chunk, threads per CTA and CTAs per SM that fit shared memory.
+struct DensePlan { int DH, threads, per_sm; size_t smem; };
+
 // A template set's descriptor for K4 / K4D (valid: built and on the device) and the launch geometry it has alone
 struct DenseSetHost {
     bool valid = false;
-    int DH = 0, threads = 0, per_sm = 0;
-    size_t smem = 0;
+    DensePlan plan{};
     DenseSetDev dev{};
 };
 
@@ -147,27 +149,15 @@ struct ewk_ctx {
     cudaEvent_t ev_pos[2] = {nullptr, nullptr};
     bool ev_pos_valid[2] = {false, false};
     int pos_idx = 0;
-    // per-row descriptors of a ragged K4 call (ewk_dense_scores_streams, ewk_dense_ready): two slots of the same kind
-    ewk::DenseRow* h_drow[2] = {nullptr, nullptr};
-    ewk::DevBuf b_drow[2]{{&pool, "b_drow", false}, {&pool, "b_drow", false}};
-    cudaEvent_t ev_drow[2] = {nullptr, nullptr};
-    bool ev_drow_valid[2] = {false, false};
-    int drow_idx = 0;
-    // per-row descriptors of K4D (ewk_dense_detect): two slots of the same kind
-    ewk::DetRow* h_ddet[2] = {nullptr, nullptr};
-    ewk::DevBuf b_ddet[2]{{&pool, "b_ddet", false}, {&pool, "b_ddet", false}};
-    cudaEvent_t ev_ddet[2] = {nullptr, nullptr};
-    bool ev_ddet_valid[2] = {false, false};
-    int ddet_idx = 0;
     ewk::DevBuf b_det_state{&pool, "b_det_state", false};                 // K4D's DetState [n_streams], allocated (zeroed) by the first detect call
-    // per-row template sets (ewk_dense_*_sets): the descriptor of set [first, first + count) sits at index
+    // the template sets of K4 row calls and K4D: the descriptor of set [first, first + count) sits at index
     // first * DENSE_MAX_T + count - 1 of a device table; h_dset mirrors it.  A set is built and uploaded on first use and
     // kept until a template slot of its range changes (dense_sets_forget).  New descriptors go through dset_stage.
     std::vector<ewk::DenseSetHost> h_dset;
     ewk::DevBuf b_dset{&pool, "b_dset", false};
     ewk::SlotPair<ewk::DenseSetDev> dset_stage{&pool, "dset_stage"};
-    ewk::SlotPair<ewk::DenseRowSet> drow_sets{&pool, "drow_sets"};   // K4 row descriptors of a per-row-set call
-    ewk::SlotPair<ewk::DetRowSet> ddet_sets{&pool, "ddet_sets"};     // K4D row descriptors of ewk_dense_detect_sets
+    ewk::SlotPair<ewk::DenseRow> drows{&pool, "drows"};   // K4 row descriptors of a row call
+    ewk::SlotPair<ewk::DetRow> ddets{&pool, "ddets"};     // K4D row descriptors
     void dense_sets_forget(int slot);
     // K4D's output, pinned and mapped into the device: per-row record counts [n_streams], then records (row i at its offset)
     void* h_det_map = nullptr;

@@ -74,32 +74,12 @@ struct DenseTmplDev {
     double inv_f;                      // 1 / F (IEEE double division: the same bits on host and device)
 };
 
-// One row of a ragged call (ewk_dense_scores_streams / ewk_dense_ready): CTA x scores stream `stream` at hops
-// [hop0, hop0 + n_hops) into out[out, out + n_hops T), laid out [n_hops][T]
-struct DenseRow {
-    long long hop0, out;
-    int stream, n_hops;
-};
-
-// The template-dependent part of DenseArgs for one template set [slot0, slot0 + T) (fields as there).  The context
-// keeps a table of them (ewk_dense_*_sets); a SETS-instance CTA takes its set from its row descriptor.
+// The template-dependent part of K4's arguments for one template set [slot0, slot0 + T).  The context keeps a table of
+// them; a per-row-set CTA takes its set from its row descriptor, the other instances from DenseArgs (whose layout the
+// order of these fields serves, see there).
 struct DenseSetDev {
-    int T, DG, DLE, n_re_u, n_min, n_max, g_back, slot0;
-    int re_goff[DENSE_MAX_RE], re_delta[DENSE_MAX_RE], re_rep[DENSE_MAX_RE], re_rep_e[DENSE_MAX_RE], re_nfirst[DENSE_MAX_RE];
-    DenseTmplDev t[DENSE_MAX_T];
-};
-
-// A row of a per-row-set call: the row and its set in the context's table
-struct DenseRowSet {
-    DenseRow r;
-    const DenseSetDev* set;
-};
-
-struct DenseArgs {
-    long long hop0;                    // first hop scored (hop h <-> 160 h samples of the stream); uniform instance only
-    int n_hops;
-    int T;
-    int DH;                            // hops per sub-chunk (32 or 64)
+    int slot0, T;
+    int DH;                            // hops per sub-chunk (32 or 64) of the geometry the set has alone
     int DG;                            // rows of the grid-frame ring (>= DH + n_max + 2)
     int DLE;                           // starts held by the left-edge rings (>= DH + n_max - n_min)
     int n_re_u;                        // distinct right-edge frames per hop
@@ -110,10 +90,30 @@ struct DenseArgs {
     // a template and edge index that use it (window view of the generic loader); n_first: the shortest window using it
     int re_goff[DENSE_MAX_RE], re_delta[DENSE_MAX_RE], re_rep[DENSE_MAX_RE], re_rep_e[DENSE_MAX_RE], re_nfirst[DENSE_MAX_RE];
     DenseTmplDev t[DENSE_MAX_T];
+};
+
+// One row of a row call (ewk_dense_scores_streams, ewk_dense_ready, ewk_dense_detect and their _sets forms): CTA x scores
+// stream `stream` at hops [hop0, hop0 + n_hops) against `set` (in the context's table) into out[out, out + n_hops T), laid
+// out [n_hops][T]
+struct DenseRow {
+    long long hop0, out;
+    int stream, n_hops;
+    const DenseSetDev* set;
+};
+
+// The uniform instance reads its hops and set from here, the one-set row instance its set.  hop0 and set lead: at these
+// parameter offsets those instances (the uniform one is bench.py's dense path) compile to their fewest spills; other
+// orders of the same fields spill up to 24 bytes more.
+struct DenseArgs {
+    long long hop0;                    // uniform instance: first hop scored (hop h <-> 160 h samples of the stream)
+    DenseSetDev set;                   // uniform and one-set row instances: the launch's template set
+    int n_hops;                        // uniform instance
+    int DH;                            // per-row-set instance: hops per sub-chunk of the launch (that of each of its sets)
+    int DG;                            // per-row-set instance: the g2 stride, the largest DG of the launch's sets
     float* out;                        // uniform: [n_streams][n_hops][T]; rows: packed as their descriptors say
-    const DenseRow* rows;              // ROWS instance: one descriptor per CTA (SETS instance: DenseRowSet descriptors)
+    const DenseRow* rows;              // row instance: one descriptor per CTA
     float* g2;                         // [n_streams][DENSE_WAYS][DG][20]: grid rows floored with a way's floor (tags in shared memory);
-                                       // SETS instance: streams DG (the launch's largest) apart, a set's own DG within
+                                       // streams DG apart (per-row-set instance: A.DG), a set's own DG within
     // carry-over between consecutive calls: the newest stream-grid rows of every stream (functions of the PCM only)
     float* keep_rows;                  // [n_streams][DENSE_KEEP][ROW], row of grid frame g at g % DENSE_KEEP
     long long* keep_end;               // [n_streams][2]: grid frames [keep_end[2s], keep_end[2s+1]) are stored (0, 0: nothing)
@@ -263,24 +263,20 @@ __device__ __forceinline__ int next_task(int* counter, int lane) {
 
 __device__ __forceinline__ int wrap1(int r, int n) { return r >= n ? r - n : r; }
 
-// ROWS = false: CTA s scores stream s at the call's hops [A.hop0, A.hop0 + A.n_hops).  ROWS = true: CTA x takes
-// descriptor A.rows[x] (its stream, hop range and output block); the body is the same.  SETS = true (with ROWS): the
-// descriptors are DenseRowSet, and each CTA takes the template-dependent fields (T, DG, DLE, n_re_u, n_min, n_max,
-// g_back, re_*, t[]) from its row's set instead of A; A.DH is the launch's, A.DG the g2 stride.
-template <bool PRE, bool ROWS, bool SETS = false>
+// ROWS = false: CTA s scores stream s at the call's hops [A.hop0, A.hop0 + A.n_hops) against the set A.set.  ROWS = true:
+// CTA x takes descriptor A.rows[x] (its stream, hop range and output block); the body is the same.  SETS = true (with
+// ROWS): each CTA takes its set from its descriptor; SETS = false: every row's set is A.set (the descriptors' set pointers
+// are not read), whose fields are kernel parameters rather than global loads and spill less.
+template <bool PRE, bool ROWS, bool SETS>
 __global__ void __launch_bounds__(1024, 1)
 dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const TemplateFeat* __restrict__ tmpl, DenseArgs A) {
-    static_assert(ROWS || !SETS, "per-row sets need row descriptors");
     extern __shared__ __align__(16) float smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5, nthr = blockDim.x;
-    // the row's set is re-read where it is used, as the row's hops are
-    auto row = [&]() -> const DenseRow& {
-        if constexpr (SETS) return reinterpret_cast<const DenseRowSet*>(A.rows)[blockIdx.x].r;
-        else return A.rows[blockIdx.x];
-    };
-    auto set = [&]() -> const DenseSetDev& { return *reinterpret_cast<const DenseRowSet*>(A.rows)[blockIdx.x].set; };
-#define DSET(f) (SETS ? set().f : A.f)
-    const int DH = A.DH, DG = DSET(DG), DLE = DSET(DLE), NT = DSET(T);
+    static_assert(ROWS || !SETS, "per-row sets need row descriptors");
+    // the row and its set are re-read where they are used: values kept live across the kernel would cost registers
+    auto row = [&]() -> const DenseRow& { return A.rows[blockIdx.x]; };
+#define DSET(f) (SETS ? row().set->f : A.set.f)
+    const int DH = SETS ? A.DH : A.set.DH, DG = DSET(DG), DLE = DSET(DLE), NT = DSET(T);
     FrameTables* ft = reinterpret_cast<FrameTables*>(smem);
     float* scratch = smem + sizeof(FrameTables) / sizeof(float);
     float2* MS = reinterpret_cast<float2*>(scratch + (size_t)nwarps * SCR_WARP);   // [T][20][DH] (mean, std) of a coefficient
@@ -301,7 +297,6 @@ dense_score_kernel(const DeviceTables* __restrict__ T, BankView B, const Templat
     int* WAYMASK = ctl + 40;
     int* COMBO = ctl + 56;
     const int s = ROWS ? row().stream : blockIdx.x;
-    // the row's hops are re-read where they are used: values kept live across the kernel would cost registers
     auto hop0 = [&]() -> long long { return ROWS ? row().hop0 : A.hop0; };
     auto n_hops = [&]() -> int { return ROWS ? row().n_hops : A.n_hops; };
     // score of hop (hs + hl), template k
@@ -732,22 +727,16 @@ struct DetRecord {                     // mirrors ewk_detection (include/ewk.h)
 };
 
 // One non-empty row of a detect call: stream `stream`, hops [hop0, hop0 + n_hops), scores at `scores` ([n_hops][T]
-// floats into the call's packed K4 output); its records go to rec[det, det + ceil(n_hops / 2)) and their count to
-// counts[row] (row: the stream's index in the call's list)
+// floats into the call's packed K4 output) against `set` (T, slot0, per-template n and L, in the context's table); its
+// records go to rec[det, det + ceil(n_hops / 2)) and their count to counts[row] (row: the stream's index in the call's list)
 struct DetRow {
     long long hop0, scores, det;
     int stream, n_hops, row, pad;
-};
-
-// A row of a per-row-set detect call: the row and its set (T, slot0, per-template n and L) in the context's table
-struct DetRowSet {
-    DetRow r;
     const DenseSetDev* set;
 };
 
 struct DetArgs {
-    int T, slot0, hold, refractory;    // templates [slot0, slot0 + T) of the call
-    int n[DENSE_MAX_T], L[DENSE_MAX_T]; // per template: window in hops (ceil(L / 160)) and samples
+    int hold, refractory;
     const DetRow* rows;
     int n_rows;
     const float* scores;
@@ -756,15 +745,13 @@ struct DetArgs {
     int* counts;                       // host-mapped [list length]
 };
 
-// SETS = true: A.rows holds DetRowSet descriptors, and each row takes T, slot0, n and L from its set instead of A
-template <bool SETS = false>
 __global__ void __launch_bounds__(32 * DETECT_WARPS)
 dense_detect_kernel(const StreamParams* __restrict__ prm, DetArgs A) {
     const int lane = threadIdx.x & 31, w = blockIdx.x * DETECT_WARPS + (threadIdx.x >> 5);
     if (w >= A.n_rows) return;
-    const DetRow r = SETS ? reinterpret_cast<const DetRowSet*>(A.rows)[w].r : A.rows[w];
-    const DenseSetDev* __restrict__ set = SETS ? reinterpret_cast<const DetRowSet*>(A.rows)[w].set : nullptr;
-    const int T = SETS ? set->T : A.T, slot0 = SETS ? set->slot0 : A.slot0;
+    const DetRow r = A.rows[w];
+    const DenseSetDev* __restrict__ set = r.set;
+    const int T = set->T, slot0 = set->slot0;
     const float thr = prm[r.stream].similarity_threshold;
     const float* __restrict__ sc = A.scores + r.scores;
     DetRecord* __restrict__ out = A.rec + r.det;
@@ -786,13 +773,7 @@ dense_detect_kernel(const StreamParams* __restrict__ prm, DetArgs A) {
             const float bh = __shfl_sync(FULL, b, i);
             const int kh = __shfl_sync(FULL, kb, i);
             const long long h = r.hop0 + base + i;
-            int nk = 0, Lk = 0;                                  // window of k* (selects: no local copy of A)
-            if (SETS) { nk = set->t[kh].n; Lk = set->t[kh].L; }
-            else {
-#pragma unroll
-                for (int t = 0; t < DENSE_MAX_T; t++)
-                    if (t == kh) { nk = A.n[t]; Lk = A.L[t]; }
-            }
+            const int nk = set->t[kh].n, Lk = set->t[kh].L;     // window of k*
             const bool above = bh >= thr;
             bool emit = false;
             if (st.mode == DET_IDLE) {

@@ -7,8 +7,8 @@ Bank: 4096 slots, 10 s int16 rings of synthetic speech-like audio (synth.stream_
 1. Equal hop ranges: 4096 streams x 100 hops through the uniform and the ragged entry point, alternated call by call in
    one process, for one template (the bundled word) and for bench.py's 4-template sweep set.
 2. Occupancy: 100 / 50 / 10 % of the slots active (a scattered random subset), each with its own row of U(50, 150) hops
-   (U(0.5, 1.5) s of audio), through ewk_dense_scores_streams with the rows longest first (the default) and in list order
-   (EWK_DENSE_LONGEST_FIRST=0), alternated.
+   (U(0.5, 1.5) s of audio), through ewk_dense_scores_streams (which runs the rows longest first: r06_ragged_dense.json
+   measured that order against list order).
 3. A live step at those occupancies: push_streams of U(0.5, 1.5) s per active slot from pinned host memory, tick_ready
    until nothing is due, dense_ready until nothing is due, poll.
 Call and step times are host clocks around work that ends in a synchronise; K4 times per launch come from ewk_profile
@@ -100,19 +100,10 @@ def occupancy(ctx, occ, reps, rng):
     def call():
         ctx.dense_scores_streams(st, h0, nh, 0, 1, out_device_ptr=out.data_ptr())
 
-    res = {}
-    times = {"longest_first": [], "list_order": []}
-    for i in range(reps + 2):
-        for key, env in (("longest_first", "1"), ("list_order", "0")):
-            os.environ["EWK_DENSE_LONGEST_FIRST"] = env
-            t = timed(call, ctx)
-            if i >= 2:
-                times[key].append(t)
-    for key, env in (("longest_first", "1"), ("list_order", "0")):
-        os.environ["EWK_DENSE_LONGEST_FIRST"] = env
-        k4 = k4_profile(ctx, call, 5)
-        res[key] = {"call_ms_median": float(np.median(times[key])) * 1e3, "k4_ms": k4, "windows_per_s_k4": windows / (k4 * 1e-3)}
-    os.environ["EWK_DENSE_LONGEST_FIRST"] = "1"
+    times = [timed(call, ctx) for _ in range(reps + 2)][2:]
+    k4 = k4_profile(ctx, call, 5)
+    res = {"longest_first": {"call_ms_median": float(np.median(times)) * 1e3, "k4_ms": k4,
+                             "windows_per_s_k4": windows / (k4 * 1e-3)}}
     res["active_streams"], res["windows"] = n_act, windows
     return res
 

@@ -1,6 +1,6 @@
 """GPU: per-row template sets in dense scoring and detection (ewk_dense_scores_sets, ewk_dense_ready_sets,
 ewk_dense_detect_sets).  Every row equals, bit for bit (np.array_equal(equal_nan=True)), the single-set call of that row
-alone with its set, and on a subset oracle/dense_model.py; paced calls equal per-set grouped ewk_dense_ready /
+alone with its set and the uniform ewk_dense_scores (K4's other instance), and on a subset oracle/dense_model.py; paced calls equal per-set grouped ewk_dense_ready /
 ewk_dense_detect calls and oracle/dense_detect.py record for record; one K4 launch per geometry plus one K4D; resets,
 migration, cache invalidation and every error."""
 import ctypes
@@ -100,8 +100,8 @@ def assert_rows(got, want, what):
                          ids=["i16", "f32", "i16-pre-mfcc13"])
 def test_scores_sets_equal_single_set_rows(word, fmt, kw):
     """Random stream lists, each row with a random set (shared, overlapping, identical, disjoint; every geometry; one-
-    template sets of all 64 slots): every row equals ewk_dense_scores_streams of that row alone with its set, host and
-    device output, and the model on a subset.  Launches: one K4 per geometry among the non-empty rows."""
+    template sets of all 64 slots): every row equals ewk_dense_scores_streams of that row alone with its set and the
+    uniform ewk_dense_scores of its hops and set, host and device output, and the model on a subset.  Launches: one K4 per geometry among the non-empty rows."""
     import torch
     from easywakeword_b200 import _lib
     lens, sets, _, word_slot = layout(word)
@@ -116,6 +116,14 @@ def test_scores_sets_equal_single_set_rows(word, fmt, kw):
     one_slot_sets = set()
     model_rows = 0
     frames = lambda pcm: ctx.extract_mfcc(pcm, want_frames=True)[2]
+
+    def alone(s, a, n, f, c):
+        """row s alone through ewk_dense_scores_streams, checked against the uniform instance (every stream has the same
+        length, so every stream holds these hops)"""
+        row = ctx.dense_scores_streams([s], [a], [n], f, c)[0]
+        assert_rows([row], [ctx.dense_scores(a, n, f, c)[s] if n else np.zeros((0, c), np.float32)],
+                    f"uniform stream {s} hops {a}+{n} set {f}+{c}")
+        return row
     for call in range(10):
         k = int(rng.integers(1, N + 1))
         streams = [int(s) for s in rng.choice(N, k, replace=False)]
@@ -140,7 +148,7 @@ def test_scores_sets_equal_single_set_rows(word, fmt, kw):
         assert ctx.launch_count() - n0 == len(groups), (call, ctx.launch_count() - n0, groups)
         if groups:
             assert ctx.dense_last_plan()[:3] == list(groups)[-1]
-        want = [ctx.dense_scores_streams([s], [a], [n], f, c)[0] for s, a, n, f, c in zip(streams, h0, nh, fs, cs)]
+        want = [alone(s, a, n, f, c) for s, a, n, f, c in zip(streams, h0, nh, fs, cs)]
         assert_rows(got, want, f"call {call}")
         # device output, packed as the header says
         off, total = _lib.sets_offsets(nh, cs)
@@ -160,7 +168,7 @@ def test_scores_sets_equal_single_set_rows(word, fmt, kw):
         for base in range(0, NT, N):
             fs = [(base + i) % NT for i in range(N)]
             got = ctx.dense_scores_sets(list(range(N)), [10] * N, [30] * N, fs, [1] * N)
-            want = [ctx.dense_scores_streams([s], [10], [30], f, 1)[0] for s, f in zip(range(N), fs)]
+            want = [alone(s, 10, 30, f, 1) for s, f in zip(range(N), fs)]
             assert_rows(got, want, f"one-slot sets from {base}")
             one_slot_sets.update(fs)
         assert len(one_slot_sets) >= 64
@@ -170,7 +178,7 @@ def test_scores_sets_equal_single_set_rows(word, fmt, kw):
     for s, (f, c) in enumerate(own):
         ctx.set_stream_params(s, frame_size=1600, template_first=f, template_count=c, live=1)
     got = ctx.dense_scores_sets(list(range(N)), [5] * N, [50] * N)
-    want = [ctx.dense_scores_streams([s], [5], [50], f, c)[0] for s, (f, c) in enumerate(own)]
+    want = [alone(s, 5, 50, f, c) for s, (f, c) in enumerate(own)]
     assert_rows(got, want, "own ranges")
     ctx.close()
 

@@ -271,12 +271,12 @@ def k3_forms(r, word):
 
 
 def dense(r, word):
-    """reaches: dense_score_kernel<false, false> (dense_scores at every geometry ewk_dense_plan can choose),
-    <false, true> (dense_scores_streams with an empty row, rows in descending hop order and rows that overlap in hops;
-    dense_ready), <false, true, true>
-    (the _sets forms), dense_detect_kernel<false> / <true> (dense_detect, dense_detect_sets), and with preemphasis the
-    <true, false>, <true, true>, <true, true, true> instances; calls whose DG differs from the previous call's; a set
-    switch and a template change that rebuilds cached sets"""
+    """reaches: dense_score_kernel<false, false, false> (dense_scores at every geometry ewk_dense_plan can choose),
+    <false, true, false> (dense_scores_streams with an empty row, rows in descending hop order and rows that overlap in
+    hops; dense_ready; geometry groups of the _sets forms whose rows share one set), <false, true, true> (a _sets call
+    with three sets of one geometry), dense_detect_kernel (dense_detect, dense_detect_sets), and with preemphasis the
+    <true, ...> instances; calls whose DG differs from the previous call's; a set switch and a template change that
+    rebuilds cached sets"""
     import helpers
     from easywakeword_b200 import _lib, synth
     geo = helpers.dense_geometry_sets(_lib.dense_plan)
@@ -303,6 +303,7 @@ def dense(r, word):
         c.set_stream_params(0, frame_size=1600, template_first=0, template_count=2, similarity_threshold=0.0)
         c.set_stream_params(1, frame_size=1600, template_first=1, template_count=3, similarity_threshold=0.0)
         r.add(f"{pre} sets", c.dense_scores_sets([0, 1, 2], [4, 4, 4], [30, 30, 30]))
+        r.add(f"{pre} sets one geometry", c.dense_scores_sets([0, 1, 2], [4, 4, 4], [30, 30, 30], [0, 1, 3], [1, 1, 1]))
         r.add(f"{pre} ready sets", c.dense_ready_sets(None, 50))
         r.add(f"{pre} detect sets", c.dense_detect_sets(None, 80, scores=True))
         c.set_template(2, word[::-1].copy())                 # rebuilds the cached sets that contain slot 2
